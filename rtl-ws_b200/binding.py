@@ -233,6 +233,26 @@ class SpectrumPlan:
     def rows(self, n_samples: int) -> int:
         return int(lib().b200_spectrum_plan_rows(self.h, n_samples))
 
+    def _run(self, fn, x, n_rows, db, power, db_u8, out, stream) -> dict:
+        """Allocate the requested [n_streams, n_rows, N] outputs (unless `out` has them) and call the C exec `fn`
+        on x[s] (stream s starts x.stride(0) elements after stream s - 1)."""
+        torch = _torch()
+        n_streams, n_samples = x.shape[0], x.shape[1]
+        if n_rows is None:
+            n_rows = self.rows(n_samples)
+        res = {} if out is None else out
+        if db and "db" not in res:
+            res["db"] = torch.empty((n_streams, n_rows, self.N), dtype=torch.float32, device=x.device)
+        if power and "power" not in res:
+            res["power"] = torch.empty((n_streams, n_rows, self.N), dtype=torch.float32, device=x.device)
+        if db_u8 and "db_u8" not in res:
+            res["db_u8"] = torch.empty((n_streams, n_rows, self.N), dtype=torch.uint8, device=x.device)
+        ptr = lambda k: C.c_void_p(res[k].data_ptr()) if k in res else None
+        stride = x.stride(0) * x.element_size() if n_streams > 1 else 0
+        _check(fn(self.h, C.c_void_p(x.data_ptr()), stride, n_streams, n_rows, ptr("db"), ptr("power"), ptr("db_u8"),
+                  _stream_ptr(stream)), fn.__name__)
+        return res
+
     def exec(self, iq, n_rows: int | None = None, db: bool = True, power: bool = False, db_u8: bool = False,
              out: dict | None = None, stream=None) -> dict:
         """iq: cuda uint8 tensor [n_streams, n_samples, 2] (rows may be strided views).
@@ -241,46 +261,24 @@ class SpectrumPlan:
         torch = _torch()
         assert iq.is_cuda and iq.dtype == torch.uint8 and iq.dim() == 3 and iq.shape[2] == 2
         assert iq.stride(2) == 1 and iq.stride(1) == 2
-        n_streams, n_samples = iq.shape[0], iq.shape[1]
-        if n_rows is None:
-            n_rows = self.rows(n_samples)
-        res = {} if out is None else out
-        if db and "db" not in res:
-            res["db"] = torch.empty((n_streams, n_rows, self.N), dtype=torch.float32, device=iq.device)
-        if power and "power" not in res:
-            res["power"] = torch.empty((n_streams, n_rows, self.N), dtype=torch.float32, device=iq.device)
-        if db_u8 and "db_u8" not in res:
-            res["db_u8"] = torch.empty((n_streams, n_rows, self.N), dtype=torch.uint8, device=iq.device)
-        ptr = lambda k: C.c_void_p(res[k].data_ptr()) if k in res else None
-        stride = iq.stride(0) if n_streams > 1 else 0
-        _check(lib().b200_spectrum_exec(self.h, C.c_void_p(iq.data_ptr()), stride, n_streams, n_rows,
-                                        ptr("db"), ptr("power"), ptr("db_u8"), _stream_ptr(stream)),
-               "b200_spectrum_exec")
-        return res
+        return self._run(lib().b200_spectrum_exec, iq, n_rows, db, power, db_u8, out, stream)
 
-    def exec_cs32(self, x, n_rows: int | None = None, stream=None) -> dict:
-        """x: cuda int32 tensor [n_streams, n_samples, 2] (spectrum_add_cmplx_s32 semantics)."""
+    def exec_cs32(self, x, n_rows: int | None = None, db: bool = False, power: bool = True, db_u8: bool = False,
+                  out: dict | None = None, stream=None) -> dict:
+        """x: cuda int32 tensor [n_streams, n_samples, 2] (spectrum_add_cmplx_s32 semantics; rows may be strided
+        views).  Outputs as for exec(); power only by default."""
         torch = _torch()
-        assert x.is_cuda and x.dtype == torch.int32 and x.is_contiguous()
-        n_streams, n_samples = x.shape[0], x.shape[1]
-        n_rows = self.rows(n_samples) if n_rows is None else n_rows
-        power = torch.empty((n_streams, n_rows, self.N), dtype=torch.float32, device=x.device)
-        _check(lib().b200_spectrum_exec_cs32(self.h, C.c_void_p(x.data_ptr()), n_samples * 8, n_streams, n_rows,
-                                             None, C.c_void_p(power.data_ptr()), None, _stream_ptr(stream)),
-               "b200_spectrum_exec_cs32")
-        return {"power": power}
+        assert x.is_cuda and x.dtype == torch.int32 and x.dim() == 3 and x.shape[2] == 2
+        assert x.stride(2) == 1 and x.stride(1) == 2
+        return self._run(lib().b200_spectrum_exec_cs32, x, n_rows, db, power, db_u8, out, stream)
 
-    def exec_rf32(self, x, n_rows: int | None = None, stream=None) -> dict:
-        """x: cuda float32 tensor [n_streams, n_samples] (spectrum_add_real_f32 semantics)."""
+    def exec_rf32(self, x, n_rows: int | None = None, db: bool = False, power: bool = True, db_u8: bool = False,
+                  out: dict | None = None, stream=None) -> dict:
+        """x: cuda float32 tensor [n_streams, n_samples] (spectrum_add_real_f32 semantics; rows may be strided
+        views).  Outputs as for exec(); power only by default."""
         torch = _torch()
-        assert x.is_cuda and x.dtype == torch.float32 and x.is_contiguous()
-        n_streams, n_samples = x.shape[0], x.shape[1]
-        n_rows = self.rows(n_samples) if n_rows is None else n_rows
-        power = torch.empty((n_streams, n_rows, self.N), dtype=torch.float32, device=x.device)
-        _check(lib().b200_spectrum_exec_rf32(self.h, C.c_void_p(x.data_ptr()), n_samples * 4, n_streams, n_rows,
-                                             None, C.c_void_p(power.data_ptr()), None, _stream_ptr(stream)),
-               "b200_spectrum_exec_rf32")
-        return {"power": power}
+        assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 2 and x.stride(1) == 1
+        return self._run(lib().b200_spectrum_exec_rf32, x, n_rows, db, power, db_u8, out, stream)
 
 
 # --------------------------------------------------------------------------------------
