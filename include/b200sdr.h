@@ -120,6 +120,39 @@ int b200_fm_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams
                  float* d_audio, int64_t audio_stride, int32_t* d_decimated, int64_t dec_stride,
                  void* cuda_stream);
 
+/* ---- FM channels: several stations at frequency offsets inside one dongle's band ----------------
+ *
+ * The reference demodulates whatever sits at the tuned frequency (resample.c:21-40, audio_main.c:110-139), and
+ * its `freq` command retunes the dongle (main.c:139-171), which moves every listener of that dongle.  Here the
+ * band stays put and each channel gets the same chain re-centred digitally.  Channel c of stream s has a 32-bit
+ * phase increment inc; a signal at baseband +f Hz (RF = dongle frequency + f) is brought to DC by the increment
+ * of +f.  With n the int64 index of an input sample from stream start (the history has n < 0):
+ *   phi(n) = (uint32)(inc * (uint64) n),   y[n] = ((re - 128) + j (im - 128)) * exp(-j 2 pi phi(n) / 2^32)
+ *   b[m]   = sum_{k<R} y[mR + k]           the CIC boxcar of resample.c:21-40 at its own scale, no 1/128
+ *   audio  = atan2_approx, first difference, +-1 limiter, two half-bands (audio_main.c:110-139) on b, in f32,
+ *            one float per 4R input samples.
+ * At inc = 0, b is exactly the integer cic_decimate output and the audio is b200_fm_exec's.  The only state is
+ * the input history b200_fm_exec already carries plus the absolute index of the batch's first sample, which the
+ * caller passes: an all-128 history mixes to zero, so stream start reproduces the reference's zeroed delay lines.
+ * All channels of one call share R.  The filter in front of the demodulator is the reference's boxcar and no
+ * sharper: a strong neighbour within fs / R of the channel leaks into it as it would into the reference. */
+#define B200_FM_MAX_CHANNELS 32
+/* round(offset_hz / sample_rate_hz * 2^32) as a two's-complement uint32; B200_ERR_ARG if |offset| > fs/2, fs <= 0 or NaN.
+   Pure host arithmetic: works without a device. */
+int b200_fm_channel_tune(double offset_hz, double sample_rate_hz, uint32_t* phase_inc);
+/* Layout and history as b200_fm_exec; first_sample >= 0, a multiple of 4R (absolute index of d_iq's first batch sample);
+   d_phase_inc: device [n_streams][n_channels]; d_audio row s*n_channels + c (audio_stride floats apart);
+   d_baseband (nullable): float (re, im) pairs, row s*n_channels + c, n_samples/R per row, baseband_stride in complex samples.
+   n_channels in [1, B200_FM_MAX_CHANNELS], R in [1, 256], n_samples a multiple of 4R and of 8.  Arguments are checked
+   before anything is launched: B200_ERR_ARG for counts, R, first_sample, n_samples or NULL pointers, B200_ERR_ALIGN for
+   an IQ pointer or stride that is not 16-byte aligned (or d_audio / d_phase_inc not 4-, d_baseband not 8-byte aligned).
+   The audio rows are [n_streams * n_channels][...], so b200_wire_audio_messages turns them into websocket audio
+   messages with n_streams * n_channels rows, one per listener; no other wire call is needed. */
+int b200_fm_channels_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                          int64_t first_sample, const uint32_t* d_phase_inc, int n_channels,
+                          float* d_audio, int64_t audio_stride, float* d_baseband, int64_t baseband_stride,
+                          void* cuda_stream);
+
 /* The same demodulator for DECIMATED input -- the signature of the reference's own callback,
  * audio_fm_demodulator(const cmplx_s32*, int) (audio_main.h:12, audio_main.c:74-145), with its three
  * function statics (audio_main.c:77-79) made explicit.  d_state: B200_FM_STATE_FLOATS floats per stream on
@@ -214,6 +247,12 @@ int b200_session_chain(b200_session* s, const uint8_t* h_iq, int64_t n_samples, 
  * over PCIe instead of 4.1.  h_avg_u8: [n_streams][1024]. */
 int b200_session_products(b200_session* s, const uint8_t* h_iq, int64_t n_samples, int gain_db, int K_avg,
                           float* h_audio, uint8_t* h_avg_u8);
+/* b200_fm_channels_exec on host buffers: h_phase_inc [n_streams][n_channels] (host), h_audio
+ * [n_streams][n_channels][n_samples / (4R)]; batch rules as b200_session_chain.  The session counts the samples
+ * every call has consumed (chain, products, channels; b200_session_reset sets it back to 0), so channel calls may
+ * be interleaved with the others and each batch is mixed at its absolute position in the stream. */
+int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_samples, const uint32_t* h_phase_inc,
+                          int n_channels, float* h_audio);
 /* ---- push-style streaming: what a signal_source callback calls ------------------------------
  *
  * signal_source.c:29-35 hands every registered callback a BORROWED buffer of cmplx_u8 and its

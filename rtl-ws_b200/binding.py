@@ -26,8 +26,10 @@ EXPORTED_SYMBOLS = [
     "b200_spectrum_plan_create", "b200_spectrum_plan_destroy", "b200_spectrum_plan_rows", "b200_spectrum_exec",
     "b200_spectrum_exec_cs32", "b200_spectrum_exec_rf32",
     "b200_fm_history_samples", "b200_fm_history_reset", "b200_fm_history_carry", "b200_fm_exec",
+    "b200_fm_channel_tune", "b200_fm_channels_exec",
     "b200_chain_exec", "b200_chain_exec_r", "b200_chain_tile_samples",
     "b200_session_create", "b200_session_create_r", "b200_session_destroy", "b200_session_reset", "b200_session_chain", "b200_session_products",
+    "b200_session_channels",
     "b200_stream_create", "b200_stream_create_r", "b200_stream_destroy", "b200_stream_set_sinks", "b200_stream_set_payload_sink", "b200_stream_push", "b200_stream_poll",
     "b200_stream_flush", "b200_stream_pending_samples",
     "b200_wire_spectrum_header", "b200_wire_spectrum_message", "b200_wire_spectrum_messages",
@@ -91,6 +93,8 @@ def lib() -> C.CDLL:
     L.b200_fm_history_reset.argtypes = [vp, i64, i32, i32, vp]
     L.b200_fm_history_carry.argtypes = [vp, i64, i32, i64, i32, vp]
     L.b200_fm_exec.argtypes = [vp, i64, i32, i64, i32, f32p, i64, vp, i64, vp]
+    L.b200_fm_channel_tune.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_uint32)]
+    L.b200_fm_channels_exec.argtypes = [vp, i64, i32, i64, i32, i64, vp, i32, f32p, i64, f32p, i64, vp]
     L.b200_chain_exec.argtypes = [vp, i64, i32, i64, i32, f32p, f32p, i64, vp, i32, vp]
     L.b200_chain_exec_r.argtypes = [vp, i64, i32, i64, i32, i32, f32p, f32p, i64, vp, i32, vp]
     L.b200_chain_tile_samples.restype = i64
@@ -105,6 +109,7 @@ def lib() -> C.CDLL:
     L.b200_session_reset.argtypes = [vp]
     L.b200_session_chain.argtypes = [vp, vp, i64, i32, vp, vp]
     L.b200_session_products.argtypes = [vp, vp, i64, i32, i32, vp, vp]
+    L.b200_session_channels.argtypes = [vp, vp, i64, vp, i32, vp]
     L.b200_stream_create.restype = vp
     L.b200_stream_create.argtypes = [i32, i64, i32]
     L.b200_stream_destroy.argtypes = [vp]
@@ -333,6 +338,40 @@ def fm_exec(ring: StreamRing, audio=None, decimated: bool = False, stream=None):
     return audio, dec
 
 
+FM_MAX_CHANNELS = 32
+
+
+def fm_channel_tune(offset_hz: float, fs: float) -> int:
+    """b200_fm_channel_tune: the phase increment (uint32) that brings baseband +offset_hz to DC; host arithmetic."""
+    inc = C.c_uint32()
+    _check(lib().b200_fm_channel_tune(float(offset_hz), float(fs), C.byref(inc)), "b200_fm_channel_tune")
+    return int(inc.value)
+
+
+def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None, baseband: bool = False, stream=None):
+    """b200_fm_channels_exec over a StreamRing: phase_inc is a cuda int32 tensor [n_streams, n_channels] holding the
+    uint32 increments' bits; first_sample is the absolute index of the batch's first sample (a multiple of 4R).
+    -> (audio [S, C, n/(4R)] f32, baseband [S, C, n/R, 2] f32 | None)."""
+    torch = _torch()
+    assert phase_inc.is_cuda and phase_inc.dtype == torch.int32 and phase_inc.dim() == 2
+    assert phase_inc.shape[0] == ring.n_streams and phase_inc.is_contiguous()
+    S, Ch = phase_inc.shape
+    n_audio = ring.n_samples // (4 * ring.R)
+    if audio is None:
+        audio = torch.empty((S, Ch, n_audio), dtype=torch.float32, device=ring.buf.device)
+    assert audio.shape == (S, Ch, n_audio) and audio.stride(2) == 1 and audio.stride(0) == Ch * audio.stride(1)
+    bb = None
+    if baseband:
+        bb = torch.empty((S, Ch, ring.n_samples // ring.R, 2), dtype=torch.float32, device=ring.buf.device)
+    _check(lib().b200_fm_channels_exec(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
+                                       ring.n_samples, ring.R, first_sample, C.c_void_p(phase_inc.data_ptr()), Ch,
+                                       C.c_void_p(audio.data_ptr()), audio.stride(1),
+                                       C.c_void_p(bb.data_ptr()) if bb is not None else None,
+                                       bb.stride(1) // 2 if bb is not None else 0, _stream_ptr(stream)),
+           "b200_fm_channels_exec")
+    return audio, bb
+
+
 def chain_exec(ring: StreamRing, gain_db: int = 0, db=None, audio=None, avg_u8=None, K_avg: int = 6, stream=None):
     """b200_chain_exec: per-frame dB spectra (N = 1024) + FM audio from one pass over the ring's batch."""
     torch = _torch()
@@ -552,6 +591,19 @@ class Session:
             return C.c_void_p(x.data_ptr() if hasattr(x, "data_ptr") else x.ctypes.data)
         _check(lib().b200_session_products(self.h, hp(h_iq), n_samples, gain_db, K_avg, hp(h_audio), hp(h_avg_u8)),
                "b200_session_products")
+
+    def channels(self, h_iq, n_samples: int, phase_inc, h_audio=None):
+        """b200_session_channels: phase_inc [n_streams, n_channels] (host, uint32 bits) -> h_audio
+        [n_streams, n_channels, n_samples / (4R)] f32 (allocated if not given), mixed at the session's position."""
+        inc = np.ascontiguousarray(np.asarray(phase_inc).astype(np.int64) & 0xFFFFFFFF, dtype=np.uint32)
+        assert inc.ndim == 2 and inc.shape[0] == self.n_streams
+        if h_audio is None:
+            h_audio = np.empty((self.n_streams, inc.shape[1], n_samples // (4 * self.R)), np.float32)
+        h_iq = np.ascontiguousarray(h_iq, dtype=np.uint8) if isinstance(h_iq, np.ndarray) else h_iq
+        p = lambda x: C.c_void_p(x.data_ptr() if hasattr(x, "data_ptr") else x.ctypes.data)
+        _check(lib().b200_session_channels(self.h, p(h_iq), n_samples, inc.ctypes.data, inc.shape[1], p(h_audio)),
+               "b200_session_channels")
+        return h_audio
 
 
 class PushStream:

@@ -90,6 +90,9 @@ int launch_fm_chain(const FmParams& p, cudaStream_t stream);
 int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
 int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
 int fm_history_samples(int R);
+int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                       int64_t first_sample, const uint32_t* phase_inc, int n_channels, float* audio,
+                       int64_t audio_stride, float* baseband, int64_t baseband_stride, cudaStream_t stream);
 
 }  // namespace b200
 
@@ -501,6 +504,30 @@ int b200_fm_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams
     p.decimated = d_decimated;
     p.dec_stride = dec_stride;
     return launch_fm_chain(p, reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+int b200_fm_channel_tune(double offset_hz, double sample_rate_hz, uint32_t* phase_inc)
+{
+    // !(a <= b) also refuses NaN
+    if (phase_inc == nullptr || !(sample_rate_hz > 0.0) || !isfinite(sample_rate_hz) ||
+        !(fabs(offset_hz) <= 0.5 * sample_rate_hz)) {
+        set_error("fm channel tune: offset %g Hz outside +-fs/2 or sample rate %g Hz not positive", offset_hz,
+                  sample_rate_hz);
+        return B200_ERR_ARG;
+    }
+    // |offset / fs| <= 1/2, so the rounded value lies in [-2^31, 2^31] and its low 32 bits are the increment
+    const int64_t v = (int64_t) llround(offset_hz / sample_rate_hz * 4294967296.0);
+    *phase_inc = (uint32_t) (uint64_t) v;
+    return B200_OK;
+}
+
+int b200_fm_channels_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                          int64_t first_sample, const uint32_t* d_phase_inc, int n_channels, float* d_audio,
+                          int64_t audio_stride, float* d_baseband, int64_t baseband_stride, void* cuda_stream)
+{
+    return launch_fm_channels(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
+                              n_channels, d_audio, audio_stride, d_baseband, baseband_stride,
+                              reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- pinned host memory --------------------------------------------------------------------

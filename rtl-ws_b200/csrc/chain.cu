@@ -150,6 +150,10 @@ struct b200_session {
     float* d_db;               // [n_streams][max_samples]            (1024 bins per 1024 samples)
     float* d_audio;            // [n_streams][max_samples / (4R)]
     uint8_t* d_avg;            // [n_streams][1024] payload rows, allocated on first use (b200_session_products)
+    int64_t position;          // samples per stream consumed since create / reset (index of the next batch's first)
+    uint32_t* d_phase_inc;     // [n_streams][ch_cap], b200_session_channels, allocated on first use
+    float* d_ch_audio;         // [n_streams][ch_cap][max_samples / (4R)]
+    int ch_cap;                // channels the two buffers above hold
     static constexpr int LANES = 4;
     cudaStream_t streams[LANES];
     int device;
@@ -199,6 +203,7 @@ int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_
         const int rc2 = launch_fm_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->R, st);
         if (rc2) return rc2;
     }
+    s->position += n_samples;
     return B200_OK;
 }
 
@@ -263,6 +268,8 @@ void b200_session_destroy(b200_session* s)
     if (s->d_db) cudaFree(s->d_db);
     if (s->d_audio) cudaFree(s->d_audio);
     if (s->d_avg) cudaFree(s->d_avg);
+    if (s->d_phase_inc) cudaFree(s->d_phase_inc);
+    if (s->d_ch_audio) cudaFree(s->d_ch_audio);
     delete s;
 }
 
@@ -272,6 +279,66 @@ void b200_session_reset(b200_session* s)
     launch_fm_history_reset(s->d_ring + 2 * (int64_t) s->hist_samples, s->stride_bytes, s->n_streams, s->R,
                             s->streams[0]);
     cudaStreamSynchronize(s->streams[0]);
+    s->position = 0;
+}
+
+int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_samples, const uint32_t* h_phase_inc,
+                          int n_channels, float* h_audio)
+{
+    if (s == nullptr || h_iq == nullptr || h_phase_inc == nullptr || h_audio == nullptr) {
+        set_error("session channels: null argument");
+        return B200_ERR_ARG;
+    }
+    if (n_channels < 1 || n_channels > B200_FM_MAX_CHANNELS) {
+        set_error("session channels: n_channels %d outside [1, %d]", n_channels, B200_FM_MAX_CHANNELS);
+        return B200_ERR_ARG;
+    }
+    if (n_samples < 0 || n_samples > s->max_samples || n_samples % s->tile != 0) {
+        set_error("session channels: n_samples %lld must be a multiple of %lld and at most %lld", (long long) n_samples,
+                  (long long) s->tile, (long long) s->max_samples);
+        return B200_ERR_ARG;
+    }
+    if (n_samples == 0) return B200_OK;
+    if (n_channels > s->ch_cap) {       // every earlier call has finished: the session calls wait for their work
+        if (s->d_phase_inc) cudaFree(s->d_phase_inc);
+        if (s->d_ch_audio) cudaFree(s->d_ch_audio);
+        s->d_phase_inc = nullptr;
+        s->d_ch_audio = nullptr;
+        s->ch_cap = 0;
+        const size_t rows = (size_t) s->n_streams * (size_t) n_channels;
+        B200_CUDA_TRY(cudaMalloc((void**) &s->d_phase_inc, sizeof(uint32_t) * rows));
+        B200_CUDA_TRY(cudaMalloc((void**) &s->d_ch_audio, sizeof(float) * rows * (size_t) (s->max_samples / (4 * s->R))));
+        s->ch_cap = n_channels;
+    }
+    const int lanes = b200_session::LANES;
+    int group = (s->n_streams + 4 * lanes - 1) / (4 * lanes);
+    if (group < 1) group = 1;
+    const int64_t n_audio = n_samples / (4 * s->R);
+    int lane = 0;
+    for (int s0 = 0; s0 < s->n_streams; s0 += group, lane = (lane + 1) % lanes) {
+        const int ns = (s->n_streams - s0) < group ? (s->n_streams - s0) : group;
+        cudaStream_t st = s->streams[lane];
+        uint8_t* d_batch = s->d_ring + (int64_t) s0 * s->stride_bytes + 2 * (int64_t) s->hist_samples;
+        const size_t row0 = (size_t) s0 * (size_t) n_channels;
+        const size_t rows = (size_t) ns * (size_t) n_channels;
+        uint32_t* d_inc = s->d_phase_inc + row0;
+        float* d_audio = s->d_ch_audio + row0 * (size_t) n_audio;
+        B200_CUDA_TRY(cudaMemcpy2DAsync(d_batch, (size_t) s->stride_bytes, h_iq + (size_t) s0 * 2 * (size_t) n_samples,
+                                        (size_t) (2 * n_samples), (size_t) (2 * n_samples), (size_t) ns,
+                                        cudaMemcpyHostToDevice, st));
+        B200_CUDA_TRY(cudaMemcpyAsync(d_inc, h_phase_inc + row0, sizeof(uint32_t) * rows, cudaMemcpyHostToDevice, st));
+        const int rc = b200_fm_channels_exec(d_batch, s->stride_bytes, ns, n_samples, s->R, s->position, d_inc,
+                                             n_channels, d_audio, n_audio, nullptr, 0, st);
+        if (rc) return rc;
+        B200_CUDA_TRY(cudaMemcpyAsync(h_audio + row0 * (size_t) n_audio, d_audio, sizeof(float) * rows * (size_t) n_audio,
+                                      cudaMemcpyDeviceToHost, st));
+        const int rc2 = launch_fm_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->R, st);
+        if (rc2) return rc2;
+    }
+    const int rc = b200::session_wait(s);
+    if (rc) return rc;
+    s->position += n_samples;
+    return B200_OK;
 }
 
 int b200_session_chain(b200_session* s, const uint8_t* h_iq, int64_t n_samples, int gain_db, float* h_db,

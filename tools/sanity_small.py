@@ -40,6 +40,11 @@ pkg.audio_post(audio[:, :368], st, pkg.AUDIO_DEEMPH_50US | pkg.AUDIO_RESAMPLE_48
 r7 = pkg.StreamRing(2, 4 * 7 * 8 * 9, R=7)
 r7.load(np.stack([pkg.synth.s1_noise(4 * 7 * 8 * 9, seed=s) for s in range(2)]))
 pkg.fm_exec(r7, decimated=True)
+# FM channels at offsets: the R = 10 kernel and the general one (R = 7)
+inc = torch.tensor([[0, pkg.fm_channel_tune(200e3, 2.048e6), pkg.fm_channel_tune(-1.024e6, 2.048e6) - 2**32]] * 3,
+                   dtype=torch.int32, device="cuda")
+pkg.fm_channels_exec(ring, inc, 0, baseband=True)
+pkg.fm_channels_exec(r7, inc[:2, :2].contiguous(), 4 * 7 * 10, baseband=True)
 sess = pkg.Session(3, n)
 hdb = np.empty((3, n // 1024, 1024), np.float32)
 hau = np.empty((3, n // 40), np.float32)
