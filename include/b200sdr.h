@@ -192,7 +192,10 @@ int b200_debug_atan2(const int32_t* d_yx, int n, float* d_out, int which, void* 
  *   B200_AUDIO_RESAMPLE_48K         15/16 polyphase FIR (240-tap Blackman-windowed sinc, 16 taps per phase):
  *                                   16 input samples -> 15 output samples; n_audio must be a multiple of 16
  * De-emphasis runs first.  d_state: B200_AUDIO_POST_STATE_FLOATS floats per stream, in/out, zero = stream
- * start.  d_out may not alias d_audio.  The test oracle restates both as plain sequential loops. */
+ * start.  d_out may not alias d_audio.  The test oracle restates both as plain sequential loops.
+ * De-emphasis is computed in parallel: each output is started ceil(ln(1e-7) / ln(1 - alpha)) samples early (at
+ * least 96), which grows with audio_rate_hz.  Where that run-in would exceed 1024 samples -- audio_rate_hz above
+ * about 850 kHz with 75 us, 1.27 MHz with 50 us -- the call returns B200_ERR_ARG before launching anything. */
 #define B200_AUDIO_DEEMPH_50US 1
 #define B200_AUDIO_DEEMPH_75US 2
 #define B200_AUDIO_RESAMPLE_48K 4

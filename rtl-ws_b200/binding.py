@@ -322,15 +322,18 @@ class StreamRing:
         self.batch.copy_(t.reshape(self.n_streams, self.n_samples, 2), non_blocking=True)
 
 
-def fm_exec(ring: StreamRing, audio=None, decimated: bool = False, stream=None):
-    """b200_fm_exec over a StreamRing -> (audio [n_streams, n/(4R)] f32, decimated [n_streams, n/R, 2] i32 | None)."""
+def fm_exec(ring: StreamRing, audio=None, decimated: bool = False, dec=None, stream=None):
+    """b200_fm_exec over a StreamRing -> (audio [n_streams, n/(4R)] f32, decimated [n_streams, n/R, 2] i32 | None).
+    `audio` / `dec` may be given, also as row slices of wider tensors; a given `dec` implies decimated=True."""
     torch = _torch()
     n_audio = ring.n_samples // (4 * ring.R)
     if audio is None:
         audio = torch.empty((ring.n_streams, n_audio), dtype=torch.float32, device=ring.buf.device)
-    dec = None
-    if decimated:
+    if dec is None and decimated:
         dec = torch.empty((ring.n_streams, ring.n_samples // ring.R, 2), dtype=torch.int32, device=ring.buf.device)
+    if dec is not None:
+        assert dec.dtype == torch.int32 and dec.shape == (ring.n_streams, ring.n_samples // ring.R, 2)
+        assert dec.stride(2) == 1 and dec.stride(1) == 2 and dec.stride(0) % 2 == 0
     _check(lib().b200_fm_exec(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams, ring.n_samples,
                               ring.R, C.c_void_p(audio.data_ptr()), audio.stride(0),
                               C.c_void_p(dec.data_ptr()) if dec is not None else None,

@@ -14,11 +14,15 @@
 //                 h = 240-tap Blackman-windowed sinc, cutoff 24 kHz at the 768 kHz interpolated rate,
 //                 DC gain 15 (unity per phase); x[<0] = 0.  16 input samples -> 15 output samples.
 //
-// The recursion is a scan, but a short-memory one: (1 - alpha)^96 < 2e-11 for both time constants, so a
-// thread that starts 96 samples early from y = 0 reproduces the sequential result far inside f32
-// rounding.  Each thread produces 8 samples after such a run-in; only a batch's first samples use the
-// carried y[-1] itself.  The audio is 1/40 of the input sample rate (0.1 B per input sample), so this
-// pass costs nothing next to the chain kernel.
+// The recursion is a scan, but a short-memory one: a thread that starts L samples early from y = 0 is off
+// by at most (1 - alpha)^L times the signal's peak, so the host picks the run-in
+//   L = max(96, ceil(ln(1e-7) / ln(1 - alpha)) rounded up to a multiple of 8)
+// and the result matches the sequential one within f32 rounding.  At the reference's 51.2 kHz L is 96 for both
+// time constants ((1 - alpha)^96 < 2e-11 there); alpha shrinks as the rate grows, so L grows with it: 312 at
+// 256 kHz and 624 at 512 kHz with 75 us.  De-emphasis is refused when L would exceed AP_MAX_RUNIN (above about
+// 850 kHz at 75 us and 1.27 MHz at 50 us).  Each thread produces 8 samples after its run-in; only a batch's
+// first samples use the carried y[-1] itself.  At 51.2 kHz the audio is 1/40 of the input sample rate (0.1 B
+// per input sample), so this pass costs nothing next to the chain kernel.
 #include <math.h>
 #include <string.h>
 
@@ -34,7 +38,8 @@ constexpr int AP_PER_THREAD = 8;
 constexpr int AP_CHUNK = 1024;                 // input samples per CTA
 constexpr int AP_HALO = 16;                    // e[] samples in front of the chunk (15 needed)
 constexpr int AP_THREADS = 160;                // >= (AP_CHUNK + AP_HALO) / AP_PER_THREAD = 130
-constexpr int AP_RUNIN = 96;
+constexpr int AP_MIN_RUNIN = 96;
+constexpr int AP_MAX_RUNIN = 1024;
 constexpr int AP_TAPS = 240;
 constexpr int AP_T = 16;                       // taps per phase
 
@@ -55,6 +60,7 @@ struct PostParams {
     int64_t out_stride;
     float* state;               // [n_streams][B200_AUDIO_POST_STATE_FLOATS]
     float alpha;                // 0 = no de-emphasis
+    int runin;                  // de-emphasis samples each thread runs before its first output
     int resample;
 };
 
@@ -79,7 +85,7 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
         if (i0 < n_here + AP_HALO) {
             if (p.alpha > 0.0f) {
                 float y;
-                int64_t g = g0 - AP_RUNIN;
+                int64_t g = g0 - p.runin;
                 if (g <= 0) {                                       // the run-in would cross the batch start: exact state
                     y = st[APS_Y];
                     g = 0;
@@ -214,6 +220,21 @@ int b200_audio_post(const float* d_audio, int64_t audio_stride, int n_streams, i
         set_error("audio post: the 15/16 resampler takes multiples of 16 samples, not %lld", (long long) n_audio);
         return B200_ERR_ARG;
     }
+    float alpha = 0.0f;
+    int runin = AP_MIN_RUNIN;
+    if (de) {
+        const double tau = de == B200_AUDIO_DEEMPH_50US ? 50e-6 : 75e-6;
+        alpha = (float) (1.0 - exp(-1.0 / (audio_rate_hz * tau)));
+        // run-in after which a start from y = 0 is off by (1 - alpha)^L <= 1e-7 of the signal's peak (alpha = 0,
+        // a rate so high that alpha rounds away, would need an endless one)
+        const double need = ceil(log(1e-7) / log1p(-(double) alpha));
+        if (!(alpha > 0.0f) || !(need <= AP_MAX_RUNIN)) {
+            set_error("audio post: de-emphasis at %g Hz needs a run-in of %g samples, more than %d", audio_rate_hz,
+                      need, AP_MAX_RUNIN);
+            return B200_ERR_ARG;
+        }
+        runin = (int) need > AP_MIN_RUNIN ? ((int) need + 7) / 8 * 8 : AP_MIN_RUNIN;
+    }
     if (n_streams == 0 || n_audio == 0) return B200_OK;
     if (n_streams > 65535 || (n_audio + AP_CHUNK - 1) / AP_CHUNK >= (1ll << 31)) {
         set_error("audio post: too large for one launch");
@@ -228,11 +249,8 @@ int b200_audio_post(const float* d_audio, int64_t audio_stride, int n_streams, i
     p.out_stride = out_stride;
     p.state = d_state;
     p.resample = (flags & B200_AUDIO_RESAMPLE_48K) != 0;
-    p.alpha = 0.0f;
-    if (de) {
-        const double tau = de == B200_AUDIO_DEEMPH_50US ? 50e-6 : 75e-6;
-        p.alpha = (float) (1.0 - exp(-1.0 / (audio_rate_hz * tau)));
-    }
+    p.alpha = alpha;
+    p.runin = runin;
     if (p.resample)
         if (int rc = ensure_taps()) return rc;
     const unsigned chunks = (unsigned) ((n_audio + AP_CHUNK - 1) / AP_CHUNK);

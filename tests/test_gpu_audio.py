@@ -224,8 +224,12 @@ def test_unmodified_main_c_with_gpu_demodulator_on_the_wire(pkg, cuda, po, synth
 
 # ---- opt-in extensions: de-emphasis and the 15/16 resampler ---------------------------------------------------
 
-@pytest.mark.parametrize("flags_name", ["AUDIO_DEEMPH_50US", "AUDIO_DEEMPH_75US", "AUDIO_RESAMPLE_48K", "both"])
-def test_audio_post_matches_definition_across_batches(pkg, cuda, po, flags_name):
+@pytest.mark.parametrize("flags_name,rate", [pytest.param(f, 51200.0, id=f) for f in
+                                               ("AUDIO_DEEMPH_50US", "AUDIO_DEEMPH_75US", "AUDIO_RESAMPLE_48K", "both")] +
+                         [pytest.param(f, r, id=f"{f}-{r:.0f}") for r in (128000.0, 512000.0, 800000.0)
+                          for f in ("AUDIO_DEEMPH_50US", "AUDIO_DEEMPH_75US", "both")])
+def test_audio_post_matches_definition_across_batches(pkg, cuda, po, flags_name, rate):
+    """rate: the audio rate fs / (4R) the de-emphasis is designed for (51.2 kHz at the reference's R = 10)."""
     torch = cuda
     flags = pkg.AUDIO_DEEMPH_75US | pkg.AUDIO_RESAMPLE_48K if flags_name == "both" else getattr(pkg, flags_name)
     rng = np.random.default_rng(11)
@@ -238,11 +242,11 @@ def test_audio_post_matches_definition_across_batches(pkg, cuda, po, flags_name)
     tau = 50e-6 if flags & pkg.AUDIO_DEEMPH_50US else 75e-6
     pos = 0
     for n in batches:
-        got = pkg.audio_post(torch.as_tensor(x[:, pos:pos + n]).cuda().contiguous(), state, flags).cpu().numpy()
+        got = pkg.audio_post(torch.as_tensor(x[:, pos:pos + n]).cuda().contiguous(), state, flags, rate).cpu().numpy()
         for s in range(n_streams):
             want = x[s, pos:pos + n]
             if flags & (pkg.AUDIO_DEEMPH_50US | pkg.AUDIO_DEEMPH_75US):
-                want, y_state[s] = po.deemphasis(want, 51200.0, tau, y_state[s])
+                want, y_state[s] = po.deemphasis(want, rate, tau, y_state[s])
             if flags & pkg.AUDIO_RESAMPLE_48K:
                 want, hist[s] = po.resample_15_16(want, hist[s])
             assert got[s].shape == want.shape

@@ -23,7 +23,7 @@ def oracle_stream(po, iq, R=10):
     return dec, audio
 
 
-@pytest.mark.parametrize("R", [10, 5, 12, 16, 1, 7, 64, 3, 4, 6, 8, 9, 11, 13, 14, 15, 2, 17])
+@pytest.mark.parametrize("R", [10, 5, 12, 16, 1, 7, 64, 3, 4, 6, 8, 9, 11, 13, 14, 15, 2, 17, 103, 171, 255, 256])
 def test_fm_exec_matches_oracle(pkg, cuda, po, synth, R):
     torch = cuda
     n = 4 * R * 8 * 61              # whole audio samples, multiple of 8, not a multiple of the tile
@@ -116,31 +116,47 @@ def test_fm_argument_errors(pkg, cuda):
         pkg.StreamRing(1, 5120, R=0)
 
 
-def test_chain_exec_matches_oracle(pkg, cuda, po, synth):
-    torch = cuda
-    n = 5120 * 9
+def check_chain_exec(pkg, torch, po, synth, R, K_avg, gain_db):
+    """b200_chain_exec_r on 7 streams against the oracle: per-frame dB, audio and the K_avg-frame payload bytes.
+    K_avg None: every frame of the batch (n / 1024, the most the argument check admits)."""
+    tile = int(pkg.lib().b200_chain_tile_samples(R))
+    n = tile * -(-5120 * 9 // tile)
+    K_avg = n // 1024 if K_avg is None else K_avg
     n_streams = 7
     iqs = np.stack([synth.s3_fm(n, seed=70 + s, carrier=(0.0, 50e3)[s % 2]) for s in range(n_streams)])
-    ring = pkg.StreamRing(n_streams, n)
+    ring = pkg.StreamRing(n_streams, n, R=R)
     ring.load(iqs)
     avg = torch.zeros((n_streams, 1024), dtype=torch.uint8, device="cuda")
     before = pkg.launch_count()
-    db, audio = pkg.chain_exec(ring, gain_db=20, avg_u8=avg, K_avg=6)
+    db, audio = pkg.chain_exec(ring, gain_db=gain_db, avg_u8=avg, K_avg=K_avg)
     torch.cuda.synchronize()
     assert pkg.launch_count() > before
     db, audio, avg = db.cpu().numpy(), audio.cpu().numpy(), avg.cpu().numpy()
+    gain = 10.0 ** int(gain_db / 10)
     for s in range(n_streams):
         rows = po.Spectrum(1024).rows(iqs[s])
         with np.errstate(divide="ignore"):
-            want_db = 10 * np.log10(100.0 * rows)
+            want_db = 10 * np.log10(gain * rows)
         ok = rows > 1e-6 * rows.mean(axis=1, keepdims=True)
         assert np.abs(db[s][ok] - want_db[ok]).max() <= 0.01
-        _, want_audio = oracle_stream(po, iqs[s])
+        _, want_audio = oracle_stream(po, iqs[s], R)
         assert np.abs(audio[s] - want_audio).max() <= AUDIO_TOL
-        rows6 = po.Spectrum(1024).rows(iqs[s], K=6)[0]
-        want_u8, dbf = po.db_payload(rows6, 6, 20)
+        rows_k = po.Spectrum(1024).rows(iqs[s], K=K_avg)[0]
+        want_u8, dbf = po.db_payload(rows_k, K_avg, gain_db)
         diff = avg[s] != want_u8
         assert diff.mean() < 0.01 and (np.abs(dbf[diff] - np.rint(dbf[diff])) <= 0.01).all()
+
+
+def test_chain_exec_matches_oracle(pkg, cuda, po, synth):
+    check_chain_exec(pkg, cuda, po, synth, R=10, K_avg=6, gain_db=20)
+
+
+@pytest.mark.parametrize("R,K_avg,gain_db", [(R, K, g) for R in (10, 1, 7, 100, 256)
+                                             for K, g in ((6, 20), (1, -15), (None, 20)) if (R, K, g) != (10, 6, 20)])
+def test_chain_exec_r_matches_oracle(pkg, cuda, po, synth, R, K_avg, gain_db):
+    """The fused kernel at R = 10, spectrum + b200_fm_exec otherwise; one frame and every frame per payload row;
+    gain_db = -15 scales by 10^-1, C's integer division (cbb_main.c:112)."""
+    check_chain_exec(pkg, cuda, po, synth, R, K_avg, gain_db)
 
 
 def test_chain_full_size_properties(pkg, cuda):
