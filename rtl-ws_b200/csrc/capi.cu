@@ -2,7 +2,6 @@
 // Host code only; every arithmetic step happens in the kernels of this directory.
 #include <math.h>
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <map>
@@ -83,9 +82,8 @@ int launch_spectrum_generic(const SpecParams& p, int N, int kind, float2* scratc
 int spectrum_generic_scratch_ctas();
 int launch_spectrum4096(const SpecParams& p, cudaStream_t stream);
 int launch_spectrum2048(const SpecParams& p, cudaStream_t stream);
-int launch_spectrum_mx1024(const SpecParams& p, int N, cudaStream_t stream);
+int launch_spectrum_mx1024(const SpecParams& p, cudaStream_t stream);
 int launch_spectrum64k(const SpecParams& p, const Spec64kExtra& x, int N, cudaStream_t stream);
-int launch_spectrum64k_cluster(const SpecParams& p, const Spec64kExtra& x, cudaStream_t stream);
 int launch_fm_chain(const FmParams& p, cudaStream_t stream);
 int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
 int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
@@ -107,8 +105,8 @@ struct b200_spectrum_plan {
     int gain_db;
     float db_offset;
     float2* d_twiddle;             // N-point table
-    float2* d_twiddle1024;         // 1024-point table (N = 2048 / 4096 / 8192 run M branches of 1024)
-    float2* d_twiddle_rk;          // [M][1024]: W_N^(r k), the layout spectrum_mx1024.cu reads with immediate offsets
+    float2* d_twiddle1024;         // 1024-point table (N = 8192 and the four-step sizes run branches of 1024)
+    float2* d_twiddle_rk;          // N = 8192: [8][1024] W_N^(r k), the layout spectrum_mx1024.cu reads with immediate offsets
     float2* d_twiddle_4k;          // N = 4096: [64][64] W_4096^(n2 k1), the inter-pass table of spectrum4096.cu
                                    // N = 2048: [32][64] W_2048^(n2 k1), the inter-pass table of spectrum2048.cu
     float* d_window;
@@ -236,7 +234,7 @@ b200_spectrum_plan* b200_spectrum_plan_create(int N, int hop, int K, int64_t row
     pl->gen_ctas = 0;
     pl->d_twiddle = upload_twiddles(N);
     const bool four_step = (N == 16384 || N == 32768 || N == 65536);      // spectrum64k.cu, R = N / 1024 branches
-    const bool wants1024 = (N == 2048 || N == 4096 || N == 8192 || four_step);
+    const bool wants1024 = (N == 8192 || four_step);
     if (pl->d_twiddle != nullptr && wants1024) pl->d_twiddle1024 = upload_twiddles(1024);
     if (pl->d_twiddle == nullptr || (wants1024 && pl->d_twiddle1024 == nullptr)) {
         set_error("spectrum plan: twiddle upload failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -258,10 +256,9 @@ b200_spectrum_plan* b200_spectrum_plan_create(int N, int hop, int K, int64_t row
             return nullptr;
         }
     }
-    if (N == 2048 || N == 4096 || N == 8192) {
-        const int M = N / 1024;
-        std::vector<float2> trk((size_t) M * 1024);
-        for (int r = 0; r < M; ++r)
+    if (N == 8192) {
+        std::vector<float2> trk((size_t) 8 * 1024);
+        for (int r = 0; r < 8; ++r)
             for (int k = 0; k < 1024; ++k) {
                 const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double) (r * k) / (long double) N;
                 trk[(size_t) r * 1024 + k] = make_float2((float) cosl(a), (float) sinl(a));
@@ -299,14 +296,6 @@ b200_spectrum_plan* b200_spectrum_plan_create(int N, int hop, int K, int64_t row
             }
         bool ok = cudaMalloc((void**) &pl->x64.twiddle_rk, sizeof(float2) * trk.size()) == cudaSuccess &&
                   cudaMemcpy((void*) pl->x64.twiddle_rk, trk.data(), sizeof(float2) * trk.size(), cudaMemcpyHostToDevice) == cudaSuccess;
-        std::vector<float2> t32((size_t) 32 * 32);
-        for (int n2 = 0; n2 < 32; ++n2)
-            for (int k1 = 0; k1 < 32; ++k1) {
-                const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double) (n2 * k1) / 1024.0L;
-                t32[(size_t) n2 * 32 + k1] = make_float2((float) cosl(a), (float) sinl(a));
-            }
-        ok = ok && cudaMalloc((void**) &pl->x64.twiddle_32x32, sizeof(float2) * t32.size()) == cudaSuccess &&
-             cudaMemcpy((void*) pl->x64.twiddle_32x32, t32.data(), sizeof(float2) * t32.size(), cudaMemcpyHostToDevice) == cudaSuccess;
         pl->x64.scratch_ctas = sm_count();
         ok = ok && cudaMalloc((void**) &pl->x64.scratch, sizeof(float2) * (size_t) N * (size_t) pl->x64.scratch_ctas) == cudaSuccess;
         if (ok && K > 1) ok = cudaMalloc((void**) &pl->x64.acc, sizeof(float) * (size_t) N * (size_t) pl->x64.scratch_ctas) == cudaSuccess;
@@ -328,7 +317,6 @@ void b200_spectrum_plan_destroy(b200_spectrum_plan* plan)
     if (plan->d_twiddle_4k) cudaFree(plan->d_twiddle_4k);
     if (plan->d_window) cudaFree(plan->d_window);
     if (plan->x64.twiddle_rk) cudaFree((void*) plan->x64.twiddle_rk);
-    if (plan->x64.twiddle_32x32) cudaFree((void*) plan->x64.twiddle_32x32);
     if (plan->x64.scratch) cudaFree(plan->x64.scratch);
     if (plan->x64.acc) cudaFree(plan->x64.acc);
     if (plan->gen_scratch) cudaFree(plan->gen_scratch);
@@ -384,34 +372,28 @@ static int spectrum_exec_kind(b200_spectrum_plan* plan, const void* d_in, int64_
         }
         return launch_spectrum1024(p, stream);
     }
-    if (kind == 0 && plan->d_twiddle1024 != nullptr) {
+    if (kind == 0 && plan->N >= 2048) {
         if ((reinterpret_cast<uintptr_t>(d_in) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
             set_error("spectrum exec: IQ pointer and stream stride must be 16-byte aligned");
             return B200_ERR_ALIGN;
-        }
-        p.twiddle = plan->d_twiddle1024;
-        const bool four_step = plan->x64.twiddle_rk != nullptr;
-        p.twiddle_n = four_step ? plan->d_twiddle : plan->d_twiddle_rk;
-        if (four_step) {
-            // B200_S64K_CLUSTER=1 selects the four-CTA cluster kernel (Z in distributed shared memory, K = 1 rows;
-            // spectrum64k_cluster.cu): DRAM traffic 1.0x algorithmic but 111 vs 123 Gsamples/s, so it is not the default.
-            const char* env = getenv("B200_S64K_CLUSTER");
-            if (plan->N == 65536 && plan->K == 1 && env != nullptr && atoi(env) != 0)
-                return launch_spectrum64k_cluster(p, plan->x64, stream);
-            return with_plan_scratch(plan, stream, [&] { return launch_spectrum64k(p, plan->x64, plan->N, stream); });
-        }
-        if (plan->N == 4096) {
-            p.twiddle_n = plan->d_twiddle_4k;
-            return launch_spectrum4096(p, stream);
         }
         if (plan->N == 2048) {
             p.twiddle_n = plan->d_twiddle_4k;
             return launch_spectrum2048(p, stream);
         }
-        return launch_spectrum_mx1024(p, plan->N, stream);
+        if (plan->N == 4096) {
+            p.twiddle_n = plan->d_twiddle_4k;
+            return launch_spectrum4096(p, stream);
+        }
+        p.twiddle = plan->d_twiddle1024;
+        if (plan->N == 8192) {
+            p.twiddle_n = plan->d_twiddle_rk;
+            return launch_spectrum_mx1024(p, stream);
+        }
+        return with_plan_scratch(plan, stream, [&] { return launch_spectrum64k(p, plan->x64, plan->N, stream); });
     }
     if (plan->N <= 8192) return launch_spectrum_generic(p, plan->N, kind, nullptr, nullptr, 0, stream);
-    // N > 8192 on the generic kernel (16384 / 32768 from bytes, any N > 8192 from s32 / f32 input): its per-CTA work
+    // N > 8192 from s32 / f32 input on the generic kernel: its per-CTA work
     // arrays live in the plan, on the plan's device, allocated on first use
     {
         std::lock_guard<std::mutex> lock(plan->scratch_mutex);

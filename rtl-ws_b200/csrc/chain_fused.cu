@@ -6,20 +6,18 @@
 //
 // Tile = 5120 samples = lcm(1024, 4 * 10): 5 frames and 128 audio samples, plus the FM
 // branch's 320-sample history (32 decimated samples) in front: 10880 bytes, fetched by one
-// TMA bulk copy into a four-deep ring with full/empty mbarriers.  A CTA is 6 symmetric warps
-// that never meet at a block barrier.  For every tile each warp
-//   - does a third of a sixth... precisely 3 of the tile's 18 discriminator chunks (CIC sums
-//     with dp4a, atan2_approx, difference + limiter -> demod[], four buffers deep),
-//   - and 5 of the 6 warps unpack one frame each into registers, release the stage, run the
-//     32x32 two-pass transform, |X|^2, dB and store 4 KB of spectrum;
-//   - the sixth warp (rotating: tile index mod 6) is the tile's service warp: it re-arms the
-//     TMA producer and runs the two half-band decimators of the PREVIOUS tile -> 128 audio
-//     floats.  Its job is about a third of a transform, so it simply gets ahead.
-// All 12 warps an SM holds (two CTAs at <= 168 registers) are transform-capable; none idles
-// on a role.  Tiles are independent (a tile's audio depends on input bytes only, through the
-// history), so CTAs stride over (stream, tile) with no inter-CTA communication.
-#include <stdlib.h>
-
+// TMA bulk copy into a four-deep ring with full/empty mbarriers.  A tile is six jobs:
+//   - five frame jobs: 3 of the tile's 18 discriminator chunks (CIC sums with dp4a,
+//     atan2_approx, difference + limiter -> demod[], four buffers deep), then unpack one frame
+//     into registers, release the stage, run the 32x32 two-pass transform, |X|^2, dB and store
+//     4 KB of spectrum;
+//   - one service job: 3 chunks, re-arm the TMA producer and run the two half-band decimators
+//     of the PREVIOUS tile -> 128 audio floats.
+// One CTA per SM of 18 warps; each warp takes the next job from a shared counter, so no warp is
+// tied to a role and none meets another at a block barrier.  The inter-pass twiddles come from
+// an 8 KB shared table instead of 62 registers per lane, which is what lets 18 warps fit.
+// Tiles are independent (a tile's audio depends on input bytes only, through the history), so
+// CTAs stride over (stream, tile) with no inter-CTA communication.
 #include "b200_common.cuh"
 #include "fft1024_warp.cuh"
 #include "fm_kernels.cuh"
@@ -28,22 +26,36 @@ namespace b200 {
 
 namespace {
 
-constexpr int CF_WARPS = 6;                         // warps per group: 5 transforms + 1 service per tile
-constexpr int CF_GROUPS = 2;                        // independent groups per CTA (see kernel comment)
-constexpr int CF_THREADS = CF_GROUPS * CF_WARPS * 32;
-constexpr int CF_STAGES = 4;
+constexpr int CF_WARPS = 18;
+constexpr int CF_THREADS = CF_WARPS * 32;
+constexpr int CF_STAGES = 4;                        // TMA ring
 constexpr int CF_DBUF = 4;                          // demod[] / work[] buffers: tiles a fast warp may run ahead
 constexpr int CF_TILE = 5120;                       // samples
 constexpr int CF_HIST = 320;                        // samples of history in front of a tile
 constexpr int CF_STAGE_BYTES = 2 * (CF_TILE + CF_HIST);   // 10880
-constexpr int CF_ND = (CF_TILE + CF_HIST) / 10;     // 544 decimated samples per tile
-constexpr int CF_ND_PAD = 576;                      // demod[] pitch: the 18 chunks of 31 cover indices up to 557
+constexpr int CF_ND_PAD = 576;                      // demod[] pitch: 544 decimated samples per tile, but the
+                                                    // 18 chunks of 31 cover indices up to 557
 constexpr int CF_NW = 2 * 128 + 10;                 // 266 first-stage outputs per tile
 constexpr int CF_WORK = 272;                        // CF_NW padded
-constexpr int CF_GROUP_SMEM = CF_STAGES * CF_STAGE_BYTES + CF_WARPS * FFT1024_XCH_BYTES + CF_DBUF * CF_ND_PAD * 4 +
-                              CF_DBUF * CF_WORK * 4 + (2 * CF_STAGES + 2 * CF_DBUF) * 8;
-static_assert(CF_GROUP_SMEM % 128 == 0, "group shared memory must keep the TMA destinations 128-byte aligned");
-constexpr int CF_SMEM = CF_GROUPS * CF_GROUP_SMEM;
+
+constexpr int CF_RING_BYTES = CF_STAGES * CF_STAGE_BYTES;
+constexpr int CF_XCH_BYTES = CF_WARPS * FFT1024_XCH_BYTES;
+constexpr int CF_DEMOD_BYTES = CF_DBUF * CF_ND_PAD * 4;
+constexpr int CF_WORK_BYTES = CF_DBUF * CF_WORK * 4;
+constexpr int CF_BAR_BYTES = (2 * CF_STAGES + 2 * CF_DBUF) * 8 + 8;     // + the job counter
+constexpr int CF_TW_OFFSET = (CF_RING_BYTES + CF_XCH_BYTES + CF_DEMOD_BYTES + CF_WORK_BYTES + CF_BAR_BYTES + 127) / 128 * 128;
+constexpr int CF_SMEM = CF_TW_OFFSET + 32 * 32 * 8;                     // + the [n2][k1] twiddle table
+static_assert(CF_SMEM <= 232448, "more shared memory than a CTA may have on sm_100");
+static_assert(CF_STAGE_BYTES % 128 == 0, "ring stages must stay 128-byte aligned");
+// A waiter tests the PARITY of a barrier phase, so it must never get two phases ahead of the barrier: no job of
+// tile it + S (or it + D) may be claimed while a job of tile it is still running.  Jobs are claimed in order and
+// at most W are in flight, so the first job of tile it + S (number 6 (it + S)) is claimed after job
+// 6 (it + S) - W + 1 - 1 has been claimed and ... finished only if it is older than every running job:
+// 6 (it + S) - (W - 1) > 6 it + 5.  (W = 20, S = 3 broke exactly this at kernel start: measured, 78 dB off.)
+static_assert(CF_WARPS <= 6 * CF_STAGES - 5, "ring too shallow for this many warps: a full[] waiter could lap the barrier");
+// demod[] buffers: the audio job of tile it (job 6 (it + 1)) waits for phase it / D of demod_full[it % D]; it would
+// pass a phase early if the audio job of tile it - D (6 D jobs older) had not passed its own wait yet
+static_assert(CF_WARPS <= 6 * CF_DBUF, "too few demod buffers for this many warps");
 
 struct ChainParams {
     const uint8_t* iq;             // stream 0, first sample of the batch (history lies before it)
@@ -59,37 +71,41 @@ struct ChainParams {
     const float2* twiddle;
 };
 
-// One CTA per SM holds TWO independent six-warp groups (own ring, own barriers, own tiles):
-// warps are assigned to the four schedulers by warp index mod 4, so a lone six-warp CTA would
-// load them 2-2-1-1 (and two such CTAs 4-4-2-2); twelve warps in one CTA land 3-3-3-3.
-__global__ void __launch_bounds__(CF_THREADS, 1) chain_fused_kernel(const ChainParams p)
+// The six jobs of a tile (service + five frames) are not tied to particular warps: every warp takes the next job
+// from a shared counter, and a warp that drew the short service job simply comes back sooner.  Jobs are claimed in
+// order and only ever wait for lower-numbered jobs (ring refills, demod hand-off), so the lowest unfinished job can
+// always run: no deadlock whatever the interleaving.  The inter-pass twiddles W_1024^(n2 k1) come from a shared
+// [n2][k1] table (one LDS.64 per pair member, conflict-free).
+__global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainParams p)
 {
-    extern __shared__ __align__(128) uint8_t smem_all[];
+    extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x;
     const int lane = tid & 31;
-    const int group = (tid >> 5) / CF_WARPS;
-    const int warp = (tid >> 5) % CF_WARPS;
-    uint8_t* smem = smem_all + group * CF_GROUP_SMEM;
+    const int warp = tid >> 5;
     uint8_t* ring = smem;
-    uint8_t* xch_base = smem + CF_STAGES * CF_STAGE_BYTES;
-    float2* xch = reinterpret_cast<float2*>(xch_base + warp * FFT1024_XCH_BYTES);
-    float* demod_base = reinterpret_cast<float*>(xch_base + CF_WARPS * FFT1024_XCH_BYTES);   // [CF_DBUF][CF_ND_PAD]
+    float2* xch = reinterpret_cast<float2*>(smem + CF_RING_BYTES + warp * FFT1024_XCH_BYTES);
+    float* demod_base = reinterpret_cast<float*>(smem + CF_RING_BYTES + CF_XCH_BYTES);         // [CF_DBUF][CF_ND_PAD]
     float* work_base = demod_base + CF_DBUF * CF_ND_PAD;                                         // [CF_DBUF][CF_WORK]
     uint64_t* full = reinterpret_cast<uint64_t*>(work_base + CF_DBUF * CF_WORK);
     uint64_t* empty = full + CF_STAGES;
-    uint64_t* demod_full = empty + CF_STAGES;       // [CF_DBUF]
-    uint64_t* demod_empty = demod_full + CF_DBUF;   // [CF_DBUF]
+    uint64_t* demod_full = empty + CF_STAGES;
+    uint64_t* demod_empty = demod_full + CF_DBUF;
+    uint32_t* next_job = reinterpret_cast<uint32_t*>(demod_empty + CF_DBUF);
+    float2* tws = reinterpret_cast<float2*>(smem + CF_TW_OFFSET);                               // [n2][k1]
 
-    const uint32_t tps = (uint32_t) p.tiles_per_stream;
-    const uint32_t total_tiles = (uint32_t) p.n_streams * tps;
-    const uint32_t first = blockIdx.x * CF_GROUPS + group;           // groups stride over tiles like CTAs would
-    const uint32_t stride = gridDim.x * CF_GROUPS;
+    const uint32_t total_tiles = (uint32_t) p.n_streams * (uint32_t) p.tiles_per_stream;
+    const uint32_t first = blockIdx.x;
+    const uint32_t stride = gridDim.x;
     const uint32_t n_mine = first < total_tiles ? (total_tiles - first + stride - 1) / stride : 0;
 
+    // tile -> (stream, tile in stream) without a division: tile * magic >> shift (exact below 2^31)
+    auto locate = [&](uint32_t tile, uint32_t& s, uint32_t& t) {
+        s = (uint32_t) (((uint64_t) tile * p.tps_magic) >> p.tps_shift);
+        t = tile - s * (uint32_t) p.tiles_per_stream;
+    };
     auto issue = [&](uint32_t it) {
-        const uint32_t tile = first + it * stride;
-        const uint32_t s = tile / tps;
-        const uint32_t t = tile - s * tps;
+        uint32_t s, t;
+        locate(first + it * stride, s, t);
         const int st = it % CF_STAGES;
         const uint8_t* src = p.iq + (int64_t) s * p.stream_stride_bytes + 2 * ((int64_t) t * CF_TILE - CF_HIST);
         mbar_arrive_expect_tx(&full[st], CF_STAGE_BYTES);
@@ -97,9 +113,8 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_fused_kernel(const ChainP
     };
     // the two half-band decimators of local tile `it` (audio_main.c:133,139); one warp
     auto audio_job = [&](uint32_t it) {
-        const uint32_t tile = first + it * stride;
-        const uint32_t s = tile / tps;
-        const uint32_t t = tile - s * tps;
+        uint32_t s, t;
+        locate(first + it * stride, s, t);
         const int buf = it % CF_DBUF;
         const float* demod = demod_base + buf * CF_ND_PAD;
         float* work = work_base + buf * CF_WORK;
@@ -116,201 +131,18 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_fused_kernel(const ChainP
     if (warp == 0 && lane == 0) {
         for (int i = 0; i < CF_STAGES; ++i) {
             mbar_init(&full[i], 1);
-            mbar_init(&empty[i], CF_WARPS);
-        }
-        for (int i = 0; i < CF_DBUF; ++i) {
-            mbar_init(&demod_full[i], CF_WARPS);
-            mbar_init(&demod_empty[i], 1);
-        }
-        fence_mbar_init();
-        for (uint32_t it = 0; it < CF_STAGES - 1 && it < n_mine; ++it) issue(it);
-    }
-    __syncthreads();
-
-    float2 tw[32];
-    fft1024_load_twiddles(p.twiddle, lane, tw);
-
-    int service = 0;                      // which warp serves this tile: it mod 6
-    for (uint32_t it = 0; it < n_mine; ++it) {
-        const int st = it % CF_STAGES;
-        const uint32_t tile = first + it * stride;
-        const uint32_t s = tile / tps;
-        const uint32_t t = tile - s * tps;
-        const int buf = it % CF_DBUF;
-        float* demod = demod_base + buf * CF_ND_PAD;
-        const bool serving = (warp == service);
-        // frames 0..4 go to the five other warps in rotation order
-        int slot = warp - service - 1;
-        if (slot < 0) slot += CF_WARPS;
-
-        mbar_wait(&full[st], (it / CF_STAGES) & 1);
-        const uint8_t* in = ring + st * CF_STAGE_BYTES;
-
-        // ---- discriminator share: 3 chunks of 31 outputs (lane 0 only supplies phase[j-1]);
-        //      demod[buf] must have been drained by the audio job of tile it - CF_DBUF ----
-        if (it >= CF_DBUF) mbar_wait(&demod_empty[buf], ((it - CF_DBUF) / CF_DBUF) & 1);
-#pragma unroll
-        for (int c3 = 0; c3 < 3; ++c3) {
-            const int j = 31 * (warp + CF_WARPS * c3) + lane;
-            // straight-line on purpose (the three chunks interleave): the last chunk's lanes 17..31
-            // read up to 280 bytes past the stage -- still inside this group's shared memory -- and
-            // write demod[544..557], padding that is never read
-            uint32_t ure, uim;
-            cic10_sum(reinterpret_cast<const uint32_t*>(in + j * 20), ure, uim);
-            const float ph = atan2_approx_dev(__uint_as_float(uim) - CIC_MAGIC, __uint_as_float(ure) - CIC_MAGIC);
-            const float prev = __shfl_up_sync(0xffffffffu, ph, 1);
-            if (lane > 0) demod[j] = fm_limit(ph, prev);                   // demod[0] is never read
-        }
-
-        if (!serving) {
-            c64 a[32];
-            fft1024_load<false>(reinterpret_cast<const uint16_t*>(in + 2 * CF_HIST + 2048 * slot), nullptr, lane, a);
-            __syncwarp();
-            if (lane == 0) {
-                mbar_arrive(&empty[st]);
-                mbar_arrive(&demod_full[buf]);
-            }
-            float pw[32];
-            fft1024_core<true>(a, tw, xch, lane, pw);
-            // DC-position patch (spectrum.c:30-33): display index 512 takes display index 511's value
-            const float left = __shfl_sync(0xffffffffu, pw[31], 31);
-            if (lane == 0) pw[0] = left;
-            float* out = p.db + ((size_t) s * tps * 5 + (size_t) t * 5 + slot) * 1024 + lane;
-#pragma unroll
-            for (int k2 = 0; k2 < 32; ++k2)
-                __stcs(out + fft1024_col(k2), fmaf(DB_PER_LOG2, lg2_ftz(pw[k2]), p.dboff));
-        } else {
-            __syncwarp();
-            if (lane == 0) {
-                mbar_arrive(&empty[st]);
-                mbar_arrive(&demod_full[buf]);
-                // keep the ring full: tile it + STAGES - 1 goes into the stage tile it - 1 used
-                if (it + CF_STAGES - 1 < n_mine) {
-                    if (it > 0) mbar_wait(&empty[(it - 1) % CF_STAGES], ((it - 1) / CF_STAGES) & 1);
-                    issue(it + CF_STAGES - 1);
-                }
-            }
-            __syncwarp();
-            if (it > 0) audio_job(it - 1);
-        }
-        service = (service + 1 == CF_WARPS) ? 0 : service + 1;
-    }
-    // the last tile's audio: the warp that would serve tile n_mine
-    if (n_mine > 0 && warp == service) audio_job(n_mine - 1);
-}
-
-// ---- the job-queue form ----------------------------------------------------------------------
-// Same tile, same ring, same barriers, same arithmetic as chain_fused_kernel, but the six jobs of
-// a tile (service + five frames) are no longer tied to six particular warps: every warp of a group
-// takes the next job from a shared counter.  That decouples the warp count from the tile shape, so
-// a group can be 8 warps (two groups) or 16 (one group) per SM -- four warps per scheduler
-// instead of three -- and a warp that drew the short service job simply comes back sooner.  Jobs
-// are claimed in order and only ever wait for lower-numbered jobs (ring refills, demod hand-off), so
-// the lowest unfinished job can always run: no deadlock whatever the interleaving.
-// With TWS the inter-pass twiddles W_1024^(n2 k1) come from a shared [n2][k1] table (8 KB per
-// CTA, one LDS.64 per pair member, conflict-free) instead of 62 registers per lane; that is what
-// lets 16 warps fit at 128 registers.
-template <int W, int G, int S, int D, bool TWS>
-struct ChainJobsCfg {
-    static constexpr int THREADS = W * G * 32;
-    static constexpr int RING_BYTES = S * CF_STAGE_BYTES;
-    static constexpr int XCH_BYTES = W * FFT1024_XCH_BYTES;
-    static constexpr int DEMOD_BYTES = D * CF_ND_PAD * 4;
-    static constexpr int WORK_BYTES = D * CF_WORK * 4;
-    static constexpr int BAR_BYTES = (2 * S + 2 * D) * 8 + 8;          // + the job counter
-    static constexpr int GROUP_SMEM = (RING_BYTES + XCH_BYTES + DEMOD_BYTES + WORK_BYTES + BAR_BYTES + 127) / 128 * 128;
-    static constexpr int TW_BYTES = TWS ? 32 * 32 * 8 : 0;
-    static constexpr int SMEM = G * GROUP_SMEM + TW_BYTES;
-    static_assert(SMEM <= 232448, "more shared memory than a CTA may have on sm_100");
-    static_assert(CF_STAGE_BYTES % 128 == 0, "ring stages must stay 128-byte aligned");
-    // A waiter tests the PARITY of a barrier phase, so it must never get two phases ahead of the barrier: no job of
-    // tile it + S (or it + D) may be claimed while a job of tile it is still running.  Jobs are claimed in order and
-    // at most W are in flight, so the first job of tile it + S (number 6 (it + S)) is claimed after job
-    // 6 (it + S) - W + 1 - 1 has been claimed and ... finished only if it is older than every running job:
-    // 6 (it + S) - (W - 1) > 6 it + 5.  (W = 20, S = 3 broke exactly this at kernel start: measured, 78 dB off.)
-    static_assert(W <= 6 * S - 5, "ring too shallow for this many warps: a full[] waiter could lap the barrier");
-    // demod[] buffers: the audio job of tile it (job 6 (it + 1)) waits for phase it / D of demod_full[it % D]; it would
-    // pass a phase early if the audio job of tile it - D (6 D jobs older) had not passed its own wait yet
-    static_assert(W <= 6 * D, "too few demod buffers for this many warps");
-};
-
-template <int W, int G, int S, int D, bool TWS>
-__global__ void __launch_bounds__(W * G * 32, 1) chain_jobs_kernel(const ChainParams p)
-{
-    using C = ChainJobsCfg<W, G, S, D, TWS>;
-    extern __shared__ __align__(128) uint8_t smem_all[];
-    const int tid = threadIdx.x;
-    const int lane = tid & 31;
-    const int group = (tid >> 5) / W;
-    const int warp = (tid >> 5) % W;
-    uint8_t* smem = smem_all + group * C::GROUP_SMEM;
-    uint8_t* ring = smem;
-    float2* xch = reinterpret_cast<float2*>(smem + C::RING_BYTES + warp * FFT1024_XCH_BYTES);
-    float* demod_base = reinterpret_cast<float*>(smem + C::RING_BYTES + C::XCH_BYTES);       // [D][CF_ND_PAD]
-    float* work_base = demod_base + D * CF_ND_PAD;                                            // [D][CF_WORK]
-    uint64_t* full = reinterpret_cast<uint64_t*>(work_base + D * CF_WORK);
-    uint64_t* empty = full + S;
-    uint64_t* demod_full = empty + S;
-    uint64_t* demod_empty = demod_full + D;
-    uint32_t* next_job = reinterpret_cast<uint32_t*>(demod_empty + D);
-    const float2* tws = reinterpret_cast<const float2*>(smem_all + G * C::GROUP_SMEM);      // [n2][k1]
-
-    const uint32_t total_tiles = (uint32_t) p.n_streams * (uint32_t) p.tiles_per_stream;
-    const uint32_t first = blockIdx.x * G + group;
-    const uint32_t stride = gridDim.x * G;
-    const uint32_t n_mine = first < total_tiles ? (total_tiles - first + stride - 1) / stride : 0;
-
-    // tile -> (stream, tile in stream) without a division: tile * magic >> shift (exact below 2^31)
-    auto locate = [&](uint32_t tile, uint32_t& s, uint32_t& t) {
-        s = (uint32_t) (((uint64_t) tile * p.tps_magic) >> p.tps_shift);
-        t = tile - s * (uint32_t) p.tiles_per_stream;
-    };
-    auto issue = [&](uint32_t it) {
-        uint32_t s, t;
-        locate(first + it * stride, s, t);
-        const int st = it % S;
-        const uint8_t* src = p.iq + (int64_t) s * p.stream_stride_bytes + 2 * ((int64_t) t * CF_TILE - CF_HIST);
-        mbar_arrive_expect_tx(&full[st], CF_STAGE_BYTES);
-        tma_load_1d(ring + st * CF_STAGE_BYTES, src, CF_STAGE_BYTES, &full[st]);
-    };
-    // the two half-band decimators of local tile `it` (audio_main.c:133,139); one warp
-    auto audio_job = [&](uint32_t it) {
-        uint32_t s, t;
-        locate(first + it * stride, s, t);
-        const int buf = it % D;
-        const float* demod = demod_base + buf * CF_ND_PAD;
-        float* work = work_base + buf * CF_WORK;
-        mbar_wait(&demod_full[buf], (it / D) & 1);
-        for (int m = lane; m < CF_NW; m += 32)              // work index 0 <-> 2*n0 - 10
-            work[m] = halfband_from(demod + 2 * m + 2);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&demod_empty[buf]);
-        float* out = p.audio + (int64_t) s * p.audio_stride + (int64_t) t * 128;
-#pragma unroll
-        for (int r = 0; r < 4; ++r) out[32 * r + lane] = halfband_from(work + 2 * (32 * r + lane));
-    };
-
-    if (warp == 0 && lane == 0) {
-        for (int i = 0; i < S; ++i) {
-            mbar_init(&full[i], 1);
             mbar_init(&empty[i], 6);
         }
-        for (int i = 0; i < D; ++i) {
+        for (int i = 0; i < CF_DBUF; ++i) {
             mbar_init(&demod_full[i], 6);
             mbar_init(&demod_empty[i], 1);
         }
         *next_job = 0;
         fence_mbar_init();
-        for (uint32_t it = 0; it < S - 1 && it < n_mine; ++it) issue(it);
+        for (uint32_t it = 0; it < CF_STAGES - 1 && it < n_mine; ++it) issue(it);
     }
-    if (TWS) {
-        float2* t = const_cast<float2*>(tws);
-        for (int i = tid; i < 1024; i += C::THREADS) t[i] = __ldg(&p.twiddle[((i >> 5) * (i & 31)) & 1023]);
-    }
+    for (int i = tid; i < 1024; i += CF_THREADS) tws[i] = __ldg(&p.twiddle[((i >> 5) * (i & 31)) & 1023]);
     __syncthreads();
-
-    float2 tw[32];
-    if (!TWS) fft1024_load_twiddles(p.twiddle, lane, tw);
 
     // jobs 6*it + pos: pos 0 = the tile's service job, 1..5 = frames 0..4; job 6*n_mine = the last tile's audio
     const uint32_t n_jobs = n_mine > 0 ? 6 * n_mine + 1 : 0;
@@ -325,21 +157,21 @@ __global__ void __launch_bounds__(W * G * 32, 1) chain_jobs_kernel(const ChainPa
             audio_job(n_mine - 1);
             break;
         }
-        const int st = it % S;
-        const int buf = it % D;
+        const int st = it % CF_STAGES;
+        const int buf = it % CF_DBUF;
         float* demod = demod_base + buf * CF_ND_PAD;
 
-        mbar_wait(&full[st], (it / S) & 1);
+        mbar_wait(&full[st], (it / CF_STAGES) & 1);
         const uint8_t* in = ring + st * CF_STAGE_BYTES;
 
         // ---- discriminator share: 3 of the tile's 18 chunks of 31 outputs (lane 0 only supplies
-        //      phase[j-1]); demod[buf] must have been drained by the audio job of tile it - D ----
-        if (it >= (uint32_t) D) mbar_wait(&demod_empty[buf], ((it / D) - 1) & 1);
+        //      phase[j-1]); demod[buf] must have been drained by the audio job of tile it - CF_DBUF ----
+        if (it >= (uint32_t) CF_DBUF) mbar_wait(&demod_empty[buf], ((it / CF_DBUF) - 1) & 1);
 #pragma unroll
         for (int c3 = 0; c3 < 3; ++c3) {
             const int j = 31 * (pos + 6 * c3) + lane;
             // the last chunk's lanes 17..31 read up to 280 bytes past the stage -- still inside this
-            // group's shared memory -- and write demod[544..557], padding that is never read
+            // CTA's shared memory -- and write demod[544..557], padding that is never read
             uint32_t ure, uim;
             cic10_sum(reinterpret_cast<const uint32_t*>(in + j * 20), ure, uim);
             const float ph = atan2_approx_dev2(__uint_as_float(uim) - CIC_MAGIC, __uint_as_float(ure) - CIC_MAGIC);
@@ -358,10 +190,7 @@ __global__ void __launch_bounds__(W * G * 32, 1) chain_jobs_kernel(const ChainPa
             }
             fft1024_pass1<true>(a);
             c64 b[32];
-            if (TWS)
-                fft1024_pass2_smem_tw<false>(a, tws + lane, xch, lane, b);
-            else
-                fft1024_pass2(a, tw, xch, lane, b);
+            fft1024_pass2_smem_tw<false>(a, tws + lane, xch, lane, b);
             float pw[32];
             fft1024_power(b, pw);
             // DC-position patch (spectrum.c:30-33): display index 512 takes display index 511's value
@@ -374,30 +203,16 @@ __global__ void __launch_bounds__(W * G * 32, 1) chain_jobs_kernel(const ChainPa
             if (lane == 0) {
                 mbar_arrive(&empty[st]);
                 mbar_arrive(&demod_full[buf]);
-                // keep the ring full: tile it + S - 1 goes into the stage tile it - 1 used
-                if (it + S - 1 < n_mine) {
-                    if (it > 0) mbar_wait(&empty[(it - 1) % S], ((it - 1) / S) & 1);
-                    issue(it + S - 1);
+                // keep the ring full: tile it + CF_STAGES - 1 goes into the stage tile it - 1 used
+                if (it + CF_STAGES - 1 < n_mine) {
+                    if (it > 0) mbar_wait(&empty[(it - 1) % CF_STAGES], ((it - 1) / CF_STAGES) & 1);
+                    issue(it + CF_STAGES - 1);
                 }
             }
             __syncwarp();
             if (it > 0) audio_job(it - 1);
         }
     }
-}
-
-template <int W, int G, int S, int D, bool TWS>
-int launch_chain_jobs(const ChainParams& p, int64_t total, cudaStream_t stream)
-{
-    using C = ChainJobsCfg<W, G, S, D, TWS>;
-    auto kern = chain_jobs_kernel<W, G, S, D, TWS>;
-    if (int rc = ensure_dynamic_smem((const void*) kern, C::SMEM)) return rc;
-    int64_t grid = sm_count();
-    const int64_t needed = (total + G - 1) / G;
-    if (grid > needed) grid = needed;
-    kern<<<(unsigned) grid, C::THREADS, C::SMEM, stream>>>(p);
-    B200_LAUNCH_CHECK();
-    return B200_OK;
 }
 
 }  // namespace
@@ -429,23 +244,10 @@ int launch_chain_fused(const uint8_t* d_iq, int64_t stride, int n_streams, int64
     while ((1ll << L) < tiles_per_stream) ++L;
     p.tps_magic = (uint32_t) (((1ull << (31 + L)) + (uint64_t) tiles_per_stream - 1) / (uint64_t) tiles_per_stream);
     p.tps_shift = 31 + L;
-    const char* venv = getenv("B200_CHAIN_VARIANT");       // tuning knob while the variants are being measured
-    const int variant = venv ? atoi(venv) : 6;
-    switch (variant) {
-        case 1: return launch_chain_jobs<16, 1, 5, 5, true>(p, total, stream);
-        case 2: return launch_chain_jobs<8, 2, 3, 2, true>(p, total, stream);
-        case 3: return launch_chain_jobs<6, 2, 4, 4, false>(p, total, stream);
-        case 4: return launch_chain_jobs<6, 2, 4, 4, true>(p, total, stream);
-        case 5: return launch_chain_jobs<14, 1, 5, 5, true>(p, total, stream);
-        case 6: return launch_chain_jobs<18, 1, 4, 4, true>(p, total, stream);
-        default: break;
-    }
-    if (int rc = ensure_dynamic_smem((const void*) chain_fused_kernel, CF_SMEM)) return rc;
-    const int ctas_per_sm = cached_occupancy((const void*) chain_fused_kernel, CF_THREADS, CF_SMEM);
-    int64_t grid = (int64_t) sm_count() * ctas_per_sm;
-    const int64_t needed = (total + CF_GROUPS - 1) / CF_GROUPS;
-    if (grid > needed) grid = needed;
-    chain_fused_kernel<<<(unsigned) grid, CF_THREADS, CF_SMEM, stream>>>(p);
+    if (int rc = ensure_dynamic_smem((const void*) chain_jobs_kernel, CF_SMEM)) return rc;
+    int64_t grid = sm_count();
+    if (grid > total) grid = total;
+    chain_jobs_kernel<<<(unsigned) grid, CF_THREADS, CF_SMEM, stream>>>(p);
     B200_LAUNCH_CHECK();
     return B200_OK;
 }

@@ -219,7 +219,7 @@ __device__ __forceinline__ void fft_dit32(c64 (&a)[32], const float2 (&tw)[32])
 // The same 32-point transform with the pre-multipliers read just in time from shared memory:
 // x[n] is multiplied by twp[32 * n] (n = 0 taken as 1).  twp already points at this lane's column
 // of a [32][32] table, so a warp load is 256 contiguous bytes.  Frees the 62 registers a
-// lane-private copy costs (chain_fused.cu runs 16 warps per SM at 128 registers with it).
+// lane-private copy costs (chain_fused.cu runs 18 warps per SM at 95 registers with it).
 __device__ __forceinline__ void fft_dit32_pretwiddled_smem(c64 (&a)[32], const float2* twp)
 {
 #pragma unroll
@@ -228,28 +228,6 @@ __device__ __forceinline__ void fft_dit32_pretwiddled_smem(c64 (&a)[32], const f
         const int nb = bitrev<32>(g + 1);
         const float2 ta = na == 0 ? make_float2(1.0f, 0.0f) : twp[32 * na];
         const float2 tb = twp[32 * nb];
-        dit_butterfly_pretwiddled(a[g], a[g + 1], na == 0, ta, tb);
-    }
-#pragma unroll
-    for (int half = 2; half <= 16; half <<= 1) {
-#pragma unroll
-        for (int g = 0; g < 32; g += 2 * half) {
-#pragma unroll
-            for (int k = 0; k < half; ++k) dit_butterfly(a[g + k], a[g + k + half], k * (16 / half));
-        }
-    }
-}
-
-// The same with the table in GLOBAL memory (8 KB, read through L1 with ld.global.nc): for kernels that have neither
-// 62 registers nor 8 KB of shared memory to spare (spectrum64k_cluster.cu).
-__device__ __forceinline__ void fft_dit32_pretwiddled_ldg(c64 (&a)[32], const float2* __restrict__ twp)
-{
-#pragma unroll
-    for (int g = 0; g < 32; g += 2) {
-        const int na = bitrev<32>(g);
-        const int nb = bitrev<32>(g + 1);
-        const float2 ta = na == 0 ? make_float2(1.0f, 0.0f) : __ldg(twp + 32 * na);
-        const float2 tb = __ldg(twp + 32 * nb);
         dit_butterfly_pretwiddled(a[g], a[g + 1], na == 0, ta, tb);
     }
 #pragma unroll

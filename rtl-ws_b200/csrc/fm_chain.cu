@@ -33,29 +33,21 @@ __host__ __device__ inline int fm_tile_audio(int R)
 
 // One warp-wide step of the discriminator: lane handles local decimated index j (bytes at
 // in + j * 2R); returns the phase (0 for j outside [0, nd)), and writes the CIC sums.
-template <int RT>
 __device__ __forceinline__ float fm_phase_at(const uint8_t* in, int R, int j, int nd, int& sre, int& sim)
 {
     uint32_t ure = CIC_MAGIC_BITS, uim = CIC_MAGIC_BITS;
-    if (j >= 0 && j < nd) {
-        if (RT == 10)
-            cic10_sum(reinterpret_cast<const uint32_t*>(in + j * 20), ure, uim);
-        else
-            cic_sum(reinterpret_cast<const uint16_t*>(in) + (size_t) j * R, R, ure, uim);
-    }
+    if (j >= 0 && j < nd) cic_sum(reinterpret_cast<const uint16_t*>(in) + (size_t) j * R, R, ure, uim);
     sre = (int) (ure - CIC_MAGIC_BITS);
     sim = (int) (uim - CIC_MAGIC_BITS);
     return atan2_approx_dev(__uint_as_float(uim) - CIC_MAGIC, __uint_as_float(ure) - CIC_MAGIC);
 }
 
-// RT = 10: the default decimation (cbb_main.c:80), word loads + dp4a, fully unrolled.
-// RT = 0:  any R, sample-wise.
-template <int RT>
+// Any R, sample-wise: the down factors 1, 2 and above 16 (3 <= R <= 16 take fm_chain_warp_kernel below).
 __global__ void __launch_bounds__(FM_THREADS) fm_chain_kernel(const FmParams p, const int T, const int tiles_per_stream,
                                                               const int stage_bytes)
 {
     extern __shared__ __align__(128) uint8_t smem[];
-    const int R = RT ? RT : p.R;
+    const int R = p.R;
     const int tid = threadIdx.x;
     const int lane = tid & 31;
     uint8_t* ring = smem;
@@ -105,11 +97,11 @@ __global__ void __launch_bounds__(FM_THREADS) fm_chain_kernel(const FmParams p, 
         for (int j0 = (tid & ~31); j0 < nd; j0 += FM_THREADS) {
             const int j = j0 + lane;
             int sre, sim;
-            const float ph = fm_phase_at<RT>(in, R, j, nd, sre, sim);
+            const float ph = fm_phase_at(in, R, j, nd, sre, sim);
             float prev = __shfl_up_sync(0xffffffffu, ph, 1);
             if (lane == 0) {
                 int a, b;
-                prev = fm_phase_at<RT>(in, R, j - 1, nd, a, b);
+                prev = fm_phase_at(in, R, j - 1, nd, a, b);
             }
             if (j < nd) {
                 demod[j] = fm_limit(ph, prev);
@@ -360,13 +352,12 @@ int launch_fm_chain(const FmParams& p, cudaStream_t stream)
     }
     const int stage_bytes = (4 * T + 32) * 2 * p.R;
     const int smem = 2 * stage_bytes + (4 * T + 32) * 4 + (2 * T + 16) * 4 + 16;
-    auto kern = fm_chain_kernel<0>;
-    if (int rc = ensure_dynamic_smem((const void*) kern, 2 * 32768 + 8192)) return rc;
-    const int ctas_per_sm = cached_occupancy((const void*) kern, FM_THREADS, smem);
+    if (int rc = ensure_dynamic_smem((const void*) fm_chain_kernel, 2 * 32768 + 8192)) return rc;
+    const int ctas_per_sm = cached_occupancy((const void*) fm_chain_kernel, FM_THREADS, smem);
     int64_t grid = (int64_t) sm_count() * ctas_per_sm;
     const int64_t total_tiles = (int64_t) p.n_streams * tiles_per_stream;
     if (grid > total_tiles) grid = total_tiles;
-    kern<<<(unsigned) grid, FM_THREADS, smem, stream>>>(p, T, (int) tiles_per_stream, stage_bytes);
+    fm_chain_kernel<<<(unsigned) grid, FM_THREADS, smem, stream>>>(p, T, (int) tiles_per_stream, stage_bytes);
     B200_LAUNCH_CHECK();
     return B200_OK;
 }

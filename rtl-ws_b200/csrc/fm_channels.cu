@@ -24,8 +24,6 @@
 #include "fft_regs.cuh"
 #include "fm_kernels.cuh"
 
-#include <stdlib.h>
-
 namespace b200 {
 
 namespace {
@@ -290,17 +288,9 @@ int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_str
     p.audio_stride = audio_stride;
     p.baseband = reinterpret_cast<float2*>(baseband);
     p.baseband_stride = baseband_stride;
-    if (R != 10) return launch_fc<0, 4>(p, tps, stream);
-    // channels per group at R = 10: 8 measured fastest (DESIGN.md 4.3a); B200_FM_CHANNELS_GROUP = 1 / 2 / 4 selects
-    // another for measurement (the bits do not change)
-    const char* env = getenv("B200_FM_CHANNELS_GROUP");
-    const int G = env != nullptr ? atoi(env) : 8;
-    switch (G) {
-        case 1: return launch_fc<10, 1>(p, tps, stream);
-        case 2: return launch_fc<10, 2>(p, tps, stream);
-        case 4: return launch_fc<10, 4>(p, tps, stream);
-        default: return launch_fc<10, 8>(p, tps, stream);
-    }
+    // channels per group at R = 10: 8 measured fastest at every channel count (DESIGN.md 4.3a)
+    if (R == 10) return launch_fc<10, 8>(p, tps, stream);
+    return launch_fc<0, 4>(p, tps, stream);
 }
 
 }  // namespace b200

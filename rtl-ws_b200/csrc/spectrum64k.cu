@@ -229,7 +229,8 @@ __global__ void __launch_bounds__(S64_THREADS, 1) spectrum64k_kernel(const SpecP
 // persisting property over the 74 MB, backed by a set-aside of the same size.  DRAM writes went UP (6.9 -> 11.9 GB per
 // 524 M samples: what is left of the L2 no longer absorbs the streaming rows) and the kernel lost 3 % (123 -> 119
 // Gsamples/s).  A sweep of the set-aside (32 / 64 / 79 MB = the device's maximum, misses left at normal priority) gave
-// 7.6 / 11.9 / 11.9 GB of DRAM writes against 7.0 without it: no size helps.  The four-CTA cluster kernel (spectrum64k_cluster.cu) removes the scratch altogether.
+// 7.6 / 11.9 / 11.9 GB of DRAM writes against 7.0 without it: no size helps.  A four-CTA cluster kernel that keeps Z in
+// distributed shared memory removes the scratch altogether, but measured slower (DESIGN.md 4.6).
 template <int R>
 static int launch_scratch(const SpecParams& p, const Spec64kExtra& x, cudaStream_t stream)
 {

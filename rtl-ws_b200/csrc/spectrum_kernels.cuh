@@ -18,8 +18,10 @@ struct SpecParams {
     float* power;                 // [n_streams][n_rows][N] or null
     uint8_t* db_u8;               // [n_streams][n_rows][N] or null
     float db_offset;              // 10*log10(g / (K * 2^14)): folds gain, /count and the 1/128 input scale
-    const float2* twiddle;        // exp(-2*pi*i*k/N), k = 0..N-1 (device); the 1024-point table for N = M * 1024
-    const float2* twiddle_n;      // N = 65536: the N-point table; N = M * 1024 <= 8192: [M][1024] W_N^(r k); else null
+    const float2* twiddle;        // exp(-2*pi*i*k/N), k = 0..N-1 (device); the 1024-point table for u8 input at
+                                  // N = 8192 and the four-step sizes (16384..65536)
+    const float2* twiddle_n;      // u8 input, N = 8192: [8][1024] W_N^(r k); N = 2048 / 4096: [N/64][64] W_N^(n2 k1);
+                                  // else null
     const float* window;          // N floats (device) or null = rectangular
 };
 
@@ -28,7 +30,6 @@ struct Spec64kExtra {
     float2* scratch;              // [scratch_ctas][64][1024] complex: Z[r][k], L2-resident
     float* acc;                   // [scratch_ctas][65536] power accumulators (K > 1), else null
     const float2* twiddle_rk;     // [64][1024]: exp(-2*pi*i*r*k/65536)
-    const float2* twiddle_32x32;  // [32][32]: exp(-2*pi*i*n2*k1/1024), the inter-pass table of the 1024-point transform
     int scratch_ctas;
 };
 

@@ -1,8 +1,7 @@
-// spectrum_mx1024.cu -- batched power spectra for N = M * 1024, M in {2, 4, 8} (sm_100a):
-// the frame lengths between the reference's 1024 and what still fits one CTA's shared memory.
-// The library routes N = 8192 here; 2048 and 4096 (BASELINE config 2's second size) have their own
-// kernels with a single shared-memory round trip (spectrum2048.cu, spectrum4096.cu); M = 2 and 4 are
-// kept as the general form (what those kernels were measured against: 517 vs 637 and 490 vs 675
+// spectrum_mx1024.cu -- batched power spectra for N = 8192 = M * 1024, M = 8 (sm_100a): the
+// largest frame that still fits one CTA's shared memory.  2048 and 4096 (BASELINE config 2's second
+// size) have their own kernels with a single shared-memory round trip (spectrum2048.cu,
+// spectrum4096.cu), which measured faster than this form at M = 2 and 4 (637 vs 517 and 675 vs 490
 // Gsamples/s).
 //
 // Decimation in time by M:  X[k + 1024 q] = sum_{r<M} W_M^(r q) * ( W_N^(r k) * F_r[k] ),
@@ -25,31 +24,26 @@ namespace b200 {
 
 namespace {
 
-template <int M>
-struct MxCfg {
-    static constexpr int N = M * 1024;
-    static constexpr int FRAME_BYTES = 2 * N;
-    static constexpr int THREADS = M * 32;
-    static constexpr int KPW = 32 / M;                       // k-groups of 32 per warp in the combine
-    static constexpr int STAGES = 2;                         // TMA ring
-    static constexpr int TILE_SETS = 2;                      // exchange tiles alternate between frames
-    static constexpr int BAR_OFFSET = STAGES * FRAME_BYTES + TILE_SETS * M * FFT1024_XCH_BYTES;
-    static constexpr int SMEM = BAR_OFFSET + 64;
-    static constexpr int CTAS_PER_SM = 8 / M;                 // 8 warps per SM: room for 255 registers per thread
-};
+constexpr int M = 8;                                 // polyphase branches = warps per CTA
+constexpr int N = M * 1024;
+constexpr int MX_FRAME_BYTES = 2 * N;
+constexpr int MX_THREADS = M * 32;
+constexpr int MX_KPW = 32 / M;                       // k-groups of 32 per warp in the combine
+constexpr int MX_STAGES = 2;                         // TMA ring
+constexpr int MX_TILE_SETS = 2;                      // exchange tiles alternate between frames
+constexpr int MX_BAR_OFFSET = MX_STAGES * MX_FRAME_BYTES + MX_TILE_SETS * M * FFT1024_XCH_BYTES;
+constexpr int MX_SMEM = MX_BAR_OFFSET + 64;
 
-// 32 output values of one warp (index g * M + q: bin = (r * KPW + g) * 32 + lane + 1024 q) -> the
+// 32 output values of one warp (index g * M + q: bin = (r * MX_KPW + g) * 32 + lane + 1024 q) -> the
 // requested arrays in display order (fftshift of spectrum.c:25: bin + N/2 mod N moves the q digit
-// by M/2).  `base` = row * N + r * KPW * 32 + lane: every store is base + a compile-time offset
+// by M/2).  `base` = row * N + r * MX_KPW * 32 + lane: every store is base + a compile-time offset
 // and a warp store covers 128 contiguous bytes.
-template <int M>
 __device__ __forceinline__ void store_bins(const SpecParams& p, float dboff, size_t base, const float (&pw)[32])
 {
-    constexpr int KPW = 32 / M;
     if (p.db != nullptr) {
         float* out = p.db + base;
 #pragma unroll
-        for (int g = 0; g < KPW; ++g)
+        for (int g = 0; g < MX_KPW; ++g)
 #pragma unroll
             for (int q = 0; q < M; ++q)
                 __stcs(out + 32 * g + 1024 * ((q + M / 2) % M), fmaf(DB_PER_LOG2, lg2_ftz(pw[g * M + q]), dboff));
@@ -57,14 +51,14 @@ __device__ __forceinline__ void store_bins(const SpecParams& p, float dboff, siz
     if (p.power != nullptr) {
         float* out = p.power + base;
 #pragma unroll
-        for (int g = 0; g < KPW; ++g)
+        for (int g = 0; g < MX_KPW; ++g)
 #pragma unroll
             for (int q = 0; q < M; ++q) __stcs(out + 32 * g + 1024 * ((q + M / 2) % M), pw[g * M + q] * FFT1024_POWER_SCALE);
     }
     if (p.db_u8 != nullptr) {
         uint8_t* out = p.db_u8 + base;
 #pragma unroll
-        for (int g = 0; g < KPW; ++g)
+        for (int g = 0; g < MX_KPW; ++g)
 #pragma unroll
             for (int q = 0; q < M; ++q) {
                 // cbb_main.c:125-127: (int) truncation toward zero, then clamp; -inf / NaN -> 0
@@ -82,19 +76,18 @@ __device__ __forceinline__ void store_bins(const SpecParams& p, float dboff, siz
 // unit, and (ii) had finished combining frame f - 1 before they started on f, so tile set
 // (f + 1) & 1 is free to be overwritten: nothing else needs ordering.  Between its arrival and the
 // wait a warp gathers the next frame and runs its first pass (registers only).
-template <int M, bool WINDOW, bool MULTI>
-__global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spectrum_mx1024_kernel(const SpecParams p)
+// One CTA of 8 warps per SM: room for 255 registers per thread.
+template <bool WINDOW, bool MULTI>
+__global__ void __launch_bounds__(MX_THREADS, 1) spectrum_mx1024_kernel(const SpecParams p)
 {
-    using C = MxCfg<M>;
-    constexpr int N = C::N;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x;
     const int lane = tid & 31;
     const int r = tid >> 5;                                   // polyphase branch of this warp
     uint8_t* ring = smem;
-    uint8_t* tiles = smem + C::STAGES * C::FRAME_BYTES;       // [set][branch] tiles of FFT1024_XCH_BYTES
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem + C::BAR_OFFSET);
-    uint64_t* zfull = full + C::STAGES;
+    uint8_t* tiles = smem + MX_STAGES * MX_FRAME_BYTES;       // [set][branch] tiles of FFT1024_XCH_BYTES
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + MX_BAR_OFFSET);
+    uint64_t* zfull = full + MX_STAGES;
 
     const uint32_t total_items = (uint32_t) p.n_streams * (uint32_t) p.n_rows;
     const uint32_t n_rows = (uint32_t) p.n_rows;
@@ -105,7 +98,7 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
 
     if (tid == 0) {
 #pragma unroll
-        for (int i = 0; i < C::STAGES; ++i) mbar_init(&full[i], 1);
+        for (int i = 0; i < MX_STAGES; ++i) mbar_init(&full[i], 1);
         mbar_init(&zfull[0], M);
         mbar_init(&zfull[1], M);
         fence_mbar_init();
@@ -120,9 +113,9 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
         return p.iq + (int64_t) s * p.stream_stride_bytes + 2 * ((int64_t) row * p.row_hop + (int64_t) j * p.hop);
     };
     if (tid == 0) {
-        for (uint32_t f = 0; f < (uint32_t) C::STAGES && f < n_frames; ++f) {
-            mbar_arrive_expect_tx(&full[f], C::FRAME_BYTES);
-            tma_load_1d(ring + f * C::FRAME_BYTES, frame_src(f), C::FRAME_BYTES, &full[f]);
+        for (uint32_t f = 0; f < (uint32_t) MX_STAGES && f < n_frames; ++f) {
+            mbar_arrive_expect_tx(&full[f], MX_FRAME_BYTES);
+            tma_load_1d(ring + f * MX_FRAME_BYTES, frame_src(f), MX_FRAME_BYTES, &full[f]);
         }
     }
 
@@ -142,9 +135,9 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
     // over n1, registers only)
     c64 a[32];
     auto gather_pass1 = [&](uint32_t ff) {
-        const int st = ff % C::STAGES;
-        mbar_wait(&full[st], (ff / C::STAGES) & 1);
-        const uint16_t* in16 = reinterpret_cast<const uint16_t*>(ring + st * C::FRAME_BYTES);
+        const int st = ff % MX_STAGES;
+        mbar_wait(&full[st], (ff / MX_STAGES) & 1);
+        const uint16_t* in16 = reinterpret_cast<const uint16_t*>(ring + st * MX_FRAME_BYTES);
         const c64 bias1 = cpack(8421376.0f, 8421376.0f);           // 2^23 + 256 * 128
 #pragma unroll
         for (int n1 = 0; n1 < 32; ++n1) {
@@ -165,9 +158,9 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
     uint32_t f = 0;
     for (uint32_t it = 0; it < n_items; ++it) {
         const uint32_t item = blockIdx.x + it * gridDim.x;
-        const size_t out_base = (size_t) item * N + (size_t) (r * C::KPW * 32 + lane);
+        const size_t out_base = (size_t) item * N + (size_t) (r * MX_KPW * 32 + lane);
         for (int j = 0; j < K; ++j, ++f) {
-            const int st = f % C::STAGES;
+            const int st = f % MX_STAGES;
             const int set = f & 1;
             float2* xch = reinterpret_cast<float2*>(tiles + (set * M + r) * FFT1024_XCH_BYTES);
 
@@ -188,22 +181,22 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
             if (lane == 0) mbar_arrive(&zfull[set]);
             if (f + 1 < n_frames) gather_pass1(f + 1);
             mbar_wait(&zfull[set], (f >> 1) & 1);
-            if (tid == 0 && f + C::STAGES < n_frames) {          // all branches have consumed the stage
+            if (tid == 0 && f + MX_STAGES < n_frames) {          // all branches have consumed the stage
                 fence_proxy_async_smem();
-                mbar_arrive_expect_tx(&full[st], C::FRAME_BYTES);
-                tma_load_1d(ring + st * C::FRAME_BYTES, frame_src(f + C::STAGES), C::FRAME_BYTES, &full[st]);
+                mbar_arrive_expect_tx(&full[st], MX_FRAME_BYTES);
+                tma_load_1d(ring + st * MX_FRAME_BYTES, frame_src(f + MX_STAGES), MX_FRAME_BYTES, &full[st]);
             }
 
-            // ---- combine: this warp owns k = (r * KPW + g) * 32 + lane, g < KPW ----
+            // ---- combine: this warp owns k = (r * MX_KPW + g) * 32 + lane, g < MX_KPW ----
             const uint8_t* zset = tiles + set * M * FFT1024_XCH_BYTES;
             float pw[32];
 #pragma unroll
-            for (int g = 0; g < C::KPW; ++g) {
+            for (int g = 0; g < MX_KPW; ++g) {
                 c64 z[M];
 #pragma unroll
                 for (int rr = 0; rr < M; ++rr)
                     z[bitrev<M>(rr)] =
-                        reinterpret_cast<const c64*>(zset + rr * FFT1024_XCH_BYTES)[(r * C::KPW + g) * 32 + lane];
+                        reinterpret_cast<const c64*>(zset + rr * FFT1024_XCH_BYTES)[(r * MX_KPW + g) * 32 + lane];
                 fft_dit_small<M>(z);
 #pragma unroll
                 for (int q = 0; q < M; ++q) {
@@ -234,12 +227,12 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
 #pragma unroll
                 for (int i = 0; i < 32; ++i) acc[i] += pw[i];
             } else {
-                store_bins<M>(p, dboff, out_base, pw);
+                store_bins(p, dboff, out_base, pw);
             }
         }
         if (MULTI) {
             if (r == 0 && lane == 0) acc[0] = dcacc;
-            store_bins<M>(p, dboff, out_base, acc);
+            store_bins(p, dboff, out_base, acc);
 #pragma unroll
             for (int i = 0; i < 32; ++i) acc[i] = 0.0f;
             dcacc = 0.0f;
@@ -247,41 +240,27 @@ __global__ void __launch_bounds__(MxCfg<M>::THREADS, MxCfg<M>::CTAS_PER_SM) spec
     }
 }
 
-template <int M>
-int launch_m(const SpecParams& p, cudaStream_t stream)
+}  // namespace
+
+// N = 8192, cmplx_u8 input.  p.twiddle must be the 1024-point table and p.twiddle_n the [8][1024] table
+// W_N^(r k) (capi.cu keeps both in the plan).
+int launch_spectrum_mx1024(const SpecParams& p, cudaStream_t stream)
 {
-    using C = MxCfg<M>;
     const uint64_t total = (uint64_t) p.n_streams * (uint64_t) p.n_rows;
+    if (total == 0) return B200_OK;
     if (total >= (1ull << 31)) {
         set_error("spectrum: n_streams * n_rows = %llu exceeds 2^31 - 1 rows per launch", (unsigned long long) total);
         return B200_ERR_ARG;
     }
-    auto kern = p.K > 1 ? (p.window ? spectrum_mx1024_kernel<M, true, true> : spectrum_mx1024_kernel<M, false, true>)
-                        : (p.window ? spectrum_mx1024_kernel<M, true, false> : spectrum_mx1024_kernel<M, false, false>);
-    if (int rc = ensure_dynamic_smem((const void*) kern, C::SMEM)) return rc;
-    const int ctas_per_sm = cached_occupancy((const void*) kern, C::THREADS, C::SMEM);
+    auto kern = p.K > 1 ? (p.window ? spectrum_mx1024_kernel<true, true> : spectrum_mx1024_kernel<false, true>)
+                        : (p.window ? spectrum_mx1024_kernel<true, false> : spectrum_mx1024_kernel<false, false>);
+    if (int rc = ensure_dynamic_smem((const void*) kern, MX_SMEM)) return rc;
+    const int ctas_per_sm = cached_occupancy((const void*) kern, MX_THREADS, MX_SMEM);
     uint64_t grid = (uint64_t) sm_count() * (uint64_t) ctas_per_sm;
     if (grid > total) grid = total;
-    kern<<<(unsigned) grid, C::THREADS, C::SMEM, stream>>>(p);
+    kern<<<(unsigned) grid, MX_THREADS, MX_SMEM, stream>>>(p);
     B200_LAUNCH_CHECK();
     return B200_OK;
-}
-
-}  // namespace
-
-// N = 2048, 4096 or 8192, cmplx_u8 input.  p.twiddle must be the 1024-point table and
-// p.twiddle_n the [M][1024] table W_N^(r k) (capi.cu keeps both in the plan).
-int launch_spectrum_mx1024(const SpecParams& p, int N, cudaStream_t stream)
-{
-    if ((uint64_t) p.n_streams * (uint64_t) p.n_rows == 0) return B200_OK;
-    switch (N) {
-        case 2048: return launch_m<2>(p, stream);
-        case 4096: return launch_m<4>(p, stream);
-        case 8192: return launch_m<8>(p, stream);
-        default:
-            set_error("spectrum_mx1024: N = %d", N);
-            return B200_ERR_ARG;
-    }
 }
 
 }  // namespace b200

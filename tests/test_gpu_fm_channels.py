@@ -283,7 +283,7 @@ def test_far_stream_positions(pkg, synth, cuda, first):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("R", [10, 12])
-def test_channels_are_independent(pkg, synth, cuda, R, monkeypatch):
+def test_channels_are_independent(pkg, synth, cuda, R):
     torch = cuda
     n = batch_len(R, 62 * 3)
     S, Ch = 2, 11
@@ -298,11 +298,6 @@ def test_channels_are_independent(pkg, synth, cuda, R, monkeypatch):
     perm = rng.permutation(Ch)
     a_p, b_p = pkg.fm_channels_exec(ring, incs_tensor(torch, incs[:, perm]), 40 * R, baseband=True)
     assert torch.equal(a_p, a_all[:, perm]) and torch.equal(b_p, b_all[:, perm])
-    # the other channel-group sizes of the R = 10 kernel (a measurement knob) compute the same bits
-    for G in ("1", "2", "4"):
-        monkeypatch.setenv("B200_FM_CHANNELS_GROUP", G)
-        a_g, b_g = pkg.fm_channels_exec(ring, incs_tensor(torch, incs), 40 * R, baseband=True)
-        assert torch.equal(a_g, a_all) and torch.equal(b_g, b_all), G
 
 
 @pytest.mark.gpu

@@ -3,8 +3,7 @@
 256 streams x 2^23 - 8 samples (the largest multiple of 4R below 2^23; 4.3 GB of IQ, far past the 126 MB L2), channel counts C = 1, 2, 4, 10, 16, 32.  Every
 number is CUDA events around >= 1 s of back-to-back launches after a warm-up.  Algorithmic bytes per input sample:
 2 (IQ) + C * 4 / (4R) (f32 audio).  Also times b200_fm_exec on the same ring, one C = 10 launch against ten C = 1
-launches, and the channels-per-group choice of the R = 10 kernel (B200_FM_CHANNELS_GROUP).  Prints one JSON line;
-with --out it is also written to that file.
+launches.  Prints one JSON line; with --out it is also written to that file.
 
     python tools/gpu/fm_channels_bench.py [--streams 256] [--samples 8388600] [--out FILE]
 """
@@ -21,7 +20,6 @@ sys.path.insert(0, ROOT)
 HBM_GBS = 6543.0          # the project's measured HBM copy bandwidth on B200 (DESIGN.md section 6)
 R = 10
 CHANNELS = (1, 2, 4, 10, 16, 32)
-GROUPS = (1, 2, 4, 8)
 
 
 def gpu_info():
@@ -111,21 +109,6 @@ def main():
     res["one_c10_vs_ten_c1"] = {"one_launch_c10_ms": round(ms10, 4), "ten_launches_c1_ms": round(ms1x10, 4),
                                 "speedup": round(ms1x10 / ms10, 3)}
     del outs1
-
-    # channels per group of the R = 10 kernel (bytes unpacked once per group of G channels)
-    groups = []
-    for C in (4, 10, 32):
-        inc = torch.as_tensor(incs_all[:, :C].copy()).cuda()
-        out = torch.empty((S, C, n_audio), dtype=torch.float32, device="cuda")
-        row = {"C": C}
-        for G in GROUPS:
-            os.environ["B200_FM_CHANNELS_GROUP"] = str(G)
-            ms, _ = timed(torch, lambda: pkg.fm_channels_exec(ring, inc, 0, audio=out), args.seconds)
-            row[f"G{G}_ms"] = round(ms, 4)
-        del os.environ["B200_FM_CHANNELS_GROUP"]
-        groups.append(row)
-        del out
-    res["group_size"] = groups
     res["gpu_after"] = gpu_info()
     line = json.dumps(res)
     print(line)

@@ -1,7 +1,5 @@
-# round 2, run 3 (after the container was re-created): variants, whole GPU suite, smoke, default bench
+# round 2, run 3 (after the container was re-created): whole GPU suite, smoke, default bench
 mkdir -p gpurun_out/r02
-timeout 600 python tools/gpu/chain_variants.py > gpurun_out/r02/variants.log 2>&1; echo "variants rc=$?"
-tail -14 gpurun_out/r02/variants.log
 timeout 1500 python -m pytest tests -m gpu -x -q > gpurun_out/r02/pytest_run3.log 2>&1; echo "pytest rc=$?"
 tail -15 gpurun_out/r02/pytest_run3.log
 timeout 300 python -c "import __graft_entry__ as g; g.smoke()" 2>&1 | tail -2

@@ -24,13 +24,9 @@ big = pkg.StreamRing(1, 65536 * 2)
 big.load(pkg.synth.s2_tones(65536 * 2, N=65536)[None])
 pkg.SpectrumPlan(65536, hop=32768, window=1).exec(big.batch, db=True)
 pkg.SpectrumPlan(65536, K=2).exec(big.batch, power=True)
-# round 2: the four-step kernel at 16 / 32 branches, the opt-in cluster kernel, the cs32 demodulator, the audio extensions
+# round 2: the four-step kernel at 16 / 32 branches, the cs32 demodulator, the audio extensions
 pkg.SpectrumPlan(16384, hop=8192, window=1).exec(big.batch, db=True, power=True, db_u8=True)
 pkg.SpectrumPlan(32768, K=2).exec(big.batch, db=True)
-os.environ["B200_S64K_CLUSTER"] = "1"
-pkg.SpectrumPlan(65536, hop=32768, window=1).exec(big.batch, db=True, power=True, db_u8=True)
-pkg.SpectrumPlan(65536).exec(big.batch, db=True)
-del os.environ["B200_S64K_CLUSTER"]
 dm = pkg.FmDemod()
 dm.block(dec[0][:4096].cpu().numpy(), want_demod=True)
 dm.block(dec[0][4096:8192].cpu().numpy(), want_audio=False)
