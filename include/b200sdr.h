@@ -114,6 +114,14 @@ int b200_fm_history_samples(int R);
 int b200_fm_history_reset(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int R, void* cuda_stream);
 int b200_fm_history_carry(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,
                           int R, void* cuda_stream);
+/* The same two calls for a history of any length: history_samples a positive multiple of 8, at most
+ * B200_IQ_MAX_HISTORY_SAMPLES (B200_ERR_ARG otherwise); b200_fm_history_reset / _carry are these with 32 R.  Carry needs
+ * n_samples >= history_samples. */
+#define B200_IQ_MAX_HISTORY_SAMPLES ((1 << 30) - 8)     /* the history's size in bytes stays an int */
+int b200_iq_history_reset(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int history_samples,
+                          void* cuda_stream);
+int b200_iq_history_carry(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,
+                          int history_samples, void* cuda_stream);
 /* d_audio: [n_streams][n_samples / (4R)] floats, row stride audio_stride (floats).
  * d_decimated (nullable): [n_streams][n_samples / R] cmplx_s32, row stride dec_stride (complex). */
 int b200_fm_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
@@ -135,7 +143,8 @@ int b200_fm_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams
  * the input history b200_fm_exec already carries plus the absolute index of the batch's first sample, which the
  * caller passes: an all-128 history mixes to zero, so stream start reproduces the reference's zeroed delay lines.
  * All channels of one call share R.  The filter in front of the demodulator is the reference's boxcar and no
- * sharper: a strong neighbour within fs / R of the channel leaks into it as it would into the reference. */
+ * sharper: a strong neighbour within fs / R of the channel leaks into it as it would into the reference.
+ * b200_fm_channels_exec_fir below replaces the boxcar with a FIR low-pass of up to 1024 taps. */
 #define B200_FM_MAX_CHANNELS 32
 /* round(offset_hz / sample_rate_hz * 2^32) as a two's-complement uint32; B200_ERR_ARG if |offset| > fs/2, fs <= 0 or NaN.
    Pure host arithmetic: works without a device. */
@@ -152,6 +161,37 @@ int b200_fm_channels_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int 
                           int64_t first_sample, const uint32_t* d_phase_inc, int n_channels,
                           float* d_audio, int64_t audio_stride, float* d_baseband, int64_t baseband_stride,
                           void* cuda_stream);
+
+/* FM channels with a sharper channel filter (opt-in; b200_fm_channels_exec is unchanged).  With y[n] the mixed
+ * sample above and h[0..T-1] real taps, the baseband is
+ *   b[m] = sum_{k<T} h[k] y[mR + R - T + k]
+ * -- the last tap sits on the last sample of the boxcar's window, so T = R with h = 1 IS the boxcar -- decimated by R,
+ * and the demodulator after b is the one above.  The filter reaches T - R samples further back than the boxcar, so a
+ * stream carries b200_fm_channels_fir_history_samples(R, T) = 32 R + max(T - R, 0), rounded up to a multiple of 8,
+ * input samples of history (b200_iq_history_reset / _carry with that length; the layout is [history | batch]).
+ * d_taps: T floats on the device, 4-byte aligned, shared by every channel and stream of the call.  T in
+ * [1, B200_FM_MAX_CHANNEL_TAPS]; every other argument as b200_fm_channels_exec, and every argument is checked before
+ * anything is launched (B200_ERR_ARG for T out of range or NULL d_taps, B200_ERR_ALIGN for a misaligned d_taps).
+ * Shared memory: a (R, T) pair that does not fit in a CTA is refused with B200_ERR_ARG; every R in [1, 256] fits
+ * with T = 1024 (the largest, R = 256, uses 159 KB for one channel at a time, 212 KB for four).
+ * Cost: T taps per decimated sample and channel instead of R (DESIGN.md 4.3b has the measured rates).
+ * Taps from b200_fm_channel_filter_design keep the boxcar's DC gain R, so the baseband keeps the scale the
+ * demodulator's range assumptions were checked at; any other real taps may be passed.  A signal outside +-fs/2 of
+ * the dongle's centre still needs the dongle retuned. */
+#define B200_FM_MAX_CHANNEL_TAPS 1024
+/* Kaiser-windowed sinc low-pass (host arithmetic, works without a device): n_taps symmetric taps with the -6 dB point
+ * at cutoff_hz, Kaiser's beta for atten_db of stopband attenuation, scaled so that the taps sum to R.  B200_ERR_ARG for
+ * R outside [1, 256], n_taps outside [1, B200_FM_MAX_CHANNEL_TAPS], cutoff outside (0, fs/2), atten_db negative,
+ * fs <= 0, a NaN or infinity, or a NULL h_taps.  Kaiser's estimate of the taps for A dB over a transition of df Hz:
+ * n_taps ~= (A - 7.95) / (2.285 * 2 pi df / fs) + 1. */
+int b200_fm_channel_filter_design(int R, int n_taps, double cutoff_hz, double atten_db, double sample_rate_hz,
+                                  float* h_taps);
+/* H(R, T) above; B200_ERR_ARG for R outside [1, 256] or n_taps outside [1, B200_FM_MAX_CHANNEL_TAPS]. */
+int b200_fm_channels_fir_history_samples(int R, int n_taps);
+int b200_fm_channels_exec_fir(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                              int64_t first_sample, const uint32_t* d_phase_inc, int n_channels,
+                              float* d_audio, int64_t audio_stride, float* d_baseband, int64_t baseband_stride,
+                              const float* d_taps, int n_taps, void* cuda_stream);
 
 /* The same demodulator for DECIMATED input -- the signature of the reference's own callback,
  * audio_fm_demodulator(const cmplx_s32*, int) (audio_main.h:12, audio_main.c:74-145), with its three
@@ -256,6 +296,15 @@ int b200_session_products(b200_session* s, const uint8_t* h_iq, int64_t n_sample
  * be interleaved with the others and each batch is mixed at its absolute position in the stream. */
 int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_samples, const uint32_t* h_phase_inc,
                           int n_channels, float* h_audio);
+/* Makes later b200_session_channels calls use the FIR channel filter h_taps (host, n_taps floats; see
+ * b200_fm_channels_exec_fir); n_taps = 0 goes back to the boxcar.  Only at stream position 0, i.e. after create or
+ * b200_session_reset, like b200_stream_set_payload_sink's "before the first push"; B200_ERR_ARG otherwise, or for n_taps
+ * outside [0, B200_FM_MAX_CHANNEL_TAPS], a NULL h_taps with n_taps > 0, or a history
+ * b200_fm_channels_fir_history_samples(R, n_taps) longer than the session's max_samples_per_batch.  The session's
+ * history grows to that length (the device ring is reallocated and reset), and every later batch of any session call
+ * must hold at least that many samples.  Chain and products read only the last 32 R history samples, so their output
+ * does not change. */
+int b200_session_set_channel_filter(b200_session* s, const float* h_taps, int n_taps);
 /* ---- push-style streaming: what a signal_source callback calls ------------------------------
  *
  * signal_source.c:29-35 hands every registered callback a BORROWED buffer of cmplx_u8 and its

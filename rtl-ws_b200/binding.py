@@ -27,6 +27,8 @@ EXPORTED_SYMBOLS = [
     "b200_spectrum_exec_cs32", "b200_spectrum_exec_rf32",
     "b200_fm_history_samples", "b200_fm_history_reset", "b200_fm_history_carry", "b200_fm_exec",
     "b200_fm_channel_tune", "b200_fm_channels_exec",
+    "b200_iq_history_reset", "b200_iq_history_carry", "b200_fm_channel_filter_design",
+    "b200_fm_channels_fir_history_samples", "b200_fm_channels_exec_fir", "b200_session_set_channel_filter",
     "b200_chain_exec", "b200_chain_exec_r", "b200_chain_tile_samples",
     "b200_session_create", "b200_session_create_r", "b200_session_destroy", "b200_session_reset", "b200_session_chain", "b200_session_products",
     "b200_session_channels",
@@ -95,6 +97,12 @@ def lib() -> C.CDLL:
     L.b200_fm_exec.argtypes = [vp, i64, i32, i64, i32, f32p, i64, vp, i64, vp]
     L.b200_fm_channel_tune.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_uint32)]
     L.b200_fm_channels_exec.argtypes = [vp, i64, i32, i64, i32, i64, vp, i32, f32p, i64, f32p, i64, vp]
+    L.b200_iq_history_reset.argtypes = [vp, i64, i32, i32, vp]
+    L.b200_iq_history_carry.argtypes = [vp, i64, i32, i64, i32, vp]
+    L.b200_fm_channel_filter_design.argtypes = [i32, i32, C.c_double, C.c_double, C.c_double, vp]
+    L.b200_fm_channels_fir_history_samples.argtypes = [i32, i32]
+    L.b200_fm_channels_exec_fir.argtypes = [vp, i64, i32, i64, i32, i64, vp, i32, f32p, i64, f32p, i64, vp, i32, vp]
+    L.b200_session_set_channel_filter.argtypes = [vp, vp, i32]
     L.b200_chain_exec.argtypes = [vp, i64, i32, i64, i32, f32p, f32p, i64, vp, i32, vp]
     L.b200_chain_exec_r.argtypes = [vp, i64, i32, i64, i32, i32, f32p, f32p, i64, vp, i32, vp]
     L.b200_chain_tile_samples.restype = i64
@@ -292,12 +300,15 @@ class SpectrumPlan:
 
 class StreamRing:
     """Device-resident IQ of `n_streams` independent dongles laid out as the FM branch wants it:
-    each row is [history (32*R samples) | batch (n_samples)], rows 16-byte aligned."""
+    each row is [history (32*R samples, or `history`) | batch (n_samples)], rows 16-byte aligned.
+    A FIR channel filter of T taps wants history=fm_channels_fir_history_samples(R, T)."""
 
-    def __init__(self, n_streams: int, n_samples: int, R: int = 10, device="cuda"):
+    def __init__(self, n_streams: int, n_samples: int, R: int = 10, device="cuda", history: int | None = None):
         torch = _torch()
         self.n_streams, self.n_samples, self.R = n_streams, n_samples, R
-        self.hist = int(lib().b200_fm_history_samples(R))
+        self.hist = int(lib().b200_fm_history_samples(R)) if history is None else int(history)
+        if self.hist < int(lib().b200_fm_history_samples(R)) or self.hist % 8 != 0:
+            raise B200Error(f"StreamRing: history {self.hist} must be a multiple of 8 and at least 32 R = {32 * R}")
         row = self.hist + n_samples
         row = (row + 7) // 8 * 8
         self.buf = torch.empty((n_streams, row, 2), dtype=torch.uint8, device=device)
@@ -307,13 +318,13 @@ class StreamRing:
 
     def reset(self, stream=None) -> None:
         """Every stream back to its start (history = 128: the reference's zeroed delay lines)."""
-        _check(lib().b200_fm_history_reset(C.c_void_p(self.batch.data_ptr()), self.stride_bytes, self.n_streams,
-                                           self.R, _stream_ptr(stream)), "b200_fm_history_reset")
+        _check(lib().b200_iq_history_reset(C.c_void_p(self.batch.data_ptr()), self.stride_bytes, self.n_streams,
+                                           self.hist, _stream_ptr(stream)), "b200_iq_history_reset")
 
     def carry(self, stream=None) -> None:
         """History <- tail of the batch (call after a batch has been processed)."""
-        _check(lib().b200_fm_history_carry(C.c_void_p(self.batch.data_ptr()), self.stride_bytes, self.n_streams,
-                                           self.n_samples, self.R, _stream_ptr(stream)), "b200_fm_history_carry")
+        _check(lib().b200_iq_history_carry(C.c_void_p(self.batch.data_ptr()), self.stride_bytes, self.n_streams,
+                                           self.n_samples, self.hist, _stream_ptr(stream)), "b200_iq_history_carry")
 
     def load(self, iq) -> None:
         """Copy a [n_streams, n_samples, 2] uint8 array/tensor into the batch area."""
@@ -351,9 +362,32 @@ def fm_channel_tune(offset_hz: float, fs: float) -> int:
     return int(inc.value)
 
 
-def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None, baseband: bool = False, stream=None):
+FM_MAX_CHANNEL_TAPS = 1024
+
+
+def fm_channel_filter(R: int, n_taps: int, cutoff_hz: float, atten_db: float = 60.0, fs: float = 2_048_000.0):
+    """b200_fm_channel_filter_design: Kaiser-windowed sinc low-pass taps (float32 numpy [n_taps], summing to R) for
+    fm_channels_exec(taps=...) / Session.set_channel_filter; host arithmetic."""
+    h = np.empty(n_taps if n_taps > 0 else 1, dtype=np.float32)
+    _check(lib().b200_fm_channel_filter_design(R, n_taps, float(cutoff_hz), float(atten_db), float(fs), h.ctypes.data),
+           "b200_fm_channel_filter_design")
+    return h
+
+
+def fm_channels_fir_history_samples(R: int, n_taps: int) -> int:
+    """History (input samples) a stream needs in front of its batch for a T-tap channel filter."""
+    h = int(lib().b200_fm_channels_fir_history_samples(R, n_taps))
+    if h < 0:
+        raise B200Error(f"b200_fm_channels_fir_history_samples({R}, {n_taps}): {last_error()}")
+    return h
+
+
+def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None, baseband: bool = False, stream=None,
+                     taps=None):
     """b200_fm_channels_exec over a StreamRing: phase_inc is a cuda int32 tensor [n_streams, n_channels] holding the
     uint32 increments' bits; first_sample is the absolute index of the batch's first sample (a multiple of 4R).
+    taps (a cuda float32 tensor [T]) selects b200_fm_channels_exec_fir, whose ring needs the longer history of
+    fm_channels_fir_history_samples(R, T).
     -> (audio [S, C, n/(4R)] f32, baseband [S, C, n/R, 2] f32 | None)."""
     torch = _torch()
     assert phase_inc.is_cuda and phase_inc.dtype == torch.int32 and phase_inc.dim() == 2
@@ -366,6 +400,19 @@ def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None,
     bb = None
     if baseband:
         bb = torch.empty((S, Ch, ring.n_samples // ring.R, 2), dtype=torch.float32, device=ring.buf.device)
+    if taps is not None:
+        assert taps.is_cuda and taps.dtype == torch.float32 and taps.dim() == 1 and taps.is_contiguous()
+        need = fm_channels_fir_history_samples(ring.R, taps.shape[0])
+        if ring.hist < need:          # the kernel would read before the rows: refuse before anything is launched
+            raise B200Error(f"fm_channels_exec: {taps.shape[0]} taps at R = {ring.R} need a ring history of {need} "
+                            f"samples, the ring has {ring.hist}")
+        _check(lib().b200_fm_channels_exec_fir(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
+                                               ring.n_samples, ring.R, first_sample, C.c_void_p(phase_inc.data_ptr()),
+                                               Ch, C.c_void_p(audio.data_ptr()), audio.stride(1),
+                                               C.c_void_p(bb.data_ptr()) if bb is not None else None,
+                                               bb.stride(1) // 2 if bb is not None else 0, C.c_void_p(taps.data_ptr()),
+                                               taps.shape[0], _stream_ptr(stream)), "b200_fm_channels_exec_fir")
+        return audio, bb
     _check(lib().b200_fm_channels_exec(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
                                        ring.n_samples, ring.R, first_sample, C.c_void_p(phase_inc.data_ptr()), Ch,
                                        C.c_void_p(audio.data_ptr()), audio.stride(1),
@@ -594,6 +641,13 @@ class Session:
             return C.c_void_p(x.data_ptr() if hasattr(x, "data_ptr") else x.ctypes.data)
         _check(lib().b200_session_products(self.h, hp(h_iq), n_samples, gain_db, K_avg, hp(h_audio), hp(h_avg_u8)),
                "b200_session_products")
+
+    def set_channel_filter(self, h_taps) -> None:
+        """b200_session_set_channel_filter: later channels() calls use these FIR taps (host float32); None or an
+        empty array goes back to the boxcar.  Only at stream position 0 (after creation or reset())."""
+        h = np.zeros(0, np.float32) if h_taps is None else np.ascontiguousarray(h_taps, dtype=np.float32).reshape(-1)
+        _check(lib().b200_session_set_channel_filter(self.h, h.ctypes.data if h.size else None, int(h.size)),
+               "b200_session_set_channel_filter")
 
     def channels(self, h_iq, n_samples: int, phase_inc, h_audio=None):
         """b200_session_channels: phase_inc [n_streams, n_channels] (host, uint32 bits) -> h_audio

@@ -87,10 +87,19 @@ int launch_spectrum64k(const SpecParams& p, const Spec64kExtra& x, int N, cudaSt
 int launch_fm_chain(const FmParams& p, cudaStream_t stream);
 int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
 int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
+int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
+                            cudaStream_t stream);
+int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
 int fm_history_samples(int R);
 int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
                        int64_t first_sample, const uint32_t* phase_inc, int n_channels, float* audio,
                        int64_t audio_stride, float* baseband, int64_t baseband_stride, cudaStream_t stream);
+int launch_fm_channels_fir(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                           int64_t first_sample, const uint32_t* phase_inc, int n_channels, const float* taps, int T,
+                           float* audio, int64_t audio_stride, float* baseband, int64_t baseband_stride,
+                           cudaStream_t stream);
+int fm_channels_fir_history_samples(int R, int T);
+int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h);
 
 }  // namespace b200
 
@@ -468,6 +477,30 @@ int b200_fm_history_carry(uint8_t* d_iq, int64_t stream_stride_bytes, int n_stre
                                    reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
+int b200_iq_history_reset(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int history_samples,
+                          void* cuda_stream)
+{
+    if (d_iq == nullptr || n_streams < 0 || history_samples < 8 || history_samples % 8 != 0 ||
+        history_samples > B200_IQ_MAX_HISTORY_SAMPLES) {
+        set_error("iq history reset: bad arguments (history_samples %d must be a positive multiple of 8, at most 2^30 - 8)", history_samples);
+        return B200_ERR_ARG;
+    }
+    return launch_iq_history_reset(d_iq, stream_stride_bytes, n_streams, history_samples,
+                                   reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+int b200_iq_history_carry(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,
+                          int history_samples, void* cuda_stream)
+{
+    if (d_iq == nullptr || n_streams < 0 || history_samples < 8 || history_samples % 8 != 0 ||
+        history_samples > B200_IQ_MAX_HISTORY_SAMPLES) {
+        set_error("iq history carry: bad arguments (history_samples %d must be a positive multiple of 8, at most 2^30 - 8)", history_samples);
+        return B200_ERR_ARG;
+    }
+    return launch_iq_history_carry(d_iq, stream_stride_bytes, n_streams, n_samples, history_samples,
+                                   reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
 int b200_fm_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
                  float* d_audio, int64_t audio_stride, int32_t* d_decimated, int64_t dec_stride, void* cuda_stream)
 {
@@ -510,6 +543,29 @@ int b200_fm_channels_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int 
     return launch_fm_channels(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
                               n_channels, d_audio, audio_stride, d_baseband, baseband_stride,
                               reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+int b200_fm_channel_filter_design(int R, int n_taps, double cutoff_hz, double atten_db, double sample_rate_hz,
+                                  float* h_taps)
+{
+    return fm_channel_filter_design(R, n_taps, cutoff_hz, atten_db, sample_rate_hz, h_taps);
+}
+
+int b200_fm_channels_fir_history_samples(int R, int n_taps)
+{
+    const int h = fm_channels_fir_history_samples(R, n_taps);
+    if (h < 0) set_error("fm channels fir history: R %d or %d taps out of range", R, n_taps);
+    return h;
+}
+
+int b200_fm_channels_exec_fir(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                              int64_t first_sample, const uint32_t* d_phase_inc, int n_channels, float* d_audio,
+                              int64_t audio_stride, float* d_baseband, int64_t baseband_stride, const float* d_taps,
+                              int n_taps, void* cuda_stream)
+{
+    return launch_fm_channels_fir(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
+                                  n_channels, d_taps, n_taps, d_audio, audio_stride, d_baseband, baseband_stride,
+                                  reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- pinned host memory --------------------------------------------------------------------

@@ -13,6 +13,10 @@ int launch_chain_fused(const uint8_t* d_iq, int64_t stride, int n_streams, int64
 int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
 int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
 int fm_history_samples(int R);
+int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
+                            cudaStream_t stream);
+int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
+int fm_channels_fir_history_samples(int R, int T);
 }  // namespace b200
 
 using namespace b200;
@@ -144,7 +148,7 @@ struct b200_session {
     int64_t max_samples;
     int R;                     // down factor of the FM branch
     int64_t tile;              // lcm(1024, 4R)
-    int hist_samples;
+    int hist_samples;          // 32 R, or the FIR channel filter's longer history (b200_session_set_channel_filter)
     int64_t stride_bytes;      // per-stream row pitch in the device ring: history + batch
     uint8_t* d_ring;           // [n_streams][stride_bytes]
     float* d_db;               // [n_streams][max_samples]            (1024 bins per 1024 samples)
@@ -154,6 +158,8 @@ struct b200_session {
     uint32_t* d_phase_inc;     // [n_streams][ch_cap], b200_session_channels, allocated on first use
     float* d_ch_audio;         // [n_streams][ch_cap][max_samples / (4R)]
     int ch_cap;                // channels the two buffers above hold
+    float* d_taps;             // FIR channel filter (b200_session_set_channel_filter), nullptr = the boxcar
+    int n_taps;
     static constexpr int LANES = 4;
     cudaStream_t streams[LANES];
     int device;
@@ -173,6 +179,11 @@ int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_
         return B200_ERR_ARG;
     }
     if (n_samples == 0) return B200_OK;
+    if (n_samples < s->hist_samples && s->n_taps > 0) {       // the carry below needs a whole history
+        set_error("session chain: a batch of %lld samples is shorter than the channel filter's history (%d samples)",
+                  (long long) n_samples, s->hist_samples);
+        return B200_ERR_ARG;
+    }
     const int lanes = b200_session::LANES;
     // stream groups small enough to pipeline H2D / kernels / D2H across the lanes
     int group = (s->n_streams + 4 * lanes - 1) / (4 * lanes);
@@ -200,7 +211,7 @@ int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_
             B200_CUDA_TRY(cudaMemcpy2DAsync(h_audio + (size_t) s0 * (size_t) audio_pitch, sizeof(float) * (size_t) audio_pitch,
                                             d_audio, sizeof(float) * (size_t) n_audio, sizeof(float) * (size_t) n_audio,
                                             (size_t) ns, cudaMemcpyDeviceToHost, st));
-        const int rc2 = launch_fm_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->R, st);
+        const int rc2 = launch_iq_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->hist_samples, st);
         if (rc2) return rc2;
     }
     s->position += n_samples;
@@ -270,13 +281,14 @@ void b200_session_destroy(b200_session* s)
     if (s->d_avg) cudaFree(s->d_avg);
     if (s->d_phase_inc) cudaFree(s->d_phase_inc);
     if (s->d_ch_audio) cudaFree(s->d_ch_audio);
+    if (s->d_taps) cudaFree(s->d_taps);
     delete s;
 }
 
 void b200_session_reset(b200_session* s)
 {
     if (s == nullptr) return;
-    launch_fm_history_reset(s->d_ring + 2 * (int64_t) s->hist_samples, s->stride_bytes, s->n_streams, s->R,
+    launch_iq_history_reset(s->d_ring + 2 * (int64_t) s->hist_samples, s->stride_bytes, s->n_streams, s->hist_samples,
                             s->streams[0]);
     cudaStreamSynchronize(s->streams[0]);
     s->position = 0;
@@ -299,6 +311,11 @@ int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_sample
         return B200_ERR_ARG;
     }
     if (n_samples == 0) return B200_OK;
+    if (n_samples < s->hist_samples && s->n_taps > 0) {
+        set_error("session channels: a batch of %lld samples is shorter than the channel filter's history (%d samples)",
+                  (long long) n_samples, s->hist_samples);
+        return B200_ERR_ARG;
+    }
     if (n_channels > s->ch_cap) {       // every earlier call has finished: the session calls wait for their work
         if (s->d_phase_inc) cudaFree(s->d_phase_inc);
         if (s->d_ch_audio) cudaFree(s->d_ch_audio);
@@ -327,17 +344,69 @@ int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_sample
                                         (size_t) (2 * n_samples), (size_t) (2 * n_samples), (size_t) ns,
                                         cudaMemcpyHostToDevice, st));
         B200_CUDA_TRY(cudaMemcpyAsync(d_inc, h_phase_inc + row0, sizeof(uint32_t) * rows, cudaMemcpyHostToDevice, st));
-        const int rc = b200_fm_channels_exec(d_batch, s->stride_bytes, ns, n_samples, s->R, s->position, d_inc,
-                                             n_channels, d_audio, n_audio, nullptr, 0, st);
+        const int rc = s->n_taps > 0
+                           ? b200_fm_channels_exec_fir(d_batch, s->stride_bytes, ns, n_samples, s->R, s->position, d_inc,
+                                                       n_channels, d_audio, n_audio, nullptr, 0, s->d_taps, s->n_taps, st)
+                           : b200_fm_channels_exec(d_batch, s->stride_bytes, ns, n_samples, s->R, s->position, d_inc,
+                                                   n_channels, d_audio, n_audio, nullptr, 0, st);
         if (rc) return rc;
         B200_CUDA_TRY(cudaMemcpyAsync(h_audio + row0 * (size_t) n_audio, d_audio, sizeof(float) * rows * (size_t) n_audio,
                                       cudaMemcpyDeviceToHost, st));
-        const int rc2 = launch_fm_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->R, st);
+        const int rc2 = launch_iq_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->hist_samples, st);
         if (rc2) return rc2;
     }
     const int rc = b200::session_wait(s);
     if (rc) return rc;
     s->position += n_samples;
+    return B200_OK;
+}
+
+int b200_session_set_channel_filter(b200_session* s, const float* h_taps, int n_taps)
+{
+    if (s == nullptr || n_taps < 0 || n_taps > B200_FM_MAX_CHANNEL_TAPS || (n_taps > 0 && h_taps == nullptr)) {
+        set_error("session channel filter: bad arguments (%d taps)", n_taps);
+        return B200_ERR_ARG;
+    }
+    if (s->position != 0) {
+        set_error("session channel filter: set it at stream position 0 (after create or b200_session_reset), "
+                  "not at %lld", (long long) s->position);
+        return B200_ERR_ARG;
+    }
+    const int hist = n_taps > 0 ? fm_channels_fir_history_samples(s->R, n_taps) : fm_history_samples(s->R);
+    if (hist > s->max_samples) {
+        set_error("session channel filter: its history of %d samples is longer than the largest batch (%lld)", hist,
+                  (long long) s->max_samples);
+        return B200_ERR_ARG;
+    }
+    // every earlier call has finished: the session calls wait for their work
+    float* d_taps = nullptr;
+    if (n_taps > 0) {
+        B200_CUDA_TRY(cudaMalloc((void**) &d_taps, sizeof(float) * (size_t) n_taps));
+        if (cudaMemcpyAsync(d_taps, h_taps, sizeof(float) * (size_t) n_taps, cudaMemcpyHostToDevice, s->streams[0]) !=
+                cudaSuccess ||
+            cudaStreamSynchronize(s->streams[0]) != cudaSuccess) {
+            set_error("session channel filter: upload failed: %s", cudaGetErrorString(cudaGetLastError()));
+            cudaFree(d_taps);
+            return B200_ERR_CUDA;
+        }
+    }
+    if (hist != s->hist_samples) {        // a ring with the new history; position 0, so nothing in it is kept
+        const int64_t stride = 2 * ((int64_t) hist + s->max_samples);
+        uint8_t* ring = nullptr;
+        if (cudaMalloc(&ring, (size_t) s->n_streams * (size_t) stride) != cudaSuccess) {
+            set_error("session channel filter: ring allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
+            if (d_taps) cudaFree(d_taps);
+            return B200_ERR_CUDA;
+        }
+        cudaFree(s->d_ring);
+        s->d_ring = ring;
+        s->stride_bytes = stride;
+        s->hist_samples = hist;
+        b200_session_reset(s);
+    }
+    if (s->d_taps) cudaFree(s->d_taps);
+    s->d_taps = d_taps;
+    s->n_taps = n_taps;
     return B200_OK;
 }
 

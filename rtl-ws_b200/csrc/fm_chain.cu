@@ -362,11 +362,14 @@ int launch_fm_chain(const FmParams& p, cudaStream_t stream)
     return B200_OK;
 }
 
-int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream)
+// History of any length (a positive multiple of 8 samples): the FM chain's 32 R, or the longer one a channel FIR
+// reaches back over (fm_channels_fir.cu)
+int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
+                            cudaStream_t stream)
 {
-    const int hist_bytes = 2 * fm_history_samples(R);
+    const int hist_bytes = 2 * hist_samples;
     if (n_samples * 2 < hist_bytes) {
-        set_error("fm: batch shorter than the history (%d samples)", fm_history_samples(R));
+        set_error("fm: batch shorter than the history (%d samples)", hist_samples);
         return B200_ERR_ARG;
     }
     if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stride & 15) != 0 || ((n_samples * 2) & 15) != 0) {
@@ -381,9 +384,9 @@ int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t 
     return B200_OK;
 }
 
-int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream)
+int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream)
 {
-    const int hist_bytes = 2 * fm_history_samples(R);
+    const int hist_bytes = 2 * hist_samples;
     if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stride & 15) != 0) return B200_ERR_ALIGN;
     if (n_streams == 0) return B200_OK;
     const int64_t total = (int64_t) n_streams * (hist_bytes / 16);
@@ -391,6 +394,16 @@ int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, c
     fm_history_reset_kernel<<<blocks, 256, 0, stream>>>(iq, stride, n_streams, hist_bytes);
     B200_LAUNCH_CHECK();
     return B200_OK;
+}
+
+int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream)
+{
+    return launch_iq_history_carry(iq, stride, n_streams, n_samples, fm_history_samples(R), stream);
+}
+
+int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream)
+{
+    return launch_iq_history_reset(iq, stride, n_streams, fm_history_samples(R), stream);
 }
 
 }  // namespace b200

@@ -1,0 +1,348 @@
+// fm_channels_fir.cu -- FM channels with a T-tap FIR low-pass in place of the boxcar (sm_100a).
+//
+// Same chain as fm_channels.cu (include/b200sdr.h), but the decimating filter in front of the demodulator is
+//   b[m] = sum_{k<T} h[k] y[mR + R - T + k],   y[n] = x[n] exp(-j 2 pi phi(n) / 2^32)
+// with real taps h: its last tap sits on the last sample of the boxcar's window, so T = R, h = 1 is the boxcar.
+// Write L = T - R (any sign).  phi(mR + d) = phi(mR) + phi(d) mod 2^32 holds for negative d too (uint32 two's
+// complement), so
+//   b[m] = exp(-j phi(mR)) * sum_{k<T} x[mR - L + k] w[k],   w[k] = h[k] exp(-j 2 pi phi(k - L) / 2^32):
+// one complex T-tap filter per channel, then the same exact-integer rotation per decimated sample as the boxcar.
+//
+// Geometry: the boxcar kernel's tile (280 decimated samples, 9 warps, one 31-output discriminator chunk per warp)
+// and TMA ring.  A stage holds 280 R + L input samples; the bulk copy starts at the 8-sample boundary at or below
+// the first one a tile needs, off = (-L) mod 8 samples ahead of it, so lane j's window starts at stage sample
+// j R + off.  The MAC reads byte pairs straight from the stage (2 bytes per sample: the stage of R = 256, T = 1024
+// is 142 KB, its floats would not fit), unpacks each once and applies it to the G channels of the group:
+// G accumulators per lane, taps [T][G] in shared memory, read as broadcasts.  G comes from the shared-memory budget
+// and the channel count (launcher).  Phases 2 and 3 (the half-bands) are the boxcar kernel's.
+#include <math.h>
+
+#include "b200_common.cuh"
+#include "fm_channels.cuh"
+#include "fm_kernels.cuh"
+
+namespace b200 {
+
+namespace {
+
+constexpr int FIR_MAX_G = 8;                       // channels per group (accumulators per lane)
+constexpr int FIR_SMEM_LIMIT = 227 * 1024;         // dynamic shared memory a B200 CTA may opt into
+
+struct FirParams {
+    FcParams c;
+    const float* taps;              // [T], shared by every channel and stream
+    int T;
+    int L;                          // T - R
+    int off;                        // (-L) mod 8: where lane 0's window starts in a stage
+};
+
+// MAC over T taps for NG channels of the group, then rotation, discriminator and limiter -> demod[g][j]
+// bb (nullable): this tile's baseband column 0 of channel 0 of the group, rows bb_stride complex samples apart
+template <int NG>
+__device__ __forceinline__ void fir_group(const uint16_t* in, const float4* taps, int T, int G, int R,
+                                          const uint32_t* incs, uint32_t m, int j, int lane, float2* bb,
+                                          int64_t bb_stride, int ta, float* demod)
+{
+    c64 acc[NG];
+#pragma unroll
+    for (int g = 0; g < NG; ++g) acc[g] = cpack(0.0f, 0.0f);
+#pragma unroll 4
+    for (int k = 0; k < T; ++k) {
+        const uint32_t v = in[k];
+        const c64 xr = byte_pair(v, 0);
+        const c64 xi = byte_pair(v, 1);
+        const float4* t = taps + k * G;
+#pragma unroll
+        for (int g = 0; g < NG; ++g) {
+            const float4 w = t[g];
+            acc[g] = cfma2(xr, cpack(w.x, w.y), acc[g]);
+            acc[g] = cfma2(xi, cpack(w.z, w.w), acc[g]);
+        }
+    }
+#pragma unroll
+    for (int g = 0; g < NG; ++g) {
+        float ar, ai, rc, rs;
+        cunpack(acc[g], ar, ai);
+        rotation(incs[g] * (uint32_t) R * m, rc, rs);
+        const float bre = fmaf(ar, rc, ai * rs);          // (ar + j ai) (rc - j rs)
+        const float bim = fmaf(ai, rc, -(ar * rs));
+        if (bb != nullptr && j >= 32 && j < 4 * ta + 32) bb[g * bb_stride + (j - 32)] = make_float2(bre, bim);
+        const float ph = atan2_approx_dev(bim, bre);
+        const float prev = __shfl_up_sync(0xffffffffu, ph, 1);
+        if (lane > 0) demod[g * FC_DEMOD + j] = fm_limit(ph, prev);
+    }
+}
+
+__global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirParams p, const int tiles_per_stream,
+                                                                     const int stage_bytes, const int n_stages,
+                                                                     const int G)
+{
+    extern __shared__ __align__(128) uint8_t smem[];
+    const int R = p.c.R;
+    const int T = p.T;
+    const int tid = threadIdx.x;
+    const int lane = tid & 31;
+    const int warp = tid >> 5;
+    uint8_t* ring = smem;
+    float4* taps = reinterpret_cast<float4*>(smem + n_stages * stage_bytes);   // [T][G]: (w.re, w.im, -w.im, w.re)
+    float* demod = reinterpret_cast<float*>(taps + T * G);                        // [G][FC_DEMOD]
+    float* work = demod + G * FC_DEMOD;                                           // [G][FC_WORK]
+    uint64_t* bars = reinterpret_cast<uint64_t*>(work + G * FC_WORK);
+
+    const int C = p.c.n_channels;
+    const int64_t n_audio = p.c.n_samples / (4 * R);
+    const int64_t total_tiles = (int64_t) p.c.n_streams * tiles_per_stream;
+    const uint32_t first_dec = (uint32_t) (p.c.first_sample / R);      // mod 2^32, like every phase below
+
+    if (tid == 0) {
+        mbar_init(&bars[0], 1);
+        mbar_init(&bars[1], 1);
+        fence_mbar_init();
+    }
+    __syncthreads();
+
+    auto issue = [&](int64_t tile, int st) {
+        const int s = (int) (tile / tiles_per_stream);
+        const int64_t n0 = (tile - (int64_t) s * tiles_per_stream) * FC_T;
+        const int ta = (int) ((n_audio - n0) < FC_T ? (n_audio - n0) : FC_T);
+        // samples from (4 n0 - 32) R - L - off (a multiple of 8: (4 n0 - 32) R is one because n0 is a multiple of 62,
+        // and L + off is one by the choice of off) up to 4 (n0 + ta) R, a multiple of 8 as in fm_channels.cu
+        const int64_t first = (4 * n0 - 32) * (int64_t) R - p.L - p.off;
+        const uint32_t bytes = (uint32_t) (2 * ((4 * (n0 + ta)) * (int64_t) R - first));
+        const uint8_t* src = p.c.iq + (int64_t) s * p.c.stream_stride_bytes + 2 * first;
+        mbar_arrive_expect_tx(&bars[st], bytes);
+        tma_load_1d(ring + st * stage_bytes, src, bytes, &bars[st]);
+    };
+
+    int64_t tile = blockIdx.x;
+    if (tid == 0)
+        for (int k = 0; k < n_stages; ++k)
+            if (tile + k * (int64_t) gridDim.x < total_tiles) issue(tile + k * (int64_t) gridDim.x, k);
+
+    for (uint32_t it = 0; tile < total_tiles; tile += gridDim.x, ++it) {
+        const int st = (int) (it % (uint32_t) n_stages);
+        const int s = (int) (tile / tiles_per_stream);
+        const int64_t n0 = (tile - (int64_t) s * tiles_per_stream) * FC_T;
+        const int ta = (int) ((n_audio - n0) < FC_T ? (n_audio - n0) : FC_T);
+        const int j = 31 * warp + lane;                                   // this lane's decimated sample
+        const uint32_t m = first_dec + (uint32_t) (4 * n0 - 32) + (uint32_t) j;
+        const uint32_t* incs = p.c.phase_inc + (int64_t) s * C;
+
+        mbar_wait(&bars[st], (it / (uint32_t) n_stages) & 1);
+        // lane j's window: input samples (4 n0 - 32 + j) R - L + k, k < T
+        const uint16_t* in = reinterpret_cast<const uint16_t*>(ring + st * stage_bytes) + j * R + p.off;
+
+        for (int c0 = 0; c0 < C; c0 += G) {
+            const int gc = (C - c0) < G ? (C - c0) : G;
+            // ---- 0. taps of the group: h[k] exp(-j 2 pi phi(k - L) / 2^32) ----
+            for (int i = tid; i < gc * T; i += FC_THREADS) {
+                const int g = i / T, k = i - g * T;
+                const uint32_t phi = incs[c0 + g] * (uint32_t) (k - p.L);
+                float sn, cs;
+                sincospif((float) (int32_t) phi * 4.65661287307739258e-10f, &sn, &cs);     // 2^-31: [-1, 1)
+                const float h = p.taps[k];
+                taps[k * G + g] = make_float4(h * cs, -(h * sn), h * sn, h * cs);
+            }
+            __syncthreads();
+
+            // ---- 1. mix + FIR, rotation, discriminator ----
+            float2* bb = p.c.baseband != nullptr
+                             ? p.c.baseband + ((int64_t) s * C + c0) * p.c.baseband_stride + 4 * n0 : nullptr;
+            const int64_t bs = p.c.baseband_stride;
+            switch (gc) {
+                case 1: fir_group<1>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                case 2: fir_group<2>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                case 3: fir_group<3>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                case 4: fir_group<4>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                case 5: fir_group<5>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                case 6: fir_group<6>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                case 7: fir_group<7>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+                default: fir_group<8>(in, taps, T, G, R, incs + c0, m, j, lane, bb, bs, ta, demod); break;
+            }
+            __syncthreads();
+            // the input stage is consumed after the last group: refill it with the tile n_stages steps ahead
+            if (c0 + G >= C && tid == 0) {
+                const int64_t nxt = tile + n_stages * (int64_t) gridDim.x;
+                if (nxt < total_tiles) {
+                    fence_proxy_async_smem();
+                    issue(nxt, st);
+                }
+            }
+
+            // ---- 2. half-band #1 (audio_main.c:133); work index 0 <-> 2*n0 - 10 ----
+            for (int i = tid; i < gc * FC_NW; i += FC_THREADS) {
+                const int g = i / FC_NW, mm = i - g * FC_NW;
+                work[g * FC_WORK + mm] = halfband_from(demod + g * FC_DEMOD + 2 * mm + 2);
+            }
+            __syncthreads();
+
+            // ---- 3. half-band #2 (audio_main.c:139) ----
+            for (int i = tid; i < gc * FC_T; i += FC_THREADS) {
+                const int g = i / FC_T, a = i - g * FC_T;
+                if (a < ta)
+                    p.c.audio[((int64_t) s * C + c0 + g) * p.c.audio_stride + n0 + a] = halfband_from(work + g * FC_WORK + 2 * a);
+            }
+            // taps[], demod[] and work[] are reused under the same barriers as in fm_channels.cu
+        }
+    }
+}
+
+int fir_stage_bytes(int R, int T)
+{
+    const int L = T - R;
+    return 2 * (FC_ND * R + L + ((-L) & 7));
+}
+
+int fir_smem_bytes(int stage_bytes, int n_stages, int T, int G)
+{
+    return n_stages * stage_bytes + T * G * 16 + G * (FC_DEMOD + FC_WORK) * 4 + 16;
+}
+
+// Channels per group for C channels: the fewest groups the shared-memory budget allows (at most FIR_MAX_G
+// channels each), then the channels spread evenly over them.  0 if not even one channel fits.
+int fir_group_size(int stage_bytes, int n_stages, int T, int C)
+{
+    int gmax = C < FIR_MAX_G ? C : FIR_MAX_G;
+    while (gmax > 0 && fir_smem_bytes(stage_bytes, n_stages, T, gmax) > FIR_SMEM_LIMIT) --gmax;
+    if (gmax == 0) return 0;
+    const int groups = (C + gmax - 1) / gmax;
+    return (C + groups - 1) / groups;
+}
+
+}  // namespace
+
+int fm_channels_fir_history_samples(int R, int T)
+{
+    if (R < 1 || R > 256 || T < 1 || T > B200_FM_MAX_CHANNEL_TAPS) return B200_ERR_ARG;
+    const int h = 32 * R + (T > R ? T - R : 0);
+    return (h + 7) / 8 * 8;
+}
+
+int launch_fm_channels_fir(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                           int64_t first_sample, const uint32_t* phase_inc, int n_channels, const float* taps, int T,
+                           float* audio, int64_t audio_stride, float* baseband, int64_t baseband_stride,
+                           cudaStream_t stream)
+{
+    if (n_streams < 0 || iq == nullptr || phase_inc == nullptr || audio == nullptr || taps == nullptr) {
+        set_error("fm channels fir: null pointer or negative stream count");
+        return B200_ERR_ARG;
+    }
+    if (n_channels < 1 || n_channels > B200_FM_MAX_CHANNELS) {
+        set_error("fm channels fir: n_channels %d outside [1, %d]", n_channels, B200_FM_MAX_CHANNELS);
+        return B200_ERR_ARG;
+    }
+    if (R < 1 || R > 256) {
+        set_error("fm channels fir: down factor %d outside [1, 256]", R);
+        return B200_ERR_ARG;
+    }
+    if (T < 1 || T > B200_FM_MAX_CHANNEL_TAPS) {
+        set_error("fm channels fir: %d taps outside [1, %d]", T, B200_FM_MAX_CHANNEL_TAPS);
+        return B200_ERR_ARG;
+    }
+    if (n_samples < 0 || n_samples % (4 * R) != 0 || n_samples % 8 != 0) {
+        set_error("fm channels fir: n_samples %lld must be a multiple of 4*R and of 8", (long long) n_samples);
+        return B200_ERR_ARG;
+    }
+    if (first_sample < 0 || first_sample % (4 * R) != 0) {
+        set_error("fm channels fir: first_sample %lld must be a non-negative multiple of 4*R", (long long) first_sample);
+        return B200_ERR_ARG;
+    }
+    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
+        set_error("fm channels fir: IQ pointer and stream stride must be 16-byte aligned");
+        return B200_ERR_ALIGN;
+    }
+    if ((reinterpret_cast<uintptr_t>(phase_inc) & 3) != 0 || (reinterpret_cast<uintptr_t>(audio) & 3) != 0 ||
+        (reinterpret_cast<uintptr_t>(taps) & 3) != 0 || (reinterpret_cast<uintptr_t>(baseband) & 7) != 0) {
+        set_error("fm channels fir: phase increments, taps and audio must be 4-byte aligned, baseband 8-byte aligned");
+        return B200_ERR_ALIGN;
+    }
+    const int stage_bytes = fir_stage_bytes(R, T);
+    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;       // as fm_channels.cu
+    const int G = fir_group_size(stage_bytes, n_stages, T, n_channels);
+    if (G == 0) {
+        set_error("fm channels fir: R = %d with %d taps does not fit in shared memory", R, T);
+        return B200_ERR_ARG;
+    }
+    if (n_streams == 0 || n_samples == 0) return B200_OK;
+    const int64_t tps = (n_samples / (4 * R) + FC_T - 1) / FC_T;
+    if ((int64_t) n_streams * tps >= (1ll << 31)) {
+        set_error("fm channels fir: batch too long");
+        return B200_ERR_ARG;
+    }
+    FirParams p;
+    p.c.iq = iq;
+    p.c.stream_stride_bytes = stream_stride_bytes;
+    p.c.n_streams = n_streams;
+    p.c.n_samples = n_samples;
+    p.c.R = R;
+    p.c.first_sample = first_sample;
+    p.c.phase_inc = phase_inc;
+    p.c.n_channels = n_channels;
+    p.c.audio = audio;
+    p.c.audio_stride = audio_stride;
+    p.c.baseband = reinterpret_cast<float2*>(baseband);
+    p.c.baseband_stride = baseband_stride;
+    p.taps = taps;
+    p.T = T;
+    p.L = T - R;
+    p.off = (R - T) & 7;
+    const int smem = fir_smem_bytes(stage_bytes, n_stages, T, G);
+    auto kern = fm_channels_fir_kernel;
+    if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
+    const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
+    int64_t grid = (int64_t) sm_count() * per_sm;
+    const int64_t total = (int64_t) n_streams * tps;
+    if (grid > total) grid = total;
+    kern<<<(unsigned) grid, FC_THREADS, smem, stream>>>(p, (int) tps, stage_bytes, n_stages, G);
+    B200_LAUNCH_CHECK();
+    return B200_OK;
+}
+
+// Kaiser-windowed sinc (host): I0 by its power series, which converges for every beta used here (< 120)
+static double bessel_i0(double x)
+{
+    double sum = 1.0, term = 1.0;
+    const double q = 0.25 * x * x;
+    for (int k = 1; k < 500; ++k) {
+        term *= q / ((double) k * (double) k);
+        sum += term;
+        if (term < 1e-17 * sum) break;
+    }
+    return sum;
+}
+
+int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h)
+{
+    // !(a < b) also refuses NaN
+    if (h == nullptr || R < 1 || R > 256 || T < 1 || T > B200_FM_MAX_CHANNEL_TAPS || !(fs > 0.0) || !isfinite(fs) ||
+        !(cutoff_hz > 0.0) || !(cutoff_hz < 0.5 * fs) || !(atten_db >= 0.0) || !isfinite(atten_db)) {
+        set_error("fm channel filter design: R %d, %d taps, cutoff %g Hz, attenuation %g dB, rate %g Hz", R, T,
+                  cutoff_hz, atten_db, fs);
+        return B200_ERR_ARG;
+    }
+    const double A = atten_db;
+    const double beta = A > 50.0 ? 0.1102 * (A - 8.7) : A >= 21.0 ? 0.5842 * pow(A - 21.0, 0.4) + 0.07886 * (A - 21.0) : 0.0;
+    const double fc = cutoff_hz / fs;                        // cycles per sample; the -6 dB point of the windowed sinc
+    const double mid = 0.5 * (T - 1);
+    const double pi = 3.14159265358979323846;
+    const double i0b = bessel_i0(beta);
+    double v[B200_FM_MAX_CHANNEL_TAPS];
+    double sum = 0.0;
+    for (int k = 0; k < T; ++k) {
+        const double t = k - mid;
+        const double sinc = t == 0.0 ? 2.0 * fc : sin(2.0 * pi * fc * t) / (pi * t);
+        const double r = T > 1 ? (k - mid) / mid : 0.0;
+        const double w = bessel_i0(beta * sqrt(fmax(0.0, 1.0 - r * r))) / i0b;
+        v[k] = sinc * w;
+        sum += v[k];
+    }
+    if (!(fabs(sum) > 0.0)) {
+        set_error("fm channel filter design: the taps sum to zero");
+        return B200_ERR_ARG;
+    }
+    // the boxcar's DC gain R, so the baseband keeps the scale the demodulator was checked at
+    for (int k = 0; k < T; ++k) h[k] = (float) (v[k] * (double) R / sum);
+    return B200_OK;
+}
+
+}  // namespace b200
