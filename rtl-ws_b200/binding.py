@@ -422,14 +422,30 @@ def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None,
     return audio, bb
 
 
+def _check_output(what: str, t, dtype, shape: tuple, device, row_slices: bool = False) -> None:
+    """Refuse an output tensor the kernels would write past: they see only its data pointer (and row stride).
+    row_slices: rows may be slices of wider rows (unit column stride); otherwise the tensor must be contiguous."""
+    layout_ok = t.stride(-1) == 1 if row_slices else t.is_contiguous()
+    if t.dtype != dtype or tuple(t.shape) != shape or not layout_ok or t.device != device:
+        raise B200Error(f"{what}: want {dtype} {shape} {'with unit column stride' if row_slices else 'contiguous'} "
+                        f"on {device}, got {t.dtype} {tuple(t.shape)} strides {t.stride()} on {t.device}")
+
+
 def chain_exec(ring: StreamRing, gain_db: int = 0, db=None, audio=None, avg_u8=None, K_avg: int = 6, stream=None):
-    """b200_chain_exec: per-frame dB spectra (N = 1024) + FM audio from one pass over the ring's batch."""
+    """b200_chain_exec: per-frame dB spectra (N = 1024) + FM audio from one pass over the ring's batch.
+    Given outputs must be on the ring's device: db contiguous float32 [n_streams, n/1024, 1024], audio float32
+    [n_streams, n/(4R)] (rows may be slices of wider rows), avg_u8 contiguous uint8 [n_streams, 1024]."""
     torch = _torch()
+    S, dev = ring.n_streams, ring.buf.device
     n_audio = ring.n_samples // (4 * ring.R)
     if db is None:
-        db = torch.empty((ring.n_streams, ring.n_samples // 1024, 1024), dtype=torch.float32, device=ring.buf.device)
+        db = torch.empty((S, ring.n_samples // 1024, 1024), dtype=torch.float32, device=dev)
     if audio is None:
-        audio = torch.empty((ring.n_streams, n_audio), dtype=torch.float32, device=ring.buf.device)
+        audio = torch.empty((S, n_audio), dtype=torch.float32, device=dev)
+    _check_output("chain_exec db", db, torch.float32, (S, ring.n_samples // 1024, 1024), dev)
+    _check_output("chain_exec audio", audio, torch.float32, (S, n_audio), dev, row_slices=True)
+    if avg_u8 is not None:
+        _check_output("chain_exec avg_u8", avg_u8, torch.uint8, (S, 1024), dev)
     _check(lib().b200_chain_exec_r(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
                                    ring.n_samples, ring.R, gain_db, C.c_void_p(db.data_ptr()), C.c_void_p(audio.data_ptr()),
                                    audio.stride(0), C.c_void_p(avg_u8.data_ptr()) if avg_u8 is not None else None,
