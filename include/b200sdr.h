@@ -193,6 +193,32 @@ int b200_fm_channels_exec_fir(const uint8_t* d_iq, int64_t stream_stride_bytes, 
                               float* d_audio, int64_t audio_stride, float* d_baseband, int64_t baseband_stride,
                               const float* d_taps, int n_taps, void* cuda_stream);
 
+/* FM channels over a ragged table of RUNS: one launch for rows that each have their own channel count, increments and
+ * stream position (the push stream's dongles are at different batches and have different listener sets).  Run k
+ * demodulates IQ row `stream` (d_iq + stream * stream_stride_bytes, history in front as above) as if it were at
+ * absolute sample first_sample, for its n_channels increments; channel c goes to audio row audio_row + c of d_audio
+ * (audio_stride floats apart, n_audio_rows rows, each at least n_samples / (4R) floats).  Each run's audio is bit for
+ * bit what b200_fm_channels_exec (d_taps == NULL, n_taps == 0) or b200_fm_channels_exec_fir (T = n_taps device taps;
+ * the rows then need b200_fm_channels_fir_history_samples(R, T) of history) gives on that row at that position with
+ * those increments.  All runs share n_samples and R.  h_runs is host memory, read during the call only.  There is no
+ * baseband output.  Checked before anything is launched (B200_ERR_ARG, or B200_ERR_ALIGN for alignment): n_runs in
+ * [1, B200_FM_MAX_RUNS]; per run, stream in [0, n_streams), n_channels in [1, B200_FM_MAX_CHANNELS] (a run without
+ * channels is left out of the table), first_sample a non-negative multiple of 4R, audio_row >= 0 and
+ * audio_row + n_channels <= n_audio_rows; the audio rows of two runs may not overlap; R, n_samples, taps and
+ * alignment as for the calls above; n_runs times the tiles of a row below 2^31. */
+#define B200_FM_MAX_RUNS 64
+typedef struct {
+    int32_t stream;                                  /* row of d_iq */
+    int32_t n_channels;                              /* [1, B200_FM_MAX_CHANNELS] */
+    int64_t first_sample;                            /* >= 0, a multiple of 4R: absolute index of the row's first batch sample */
+    int64_t audio_row;                               /* channel c -> audio row audio_row + c */
+    uint32_t phase_inc[B200_FM_MAX_CHANNELS];        /* b200_fm_channel_tune */
+} b200_fm_channel_run;
+int b200_fm_channels_exec_runs(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,
+                               int R, const b200_fm_channel_run* h_runs, int n_runs,
+                               float* d_audio, int64_t audio_stride, int64_t n_audio_rows,
+                               const float* d_taps, int n_taps, void* cuda_stream);
+
 /* The same demodulator for DECIMATED input -- the signature of the reference's own callback,
  * audio_fm_demodulator(const cmplx_s32*, int) (audio_main.h:12, audio_main.c:74-145), with its three
  * function statics (audio_main.c:77-79) made explicit.  d_state: B200_FM_STATE_FLOATS floats per stream on
@@ -342,6 +368,30 @@ int b200_stream_push(b200_stream* s, int stream, const uint8_t* samples, int len
 int b200_stream_poll(b200_stream* s);           /* submit what is waiting, deliver what has finished; never blocks */
 int b200_stream_flush(b200_stream* s);          /* wait for and deliver every submitted batch */
 int64_t b200_stream_pending_samples(const b200_stream* s, int stream);   /* buffered, not yet a whole batch */
+/* FM channels on the push stream: listeners at offsets inside each dongle's band (b200_fm_channels_exec).
+ * b200_stream_set_channel_sink: up to max_channels ([1, B200_FM_MAX_CHANNELS]) channels per dongle; the first call with
+ * a sink allocates the channel audio buffers, a later call with another capacity is refused.  A NULL sink stops channel
+ * work: batches submitted without a sink deliver nothing for channels.  The sink gets the `user` of
+ * b200_stream_set_sinks and, per batch and channel, n floats at fs / (4R) starting at audio sample first_sample (counted
+ * as for the audio sink), after that batch's audio sink call.
+ * b200_stream_set_channels replaces dongle `stream`'s listener set (from the stream's producer thread, or serialised
+ * with its pushes like any other b200_stream_* call): n_channels increments (b200_fm_channel_tune) and
+ * caller-chosen distinct ids, which the sink reports; n_channels = 0 clears the set, and a dongle without channels costs
+ * nothing.  B200_ERR_ARG for a bad stream index, n_channels above the capacity, a repeated id or no channel sink.  A batch
+ * uses the set that was current when its LAST sample was pushed: a change made while a batch is partly filled
+ * (b200_stream_pending_samples) applies to that batch, and a full batch waiting for its group keeps its set.  A channel's
+ * audio depends only on the input and its absolute position, so a channel added or retuned at batch b gives exactly
+ * what an always-present channel at that offset gives from batch b on.
+ * b200_stream_set_channel_filter: the FIR channel filter of b200_fm_channels_exec_fir for every channel of the stream
+ * (h_taps: n_taps host floats, n_taps = 0 goes back to the boxcar); only before anything is pushed.  The dongle rows
+ * get the history b200_fm_channels_fir_history_samples(R, n_taps); B200_ERR_ARG if that exceeds batch_samples or the
+ * (R, n_taps) pair does not fit.  Spectra, payloads and centre audio do not change. */
+typedef void (*b200_channel_audio_sink)(void* user, int stream, int32_t channel_id, int64_t first_sample, int n,
+                                        const float* audio);
+int b200_stream_set_channel_sink(b200_stream* s, int max_channels, b200_channel_audio_sink sink);
+int b200_stream_set_channels(b200_stream* s, int stream, int n_channels, const uint32_t* h_phase_inc,
+                             const int32_t* h_channel_ids);
+int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_taps);
 
 /* ---- websocket wire formats: what the reference's main.c puts on the socket ----------------
  *

@@ -29,6 +29,8 @@ EXPORTED_SYMBOLS = [
     "b200_fm_channel_tune", "b200_fm_channels_exec",
     "b200_iq_history_reset", "b200_iq_history_carry", "b200_fm_channel_filter_design",
     "b200_fm_channels_fir_history_samples", "b200_fm_channels_exec_fir", "b200_session_set_channel_filter",
+    "b200_fm_channels_exec_runs", "b200_stream_set_channel_sink", "b200_stream_set_channels",
+    "b200_stream_set_channel_filter",
     "b200_chain_exec", "b200_chain_exec_r", "b200_chain_tile_samples",
     "b200_session_create", "b200_session_create_r", "b200_session_destroy", "b200_session_reset", "b200_session_chain", "b200_session_products",
     "b200_session_channels",
@@ -66,6 +68,16 @@ RF_CALLBACK = C.CFUNCTYPE(None, C.POINTER(CmplxS32), C.c_int)
 SPECTRUM_SINK = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.POINTER(C.c_float))
 AUDIO_SINK = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.POINTER(C.c_float))
 PAYLOAD_SINK = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.POINTER(C.c_ubyte))
+CHANNEL_SINK = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int32, C.c_int64, C.c_int, C.POINTER(C.c_float))
+
+FM_MAX_CHANNELS = 32
+FM_MAX_RUNS = 64
+
+
+class FmChannelRun(C.Structure):
+    """b200_fm_channel_run: one row of the runs table of b200_fm_channels_exec_runs."""
+    _fields_ = [("stream", C.c_int32), ("n_channels", C.c_int32), ("first_sample", C.c_int64),
+                ("audio_row", C.c_int64), ("phase_inc", C.c_uint32 * FM_MAX_CHANNELS)]
 
 _lib = None
 
@@ -103,6 +115,10 @@ def lib() -> C.CDLL:
     L.b200_fm_channels_fir_history_samples.argtypes = [i32, i32]
     L.b200_fm_channels_exec_fir.argtypes = [vp, i64, i32, i64, i32, i64, vp, i32, f32p, i64, f32p, i64, vp, i32, vp]
     L.b200_session_set_channel_filter.argtypes = [vp, vp, i32]
+    L.b200_fm_channels_exec_runs.argtypes = [vp, i64, i32, i64, i32, vp, i32, f32p, i64, i64, vp, i32, vp]
+    L.b200_stream_set_channel_sink.argtypes = [vp, i32, CHANNEL_SINK]
+    L.b200_stream_set_channels.argtypes = [vp, i32, i32, vp, vp]
+    L.b200_stream_set_channel_filter.argtypes = [vp, vp, i32]
     L.b200_chain_exec.argtypes = [vp, i64, i32, i64, i32, f32p, f32p, i64, vp, i32, vp]
     L.b200_chain_exec_r.argtypes = [vp, i64, i32, i64, i32, i32, f32p, f32p, i64, vp, i32, vp]
     L.b200_chain_tile_samples.restype = i64
@@ -352,9 +368,6 @@ def fm_exec(ring: StreamRing, audio=None, decimated: bool = False, dec=None, str
     return audio, dec
 
 
-FM_MAX_CHANNELS = 32
-
-
 def fm_channel_tune(offset_hz: float, fs: float) -> int:
     """b200_fm_channel_tune: the phase increment (uint32) that brings baseband +offset_hz to DC; host arithmetic."""
     inc = C.c_uint32()
@@ -420,6 +433,42 @@ def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None,
                                        bb.stride(1) // 2 if bb is not None else 0, _stream_ptr(stream)),
            "b200_fm_channels_exec")
     return audio, bb
+
+
+def fm_channels_exec_runs(ring: StreamRing, runs, audio=None, taps=None, stream=None):
+    """b200_fm_channels_exec_runs over a StreamRing: runs is a sequence of (stream, first_sample, phase_inc list),
+    each with its own position and 1..32 uint32 increments; run k's channels get the next len(phase_inc) audio rows,
+    in order.  taps (a cuda float32 tensor [T]) selects the FIR filter, whose ring needs the history of
+    fm_channels_fir_history_samples(R, T).  -> audio [sum of the channel counts, n/(4R)] f32."""
+    torch = _torch()
+    runs = list(runs)
+    table = (FmChannelRun * max(1, len(runs)))()
+    row = 0
+    for k, (s, first, incs) in enumerate(runs):
+        incs = [int(v) & 0xFFFFFFFF for v in incs]
+        table[k].stream, table[k].n_channels, table[k].first_sample, table[k].audio_row = s, len(incs), first, row
+        for c, v in enumerate(incs[:FM_MAX_CHANNELS]):
+            table[k].phase_inc[c] = v
+        row += len(incs)
+    n_audio = ring.n_samples // (4 * ring.R)
+    if audio is None:
+        audio = torch.empty((max(row, 1), n_audio), dtype=torch.float32, device=ring.buf.device)
+    _check_output("fm_channels_exec_runs audio", audio, torch.float32, (max(row, 1), n_audio), ring.buf.device,
+                  row_slices=True)
+    T = 0
+    if taps is not None:
+        assert taps.is_cuda and taps.dtype == torch.float32 and taps.dim() == 1 and taps.is_contiguous()
+        T = taps.shape[0]
+        need = fm_channels_fir_history_samples(ring.R, T)
+        if ring.hist < need:          # the kernel would read before the rows: refuse before anything is launched
+            raise B200Error(f"fm_channels_exec_runs: {T} taps at R = {ring.R} need a ring history of {need} "
+                            f"samples, the ring has {ring.hist}")
+    _check(lib().b200_fm_channels_exec_runs(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
+                                            ring.n_samples, ring.R, table, len(runs), C.c_void_p(audio.data_ptr()),
+                                            audio.stride(0), audio.shape[0],
+                                            C.c_void_p(taps.data_ptr()) if taps is not None else None, T,
+                                            _stream_ptr(stream)), "b200_fm_channels_exec_runs")
+    return audio
 
 
 def _check_output(what: str, t, dtype, shape: tuple, device, row_slices: bool = False) -> None:
@@ -683,9 +732,11 @@ class PushStream:
     """b200_stream_*: signal_source-style pushes in, spectra and audio out through sinks."""
 
     def __init__(self, n_streams: int, batch_samples: int, gain_db: int = 0, R: int = 10, payload_K: int = 0,
-                 frames: bool = True):
+                 frames: bool = True, channel_capacity: int = 0):
         """payload_K > 0: also collect the K-frame averaged u8 payload of every batch (self.payloads);
-        frames=False: no per-frame dB sink (the rows stay on the device)."""
+        frames=False: no per-frame dB sink (the rows stay on the device);
+        channel_capacity > 0: FM channels, up to that many per dongle (set_channels), collected in
+        self.channel_audio[stream][channel id] as (first_sample, [n] copy) tuples."""
         _torch()
         self.n_streams, self.batch, self.R = n_streams, batch_samples, R
         self.h = lib().b200_stream_create_r(n_streams, batch_samples, gain_db, R)
@@ -696,6 +747,7 @@ class PushStream:
         self._payload_K = payload_K
         self.spectra = [[] for _ in range(n_streams)]      # (first_frame, [n_frames, 1024] copy)
         self.audio = [[] for _ in range(n_streams)]        # (first_sample, [n] copy)
+        self.channel_audio = [{} for _ in range(n_streams)]   # id -> [(first_sample, [n] copy)]
 
         def on_spectrum(user, stream, first, n, ptr):
             self.spectra[stream].append((first, np.ctypeslib.as_array(ptr, shape=(n, 1024)).copy()))
@@ -711,6 +763,30 @@ class PushStream:
         lib().b200_stream_set_sinks(self.h, self._cb[0], self._cb[1], None)
         if self._payload_K > 0:
             _check(lib().b200_stream_set_payload_sink(self.h, self._payload_K, self._cb[2]), "b200_stream_set_payload_sink")
+
+        def on_channel(user, stream, cid, first, n, ptr):
+            self.channel_audio[stream].setdefault(cid, []).append((first, np.ctypeslib.as_array(ptr, shape=(n,)).copy()))
+
+        self._on_channel = CHANNEL_SINK(on_channel)
+        if channel_capacity > 0:
+            _check(lib().b200_stream_set_channel_sink(self.h, channel_capacity, self._on_channel),
+                   "b200_stream_set_channel_sink")
+
+    def set_channels(self, stream: int, phase_inc, ids) -> None:
+        """b200_stream_set_channels: dongle `stream`'s listeners from now on (increments as uint32 bits, distinct
+        int32 ids); empty lists clear the set.  Takes effect with the batch whose last sample is pushed next."""
+        inc = np.ascontiguousarray(np.asarray(phase_inc, dtype=np.int64).reshape(-1) & 0xFFFFFFFF, dtype=np.uint32)
+        cid = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1), dtype=np.int32)
+        assert inc.size == cid.size
+        _check(lib().b200_stream_set_channels(self.h, stream, int(inc.size), inc.ctypes.data if inc.size else None,
+                                              cid.ctypes.data if cid.size else None), "b200_stream_set_channels")
+
+    def set_channel_filter(self, h_taps) -> None:
+        """b200_stream_set_channel_filter: FIR taps (host float32) for every channel; None or empty goes back to the
+        boxcar.  Only before anything is pushed."""
+        h = np.zeros(0, np.float32) if h_taps is None else np.ascontiguousarray(h_taps, dtype=np.float32).reshape(-1)
+        _check(lib().b200_stream_set_channel_filter(self.h, h.ctypes.data if h.size else None, int(h.size)),
+               "b200_stream_set_channel_filter")
 
     def enable_frames(self) -> None:
         """Install the per-frame dB sink on a stream that was created without one (frames=False): the library

@@ -99,6 +99,9 @@ int launch_fm_channels_fir(const uint8_t* iq, int64_t stream_stride_bytes, int n
                            float* audio, int64_t audio_stride, float* baseband, int64_t baseband_stride,
                            cudaStream_t stream);
 int fm_channels_fir_history_samples(int R, int T);
+int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                            const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
+                            int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream);
 int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h);
 
 }  // namespace b200
@@ -566,6 +569,15 @@ int b200_fm_channels_exec_fir(const uint8_t* d_iq, int64_t stream_stride_bytes, 
     return launch_fm_channels_fir(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
                                   n_channels, d_taps, n_taps, d_audio, audio_stride, d_baseband, baseband_stride,
                                   reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+int b200_fm_channels_exec_runs(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,
+                               int R, const b200_fm_channel_run* h_runs, int n_runs, float* d_audio,
+                               int64_t audio_stride, int64_t n_audio_rows, const float* d_taps, int n_taps,
+                               void* cuda_stream)
+{
+    return launch_fm_channels_runs(d_iq, stream_stride_bytes, n_streams, n_samples, R, h_runs, n_runs, d_audio,
+                                   audio_stride, n_audio_rows, d_taps, n_taps, reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- pinned host memory --------------------------------------------------------------------

@@ -20,6 +20,8 @@
 //   2. half-band #1 -> work[g][] (smem)          3. half-band #2 -> audio row s*C + c
 // At R = 10 a lane unpacks its ten byte pairs into registers once per tile and reuses them for every channel;
 // any other R reads and unpacks the bytes once per channel.
+#include <string.h>
+
 #include "b200_common.cuh"
 #include "fm_channels.cuh"
 #include "fm_kernels.cuh"
@@ -28,9 +30,12 @@ namespace b200 {
 
 namespace {
 
-template <int RT, int G>
-__global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams p, const int tiles_per_stream,
-                                                                 const int stage_bytes, const int n_stages)
+// The tile loop of both forms.  RUNS: p is an FcRunsParams, p.n_streams counts runs, and each tile takes its IQ
+// row, channel count, increments, position and audio rows from its run; no baseband.  The channel loop bound is the
+// tile's, the same for every thread of the CTA, so the three barriers per group stay uniform.
+template <int RT, int G, bool RUNS, class P>
+__device__ __forceinline__ void fm_channels_tiles(const P& p, const int tiles_per_stream, const int stage_bytes,
+                                                  const int n_stages)
 {
     extern __shared__ __align__(128) uint8_t smem[];
     const int R = RT ? RT : p.R;
@@ -43,10 +48,10 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams 
     float* work = demod + G * FC_DEMOD;                                           // [G][FC_WORK]
     uint64_t* bars = reinterpret_cast<uint64_t*>(work + G * FC_WORK);
 
-    const int C = p.n_channels;
+    const int C_all = p.n_channels;
     const int64_t n_audio = p.n_samples / (4 * R);
     const int64_t total_tiles = (int64_t) p.n_streams * tiles_per_stream;
-    const uint32_t first_dec = (uint32_t) (p.first_sample / R);      // mod 2^32, like every phase below
+    const uint32_t first_dec_all = (uint32_t) (p.first_sample / R);      // mod 2^32, like every phase below
 
     if (tid == 0) {
         mbar_init(&bars[0], 1);
@@ -56,8 +61,9 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams 
     __syncthreads();
 
     auto issue = [&](int64_t tile, int st) {
-        const int s = (int) (tile / tiles_per_stream);
-        const int64_t n0 = (tile - (int64_t) s * tiles_per_stream) * FC_T;
+        const int q = (int) (tile / tiles_per_stream);
+        const int s = RUNS ? fc_run<RUNS>(p, q)->stream : q;
+        const int64_t n0 = (tile - (int64_t) q * tiles_per_stream) * FC_T;
         const int ta = (int) ((n_audio - n0) < FC_T ? (n_audio - n0) : FC_T);
         // 8 (ta + 8) R bytes from byte 8 (n0 - 8) R: multiples of 16 (n0 is a multiple of 62; ta is even for odd R
         // because n_samples is a multiple of 8 and of 4R), as in fm_chain_warp_kernel
@@ -74,12 +80,17 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams 
 
     for (uint32_t it = 0; tile < total_tiles; tile += gridDim.x, ++it) {
         const int st = (int) (it % (uint32_t) n_stages);
-        const int s = (int) (tile / tiles_per_stream);
-        const int64_t n0 = (tile - (int64_t) s * tiles_per_stream) * FC_T;
+        const int q = (int) (tile / tiles_per_stream);
+        // the runs form: this tile's IQ row, channel count, position, increments and audio rows come from its run
+        const FcRun* run = fc_run<RUNS>(p, q);
+        const int s = RUNS ? run->stream : q;
+        const int C = RUNS ? run->n_channels : C_all;
+        const uint32_t first_dec = RUNS ? run->first_dec : first_dec_all;
+        const int64_t n0 = (tile - (int64_t) q * tiles_per_stream) * FC_T;
         const int ta = (int) ((n_audio - n0) < FC_T ? (n_audio - n0) : FC_T);
         const int j = 31 * warp + lane;                                   // this lane's decimated sample
         const uint32_t m = first_dec + (uint32_t) (4 * n0 - 32) + (uint32_t) j;
-        const uint32_t* incs = p.phase_inc + (int64_t) s * C;
+        const uint32_t* incs = RUNS ? run->phase_inc : p.phase_inc + (int64_t) s * C;
 
         mbar_wait(&bars[st], (it / (uint32_t) n_stages) & 1);
         const uint8_t* in = ring + st * stage_bytes + j * 2 * R;
@@ -136,7 +147,7 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams 
                     rotation(incs[c0 + g] * (uint32_t) R * m, rc, rs);
                     const float bre = fmaf(ar, rc, ai * rs);          // (ar + j ai) (rc - j rs)
                     const float bim = fmaf(ai, rc, -(ar * rs));
-                    if (p.baseband != nullptr && j >= 32 && j < 4 * ta + 32)
+                    if (!RUNS && p.baseband != nullptr && j >= 32 && j < 4 * ta + 32)
                         p.baseband[((int64_t) s * C + c0 + g) * p.baseband_stride + 4 * n0 + (j - 32)] = make_float2(bre, bim);
                     const float ph = atan2_approx_dev(bim, bre);
                     const float prev = __shfl_up_sync(0xffffffffu, ph, 1);
@@ -164,13 +175,28 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams 
             for (int i = tid; i < gc * FC_T; i += FC_THREADS) {
                 const int g = i / FC_T, a = i - g * FC_T;
                 if (a < ta)
-                    p.audio[((int64_t) s * C + c0 + g) * p.audio_stride + n0 + a] = halfband_from(work + g * FC_WORK + 2 * a);
+                    p.audio[((RUNS ? run->audio_row : (int64_t) s * C) + c0 + g) * p.audio_stride + n0 + a] = halfband_from(work + g * FC_WORK + 2 * a);
             }
             // taps[] are rewritten by the next group after every thread passed the phase-1 barrier; demod[] in the
             // next phase 1, after the phase-2 barrier; work[] in the next phase 2, after the next phase-1 barrier,
             // which every phase-3 reader reaches first.
         }
     }
+}
+
+template <int RT, int G>
+__global__ void __launch_bounds__(FC_THREADS) fm_channels_kernel(const FcParams p, const int tiles_per_stream,
+                                                                 const int stage_bytes, const int n_stages)
+{
+    fm_channels_tiles<RT, G, false>(p, tiles_per_stream, stage_bytes, n_stages);
+}
+
+template <int RT, int G>
+__global__ void __launch_bounds__(FC_THREADS) fm_channels_runs_kernel(const __grid_constant__ FcRunsParams p,
+                                                                      const int tiles_per_stream,
+                                                                      const int stage_bytes, const int n_stages)
+{
+    fm_channels_tiles<RT, G, true>(p, tiles_per_stream, stage_bytes, n_stages);
 }
 
 template <int RT, int G>
@@ -191,7 +217,117 @@ int launch_fc(const FcParams& p, int64_t tps, cudaStream_t stream)
     return B200_OK;
 }
 
+// the same geometry as launch_fc; p.n_streams counts runs
+template <int RT, int G>
+int launch_fc_runs(const FcRunsParams& p, int64_t tps, cudaStream_t stream)
+{
+    const int R = p.R;
+    const int stage_bytes = FC_ND * 2 * R;
+    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;
+    const int smem = n_stages * stage_bytes + G * R * 16 + G * (FC_DEMOD + FC_WORK) * 4 + 16;
+    auto kern = fm_channels_runs_kernel<RT, G>;
+    if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
+    const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
+    int64_t grid = (int64_t) sm_count() * per_sm;
+    const int64_t total = (int64_t) p.n_streams * tps;
+    if (grid > total) grid = total;
+    kern<<<(unsigned) grid, FC_THREADS, smem, stream>>>(p, (int) tps, stage_bytes, n_stages);
+    B200_LAUNCH_CHECK();
+    return B200_OK;
+}
+
 }  // namespace
+
+int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                            const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
+                            int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream)
+{
+    if (iq == nullptr || audio == nullptr || runs == nullptr || n_streams < 1) {
+        set_error("fm channels runs: null pointer or no IQ rows");
+        return B200_ERR_ARG;
+    }
+    if (n_runs < 1 || n_runs > B200_FM_MAX_RUNS) {
+        set_error("fm channels runs: n_runs %d outside [1, %d]", n_runs, B200_FM_MAX_RUNS);
+        return B200_ERR_ARG;
+    }
+    if (R < 1 || R > 256) {
+        set_error("fm channels runs: down factor %d outside [1, 256]", R);
+        return B200_ERR_ARG;
+    }
+    if (n_samples < 0 || n_samples % (4 * R) != 0 || n_samples % 8 != 0) {
+        set_error("fm channels runs: n_samples %lld must be a multiple of 4*R and of 8", (long long) n_samples);
+        return B200_ERR_ARG;
+    }
+    const int64_t n_audio = n_samples / (4 * R);
+    if (n_audio_rows < 1 || audio_stride < n_audio) {
+        set_error("fm channels runs: %lld audio rows %lld floats apart for %lld samples a row", (long long) n_audio_rows,
+                  (long long) audio_stride, (long long) n_audio);
+        return B200_ERR_ARG;
+    }
+    const bool fir = taps != nullptr || T != 0;
+    if (fir && (taps == nullptr || T < 1 || T > B200_FM_MAX_CHANNEL_TAPS)) {
+        set_error("fm channels runs: %d taps: want NULL taps and 0 (boxcar) or [1, %d] device taps", T,
+                  B200_FM_MAX_CHANNEL_TAPS);
+        return B200_ERR_ARG;
+    }
+    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
+        set_error("fm channels runs: IQ pointer and stream stride must be 16-byte aligned");
+        return B200_ERR_ALIGN;
+    }
+    if ((reinterpret_cast<uintptr_t>(audio) & 3) != 0 || (reinterpret_cast<uintptr_t>(taps) & 3) != 0) {
+        set_error("fm channels runs: audio and taps must be 4-byte aligned");
+        return B200_ERR_ALIGN;
+    }
+    int max_c = 0;
+    for (int k = 0; k < n_runs; ++k) {
+        const b200_fm_channel_run& r = runs[k];
+        if (r.stream < 0 || r.stream >= n_streams || r.n_channels < 1 || r.n_channels > B200_FM_MAX_CHANNELS ||
+            r.first_sample < 0 || r.first_sample % (4 * R) != 0 || r.audio_row < 0 ||
+            r.audio_row > n_audio_rows - r.n_channels) {
+            set_error("fm channels runs: run %d (row %d of %d, %d channels, first sample %lld, audio row %lld of %lld)",
+                      k, r.stream, n_streams, r.n_channels, (long long) r.first_sample, (long long) r.audio_row,
+                      (long long) n_audio_rows);
+            return B200_ERR_ARG;
+        }
+        // two runs writing the same audio row would race
+        for (int i = 0; i < k; ++i)
+            if (r.audio_row < runs[i].audio_row + runs[i].n_channels && runs[i].audio_row < r.audio_row + r.n_channels) {
+                set_error("fm channels runs: the audio rows of runs %d and %d overlap", i, k);
+                return B200_ERR_ARG;
+            }
+        if (r.n_channels > max_c) max_c = r.n_channels;
+    }
+    if (fir && !fm_channels_fir_fits(R, T)) {
+        set_error("fm channels runs: R = %d with %d taps does not fit in shared memory", R, T);
+        return B200_ERR_ARG;
+    }
+    const int64_t tps = (n_audio + FC_T - 1) / FC_T;
+    if ((int64_t) n_runs * tps >= (1ll << 31)) {
+        set_error("fm channels runs: batch too long");
+        return B200_ERR_ARG;
+    }
+    if (n_samples == 0) return B200_OK;
+    FcRunsParams p;
+    memset(&p, 0, sizeof(p));
+    p.iq = iq;
+    p.stream_stride_bytes = stream_stride_bytes;
+    p.n_streams = n_runs;
+    p.n_samples = n_samples;
+    p.R = R;
+    p.audio = audio;
+    p.audio_stride = audio_stride;
+    for (int k = 0; k < n_runs; ++k) {
+        FcRun& r = p.runs[k];
+        r.stream = runs[k].stream;
+        r.n_channels = runs[k].n_channels;
+        r.first_dec = (uint32_t) (runs[k].first_sample / R);
+        r.audio_row = runs[k].audio_row;
+        memcpy(r.phase_inc, runs[k].phase_inc, sizeof(r.phase_inc));
+    }
+    if (fir) return launch_fm_channels_fir_runs(p, tps, taps, T, max_c, stream);
+    if (R == 10) return launch_fc_runs<10, 8>(p, tps, stream);
+    return launch_fc_runs<0, 4>(p, tps, stream);
+}
 
 int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
                        int64_t first_sample, const uint32_t* phase_inc, int n_channels, float* audio,

@@ -30,6 +30,24 @@ struct FcParams {
     int64_t baseband_stride;        // complex samples
 };
 
+// A b200_fm_channel_run as the kernels read it: the launcher computes the first decimated sample first_sample / R
+// (mod 2^32, like every phase) once on the host, so that no tile divides a 64-bit position.
+struct FcRun {
+    int32_t stream;
+    int32_t n_channels;
+    uint32_t first_dec;
+    int64_t audio_row;
+    uint32_t phase_inc[B200_FM_MAX_CHANNELS];
+};
+
+// The runs form (b200_fm_channels_exec_runs): tile t belongs to run t / tiles_per_stream, and each run names its own
+// IQ row, channel count, increments, stream position and audio row.  The base's n_streams is the number of runs; its
+// first_sample, phase_inc, n_channels and baseband are unused.  Passed by value as a __grid_constant__ parameter
+// (~9.8 KB): per-run fields are read from the constant bank, and nothing is copied to the device.
+struct FcRunsParams : FcParams {
+    FcRun runs[B200_FM_MAX_RUNS];
+};
+
 // exp(-j theta) for theta = 2 pi phi / 2^32, phi read as int32 so theta is in [-pi, pi).  MUFU sin / cos: the
 // argument carries <= 3.1e-7 rad of rounding (int -> float and the product), sin.approx / cos.approx <= 5.1e-7 on
 // [-pi, pi]: <= 8.2e-7 absolute per component.  phi = 0 is exactly (1, 0).
@@ -49,5 +67,18 @@ __device__ __forceinline__ c64 byte_pair(uint32_t v, uint32_t sel)
     const float u = __uint_as_float(__byte_perm(v, 0x4B000000u, 0x7540u | sel));
     return cadd(cpack(u, u), cpack(-8388736.0f, -8388736.0f));
 }
+
+// the run of tile group q in the runs form (FcRunsParams / FirRunsParams); nullptr in the uniform form
+template <bool RUNS, class P>
+__device__ __forceinline__ const FcRun* fc_run(const P& p, int q)
+{
+    if constexpr (RUNS) return &p.runs[q];
+    else return nullptr;
+}
+
+// host side: the runs form's FIR launcher (fm_channels_fir.cu), called by launch_fm_channels_runs after the common checks
+int launch_fm_channels_fir_runs(const FcRunsParams& p, int64_t tiles_per_stream, const float* taps, int T,
+                                int max_channels, cudaStream_t stream);
+int fm_channels_fir_fits(int R, int T);
 
 }  // namespace b200

@@ -16,6 +16,7 @@
 // G accumulators per lane, taps [T][G] in shared memory, read as broadcasts.  G comes from the shared-memory budget
 // and the channel count (launcher).  Phases 2 and 3 (the half-bands) are the boxcar kernel's.
 #include <math.h>
+#include <string.h>
 
 #include "b200_common.cuh"
 #include "fm_channels.cuh"
@@ -34,6 +35,11 @@ struct FirParams {
     int T;
     int L;                          // T - R
     int off;                        // (-L) mod 8: where lane 0's window starts in a stage
+};
+
+// the runs form: c.n_streams counts runs (FcRunsParams)
+struct FirRunsParams : FirParams {
+    FcRun runs[B200_FM_MAX_RUNS];
 };
 
 // MAC over T taps for NG channels of the group, then rotation, discriminator and limiter -> demod[g][j]
@@ -73,9 +79,10 @@ __device__ __forceinline__ void fir_group(const uint16_t* in, const float4* taps
     }
 }
 
-__global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirParams p, const int tiles_per_stream,
-                                                                     const int stage_bytes, const int n_stages,
-                                                                     const int G)
+// the tile loop of both forms, as fm_channels_tiles in fm_channels.cu
+template <bool RUNS, class P>
+__device__ __forceinline__ void fm_channels_fir_tiles(const P& p, const int tiles_per_stream, const int stage_bytes,
+                                                      const int n_stages, const int G)
 {
     extern __shared__ __align__(128) uint8_t smem[];
     const int R = p.c.R;
@@ -89,10 +96,10 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirPa
     float* work = demod + G * FC_DEMOD;                                           // [G][FC_WORK]
     uint64_t* bars = reinterpret_cast<uint64_t*>(work + G * FC_WORK);
 
-    const int C = p.c.n_channels;
+    const int C_all = p.c.n_channels;
     const int64_t n_audio = p.c.n_samples / (4 * R);
     const int64_t total_tiles = (int64_t) p.c.n_streams * tiles_per_stream;
-    const uint32_t first_dec = (uint32_t) (p.c.first_sample / R);      // mod 2^32, like every phase below
+    const uint32_t first_dec_all = (uint32_t) (p.c.first_sample / R);      // mod 2^32, like every phase below
 
     if (tid == 0) {
         mbar_init(&bars[0], 1);
@@ -102,8 +109,9 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirPa
     __syncthreads();
 
     auto issue = [&](int64_t tile, int st) {
-        const int s = (int) (tile / tiles_per_stream);
-        const int64_t n0 = (tile - (int64_t) s * tiles_per_stream) * FC_T;
+        const int q = (int) (tile / tiles_per_stream);
+        const int s = RUNS ? fc_run<RUNS>(p, q)->stream : q;
+        const int64_t n0 = (tile - (int64_t) q * tiles_per_stream) * FC_T;
         const int ta = (int) ((n_audio - n0) < FC_T ? (n_audio - n0) : FC_T);
         // samples from (4 n0 - 32) R - L - off (a multiple of 8: (4 n0 - 32) R is one because n0 is a multiple of 62,
         // and L + off is one by the choice of off) up to 4 (n0 + ta) R, a multiple of 8 as in fm_channels.cu
@@ -121,12 +129,17 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirPa
 
     for (uint32_t it = 0; tile < total_tiles; tile += gridDim.x, ++it) {
         const int st = (int) (it % (uint32_t) n_stages);
-        const int s = (int) (tile / tiles_per_stream);
-        const int64_t n0 = (tile - (int64_t) s * tiles_per_stream) * FC_T;
+        const int q = (int) (tile / tiles_per_stream);
+        // the runs form: this tile's IQ row, channel count, position, increments and audio rows come from its run
+        const FcRun* run = fc_run<RUNS>(p, q);
+        const int s = RUNS ? run->stream : q;
+        const int C = RUNS ? run->n_channels : C_all;
+        const uint32_t first_dec = RUNS ? run->first_dec : first_dec_all;
+        const int64_t n0 = (tile - (int64_t) q * tiles_per_stream) * FC_T;
         const int ta = (int) ((n_audio - n0) < FC_T ? (n_audio - n0) : FC_T);
         const int j = 31 * warp + lane;                                   // this lane's decimated sample
         const uint32_t m = first_dec + (uint32_t) (4 * n0 - 32) + (uint32_t) j;
-        const uint32_t* incs = p.c.phase_inc + (int64_t) s * C;
+        const uint32_t* incs = RUNS ? run->phase_inc : p.c.phase_inc + (int64_t) s * C;
 
         mbar_wait(&bars[st], (it / (uint32_t) n_stages) & 1);
         // lane j's window: input samples (4 n0 - 32 + j) R - L + k, k < T
@@ -146,7 +159,7 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirPa
             __syncthreads();
 
             // ---- 1. mix + FIR, rotation, discriminator ----
-            float2* bb = p.c.baseband != nullptr
+            float2* bb = !RUNS && p.c.baseband != nullptr
                              ? p.c.baseband + ((int64_t) s * C + c0) * p.c.baseband_stride + 4 * n0 : nullptr;
             const int64_t bs = p.c.baseband_stride;
             switch (gc) {
@@ -180,11 +193,28 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirPa
             for (int i = tid; i < gc * FC_T; i += FC_THREADS) {
                 const int g = i / FC_T, a = i - g * FC_T;
                 if (a < ta)
-                    p.c.audio[((int64_t) s * C + c0 + g) * p.c.audio_stride + n0 + a] = halfband_from(work + g * FC_WORK + 2 * a);
+                    p.c.audio[((RUNS ? run->audio_row : (int64_t) s * C) + c0 + g) * p.c.audio_stride + n0 + a] = halfband_from(work + g * FC_WORK + 2 * a);
             }
             // taps[], demod[] and work[] are reused under the same barriers as in fm_channels.cu
         }
     }
+}
+
+__global__ void __launch_bounds__(FC_THREADS) fm_channels_fir_kernel(const FirParams p, const int tiles_per_stream,
+                                                                     const int stage_bytes, const int n_stages,
+                                                                     const int G)
+{
+    fm_channels_fir_tiles<false>(p, tiles_per_stream, stage_bytes, n_stages, G);
+}
+
+// three CTAs per SM, as the uniform kernel (72 registers): unbounded, the per-run values take this one to 81, which
+// leaves room for only two 288-thread CTAs
+__global__ void __launch_bounds__(FC_THREADS, 3) fm_channels_fir_runs_kernel(const __grid_constant__ FirRunsParams p,
+                                                                          const int tiles_per_stream,
+                                                                          const int stage_bytes, const int n_stages,
+                                                                          const int G)
+{
+    fm_channels_fir_tiles<true>(p, tiles_per_stream, stage_bytes, n_stages, G);
 }
 
 int fir_stage_bytes(int R, int T)
@@ -210,6 +240,45 @@ int fir_group_size(int stage_bytes, int n_stages, int T, int C)
 }
 
 }  // namespace
+
+int fm_channels_fir_fits(int R, int T)
+{
+    const int stage_bytes = fir_stage_bytes(R, T);
+    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;
+    return fir_group_size(stage_bytes, n_stages, T, 1) > 0;
+}
+
+// G from the table's largest channel count, with the budget of the uniform call; a run's audio does not depend on
+// G (each channel's MAC, rotation and demodulator are the same whatever group it is computed in)
+int launch_fm_channels_fir_runs(const FcRunsParams& runs, int64_t tps, const float* taps, int T, int max_channels,
+                                cudaStream_t stream)
+{
+    const int R = runs.R;
+    const int stage_bytes = fir_stage_bytes(R, T);
+    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;       // as fm_channels.cu
+    const int G = fir_group_size(stage_bytes, n_stages, T, max_channels);
+    if (G == 0) {
+        set_error("fm channels runs: R = %d with %d taps does not fit in shared memory", R, T);
+        return B200_ERR_ARG;
+    }
+    FirRunsParams p;
+    static_cast<FcParams&>(p.c) = static_cast<const FcParams&>(runs);
+    memcpy(p.runs, runs.runs, sizeof(p.runs));
+    p.taps = taps;
+    p.T = T;
+    p.L = T - R;
+    p.off = (R - T) & 7;
+    const int smem = fir_smem_bytes(stage_bytes, n_stages, T, G);
+    auto kern = fm_channels_fir_runs_kernel;
+    if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
+    const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
+    int64_t grid = (int64_t) sm_count() * per_sm;
+    const int64_t total = (int64_t) runs.n_streams * tps;
+    if (grid > total) grid = total;
+    kern<<<(unsigned) grid, FC_THREADS, smem, stream>>>(p, (int) tps, stage_bytes, n_stages, G);
+    B200_LAUNCH_CHECK();
+    return B200_OK;
+}
 
 int fm_channels_fir_history_samples(int R, int T)
 {

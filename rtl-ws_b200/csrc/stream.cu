@@ -16,6 +16,11 @@
 // b200_stream_push / _poll / _flush on the calling thread (no hidden threads), in submission
 // order per stream.  Re-blocking is aligned to stream start like rf_decimator.c:88-115, so
 // results do not depend on how the source chunks the samples.
+//
+// FM channels (listeners at offsets inside a dongle's band): each stream has its own set of up to `chan_max`
+// channels.  A batch takes the set that is current when its last sample is pushed (stored with the slot then), and a
+// submitted run adds one launch of the runs-table channel kernel over its streams that have channels, after the
+// chain kernel and before the history carry, and one 2-D copy back.
 #include <string.h>
 
 #include <vector>
@@ -25,9 +30,15 @@
 using namespace b200;
 
 namespace b200 {
-int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
-int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
+int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
+                            cudaStream_t stream);
+int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
 int fm_history_samples(int R);
+int fm_channels_fir_history_samples(int R, int T);
+int fm_channels_fir_fits(int R, int T);
+int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                            const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
+                            int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream);
 }  // namespace b200
 
 namespace {
@@ -42,7 +53,7 @@ struct b200_stream {
     int64_t batch;                 // samples per batch (multiple of 5120)
     int gain_db;
     int R;                         // down factor of the FM branch
-    int hist;                      // samples
+    int hist;                      // samples: 32 R, or the channel filter's H(R, T)
     int64_t row_bytes;             // device row pitch: history + batch
     uint8_t* d_rows;               // [n_streams][ST_SLOTS? no: one row per stream][row_bytes]
     float* d_db;                   // [n_streams][batch]
@@ -55,6 +66,17 @@ struct b200_stream {
     int payload_K;                 // 0 = no payload sink
     b200_payload_sink payload_sink;
     cudaStream_t lanes[ST_LANES];
+    int chan_max;                  // channel capacity per stream; 0 = no channel buffers yet
+    b200_channel_audio_sink chan_sink;
+    float* d_chan;                 // [n_streams][chan_max][batch / (4R)]
+    float* h_chan;                 // pinned [n_streams][ST_SLOTS][chan_max][batch / (4R)]
+    float* d_taps;                 // the channel filter (n_taps floats), nullptr = boxcar
+    int n_taps;
+    struct ChannelSet {
+        int n;
+        uint32_t inc[B200_FM_MAX_CHANNELS];
+        int32_t id[B200_FM_MAX_CHANNELS];
+    };
     struct PerStream {
         int64_t fill;              // samples in the current slot
         int slot;                  // slot being filled
@@ -64,6 +86,9 @@ struct b200_stream {
         bool in_flight[ST_SLOTS];
         bool ready[ST_SLOTS];      // full, not yet submitted
         bool has_db[ST_SLOTS];     // the submitted slot computed and copied per-frame dB rows
+        ChannelSet channels;       // current listener set (b200_stream_set_channels)
+        ChannelSet slot_channels[ST_SLOTS];     // the set of each full slot, taken when its last sample arrived
+        bool has_chan[ST_SLOTS];   // the submitted slot computed and copied channel audio
     };
     std::vector<PerStream> st;
     b200_spectrum_sink spectrum_sink;
@@ -91,6 +116,13 @@ static void stream_deliver(b200_stream* s, int i, bool block)
             s->spectrum_sink(s->user, i, b * (s->batch / 1024), (int) (s->batch / 1024), s->h_db + off * (size_t) s->batch);
         if (s->audio_sink)
             s->audio_sink(s->user, i, b * (s->batch / (4 * s->R)), (int) (s->batch / (4 * s->R)), s->h_audio + off * (size_t) (s->batch / (4 * s->R)));
+        if (s->chan_sink && p.has_chan[slot]) {
+            const int64_t n_audio = s->batch / (4 * s->R);
+            const b200_stream::ChannelSet& cs = p.slot_channels[slot];
+            for (int c = 0; c < cs.n; ++c)
+                s->chan_sink(s->user, i, cs.id[c], b * n_audio, (int) n_audio,
+                             s->h_chan + (off * (size_t) s->chan_max + (size_t) c) * (size_t) n_audio);
+        }
         p.in_flight[slot] = false;
         ++p.batches_delivered;
     }
@@ -118,7 +150,31 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
     int rc = b200_chain_exec_r(d_batch, s->row_bytes, n, s->batch, s->R, s->gain_db, d_db, d_audio,
                                (int64_t) n_audio, want_payload ? d_pay : nullptr, want_payload ? s->payload_K : 0, lane);
     if (rc) return rc;
-    rc = launch_fm_history_carry(d_batch, s->row_bytes, n, s->batch, s->R, lane);
+    // channels of the streams that have listeners: one runs-table launch over the group's rows
+    const bool want_chan = s->chan_sink != nullptr && s->chan_max > 0;
+    int chan_width = 0;
+    if (want_chan) {
+        b200_fm_channel_run runs[ST_GROUP];
+        int n_runs = 0;
+        for (int i = a; i < b; ++i) {
+            const b200_stream::ChannelSet& cs = s->st[i].slot_channels[slot];
+            if (cs.n == 0) continue;
+            b200_fm_channel_run& r = runs[n_runs++];
+            r.stream = i - a;
+            r.n_channels = cs.n;
+            r.first_sample = s->st[i].batches_submitted * s->batch;
+            r.audio_row = (int64_t) (i - a) * s->chan_max;
+            memcpy(r.phase_inc, cs.inc, sizeof(uint32_t) * (size_t) cs.n);
+            if (cs.n > chan_width) chan_width = cs.n;
+        }
+        if (n_runs > 0) {
+            rc = launch_fm_channels_runs(d_batch, s->row_bytes, n, s->batch, s->R, runs, n_runs,
+                                         s->d_chan + (size_t) a * (size_t) s->chan_max * n_audio, (int64_t) n_audio,
+                                         (int64_t) n * s->chan_max, s->d_taps, s->n_taps, lane);
+            if (rc) return rc;
+        }
+    }
+    rc = launch_iq_history_carry(d_batch, s->row_bytes, n, s->batch, s->hist, lane);
     if (rc) return rc;
     // the per-frame dB rows cross PCIe only if somebody listens (4 bytes per sample; the payload is 1 KB per batch)
     if (want_db)
@@ -129,12 +185,21 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
     if (want_payload)
         B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_payload + off * 1024, ST_SLOTS * 1024, d_pay, 1024, 1024, (size_t) n,
                                         cudaMemcpyDeviceToHost, lane));
+    // per stream, its first chan_width channel rows (rows past a stream's own count are not read on delivery)
+    if (chan_width > 0) {
+        const size_t block = (size_t) s->chan_max * n_audio * sizeof(float);
+        B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_chan + off * (size_t) s->chan_max * n_audio, ST_SLOTS * block,
+                                        s->d_chan + (size_t) a * (size_t) s->chan_max * n_audio, block,
+                                        (size_t) chan_width * n_audio * sizeof(float), (size_t) n,
+                                        cudaMemcpyDeviceToHost, lane));
+    }
     for (int i = a; i < b; ++i) {
         b200_stream::PerStream& p = s->st[i];
         B200_CUDA_TRY(cudaEventRecord(p.done[slot], lane));
         p.ready[slot] = false;
         p.in_flight[slot] = true;
         p.has_db[slot] = want_db;
+        p.has_chan[slot] = want_chan;
         ++p.batches_submitted;
     }
     return B200_OK;
@@ -221,6 +286,12 @@ b200_stream* b200_stream_create_r(int n_streams, int64_t batch_samples, int gain
     s->spectrum_sink = nullptr;
     s->audio_sink = nullptr;
     s->user = nullptr;
+    s->chan_max = 0;
+    s->chan_sink = nullptr;
+    s->d_chan = nullptr;
+    s->h_chan = nullptr;
+    s->d_taps = nullptr;
+    s->n_taps = 0;
     for (int i = 0; i < ST_LANES; ++i) s->lanes[i] = nullptr;
     const size_t ns = (size_t) n_streams;
     bool ok = cudaMalloc(&s->d_rows, ns * (size_t) s->row_bytes) == cudaSuccess;
@@ -236,16 +307,19 @@ b200_stream* b200_stream_create_r(int n_streams, int64_t batch_samples, int gain
         s->st[i].slot = 0;
         s->st[i].batches_submitted = 0;
         s->st[i].batches_delivered = 0;
+        s->st[i].channels.n = 0;
         for (int k = 0; k < ST_SLOTS; ++k) {
             s->st[i].done[k] = nullptr;
             s->st[i].in_flight[k] = false;
             s->st[i].ready[k] = false;
             s->st[i].has_db[k] = false;
+            s->st[i].has_chan[k] = false;
+            s->st[i].slot_channels[k].n = 0;
             if (ok) ok = cudaEventCreateWithFlags(&s->st[i].done[k], cudaEventDisableTiming) == cudaSuccess;
         }
     }
     if (ok)
-        ok = launch_fm_history_reset(s->d_rows + 2 * (size_t) s->hist, s->row_bytes, n_streams, R, s->lanes[0]) == B200_OK &&
+        ok = launch_iq_history_reset(s->d_rows + 2 * (size_t) s->hist, s->row_bytes, n_streams, s->hist, s->lanes[0]) == B200_OK &&
              cudaStreamSynchronize(s->lanes[0]) == cudaSuccess;
     if (!ok) {
         set_error("stream: allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -274,6 +348,9 @@ void b200_stream_destroy(b200_stream* s)
     if (s->h_audio) cudaFreeHost(s->h_audio);
     if (s->d_payload) cudaFree(s->d_payload);
     if (s->h_payload) cudaFreeHost(s->h_payload);
+    if (s->d_chan) cudaFree(s->d_chan);
+    if (s->h_chan) cudaFreeHost(s->h_chan);
+    if (s->d_taps) cudaFree(s->d_taps);
     delete s;
 }
 
@@ -335,6 +412,7 @@ int b200_stream_push(b200_stream* s, int stream, const uint8_t* samples, int len
         p.fill += n;
         remaining -= n;
         if (p.fill == s->batch) {
+            p.slot_channels[p.slot] = p.channels;      // the batch keeps the listener set of its last sample
             p.ready[p.slot] = true;
             p.slot = (p.slot + 1) % ST_SLOTS;
             p.fill = 0;
@@ -359,6 +437,117 @@ int b200_stream_flush(b200_stream* s)
     if (s == nullptr) return B200_ERR_ARG;
     if (int rc = stream_submit_ready(s)) return rc;
     for (int i = 0; i < s->n_streams; ++i) stream_deliver(s, i, true);
+    return B200_OK;
+}
+
+int b200_stream_set_channel_sink(b200_stream* s, int max_channels, b200_channel_audio_sink sink)
+{
+    if (s == nullptr || max_channels < 1 || max_channels > B200_FM_MAX_CHANNELS ||
+        (s->chan_max != 0 && max_channels != s->chan_max)) {
+        set_error("stream channel sink: capacity %d must be in [1, %d] and stay what it was first (%d)", max_channels,
+                  B200_FM_MAX_CHANNELS, s ? s->chan_max : 0);
+        return B200_ERR_ARG;
+    }
+    if (s->chan_max == 0 && sink != nullptr) {      // the buffers come with the first sink, like the dB rows
+        const size_t rows = (size_t) s->n_streams * (size_t) max_channels;
+        const size_t n_audio = (size_t) (s->batch / (4 * s->R));
+        bool ok = cudaMalloc(&s->d_chan, sizeof(float) * rows * n_audio) == cudaSuccess;
+        ok = ok && cudaHostAlloc(&s->h_chan, sizeof(float) * rows * ST_SLOTS * n_audio, cudaHostAllocDefault) == cudaSuccess;
+        if (!ok) {
+            set_error("stream channel sink: buffers: %s", cudaGetErrorString(cudaGetLastError()));
+            if (s->d_chan) cudaFree(s->d_chan);
+            s->d_chan = nullptr;
+            s->h_chan = nullptr;
+            return B200_ERR_CUDA;
+        }
+        s->chan_max = max_channels;
+    }
+    s->chan_sink = sink;
+    return B200_OK;
+}
+
+int b200_stream_set_channels(b200_stream* s, int stream, int n_channels, const uint32_t* h_phase_inc,
+                             const int32_t* h_channel_ids)
+{
+    if (s == nullptr || stream < 0 || stream >= s->n_streams || s->chan_sink == nullptr || n_channels < 0 ||
+        n_channels > s->chan_max || (n_channels > 0 && (h_phase_inc == nullptr || h_channel_ids == nullptr))) {
+        set_error("stream channels: stream %d, %d channels (a channel sink of capacity %d is needed first)", stream,
+                  n_channels, s ? s->chan_max : 0);
+        return B200_ERR_ARG;
+    }
+    for (int c = 0; c < n_channels; ++c)
+        for (int k = 0; k < c; ++k)
+            if (h_channel_ids[k] == h_channel_ids[c]) {
+                set_error("stream channels: channel id %d appears twice", (int) h_channel_ids[c]);
+                return B200_ERR_ARG;
+            }
+    b200_stream::ChannelSet& cs = s->st[stream].channels;
+    cs.n = n_channels;
+    for (int c = 0; c < n_channels; ++c) {
+        cs.inc[c] = h_phase_inc[c];
+        cs.id[c] = h_channel_ids[c];
+    }
+    return B200_OK;
+}
+
+int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_taps)
+{
+    if (s == nullptr || n_taps < 0 || n_taps > B200_FM_MAX_CHANNEL_TAPS || (n_taps > 0 && h_taps == nullptr)) {
+        set_error("stream channel filter: bad arguments (%d taps)", n_taps);
+        return B200_ERR_ARG;
+    }
+    for (const auto& p : s->st)
+        if (p.fill != 0 || p.batches_submitted != 0 || p.ready[0] || p.ready[1]) {
+            set_error("stream channel filter: set it before anything is pushed");
+            return B200_ERR_ARG;
+        }
+    const int hist = n_taps > 0 ? fm_channels_fir_history_samples(s->R, n_taps) : fm_history_samples(s->R);
+    if (n_taps > 0 && !fm_channels_fir_fits(s->R, n_taps)) {
+        set_error("stream channel filter: R = %d with %d taps does not fit in shared memory", s->R, n_taps);
+        return B200_ERR_ARG;
+    }
+    // the carry copies within a row: a history longer than the batch would overlap its own source
+    if (hist > s->batch) {
+        set_error("stream channel filter: its history of %d samples is longer than the batch (%lld)", hist,
+                  (long long) s->batch);
+        return B200_ERR_ARG;
+    }
+    float* d_taps = nullptr;
+    if (n_taps > 0) {
+        B200_CUDA_TRY(cudaMalloc((void**) &d_taps, sizeof(float) * (size_t) n_taps));
+        if (cudaMemcpy(d_taps, h_taps, sizeof(float) * (size_t) n_taps, cudaMemcpyHostToDevice) != cudaSuccess) {
+            set_error("stream channel filter: upload failed: %s", cudaGetErrorString(cudaGetLastError()));
+            cudaFree(d_taps);
+            return B200_ERR_CUDA;
+        }
+    }
+    if (hist != s->hist) {        // rows with the new history; nothing has been pushed, so nothing in them is kept
+        const int64_t row_bytes = 2 * ((int64_t) hist + s->batch);
+        uint8_t* rows = nullptr;
+        if (cudaMalloc(&rows, (size_t) s->n_streams * (size_t) row_bytes) != cudaSuccess) {
+            set_error("stream channel filter: row allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
+            if (d_taps) cudaFree(d_taps);
+            return B200_ERR_CUDA;
+        }
+        if (int rc = launch_iq_history_reset(rows + 2 * (size_t) hist, row_bytes, s->n_streams, hist, s->lanes[0])) {
+            cudaFree(rows);
+            if (d_taps) cudaFree(d_taps);
+            return rc;
+        }
+        if (cudaStreamSynchronize(s->lanes[0]) != cudaSuccess) {
+            set_error("stream channel filter: history reset failed: %s", cudaGetErrorString(cudaGetLastError()));
+            cudaFree(rows);
+            if (d_taps) cudaFree(d_taps);
+            return B200_ERR_CUDA;
+        }
+        cudaFree(s->d_rows);
+        s->d_rows = rows;
+        s->row_bytes = row_bytes;
+        s->hist = hist;
+    }
+    if (s->d_taps) cudaFree(s->d_taps);
+    s->d_taps = d_taps;
+    s->n_taps = n_taps;
     return B200_OK;
 }
 

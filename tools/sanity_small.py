@@ -41,11 +41,16 @@ inc = torch.tensor([[0, pkg.fm_channel_tune(200e3, 2.048e6), pkg.fm_channel_tune
                    dtype=torch.int32, device="cuda")
 pkg.fm_channels_exec(ring, inc, 0, baseband=True)
 pkg.fm_channels_exec(r7, inc[:2, :2].contiguous(), 4 * 7 * 10, baseband=True)
+# the runs-table form (boxcar and FIR) and channels on the push stream
+pkg.fm_channels_exec_runs(ring, [(0, 0, [1, 2, 3]), (2, 40 * 9, [5])])
+fr = pkg.StreamRing(2, 5120, history=pkg.fm_channels_fir_history_samples(10, 40))
+pkg.fm_channels_exec_runs(fr, [(1, 0, [7, 8])], taps=torch.ones(40, dtype=torch.float32, device="cuda"))
 sess = pkg.Session(3, n)
 hdb = np.empty((3, n // 1024, 1024), np.float32)
 hau = np.empty((3, n // 40), np.float32)
 sess.chain(np.ascontiguousarray(iq), n, hdb, hau)
-ps = pkg.PushStream(2, 5120 * 2)
+ps = pkg.PushStream(2, 5120 * 2, channel_capacity=2)
+ps.set_channels(1, [0, pkg.fm_channel_tune(200e3, 2.048e6)], [4, 5])
 for s in range(2):
     ps.push(s, iq[s])
 ps.flush()
