@@ -153,7 +153,8 @@ int b200_fm_channel_tune(double offset_hz, double sample_rate_hz, uint32_t* phas
    d_phase_inc: device [n_streams][n_channels]; d_audio row s*n_channels + c (audio_stride floats apart);
    d_baseband (nullable): float (re, im) pairs, row s*n_channels + c, n_samples/R per row, baseband_stride in complex samples.
    n_channels in [1, B200_FM_MAX_CHANNELS], R in [1, 256], n_samples a multiple of 4R and of 8.  Arguments are checked
-   before anything is launched: B200_ERR_ARG for counts, R, first_sample, n_samples or NULL pointers, B200_ERR_ALIGN for
+   before anything is launched: B200_ERR_ARG for counts, R, first_sample, n_samples, NULL pointers, or an audio_stride
+   below n_samples/(4R) or a baseband_stride below n_samples/R (the rows would overlap), B200_ERR_ALIGN for
    an IQ pointer or stride that is not 16-byte aligned (or d_audio / d_phase_inc not 4-, d_baseband not 8-byte aligned).
    The audio rows are [n_streams * n_channels][...], so b200_wire_audio_messages turns them into websocket audio
    messages with n_streams * n_channels rows, one per listener; no other wire call is needed. */
@@ -172,8 +173,8 @@ int b200_fm_channels_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int 
  * d_taps: T floats on the device, 4-byte aligned, shared by every channel and stream of the call.  T in
  * [1, B200_FM_MAX_CHANNEL_TAPS]; every other argument as b200_fm_channels_exec, and every argument is checked before
  * anything is launched (B200_ERR_ARG for T out of range or NULL d_taps, B200_ERR_ALIGN for a misaligned d_taps).
- * Shared memory: a (R, T) pair that does not fit in a CTA is refused with B200_ERR_ARG; every R in [1, 256] fits
- * with T = 1024 (the largest, R = 256, uses 159 KB for one channel at a time, 212 KB for four).
+ * Shared memory: every R in [1, 256] fits with every T up to 1024 (the largest, R = 256 with T = 1024, uses 159 KB for
+ * one channel at a time, 212 KB for four).
  * Cost: T taps per decimated sample and channel instead of R (DESIGN.md 4.3b has the measured rates).
  * Taps from b200_fm_channel_filter_design keep the boxcar's DC gain R, so the baseband keeps the scale the
  * demodulator's range assumptions were checked at; any other real taps may be passed.  A signal outside +-fs/2 of
@@ -384,8 +385,8 @@ int64_t b200_stream_pending_samples(const b200_stream* s, int stream);   /* buff
  * what an always-present channel at that offset gives from batch b on.
  * b200_stream_set_channel_filter: the FIR channel filter of b200_fm_channels_exec_fir for every channel of the stream
  * (h_taps: n_taps host floats, n_taps = 0 goes back to the boxcar); only before anything is pushed.  The dongle rows
- * get the history b200_fm_channels_fir_history_samples(R, n_taps); B200_ERR_ARG if that exceeds batch_samples or the
- * (R, n_taps) pair does not fit.  Spectra, payloads and centre audio do not change. */
+ * get the history b200_fm_channels_fir_history_samples(R, n_taps); B200_ERR_ARG if that exceeds batch_samples or
+ * n_taps is outside [0, B200_FM_MAX_CHANNEL_TAPS].  Spectra, payloads and centre audio do not change. */
 typedef void (*b200_channel_audio_sink)(void* user, int stream, int32_t channel_id, int64_t first_sample, int n,
                                         const float* audio);
 int b200_stream_set_channel_sink(b200_stream* s, int max_channels, b200_channel_audio_sink sink);

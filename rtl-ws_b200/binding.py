@@ -395,12 +395,28 @@ def fm_channels_fir_history_samples(R: int, n_taps: int) -> int:
     return h
 
 
+def _channel_taps(ring: StreamRing, taps, what: str) -> int:
+    """The tap count of an FIR channel filter (0 for the boxcar), after refusing a ring whose history is too short
+    for it: the kernel would read before the rows."""
+    if taps is None:
+        return 0
+    torch = _torch()
+    assert taps.is_cuda and taps.dtype == torch.float32 and taps.dim() == 1 and taps.is_contiguous()
+    T = taps.shape[0]
+    need = fm_channels_fir_history_samples(ring.R, T)
+    if ring.hist < need:
+        raise B200Error(f"{what}: {T} taps at R = {ring.R} need a ring history of {need} samples, the ring has "
+                        f"{ring.hist}")
+    return T
+
+
 def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None, baseband: bool = False, stream=None,
                      taps=None):
     """b200_fm_channels_exec over a StreamRing: phase_inc is a cuda int32 tensor [n_streams, n_channels] holding the
     uint32 increments' bits; first_sample is the absolute index of the batch's first sample (a multiple of 4R).
     taps (a cuda float32 tensor [T]) selects b200_fm_channels_exec_fir, whose ring needs the longer history of
-    fm_channels_fir_history_samples(R, T).
+    fm_channels_fir_history_samples(R, T).  A given audio must be float32 [S, C, n/(4R)] on the ring's device, its
+    rows may be slices of wider rows.
     -> (audio [S, C, n/(4R)] f32, baseband [S, C, n/R, 2] f32 | None)."""
     torch = _torch()
     assert phase_inc.is_cuda and phase_inc.dtype == torch.int32 and phase_inc.dim() == 2
@@ -409,29 +425,19 @@ def fm_channels_exec(ring: StreamRing, phase_inc, first_sample: int, audio=None,
     n_audio = ring.n_samples // (4 * ring.R)
     if audio is None:
         audio = torch.empty((S, Ch, n_audio), dtype=torch.float32, device=ring.buf.device)
-    assert audio.shape == (S, Ch, n_audio) and audio.stride(2) == 1 and audio.stride(0) == Ch * audio.stride(1)
+    _check_output("fm_channels_exec audio", audio, torch.float32, (S, Ch, n_audio), ring.buf.device, row_slices=True)
     bb = None
     if baseband:
         bb = torch.empty((S, Ch, ring.n_samples // ring.R, 2), dtype=torch.float32, device=ring.buf.device)
-    if taps is not None:
-        assert taps.is_cuda and taps.dtype == torch.float32 and taps.dim() == 1 and taps.is_contiguous()
-        need = fm_channels_fir_history_samples(ring.R, taps.shape[0])
-        if ring.hist < need:          # the kernel would read before the rows: refuse before anything is launched
-            raise B200Error(f"fm_channels_exec: {taps.shape[0]} taps at R = {ring.R} need a ring history of {need} "
-                            f"samples, the ring has {ring.hist}")
-        _check(lib().b200_fm_channels_exec_fir(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
-                                               ring.n_samples, ring.R, first_sample, C.c_void_p(phase_inc.data_ptr()),
-                                               Ch, C.c_void_p(audio.data_ptr()), audio.stride(1),
-                                               C.c_void_p(bb.data_ptr()) if bb is not None else None,
-                                               bb.stride(1) // 2 if bb is not None else 0, C.c_void_p(taps.data_ptr()),
-                                               taps.shape[0], _stream_ptr(stream)), "b200_fm_channels_exec_fir")
-        return audio, bb
-    _check(lib().b200_fm_channels_exec(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
-                                       ring.n_samples, ring.R, first_sample, C.c_void_p(phase_inc.data_ptr()), Ch,
-                                       C.c_void_p(audio.data_ptr()), audio.stride(1),
-                                       C.c_void_p(bb.data_ptr()) if bb is not None else None,
-                                       bb.stride(1) // 2 if bb is not None else 0, _stream_ptr(stream)),
-           "b200_fm_channels_exec")
+    T = _channel_taps(ring, taps, "fm_channels_exec")
+    args = (C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams, ring.n_samples, ring.R, first_sample,
+            C.c_void_p(phase_inc.data_ptr()), Ch, C.c_void_p(audio.data_ptr()), audio.stride(1),
+            C.c_void_p(bb.data_ptr()) if bb is not None else None, bb.stride(1) // 2 if bb is not None else 0)
+    if T:
+        _check(lib().b200_fm_channels_exec_fir(*args, C.c_void_p(taps.data_ptr()), T, _stream_ptr(stream)),
+               "b200_fm_channels_exec_fir")
+    else:
+        _check(lib().b200_fm_channels_exec(*args, _stream_ptr(stream)), "b200_fm_channels_exec")
     return audio, bb
 
 
@@ -455,14 +461,7 @@ def fm_channels_exec_runs(ring: StreamRing, runs, audio=None, taps=None, stream=
         audio = torch.empty((max(row, 1), n_audio), dtype=torch.float32, device=ring.buf.device)
     _check_output("fm_channels_exec_runs audio", audio, torch.float32, (max(row, 1), n_audio), ring.buf.device,
                   row_slices=True)
-    T = 0
-    if taps is not None:
-        assert taps.is_cuda and taps.dtype == torch.float32 and taps.dim() == 1 and taps.is_contiguous()
-        T = taps.shape[0]
-        need = fm_channels_fir_history_samples(ring.R, T)
-        if ring.hist < need:          # the kernel would read before the rows: refuse before anything is launched
-            raise B200Error(f"fm_channels_exec_runs: {T} taps at R = {ring.R} need a ring history of {need} "
-                            f"samples, the ring has {ring.hist}")
+    T = _channel_taps(ring, taps, "fm_channels_exec_runs")
     _check(lib().b200_fm_channels_exec_runs(C.c_void_p(ring.batch.data_ptr()), ring.stride_bytes, ring.n_streams,
                                             ring.n_samples, ring.R, table, len(runs), C.c_void_p(audio.data_ptr()),
                                             audio.stride(0), audio.shape[0],
@@ -473,8 +472,10 @@ def fm_channels_exec_runs(ring: StreamRing, runs, audio=None, taps=None, stream=
 
 def _check_output(what: str, t, dtype, shape: tuple, device, row_slices: bool = False) -> None:
     """Refuse an output tensor the kernels would write past: they see only its data pointer (and row stride).
-    row_slices: rows may be slices of wider rows (unit column stride); otherwise the tensor must be contiguous."""
-    layout_ok = t.stride(-1) == 1 if row_slices else t.is_contiguous()
+    row_slices: rows (the last dimension) may be slices of wider rows, with unit column stride, and the leading
+    dimensions pack them one row stride apart; otherwise the tensor must be contiguous."""
+    packed = all(t.stride(d) == t.shape[d + 1] * t.stride(d + 1) for d in range(t.dim() - 2))
+    layout_ok = t.stride(-1) == 1 and packed if row_slices else t.is_contiguous()
     if t.dtype != dtype or tuple(t.shape) != shape or not layout_ok or t.device != device:
         raise B200Error(f"{what}: want {dtype} {shape} {'with unit column stride' if row_slices else 'contiguous'} "
                         f"on {device}, got {t.dtype} {tuple(t.shape)} strides {t.stride()} on {t.device}")

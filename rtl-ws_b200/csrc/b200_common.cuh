@@ -1,5 +1,6 @@
 // b200_common.cuh -- shared device helpers (sm_100a): mbarrier + 1-D bulk TMA copies,
-// error plumbing.  No CPU fallback anywhere: a failed CUDA call surfaces as B200_ERR_CUDA.
+// error plumbing, and the one declaration of each internal host launcher and helper.
+// No CPU fallback anywhere: a failed CUDA call surfaces as B200_ERR_CUDA.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -42,6 +43,55 @@ int cached_occupancy(const void* kernel, int block_threads, int smem_bytes);
             return B200_ERR_CUDA;                                                        \
         }                                                                                \
     } while (0)
+
+// ---- host-side launchers and helpers, each implemented next to its kernels ---------------
+struct SpecParams;
+struct Spec64kExtra;
+struct FmParams;
+
+int launch_spectrum1024(const SpecParams& p, cudaStream_t stream);
+int launch_spectrum2048(const SpecParams& p, cudaStream_t stream);
+int launch_spectrum4096(const SpecParams& p, cudaStream_t stream);
+int launch_spectrum_mx1024(const SpecParams& p, cudaStream_t stream);
+int launch_spectrum64k(const SpecParams& p, const Spec64kExtra& x, int N, cudaStream_t stream);
+int launch_spectrum_generic(const SpecParams& p, int N, int kind, float2* scratch, float* acc_scratch, int scratch_ctas,
+                            cudaStream_t stream);
+int spectrum_generic_scratch_ctas();
+// the two fields of the (capi.cu-private) plan layout the fused chain launch needs
+const float2* spectrum_plan_twiddle(const b200_spectrum_plan* plan);
+float spectrum_plan_db_offset(const b200_spectrum_plan* plan);
+int launch_chain_fused(const uint8_t* d_iq, int64_t stride, int n_streams, int64_t n_samples, float db_offset,
+                       const float2* twiddle, float* d_db, float* d_audio, int64_t audio_stride, cudaStream_t stream);
+
+int launch_fm_chain(const FmParams& p, cudaStream_t stream);
+int fm_history_samples(int R);
+int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
+int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
+int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
+                            cudaStream_t stream);
+int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
+
+// FM channels: taps NULL with T = 0 is the boxcar, else T in [1, B200_FM_MAX_CHANNEL_TAPS] device taps
+int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                       int64_t first_sample, const uint32_t* phase_inc, int n_channels, float* audio,
+                       int64_t audio_stride, float* baseband, int64_t baseband_stride, const float* taps, int T,
+                       cudaStream_t stream);
+int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
+                            const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
+                            int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream);
+int fm_channels_fir_history_samples(int R, int T);
+int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h);
+// The channel filter of a block of n_rows [history | batch] rows at stream position 0, whose earlier work has all
+// finished: n_taps host taps (0 = the boxcar) replace d_taps / taps_count, and when the filter needs another history,
+// new rows with it, reset on `stream`, replace rows / row_bytes / hist.  On failure nothing changes.
+int set_channel_filter(const char* who, int R, int n_rows, int64_t max_batch, const float* h_taps, int n_taps,
+                       cudaStream_t stream, float*& d_taps, int& taps_count, uint8_t*& rows, int64_t& row_bytes,
+                       int& hist);
+
+// chain.cu: one batch of a host-buffer session, submitted without waiting (multi.cu drives one session per device)
+int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_bytes, int64_t n_samples, int gain_db,
+                         float* h_db, int64_t db_pitch, float* h_audio, int64_t audio_pitch, uint8_t* d_avg_u8, int K_avg);
+int session_wait(b200_session* s);
 
 // ---- device: mbarrier + bulk async copy (TMA, 1-D) -------------------------------------
 #ifdef __CUDACC__

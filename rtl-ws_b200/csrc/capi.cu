@@ -75,35 +75,6 @@ int cached_occupancy(const void* kernel, int block_threads, int smem_bytes)
     return n;
 }
 
-// launchers implemented next to their kernels
-int launch_spectrum1024(const SpecParams& p, cudaStream_t stream);
-int launch_spectrum_generic(const SpecParams& p, int N, int kind, float2* scratch, float* acc_scratch, int scratch_ctas,
-                            cudaStream_t stream);
-int spectrum_generic_scratch_ctas();
-int launch_spectrum4096(const SpecParams& p, cudaStream_t stream);
-int launch_spectrum2048(const SpecParams& p, cudaStream_t stream);
-int launch_spectrum_mx1024(const SpecParams& p, cudaStream_t stream);
-int launch_spectrum64k(const SpecParams& p, const Spec64kExtra& x, int N, cudaStream_t stream);
-int launch_fm_chain(const FmParams& p, cudaStream_t stream);
-int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
-int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
-int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
-                            cudaStream_t stream);
-int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
-int fm_history_samples(int R);
-int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
-                       int64_t first_sample, const uint32_t* phase_inc, int n_channels, float* audio,
-                       int64_t audio_stride, float* baseband, int64_t baseband_stride, cudaStream_t stream);
-int launch_fm_channels_fir(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
-                           int64_t first_sample, const uint32_t* phase_inc, int n_channels, const float* taps, int T,
-                           float* audio, int64_t audio_stride, float* baseband, int64_t baseband_stride,
-                           cudaStream_t stream);
-int fm_channels_fir_history_samples(int R, int T);
-int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
-                            const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
-                            int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream);
-int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h);
-
 }  // namespace b200
 
 using namespace b200;
@@ -134,6 +105,9 @@ struct b200_spectrum_plan {
     float* gen_acc;                // [gen_ctas][N]
     int gen_ctas;
 };
+
+const float2* b200::spectrum_plan_twiddle(const b200_spectrum_plan* plan) { return plan->d_twiddle; }
+float b200::spectrum_plan_db_offset(const b200_spectrum_plan* plan) { return plan->db_offset; }
 
 // Run `launch` (which enqueues a kernel using the plan's scratch on `stream`) after every earlier user of the scratch.
 template <class F>
@@ -336,10 +310,6 @@ void b200_spectrum_plan_destroy(b200_spectrum_plan* plan)
     if (plan->scratch_done) cudaEventDestroy(plan->scratch_done);
     delete plan;
 }
-
-// private accessors for chain.cu (not declared in the public header)
-const void* b200_spectrum_plan_twiddle_(const b200_spectrum_plan* plan) { return plan->d_twiddle; }
-float b200_spectrum_plan_db_offset_(const b200_spectrum_plan* plan) { return plan->db_offset; }
 
 int64_t b200_spectrum_plan_rows(const b200_spectrum_plan* plan, int64_t n_samples)
 {
@@ -544,7 +514,7 @@ int b200_fm_channels_exec(const uint8_t* d_iq, int64_t stream_stride_bytes, int 
                           int64_t audio_stride, float* d_baseband, int64_t baseband_stride, void* cuda_stream)
 {
     return launch_fm_channels(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
-                              n_channels, d_audio, audio_stride, d_baseband, baseband_stride,
+                              n_channels, d_audio, audio_stride, d_baseband, baseband_stride, nullptr, 0,
                               reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
@@ -566,9 +536,13 @@ int b200_fm_channels_exec_fir(const uint8_t* d_iq, int64_t stream_stride_bytes, 
                               int64_t audio_stride, float* d_baseband, int64_t baseband_stride, const float* d_taps,
                               int n_taps, void* cuda_stream)
 {
-    return launch_fm_channels_fir(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
-                                  n_channels, d_taps, n_taps, d_audio, audio_stride, d_baseband, baseband_stride,
-                                  reinterpret_cast<cudaStream_t>(cuda_stream));
+    if (d_taps == nullptr && n_taps == 0) {        // launch_fm_channels would take it for the boxcar
+        set_error("fm channels fir: no taps");
+        return B200_ERR_ARG;
+    }
+    return launch_fm_channels(d_iq, stream_stride_bytes, n_streams, n_samples, R, first_sample, d_phase_inc,
+                              n_channels, d_audio, audio_stride, d_baseband, baseband_stride, d_taps, n_taps,
+                              reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 int b200_fm_channels_exec_runs(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,

@@ -7,18 +7,6 @@
 #include "fm_kernels.cuh"
 #include "spectrum_kernels.cuh"
 
-namespace b200 {
-int launch_chain_fused(const uint8_t* d_iq, int64_t stride, int n_streams, int64_t n_samples, float db_offset,
-                       const float2* twiddle, float* d_db, float* d_audio, int64_t audio_stride, cudaStream_t stream);
-int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
-int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
-int fm_history_samples(int R);
-int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
-                            cudaStream_t stream);
-int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
-int fm_channels_fir_history_samples(int R, int T);
-}  // namespace b200
-
 using namespace b200;
 
 namespace {
@@ -58,10 +46,6 @@ b200_spectrum_plan* cached_plan(int K, int gain_db)
 }
 
 }  // namespace
-
-// layout of b200_spectrum_plan is private to capi.cu; the fused launcher needs two fields
-extern "C" const void* b200_spectrum_plan_twiddle_(const b200_spectrum_plan* plan);
-extern "C" float b200_spectrum_plan_db_offset_(const b200_spectrum_plan* plan);
 
 extern "C" {
 
@@ -114,9 +98,8 @@ int b200_chain_exec_r(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_st
 
     int rc;
     if (d_db != nullptr && d_audio != nullptr && R == CHAIN_R) {      // one pass over the IQ (chain_fused.cu)
-        rc = launch_chain_fused(d_iq, stream_stride_bytes, n_streams, n_samples, b200_spectrum_plan_db_offset_(pl),
-                                reinterpret_cast<const float2*>(b200_spectrum_plan_twiddle_(pl)), d_db, d_audio,
-                                audio_stride, stream);
+        rc = launch_chain_fused(d_iq, stream_stride_bytes, n_streams, n_samples, spectrum_plan_db_offset(pl),
+                                spectrum_plan_twiddle(pl), d_db, d_audio, audio_stride, stream);
         if (rc) return rc;
     } else {
         if (d_db != nullptr) {
@@ -363,8 +346,8 @@ int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_sample
 
 int b200_session_set_channel_filter(b200_session* s, const float* h_taps, int n_taps)
 {
-    if (s == nullptr || n_taps < 0 || n_taps > B200_FM_MAX_CHANNEL_TAPS || (n_taps > 0 && h_taps == nullptr)) {
-        set_error("session channel filter: bad arguments (%d taps)", n_taps);
+    if (s == nullptr) {
+        set_error("session channel filter: null session");
         return B200_ERR_ARG;
     }
     if (s->position != 0) {
@@ -372,42 +355,9 @@ int b200_session_set_channel_filter(b200_session* s, const float* h_taps, int n_
                   "not at %lld", (long long) s->position);
         return B200_ERR_ARG;
     }
-    const int hist = n_taps > 0 ? fm_channels_fir_history_samples(s->R, n_taps) : fm_history_samples(s->R);
-    if (hist > s->max_samples) {
-        set_error("session channel filter: its history of %d samples is longer than the largest batch (%lld)", hist,
-                  (long long) s->max_samples);
-        return B200_ERR_ARG;
-    }
     // every earlier call has finished: the session calls wait for their work
-    float* d_taps = nullptr;
-    if (n_taps > 0) {
-        B200_CUDA_TRY(cudaMalloc((void**) &d_taps, sizeof(float) * (size_t) n_taps));
-        if (cudaMemcpyAsync(d_taps, h_taps, sizeof(float) * (size_t) n_taps, cudaMemcpyHostToDevice, s->streams[0]) !=
-                cudaSuccess ||
-            cudaStreamSynchronize(s->streams[0]) != cudaSuccess) {
-            set_error("session channel filter: upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-            cudaFree(d_taps);
-            return B200_ERR_CUDA;
-        }
-    }
-    if (hist != s->hist_samples) {        // a ring with the new history; position 0, so nothing in it is kept
-        const int64_t stride = 2 * ((int64_t) hist + s->max_samples);
-        uint8_t* ring = nullptr;
-        if (cudaMalloc(&ring, (size_t) s->n_streams * (size_t) stride) != cudaSuccess) {
-            set_error("session channel filter: ring allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
-            if (d_taps) cudaFree(d_taps);
-            return B200_ERR_CUDA;
-        }
-        cudaFree(s->d_ring);
-        s->d_ring = ring;
-        s->stride_bytes = stride;
-        s->hist_samples = hist;
-        b200_session_reset(s);
-    }
-    if (s->d_taps) cudaFree(s->d_taps);
-    s->d_taps = d_taps;
-    s->n_taps = n_taps;
-    return B200_OK;
+    return set_channel_filter("session channel filter", s->R, s->n_streams, s->max_samples, h_taps, n_taps,
+                              s->streams[0], s->d_taps, s->n_taps, s->d_ring, s->stride_bytes, s->hist_samples);
 }
 
 int b200_session_chain(b200_session* s, const uint8_t* h_iq, int64_t n_samples, int gain_db, float* h_db,

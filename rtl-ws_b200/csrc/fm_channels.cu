@@ -199,14 +199,15 @@ __global__ void __launch_bounds__(FC_THREADS) fm_channels_runs_kernel(const __gr
     fm_channels_tiles<RT, G, true>(p, tiles_per_stream, stage_bytes, n_stages);
 }
 
-template <int RT, int G>
-int launch_fc(const FcParams& p, int64_t tps, cudaStream_t stream)
+// One launch of fm_channels_kernel or fm_channels_runs_kernel at G channels per group; p.n_streams counts IQ rows or
+// runs
+template <class P>
+int launch_fc(void (*kern)(P, int, int, int), int G, const P& p, int64_t tps, cudaStream_t stream)
 {
     const int R = p.R;
     const int stage_bytes = FC_ND * 2 * R;
     const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;      // R <= 109 double-buffers; up to R = 256 one stage
     const int smem = n_stages * stage_bytes + G * R * 16 + G * (FC_DEMOD + FC_WORK) * 4 + 16;
-    auto kern = fm_channels_kernel<RT, G>;
     if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
     const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
     int64_t grid = (int64_t) sm_count() * per_sm;
@@ -217,22 +218,46 @@ int launch_fc(const FcParams& p, int64_t tps, cudaStream_t stream)
     return B200_OK;
 }
 
-// the same geometry as launch_fc; p.n_streams counts runs
-template <int RT, int G>
-int launch_fc_runs(const FcRunsParams& p, int64_t tps, cudaStream_t stream)
+// The checks the uniform and the runs calls share.  n_rows counts IQ rows (uniform) or runs: with the tiles per
+// stream, returned in *tps, it bounds the launch's tile count.
+int check_channel_args(const char* who, const uint8_t* iq, int64_t stream_stride_bytes, int n_rows, int64_t n_samples,
+                       int R, const float* audio, int64_t audio_stride, const float* taps, int T, int64_t* tps)
 {
-    const int R = p.R;
-    const int stage_bytes = FC_ND * 2 * R;
-    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;
-    const int smem = n_stages * stage_bytes + G * R * 16 + G * (FC_DEMOD + FC_WORK) * 4 + 16;
-    auto kern = fm_channels_runs_kernel<RT, G>;
-    if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
-    const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
-    int64_t grid = (int64_t) sm_count() * per_sm;
-    const int64_t total = (int64_t) p.n_streams * tps;
-    if (grid > total) grid = total;
-    kern<<<(unsigned) grid, FC_THREADS, smem, stream>>>(p, (int) tps, stage_bytes, n_stages);
-    B200_LAUNCH_CHECK();
+    if (iq == nullptr || audio == nullptr) {
+        set_error("%s: null IQ or audio pointer", who);
+        return B200_ERR_ARG;
+    }
+    if (R < 1 || R > 256) {
+        set_error("%s: down factor %d outside [1, 256]", who, R);
+        return B200_ERR_ARG;
+    }
+    if (n_samples < 0 || n_samples % (4 * R) != 0 || n_samples % 8 != 0) {
+        set_error("%s: n_samples %lld must be a multiple of 4*R and of 8", who, (long long) n_samples);
+        return B200_ERR_ARG;
+    }
+    if ((taps != nullptr || T != 0) && (taps == nullptr || T < 1 || T > B200_FM_MAX_CHANNEL_TAPS)) {
+        set_error("%s: %d taps: want NULL taps and 0 (boxcar) or [1, %d] device taps", who, T, B200_FM_MAX_CHANNEL_TAPS);
+        return B200_ERR_ARG;
+    }
+    const int64_t n_audio = n_samples / (4 * R);
+    if (audio_stride < n_audio) {       // overlapping rows would race
+        set_error("%s: audio rows %lld floats apart for %lld samples a row", who, (long long) audio_stride,
+                  (long long) n_audio);
+        return B200_ERR_ARG;
+    }
+    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
+        set_error("%s: IQ pointer and stream stride must be 16-byte aligned", who);
+        return B200_ERR_ALIGN;
+    }
+    if ((reinterpret_cast<uintptr_t>(audio) & 3) != 0 || (reinterpret_cast<uintptr_t>(taps) & 3) != 0) {
+        set_error("%s: audio and taps must be 4-byte aligned", who);
+        return B200_ERR_ALIGN;
+    }
+    *tps = (n_audio + FC_T - 1) / FC_T;
+    if ((int64_t) n_rows * *tps >= (1ll << 31)) {
+        set_error("%s: batch too long", who);
+        return B200_ERR_ARG;
+    }
     return B200_OK;
 }
 
@@ -242,41 +267,14 @@ int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int 
                             const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
                             int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream)
 {
-    if (iq == nullptr || audio == nullptr || runs == nullptr || n_streams < 1) {
-        set_error("fm channels runs: null pointer or no IQ rows");
+    int64_t tps;
+    if (int rc = check_channel_args("fm channels runs", iq, stream_stride_bytes, n_runs, n_samples, R, audio,
+                                    audio_stride, taps, T, &tps))
+        return rc;
+    if (runs == nullptr || n_streams < 1 || n_runs < 1 || n_runs > B200_FM_MAX_RUNS || n_audio_rows < 1) {
+        set_error("fm channels runs: %d runs (table %p) over %d IQ rows, %lld audio rows; want [1, %d] runs, at least one "
+                  "row of each", n_runs, (const void*) runs, n_streams, (long long) n_audio_rows, B200_FM_MAX_RUNS);
         return B200_ERR_ARG;
-    }
-    if (n_runs < 1 || n_runs > B200_FM_MAX_RUNS) {
-        set_error("fm channels runs: n_runs %d outside [1, %d]", n_runs, B200_FM_MAX_RUNS);
-        return B200_ERR_ARG;
-    }
-    if (R < 1 || R > 256) {
-        set_error("fm channels runs: down factor %d outside [1, 256]", R);
-        return B200_ERR_ARG;
-    }
-    if (n_samples < 0 || n_samples % (4 * R) != 0 || n_samples % 8 != 0) {
-        set_error("fm channels runs: n_samples %lld must be a multiple of 4*R and of 8", (long long) n_samples);
-        return B200_ERR_ARG;
-    }
-    const int64_t n_audio = n_samples / (4 * R);
-    if (n_audio_rows < 1 || audio_stride < n_audio) {
-        set_error("fm channels runs: %lld audio rows %lld floats apart for %lld samples a row", (long long) n_audio_rows,
-                  (long long) audio_stride, (long long) n_audio);
-        return B200_ERR_ARG;
-    }
-    const bool fir = taps != nullptr || T != 0;
-    if (fir && (taps == nullptr || T < 1 || T > B200_FM_MAX_CHANNEL_TAPS)) {
-        set_error("fm channels runs: %d taps: want NULL taps and 0 (boxcar) or [1, %d] device taps", T,
-                  B200_FM_MAX_CHANNEL_TAPS);
-        return B200_ERR_ARG;
-    }
-    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
-        set_error("fm channels runs: IQ pointer and stream stride must be 16-byte aligned");
-        return B200_ERR_ALIGN;
-    }
-    if ((reinterpret_cast<uintptr_t>(audio) & 3) != 0 || (reinterpret_cast<uintptr_t>(taps) & 3) != 0) {
-        set_error("fm channels runs: audio and taps must be 4-byte aligned");
-        return B200_ERR_ALIGN;
     }
     int max_c = 0;
     for (int k = 0; k < n_runs; ++k) {
@@ -297,15 +295,6 @@ int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int 
             }
         if (r.n_channels > max_c) max_c = r.n_channels;
     }
-    if (fir && !fm_channels_fir_fits(R, T)) {
-        set_error("fm channels runs: R = %d with %d taps does not fit in shared memory", R, T);
-        return B200_ERR_ARG;
-    }
-    const int64_t tps = (n_audio + FC_T - 1) / FC_T;
-    if ((int64_t) n_runs * tps >= (1ll << 31)) {
-        set_error("fm channels runs: batch too long");
-        return B200_ERR_ARG;
-    }
     if (n_samples == 0) return B200_OK;
     FcRunsParams p;
     memset(&p, 0, sizeof(p));
@@ -324,50 +313,42 @@ int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int 
         r.audio_row = runs[k].audio_row;
         memcpy(r.phase_inc, runs[k].phase_inc, sizeof(r.phase_inc));
     }
-    if (fir) return launch_fm_channels_fir_runs(p, tps, taps, T, max_c, stream);
-    if (R == 10) return launch_fc_runs<10, 8>(p, tps, stream);
-    return launch_fc_runs<0, 4>(p, tps, stream);
+    if (taps != nullptr) return launch_fm_channels_fir_runs(p, tps, taps, T, max_c, stream);
+    if (R == 10) return launch_fc(fm_channels_runs_kernel<10, 8>, 8, p, tps, stream);
+    return launch_fc(fm_channels_runs_kernel<0, 4>, 4, p, tps, stream);
 }
 
 int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
                        int64_t first_sample, const uint32_t* phase_inc, int n_channels, float* audio,
-                       int64_t audio_stride, float* baseband, int64_t baseband_stride, cudaStream_t stream)
+                       int64_t audio_stride, float* baseband, int64_t baseband_stride, const float* taps, int T,
+                       cudaStream_t stream)
 {
-    if (n_streams < 0 || iq == nullptr || phase_inc == nullptr || audio == nullptr) {
-        set_error("fm channels: null pointer or negative stream count");
+    int64_t tps;
+    if (int rc = check_channel_args("fm channels", iq, stream_stride_bytes, n_streams, n_samples, R, audio,
+                                    audio_stride, taps, T, &tps))
+        return rc;
+    if (n_streams < 0 || phase_inc == nullptr) {
+        set_error("fm channels: null phase increments or negative stream count");
         return B200_ERR_ARG;
     }
     if (n_channels < 1 || n_channels > B200_FM_MAX_CHANNELS) {
         set_error("fm channels: n_channels %d outside [1, %d]", n_channels, B200_FM_MAX_CHANNELS);
         return B200_ERR_ARG;
     }
-    if (R < 1 || R > 256) {
-        set_error("fm channels: down factor %d outside [1, 256]", R);
-        return B200_ERR_ARG;
-    }
-    if (n_samples < 0 || n_samples % (4 * R) != 0 || n_samples % 8 != 0) {
-        set_error("fm channels: n_samples %lld must be a multiple of 4*R and of 8", (long long) n_samples);
-        return B200_ERR_ARG;
-    }
     if (first_sample < 0 || first_sample % (4 * R) != 0) {
         set_error("fm channels: first_sample %lld must be a non-negative multiple of 4*R", (long long) first_sample);
         return B200_ERR_ARG;
     }
-    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
-        set_error("fm channels: IQ pointer and stream stride must be 16-byte aligned");
-        return B200_ERR_ALIGN;
+    if (baseband != nullptr && baseband_stride < n_samples / R) {      // overlapping rows would race
+        set_error("fm channels: baseband rows %lld samples apart for %lld samples a row", (long long) baseband_stride,
+                  (long long) (n_samples / R));
+        return B200_ERR_ARG;
     }
-    if ((reinterpret_cast<uintptr_t>(phase_inc) & 3) != 0 || (reinterpret_cast<uintptr_t>(audio) & 3) != 0 ||
-        (reinterpret_cast<uintptr_t>(baseband) & 7) != 0) {
-        set_error("fm channels: phase increments and audio must be 4-byte aligned, baseband 8-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(phase_inc) & 3) != 0 || (reinterpret_cast<uintptr_t>(baseband) & 7) != 0) {
+        set_error("fm channels: phase increments must be 4-byte aligned, baseband 8-byte aligned");
         return B200_ERR_ALIGN;
     }
     if (n_streams == 0 || n_samples == 0) return B200_OK;
-    const int64_t tps = (n_samples / (4 * R) + FC_T - 1) / FC_T;
-    if ((int64_t) n_streams * tps >= (1ll << 31)) {
-        set_error("fm channels: batch too long");
-        return B200_ERR_ARG;
-    }
     FcParams p;
     p.iq = iq;
     p.stream_stride_bytes = stream_stride_bytes;
@@ -381,9 +362,10 @@ int launch_fm_channels(const uint8_t* iq, int64_t stream_stride_bytes, int n_str
     p.audio_stride = audio_stride;
     p.baseband = reinterpret_cast<float2*>(baseband);
     p.baseband_stride = baseband_stride;
+    if (taps != nullptr) return launch_fm_channels_fir(p, tps, taps, T, stream);
     // channels per group at R = 10: 8 measured fastest at every channel count (DESIGN.md 4.3a)
-    if (R == 10) return launch_fc<10, 8>(p, tps, stream);
-    return launch_fc<0, 4>(p, tps, stream);
+    if (R == 10) return launch_fc(fm_channels_kernel<10, 8>, 8, p, tps, stream);
+    return launch_fc(fm_channels_kernel<0, 4>, 4, p, tps, stream);
 }
 
 }  // namespace b200

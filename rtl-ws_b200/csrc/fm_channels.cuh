@@ -76,9 +76,10 @@ __device__ __forceinline__ const FcRun* fc_run(const P& p, int q)
     else return nullptr;
 }
 
-// host side: the runs form's FIR launcher (fm_channels_fir.cu), called by launch_fm_channels_runs after the common checks
+// host side: the FIR launchers (fm_channels_fir.cu), called by launch_fm_channels / launch_fm_channels_runs after
+// their checks; T in [1, B200_FM_MAX_CHANNEL_TAPS]
+int launch_fm_channels_fir(const FcParams& p, int64_t tiles_per_stream, const float* taps, int T, cudaStream_t stream);
 int launch_fm_channels_fir_runs(const FcRunsParams& p, int64_t tiles_per_stream, const float* taps, int T,
                                 int max_channels, cudaStream_t stream);
-int fm_channels_fir_fits(int R, int T);
 
 }  // namespace b200

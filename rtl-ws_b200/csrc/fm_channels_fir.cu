@@ -217,67 +217,75 @@ __global__ void __launch_bounds__(FC_THREADS, 3) fm_channels_fir_runs_kernel(con
     fm_channels_fir_tiles<true>(p, tiles_per_stream, stage_bytes, n_stages, G);
 }
 
-int fir_stage_bytes(int R, int T)
+constexpr int fir_stage_bytes(int R, int T)
 {
     const int L = T - R;
     return 2 * (FC_ND * R + L + ((-L) & 7));
 }
 
-int fir_smem_bytes(int stage_bytes, int n_stages, int T, int G)
+constexpr int fir_smem_bytes(int stage_bytes, int n_stages, int T, int G)
 {
     return n_stages * stage_bytes + T * G * 16 + G * (FC_DEMOD + FC_WORK) * 4 + 16;
 }
 
+// One channel per group fits at every R and T: the largest stage (R = 256, T = B200_FM_MAX_CHANNEL_TAPS, 142 KB) is
+// single-buffered, and two stages take at most 120 KB
+static_assert(fir_smem_bytes(fir_stage_bytes(256, B200_FM_MAX_CHANNEL_TAPS), 1, B200_FM_MAX_CHANNEL_TAPS, 1) <=
+                  FIR_SMEM_LIMIT, "the largest FIR channel stage does not fit in shared memory");
+
 // Channels per group for C channels: the fewest groups the shared-memory budget allows (at most FIR_MAX_G
-// channels each), then the channels spread evenly over them.  0 if not even one channel fits.
+// channels each), then the channels spread evenly over them
 int fir_group_size(int stage_bytes, int n_stages, int T, int C)
 {
     int gmax = C < FIR_MAX_G ? C : FIR_MAX_G;
-    while (gmax > 0 && fir_smem_bytes(stage_bytes, n_stages, T, gmax) > FIR_SMEM_LIMIT) --gmax;
-    if (gmax == 0) return 0;
+    while (gmax > 1 && fir_smem_bytes(stage_bytes, n_stages, T, gmax) > FIR_SMEM_LIMIT) --gmax;
     const int groups = (C + gmax - 1) / gmax;
     return (C + groups - 1) / groups;
 }
 
-}  // namespace
-
-int fm_channels_fir_fits(int R, int T)
+// One launch of fm_channels_fir_kernel or fm_channels_fir_runs_kernel: fills the filter fields of p (p.c is set;
+// p.c.n_streams counts IQ rows or runs), G from the largest channel count
+template <class P>
+int launch_fir(void (*kern)(P, int, int, int, int), P& p, int64_t tps, const float* taps, int T, int max_channels,
+               cudaStream_t stream)
 {
-    const int stage_bytes = fir_stage_bytes(R, T);
-    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;
-    return fir_group_size(stage_bytes, n_stages, T, 1) > 0;
-}
-
-// G from the table's largest channel count, with the budget of the uniform call; a run's audio does not depend on
-// G (each channel's MAC, rotation and demodulator are the same whatever group it is computed in)
-int launch_fm_channels_fir_runs(const FcRunsParams& runs, int64_t tps, const float* taps, int T, int max_channels,
-                                cudaStream_t stream)
-{
-    const int R = runs.R;
+    const int R = p.c.R;
     const int stage_bytes = fir_stage_bytes(R, T);
     const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;       // as fm_channels.cu
     const int G = fir_group_size(stage_bytes, n_stages, T, max_channels);
-    if (G == 0) {
-        set_error("fm channels runs: R = %d with %d taps does not fit in shared memory", R, T);
-        return B200_ERR_ARG;
-    }
-    FirRunsParams p;
-    static_cast<FcParams&>(p.c) = static_cast<const FcParams&>(runs);
-    memcpy(p.runs, runs.runs, sizeof(p.runs));
     p.taps = taps;
     p.T = T;
     p.L = T - R;
     p.off = (R - T) & 7;
     const int smem = fir_smem_bytes(stage_bytes, n_stages, T, G);
-    auto kern = fm_channels_fir_runs_kernel;
     if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
     const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
     int64_t grid = (int64_t) sm_count() * per_sm;
-    const int64_t total = (int64_t) runs.n_streams * tps;
+    const int64_t total = (int64_t) p.c.n_streams * tps;
     if (grid > total) grid = total;
     kern<<<(unsigned) grid, FC_THREADS, smem, stream>>>(p, (int) tps, stage_bytes, n_stages, G);
     B200_LAUNCH_CHECK();
     return B200_OK;
+}
+
+}  // namespace
+
+int launch_fm_channels_fir(const FcParams& c, int64_t tps, const float* taps, int T, cudaStream_t stream)
+{
+    FirParams p;
+    p.c = c;
+    return launch_fir(fm_channels_fir_kernel, p, tps, taps, T, c.n_channels, stream);
+}
+
+// a run's audio does not depend on G (each channel's MAC, rotation and demodulator are the same whatever group it is
+// computed in)
+int launch_fm_channels_fir_runs(const FcRunsParams& runs, int64_t tps, const float* taps, int T, int max_channels,
+                                cudaStream_t stream)
+{
+    FirRunsParams p;
+    p.c = runs;
+    memcpy(p.runs, runs.runs, sizeof(p.runs));
+    return launch_fir(fm_channels_fir_runs_kernel, p, tps, taps, T, max_channels, stream);
 }
 
 int fm_channels_fir_history_samples(int R, int T)
@@ -287,83 +295,50 @@ int fm_channels_fir_history_samples(int R, int T)
     return (h + 7) / 8 * 8;
 }
 
-int launch_fm_channels_fir(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
-                           int64_t first_sample, const uint32_t* phase_inc, int n_channels, const float* taps, int T,
-                           float* audio, int64_t audio_stride, float* baseband, int64_t baseband_stride,
-                           cudaStream_t stream)
+int set_channel_filter(const char* who, int R, int n_rows, int64_t max_batch, const float* h_taps, int n_taps,
+                       cudaStream_t stream, float*& d_taps, int& taps_count, uint8_t*& rows, int64_t& row_bytes,
+                       int& hist)
 {
-    if (n_streams < 0 || iq == nullptr || phase_inc == nullptr || audio == nullptr || taps == nullptr) {
-        set_error("fm channels fir: null pointer or negative stream count");
+    if (n_taps < 0 || n_taps > B200_FM_MAX_CHANNEL_TAPS || (n_taps > 0 && h_taps == nullptr)) {
+        set_error("%s: bad arguments (%d taps)", who, n_taps);
         return B200_ERR_ARG;
     }
-    if (n_channels < 1 || n_channels > B200_FM_MAX_CHANNELS) {
-        set_error("fm channels fir: n_channels %d outside [1, %d]", n_channels, B200_FM_MAX_CHANNELS);
+    const int h = n_taps > 0 ? fm_channels_fir_history_samples(R, n_taps) : fm_history_samples(R);
+    // the carry copies within a row: a history longer than the batch would overlap its own source
+    if (h > max_batch) {
+        set_error("%s: its history of %d samples is longer than the batch (%lld)", who, h, (long long) max_batch);
         return B200_ERR_ARG;
     }
-    if (R < 1 || R > 256) {
-        set_error("fm channels fir: down factor %d outside [1, 256]", R);
-        return B200_ERR_ARG;
+    const int64_t stride = 2 * ((int64_t) h + max_batch);
+    float* taps = nullptr;
+    uint8_t* fresh = nullptr;
+    cudaError_t e = cudaSuccess;
+    int rc = B200_OK;
+    if (n_taps > 0) {
+        e = cudaMalloc((void**) &taps, sizeof(float) * (size_t) n_taps);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(taps, h_taps, sizeof(float) * (size_t) n_taps, cudaMemcpyHostToDevice, stream);
     }
-    if (T < 1 || T > B200_FM_MAX_CHANNEL_TAPS) {
-        set_error("fm channels fir: %d taps outside [1, %d]", T, B200_FM_MAX_CHANNEL_TAPS);
-        return B200_ERR_ARG;
+    if (e == cudaSuccess && h != hist) {        // rows with the new history; at position 0 nothing in them is kept
+        e = cudaMalloc((void**) &fresh, (size_t) n_rows * (size_t) stride);
+        if (e == cudaSuccess) rc = launch_iq_history_reset(fresh + 2 * (int64_t) h, stride, n_rows, h, stream);
     }
-    if (n_samples < 0 || n_samples % (4 * R) != 0 || n_samples % 8 != 0) {
-        set_error("fm channels fir: n_samples %lld must be a multiple of 4*R and of 8", (long long) n_samples);
-        return B200_ERR_ARG;
+    if (e == cudaSuccess && rc == B200_OK) e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess || rc != B200_OK) {
+        if (e != cudaSuccess) set_error("%s: %s", who, cudaGetErrorString(e));
+        cudaFree(taps);
+        cudaFree(fresh);
+        return rc != B200_OK ? rc : B200_ERR_CUDA;
     }
-    if (first_sample < 0 || first_sample % (4 * R) != 0) {
-        set_error("fm channels fir: first_sample %lld must be a non-negative multiple of 4*R", (long long) first_sample);
-        return B200_ERR_ARG;
+    if (fresh != nullptr) {
+        cudaFree(rows);
+        rows = fresh;
+        row_bytes = stride;
+        hist = h;
     }
-    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
-        set_error("fm channels fir: IQ pointer and stream stride must be 16-byte aligned");
-        return B200_ERR_ALIGN;
-    }
-    if ((reinterpret_cast<uintptr_t>(phase_inc) & 3) != 0 || (reinterpret_cast<uintptr_t>(audio) & 3) != 0 ||
-        (reinterpret_cast<uintptr_t>(taps) & 3) != 0 || (reinterpret_cast<uintptr_t>(baseband) & 7) != 0) {
-        set_error("fm channels fir: phase increments, taps and audio must be 4-byte aligned, baseband 8-byte aligned");
-        return B200_ERR_ALIGN;
-    }
-    const int stage_bytes = fir_stage_bytes(R, T);
-    const int n_stages = 2 * stage_bytes <= 120 * 1024 ? 2 : 1;       // as fm_channels.cu
-    const int G = fir_group_size(stage_bytes, n_stages, T, n_channels);
-    if (G == 0) {
-        set_error("fm channels fir: R = %d with %d taps does not fit in shared memory", R, T);
-        return B200_ERR_ARG;
-    }
-    if (n_streams == 0 || n_samples == 0) return B200_OK;
-    const int64_t tps = (n_samples / (4 * R) + FC_T - 1) / FC_T;
-    if ((int64_t) n_streams * tps >= (1ll << 31)) {
-        set_error("fm channels fir: batch too long");
-        return B200_ERR_ARG;
-    }
-    FirParams p;
-    p.c.iq = iq;
-    p.c.stream_stride_bytes = stream_stride_bytes;
-    p.c.n_streams = n_streams;
-    p.c.n_samples = n_samples;
-    p.c.R = R;
-    p.c.first_sample = first_sample;
-    p.c.phase_inc = phase_inc;
-    p.c.n_channels = n_channels;
-    p.c.audio = audio;
-    p.c.audio_stride = audio_stride;
-    p.c.baseband = reinterpret_cast<float2*>(baseband);
-    p.c.baseband_stride = baseband_stride;
-    p.taps = taps;
-    p.T = T;
-    p.L = T - R;
-    p.off = (R - T) & 7;
-    const int smem = fir_smem_bytes(stage_bytes, n_stages, T, G);
-    auto kern = fm_channels_fir_kernel;
-    if (int rc = ensure_dynamic_smem((const void*) kern, smem)) return rc;
-    const int per_sm = cached_occupancy((const void*) kern, FC_THREADS, smem);
-    int64_t grid = (int64_t) sm_count() * per_sm;
-    const int64_t total = (int64_t) n_streams * tps;
-    if (grid > total) grid = total;
-    kern<<<(unsigned) grid, FC_THREADS, smem, stream>>>(p, (int) tps, stage_bytes, n_stages, G);
-    B200_LAUNCH_CHECK();
+    cudaFree(d_taps);
+    d_taps = taps;
+    taps_count = n_taps;
     return B200_OK;
 }
 

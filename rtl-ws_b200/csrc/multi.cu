@@ -353,13 +353,6 @@ int b200_comm_gather_rows_all(b200_comm** comms, int n, const void* const* d_sen
 // rows, no repacking), every device runs the chain on its own streams concurrently, and the per-stream
 // payload rows are gathered on device 0 by b200_comm_gather_rows_all before they go back to the host.
 
-struct b200_session;
-namespace b200 {
-int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_bytes, int64_t n_samples, int gain_db,
-                         float* h_db, int64_t db_pitch, float* h_audio, int64_t audio_pitch, uint8_t* d_avg_u8, int K_avg);
-int session_wait(b200_session* s);
-}  // namespace b200
-
 struct b200_multi {
     int G;
     int n_streams;

@@ -29,18 +29,6 @@
 
 using namespace b200;
 
-namespace b200 {
-int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
-                            cudaStream_t stream);
-int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
-int fm_history_samples(int R);
-int fm_channels_fir_history_samples(int R, int T);
-int fm_channels_fir_fits(int R, int T);
-int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
-                            const b200_fm_channel_run* runs, int n_runs, float* audio, int64_t audio_stride,
-                            int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream);
-}  // namespace b200
-
 namespace {
 constexpr int ST_R = 10;
 constexpr int ST_SLOTS = 2;
@@ -492,8 +480,8 @@ int b200_stream_set_channels(b200_stream* s, int stream, int n_channels, const u
 
 int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_taps)
 {
-    if (s == nullptr || n_taps < 0 || n_taps > B200_FM_MAX_CHANNEL_TAPS || (n_taps > 0 && h_taps == nullptr)) {
-        set_error("stream channel filter: bad arguments (%d taps)", n_taps);
+    if (s == nullptr) {
+        set_error("stream channel filter: null stream");
         return B200_ERR_ARG;
     }
     for (const auto& p : s->st)
@@ -501,54 +489,8 @@ int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_ta
             set_error("stream channel filter: set it before anything is pushed");
             return B200_ERR_ARG;
         }
-    const int hist = n_taps > 0 ? fm_channels_fir_history_samples(s->R, n_taps) : fm_history_samples(s->R);
-    if (n_taps > 0 && !fm_channels_fir_fits(s->R, n_taps)) {
-        set_error("stream channel filter: R = %d with %d taps does not fit in shared memory", s->R, n_taps);
-        return B200_ERR_ARG;
-    }
-    // the carry copies within a row: a history longer than the batch would overlap its own source
-    if (hist > s->batch) {
-        set_error("stream channel filter: its history of %d samples is longer than the batch (%lld)", hist,
-                  (long long) s->batch);
-        return B200_ERR_ARG;
-    }
-    float* d_taps = nullptr;
-    if (n_taps > 0) {
-        B200_CUDA_TRY(cudaMalloc((void**) &d_taps, sizeof(float) * (size_t) n_taps));
-        if (cudaMemcpy(d_taps, h_taps, sizeof(float) * (size_t) n_taps, cudaMemcpyHostToDevice) != cudaSuccess) {
-            set_error("stream channel filter: upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-            cudaFree(d_taps);
-            return B200_ERR_CUDA;
-        }
-    }
-    if (hist != s->hist) {        // rows with the new history; nothing has been pushed, so nothing in them is kept
-        const int64_t row_bytes = 2 * ((int64_t) hist + s->batch);
-        uint8_t* rows = nullptr;
-        if (cudaMalloc(&rows, (size_t) s->n_streams * (size_t) row_bytes) != cudaSuccess) {
-            set_error("stream channel filter: row allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
-            if (d_taps) cudaFree(d_taps);
-            return B200_ERR_CUDA;
-        }
-        if (int rc = launch_iq_history_reset(rows + 2 * (size_t) hist, row_bytes, s->n_streams, hist, s->lanes[0])) {
-            cudaFree(rows);
-            if (d_taps) cudaFree(d_taps);
-            return rc;
-        }
-        if (cudaStreamSynchronize(s->lanes[0]) != cudaSuccess) {
-            set_error("stream channel filter: history reset failed: %s", cudaGetErrorString(cudaGetLastError()));
-            cudaFree(rows);
-            if (d_taps) cudaFree(d_taps);
-            return B200_ERR_CUDA;
-        }
-        cudaFree(s->d_rows);
-        s->d_rows = rows;
-        s->row_bytes = row_bytes;
-        s->hist = hist;
-    }
-    if (s->d_taps) cudaFree(s->d_taps);
-    s->d_taps = d_taps;
-    s->n_taps = n_taps;
-    return B200_OK;
+    return set_channel_filter("stream channel filter", s->R, s->n_streams, s->batch, h_taps, n_taps, s->lanes[0],
+                              s->d_taps, s->n_taps, s->d_rows, s->row_bytes, s->hist);
 }
 
 int64_t b200_stream_pending_samples(const b200_stream* s, int stream)

@@ -350,25 +350,29 @@ def test_fir_arguments_refused_before_launch(pkg, synth, cuda):
     incs = incs_tensor(torch, np.zeros((S, 32)))
     audio = torch.empty((S * 33, n // 40 + 8), dtype=torch.float32, device="cuda")
     taps = torch.ones(1026, dtype=torch.float32, device="cuda")
+    bb = torch.empty((S * 2, n // R, 2), dtype=torch.float32, device="cuda")
     L = pkg.lib()
     iq = ring.batch.data_ptr()
 
     def call(iq=iq, stride=ring.stride_bytes, n_samples=n, first=0, inc=incs.data_ptr(), Ch=2, au=audio.data_ptr(),
-             R=R, tp=taps.data_ptr(), T=T):
+             R=R, tp=taps.data_ptr(), T=T, ast=audio.stride(0), bbp=0, bbs=0):
         return L.b200_fm_channels_exec_fir(C.c_void_p(iq), stride, S, n_samples, R, first,
                                            C.c_void_p(inc) if inc else None, Ch, C.c_void_p(au) if au else None,
-                                           audio.stride(0), None, 0, C.c_void_p(tp) if tp else None, T, None)
+                                           ast, C.c_void_p(bbp) if bbp else None, bbs,
+                                           C.c_void_p(tp) if tp else None, T, None)
 
     torch.cuda.synchronize()
     assert call() == 0
     torch.cuda.synchronize()
     before = pkg.launch_count()
-    cases = [(dict(T=0), -1), (dict(T=1025), -1), (dict(T=-3), -1), (dict(tp=0), -1), (dict(tp=taps.data_ptr() + 2), -4),
+    cases = [(dict(T=0), -1), (dict(tp=0, T=0), -1), (dict(T=1025), -1), (dict(T=-3), -1), (dict(tp=0), -1), (dict(tp=taps.data_ptr() + 2), -4),
              (dict(Ch=0), -1), (dict(Ch=33), -1), (dict(first=-40), -1), (dict(first=20), -1), (dict(first=41), -1),
              (dict(n_samples=n - 20), -1), (dict(n_samples=-40), -1),
              (dict(R=5, n_samples=60), -1), (dict(R=0), -1), (dict(R=257), -1),
              (dict(inc=0), -1), (dict(au=0), -1), (dict(iq=iq + 2), -4), (dict(stride=ring.stride_bytes + 8), -4),
-             (dict(inc=incs.data_ptr() + 2), -4), (dict(au=audio.data_ptr() + 2), -4)]
+             (dict(inc=incs.data_ptr() + 2), -4), (dict(au=audio.data_ptr() + 2), -4),
+             # rows closer than a row's length would overlap
+             (dict(ast=n // 40 - 1), -1), (dict(bbp=bb.data_ptr(), bbs=n // R - 1), -1)]
     for kw, want in cases:
         assert call(**kw) == want, kw
         assert pkg.binding.last_error()
