@@ -49,6 +49,7 @@ struct SpecParams;
 struct Spec64kExtra;
 struct FmParams;
 
+// The spectrum launchers get at least one row, and an N that b200_spectrum_plan_create accepted: capi.cu checks the rest.
 int launch_spectrum1024(const SpecParams& p, cudaStream_t stream);
 int launch_spectrum2048(const SpecParams& p, cudaStream_t stream);
 int launch_spectrum4096(const SpecParams& p, cudaStream_t stream);

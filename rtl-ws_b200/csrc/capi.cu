@@ -2,7 +2,6 @@
 // Host code only; every arithmetic step happens in the kernels of this directory.
 #include <math.h>
 #include <stdarg.h>
-#include <string.h>
 
 #include <map>
 #include <mutex>
@@ -80,40 +79,77 @@ int cached_occupancy(const void* kernel, int block_threads, int smem_bytes)
 using namespace b200;
 
 struct b200_spectrum_plan {
-    int N;
-    int hop;
-    int K;
-    int64_t row_hop;
-    int window;
-    int gain_db;
-    float db_offset;
-    float2* d_twiddle;             // N-point table
-    float2* d_twiddle1024;         // 1024-point table (N = 8192 and the four-step sizes run branches of 1024)
-    float2* d_twiddle_rk;          // N = 8192: [8][1024] W_N^(r k), the layout spectrum_mx1024.cu reads with immediate offsets
-    float2* d_twiddle_4k;          // N = 4096: [64][64] W_4096^(n2 k1), the inter-pass table of spectrum4096.cu
-                                   // N = 2048: [32][64] W_2048^(n2 k1), the inter-pass table of spectrum2048.cu
-    float* d_window;
-    Spec64kExtra x64;              // N = 65536 only (all null otherwise)
-    int device;
-    // Scratch that belongs to the plan (x64.scratch / x64.acc, and the generic kernel's global work arrays for
-    // N > 8192) is shared by every exec of the plan: execs on different CUDA streams are ordered through
-    // `scratch_done`, recorded after each launch that touched the scratch and awaited before the next one.
+    int N = 0;
+    int hop = 0;
+    int K = 0;
+    int64_t row_hop = 0;
+    float db_offset = 0.0f;
+    int device = -1;
+    float2* d_twiddle = nullptr;        // N-point table
+    float2* d_twiddle1024 = nullptr;    // 1024-point table: from N = 8192 up the u8 kernels run transforms of 1024 points
+    float2* d_twiddle_pass = nullptr;   // from N = 2048 up, the inter-pass table [N / C][C] = W_N^(r c) of the u8 kernels:
+                                        // C = 64 below N = 8192, else 1024
+    float* d_window = nullptr;
+    int four_step_ctas = 0;             // N > 8192: the grid of the four-step kernel (u8) and of the generic kernel's
+    int generic_ctas = 0;               // global-scratch form (cs32 / rf32)
+    // Scratch shared by every exec of the plan, grow-only: [four_step_ctas][N] complex + [four_step_ctas][N] floats
+    // (K > 1) for the four-step kernel, reserved at creation; [generic_ctas][2][N] complex + [generic_ctas][N] floats
+    // for the generic kernel, grown on its first exec.  Execs on different CUDA streams are ordered through
+    // `scratch_done`, recorded after each launch that used the scratch and awaited before the next one.
     std::mutex scratch_mutex;
-    cudaEvent_t scratch_done;
-    bool scratch_used;
-    float2* gen_scratch;           // [gen_ctas][2][N] complex, generic kernel, N > 8192
-    float* gen_acc;                // [gen_ctas][N]
-    int gen_ctas;
+    cudaEvent_t scratch_done = nullptr;
+    bool scratch_used = false;
+    float2* work = nullptr;
+    size_t work_n = 0;
+    float* acc = nullptr;
+    size_t acc_n = 0;
 };
 
 const float2* b200::spectrum_plan_twiddle(const b200_spectrum_plan* plan) { return plan->d_twiddle; }
 float b200::spectrum_plan_db_offset(const b200_spectrum_plan* plan) { return plan->db_offset; }
 
-// Run `launch` (which enqueues a kernel using the plan's scratch on `stream`) after every earlier user of the scratch.
+// Grow the plan's scratch to at least `work` complex and `acc` float entries.  The caller holds scratch_mutex or is
+// the plan's only user.
+static cudaError_t grow_scratch(b200_spectrum_plan* plan, size_t work, size_t acc)
+{
+    if (work <= plan->work_n && acc <= plan->acc_n) return cudaSuccess;
+    // an exec on another CUDA stream may still be reading the buffers this frees
+    if (plan->scratch_used)
+        if (cudaError_t e = cudaEventSynchronize(plan->scratch_done)) return e;
+    auto grow = [](auto*& buf, size_t& have, size_t want) {
+        if (want <= have) return cudaSuccess;
+        cudaFree(buf);
+        buf = nullptr;
+        have = 0;
+        if (cudaError_t e = cudaMalloc(&buf, want * sizeof(*buf))) {
+            buf = nullptr;
+            return e;
+        }
+        have = want;
+        return cudaSuccess;
+    };
+    if (cudaError_t e = grow(plan->work, plan->work_n, work)) return e;
+    return grow(plan->acc, plan->acc_n, acc);
+}
+
+// Run `launch` (which enqueues a kernel using the plan's scratch on `stream`) with the scratch grown to at least `work`
+// complex and `acc` float entries, after every earlier user of the scratch.
 template <class F>
-static int with_plan_scratch(b200_spectrum_plan* plan, cudaStream_t stream, F launch)
+static int launch_with_scratch(b200_spectrum_plan* plan, size_t work, size_t acc, cudaStream_t stream, F launch)
 {
     std::lock_guard<std::mutex> lock(plan->scratch_mutex);
+    if (work > plan->work_n || acc > plan->acc_n) {
+        int dev = -1;
+        B200_CUDA_TRY(cudaGetDevice(&dev));
+        if (dev != plan->device) {
+            set_error("spectrum exec: the plan was created on device %d, the current device is %d", plan->device, dev);
+            return B200_ERR_ARG;
+        }
+        if (cudaError_t e = grow_scratch(plan, work, acc)) {
+            set_error("spectrum exec: scratch allocation failed: %s", cudaGetErrorString(e));
+            return B200_ERR_CUDA;
+        }
+    }
     if (plan->scratch_done == nullptr) B200_CUDA_TRY(cudaEventCreateWithFlags(&plan->scratch_done, cudaEventDisableTiming));
     if (plan->scratch_used) B200_CUDA_TRY(cudaStreamWaitEvent(stream, plan->scratch_done, 0));
     const int rc = launch();
@@ -123,20 +159,31 @@ static int with_plan_scratch(b200_spectrum_plan* plan, cudaStream_t stream, F la
     return B200_OK;
 }
 
-static float2* upload_twiddles(int N)
+constexpr long double PI_L = 3.14159265358979323846264338327950288L;
+
+// A new device copy of `h`, or null.
+template <class T>
+static T* upload(const std::vector<T>& h)
 {
-    std::vector<float2> tw((size_t) N);
-    for (int k = 0; k < N; ++k) {
-        const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double) k / (long double) N;
-        tw[k] = make_float2((float) cosl(a), (float) sinl(a));
-    }
-    float2* d = nullptr;
-    if (cudaMalloc(&d, sizeof(float2) * (size_t) N) != cudaSuccess) return nullptr;
-    if (cudaMemcpy(d, tw.data(), sizeof(float2) * (size_t) N, cudaMemcpyHostToDevice) != cudaSuccess) {
+    T* d = nullptr;
+    if (cudaMalloc(&d, sizeof(T) * h.size()) != cudaSuccess) return nullptr;
+    if (cudaMemcpy(d, h.data(), sizeof(T) * h.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
         cudaFree(d);
         return nullptr;
     }
     return d;
+}
+
+// The N entries W_N^e(i) = exp(-2 pi i e(i) / N), i = 0..N-1, computed in long double and rounded to float.
+template <class E>
+static float2* upload_twiddles(int N, E e)
+{
+    std::vector<float2> tw((size_t) N);
+    for (int i = 0; i < N; ++i) {
+        const long double a = -2.0L * PI_L * (long double) e(i) / (long double) N;
+        tw[i] = make_float2((float) cosl(a), (float) sinl(a));
+    }
+    return upload(tw);
 }
 
 extern "C" {
@@ -191,105 +238,44 @@ b200_spectrum_plan* b200_spectrum_plan_create(int N, int hop, int K, int64_t row
         set_error("spectrum plan: unknown window %d", window);
         return nullptr;
     }
+    int device = -1;
+    if (cudaGetDevice(&device) != cudaSuccess) {
+        set_error("spectrum plan: no CUDA device");
+        return nullptr;
+    }
     b200_spectrum_plan* pl = new b200_spectrum_plan();
     pl->N = N;
     pl->hop = hop;
     pl->K = K;
     pl->row_hop = row_hop;
-    pl->window = window;
-    pl->gain_db = gain_db;
-    pl->d_twiddle = nullptr;
-    pl->d_window = nullptr;
+    pl->device = device;
     // cbb_main.c:112: pow(10, gain_db / 10) with the INTEGER quotient; cbb_main.c:125: / count.
     // 2^-14 undoes the (x - 128) / 128 input scale that the kernels leave out of the transform.
     const double g = pow(10.0, (double) (gain_db / 10));
     pl->db_offset = (float) (10.0 * log10(g / ((double) K * 16384.0)));
-    if (cudaGetDevice(&pl->device) != cudaSuccess) {
-        set_error("spectrum plan: no CUDA device");
-        delete pl;
+    auto fail = [pl](const char* what) -> b200_spectrum_plan* {
+        set_error("spectrum plan: %s: %s", what, cudaGetErrorString(cudaGetLastError()));
+        b200_spectrum_plan_destroy(pl);
         return nullptr;
-    }
-    pl->d_twiddle1024 = nullptr;
-    pl->d_twiddle_rk = nullptr;
-    pl->d_twiddle_4k = nullptr;
-    memset(&pl->x64, 0, sizeof(pl->x64));
-    pl->scratch_done = nullptr;
-    pl->scratch_used = false;
-    pl->gen_scratch = nullptr;
-    pl->gen_acc = nullptr;
-    pl->gen_ctas = 0;
-    pl->d_twiddle = upload_twiddles(N);
-    const bool four_step = (N == 16384 || N == 32768 || N == 65536);      // spectrum64k.cu, R = N / 1024 branches
-    const bool wants1024 = (N == 8192 || four_step);
-    if (pl->d_twiddle != nullptr && wants1024) pl->d_twiddle1024 = upload_twiddles(1024);
-    if (pl->d_twiddle == nullptr || (wants1024 && pl->d_twiddle1024 == nullptr)) {
-        set_error("spectrum plan: twiddle upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-        if (pl->d_twiddle) cudaFree(pl->d_twiddle);
-        delete pl;
-        return nullptr;
+    };
+    const auto identity = [](int64_t i) { return i; };
+    if ((pl->d_twiddle = upload_twiddles(N, identity)) == nullptr) return fail("twiddle upload failed");
+    if (N >= 8192 && (pl->d_twiddle1024 = upload_twiddles(1024, identity)) == nullptr) return fail("twiddle upload failed");
+    if (N >= 2048) {
+        const int64_t C = N >= 8192 ? 1024 : 64;
+        pl->d_twiddle_pass = upload_twiddles(N, [C](int64_t i) { return (i / C) * (i % C); });
+        if (pl->d_twiddle_pass == nullptr) return fail("twiddle upload failed");
     }
     if (window == B200_WINDOW_HANN) {
         std::vector<float> w((size_t) N);
-        for (int i = 0; i < N; ++i)
-            w[i] = (float) (0.5L - 0.5L * cosl(2.0L * 3.14159265358979323846264338327950288L * (long double) i /
-                                               (long double) N));
-        if (cudaMalloc(&pl->d_window, sizeof(float) * (size_t) N) != cudaSuccess ||
-            cudaMemcpy(pl->d_window, w.data(), sizeof(float) * (size_t) N, cudaMemcpyHostToDevice) != cudaSuccess) {
-            set_error("spectrum plan: window upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-            cudaFree(pl->d_twiddle);
-            if (pl->d_window) cudaFree(pl->d_window);
-            delete pl;
-            return nullptr;
-        }
+        for (int i = 0; i < N; ++i) w[i] = (float) (0.5L - 0.5L * cosl(2.0L * PI_L * (long double) i / (long double) N));
+        if ((pl->d_window = upload(w)) == nullptr) return fail("window upload failed");
     }
-    if (N == 8192) {
-        std::vector<float2> trk((size_t) 8 * 1024);
-        for (int r = 0; r < 8; ++r)
-            for (int k = 0; k < 1024; ++k) {
-                const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double) (r * k) / (long double) N;
-                trk[(size_t) r * 1024 + k] = make_float2((float) cosl(a), (float) sinl(a));
-            }
-        if (cudaMalloc((void**) &pl->d_twiddle_rk, sizeof(float2) * trk.size()) != cudaSuccess ||
-            cudaMemcpy(pl->d_twiddle_rk, trk.data(), sizeof(float2) * trk.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
-            set_error("spectrum plan: twiddle upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-            b200_spectrum_plan_destroy(pl);
-            return nullptr;
-        }
-    }
-    if (N == 4096 || N == 2048) {
-        const int rows = N / 64;                                    // n2 = 0..rows-1, k1 = 0..63
-        std::vector<float2> t4((size_t) rows * 64);
-        for (int n2 = 0; n2 < rows; ++n2)
-            for (int k1 = 0; k1 < 64; ++k1) {
-                const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double) (n2 * k1) / (long double) N;
-                t4[(size_t) n2 * 64 + k1] = make_float2((float) cosl(a), (float) sinl(a));
-            }
-        if (cudaMalloc((void**) &pl->d_twiddle_4k, sizeof(float2) * t4.size()) != cudaSuccess ||
-            cudaMemcpy(pl->d_twiddle_4k, t4.data(), sizeof(float2) * t4.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
-            set_error("spectrum plan: twiddle upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-            b200_spectrum_plan_destroy(pl);
-            return nullptr;
-        }
-    }
-    if (four_step) {
-        // tables in the layout the four-step kernel reads coalesced, and its L2-resident scratch
-        const int Rb = N / 1024;
-        std::vector<float2> trk((size_t) Rb * 1024);
-        for (int r = 0; r < Rb; ++r)
-            for (int k = 0; k < 1024; ++k) {
-                const long double a = -2.0L * 3.14159265358979323846264338327950288L * (long double) ((long long) r * k) / (long double) N;
-                trk[(size_t) r * 1024 + k] = make_float2((float) cosl(a), (float) sinl(a));
-            }
-        bool ok = cudaMalloc((void**) &pl->x64.twiddle_rk, sizeof(float2) * trk.size()) == cudaSuccess &&
-                  cudaMemcpy((void*) pl->x64.twiddle_rk, trk.data(), sizeof(float2) * trk.size(), cudaMemcpyHostToDevice) == cudaSuccess;
-        pl->x64.scratch_ctas = sm_count();
-        ok = ok && cudaMalloc((void**) &pl->x64.scratch, sizeof(float2) * (size_t) N * (size_t) pl->x64.scratch_ctas) == cudaSuccess;
-        if (ok && K > 1) ok = cudaMalloc((void**) &pl->x64.acc, sizeof(float) * (size_t) N * (size_t) pl->x64.scratch_ctas) == cudaSuccess;
-        if (!ok) {
-            set_error("spectrum plan: four-step tables / scratch: %s", cudaGetErrorString(cudaGetLastError()));
-            b200_spectrum_plan_destroy(pl);
-            return nullptr;
-        }
+    if (N > 8192) {
+        pl->four_step_ctas = sm_count();
+        pl->generic_ctas = spectrum_generic_scratch_ctas();
+        const size_t slice = (size_t) pl->four_step_ctas * N;
+        if (grow_scratch(pl, slice, K > 1 ? slice : 0) != cudaSuccess) return fail("scratch allocation failed");
     }
     return pl;
 }
@@ -297,16 +283,9 @@ b200_spectrum_plan* b200_spectrum_plan_create(int N, int hop, int K, int64_t row
 void b200_spectrum_plan_destroy(b200_spectrum_plan* plan)
 {
     if (plan == nullptr) return;
-    if (plan->d_twiddle) cudaFree(plan->d_twiddle);
-    if (plan->d_twiddle1024) cudaFree(plan->d_twiddle1024);
-    if (plan->d_twiddle_rk) cudaFree(plan->d_twiddle_rk);
-    if (plan->d_twiddle_4k) cudaFree(plan->d_twiddle_4k);
-    if (plan->d_window) cudaFree(plan->d_window);
-    if (plan->x64.twiddle_rk) cudaFree((void*) plan->x64.twiddle_rk);
-    if (plan->x64.scratch) cudaFree(plan->x64.scratch);
-    if (plan->x64.acc) cudaFree(plan->x64.acc);
-    if (plan->gen_scratch) cudaFree(plan->gen_scratch);
-    if (plan->gen_acc) cudaFree(plan->gen_acc);
+    for (void* d : std::initializer_list<void*>{plan->d_twiddle, plan->d_twiddle1024, plan->d_twiddle_pass, plan->d_window,
+                                                plan->work, plan->acc})
+        if (d != nullptr) cudaFree(d);
     if (plan->scratch_done) cudaEventDestroy(plan->scratch_done);
     delete plan;
 }
@@ -331,6 +310,18 @@ static int spectrum_exec_kind(b200_spectrum_plan* plan, const void* d_in, int64_
         set_error("spectrum exec: null input");
         return B200_ERR_ARG;
     }
+    const int N = plan->N;
+    // u8 input from 1024 points up runs a kernel made for its N, which reads 16-byte words; the rest runs the generic one
+    const bool specialised = kind == 0 && N >= 1024;
+    if (specialised && ((reinterpret_cast<uintptr_t>(d_in) & 15) != 0 || (stream_stride_bytes & 15) != 0)) {
+        set_error("spectrum exec: IQ pointer and stream stride must be 16-byte aligned");
+        return B200_ERR_ALIGN;
+    }
+    const uint64_t total = (uint64_t) n_streams * (uint64_t) n_rows;
+    if (specialised && N <= 8192 && total >= (1ull << 31)) {         // these four index rows in 32 bits
+        set_error("spectrum: n_streams * n_rows = %llu exceeds 2^31 - 1 rows per launch", (unsigned long long) total);
+        return B200_ERR_ARG;
+    }
     SpecParams p;
     p.iq = reinterpret_cast<const uint8_t*>(d_in);
     p.stream_stride_bytes = stream_stride_bytes;
@@ -343,62 +334,27 @@ static int spectrum_exec_kind(b200_spectrum_plan* plan, const void* d_in, int64_
     p.power = d_power;
     p.db_u8 = d_db_u8;
     p.db_offset = plan->db_offset;
-    p.twiddle = plan->d_twiddle;
-    p.twiddle_n = nullptr;
+    p.twiddle = specialised && N >= 8192 ? plan->d_twiddle1024 : plan->d_twiddle;
+    p.twiddle_n = specialised ? plan->d_twiddle_pass : nullptr;
     p.window = plan->d_window;
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(cuda_stream);
-    if (kind == 0 && plan->N == 1024) {
-        if ((reinterpret_cast<uintptr_t>(d_in) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
-            set_error("spectrum exec: IQ pointer and stream stride must be 16-byte aligned");
-            return B200_ERR_ALIGN;
-        }
-        return launch_spectrum1024(p, stream);
+    if (!specialised) {
+        if (N <= 8192) return launch_spectrum_generic(p, N, kind, nullptr, nullptr, 0, stream);
+        const size_t ctas = (size_t) plan->generic_ctas;
+        return launch_with_scratch(plan, ctas * 2 * N, ctas * N, stream, [&] {
+            return launch_spectrum_generic(p, N, kind, plan->work, plan->acc, plan->generic_ctas, stream);
+        });
     }
-    if (kind == 0 && plan->N >= 2048) {
-        if ((reinterpret_cast<uintptr_t>(d_in) & 15) != 0 || (stream_stride_bytes & 15) != 0) {
-            set_error("spectrum exec: IQ pointer and stream stride must be 16-byte aligned");
-            return B200_ERR_ALIGN;
-        }
-        if (plan->N == 2048) {
-            p.twiddle_n = plan->d_twiddle_4k;
-            return launch_spectrum2048(p, stream);
-        }
-        if (plan->N == 4096) {
-            p.twiddle_n = plan->d_twiddle_4k;
-            return launch_spectrum4096(p, stream);
-        }
-        p.twiddle = plan->d_twiddle1024;
-        if (plan->N == 8192) {
-            p.twiddle_n = plan->d_twiddle_rk;
-            return launch_spectrum_mx1024(p, stream);
-        }
-        return with_plan_scratch(plan, stream, [&] { return launch_spectrum64k(p, plan->x64, plan->N, stream); });
+    switch (N) {
+    case 1024: return launch_spectrum1024(p, stream);
+    case 2048: return launch_spectrum2048(p, stream);
+    case 4096: return launch_spectrum4096(p, stream);
+    case 8192: return launch_spectrum_mx1024(p, stream);
     }
-    if (plan->N <= 8192) return launch_spectrum_generic(p, plan->N, kind, nullptr, nullptr, 0, stream);
-    // N > 8192 from s32 / f32 input on the generic kernel: its per-CTA work
-    // arrays live in the plan, on the plan's device, allocated on first use
-    {
-        std::lock_guard<std::mutex> lock(plan->scratch_mutex);
-        if (plan->gen_scratch == nullptr) {
-            int dev = -1;
-            B200_CUDA_TRY(cudaGetDevice(&dev));
-            if (dev != plan->device) {
-                set_error("spectrum exec: the plan was created on device %d, the current device is %d", plan->device, dev);
-                return B200_ERR_ARG;
-            }
-            const int ctas = spectrum_generic_scratch_ctas();
-            B200_CUDA_TRY(cudaMalloc(&plan->gen_scratch, (size_t) ctas * 2 * plan->N * sizeof(float2)));
-            if (cudaMalloc(&plan->gen_acc, (size_t) ctas * plan->N * sizeof(float)) != cudaSuccess) {
-                set_error("spectrum exec: scratch allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
-                cudaFree(plan->gen_scratch);
-                plan->gen_scratch = nullptr;
-                return B200_ERR_CUDA;
-            }
-            plan->gen_ctas = ctas;
-        }
-    }
-    return with_plan_scratch(plan, stream, [&] {
-        return launch_spectrum_generic(p, plan->N, kind, plan->gen_scratch, plan->gen_acc, plan->gen_ctas, stream);
+    const size_t slice = (size_t) plan->four_step_ctas * N;
+    return launch_with_scratch(plan, slice, plan->K > 1 ? slice : 0, stream, [&] {
+        const Spec64kExtra x = {plan->work, plan->K > 1 ? plan->acc : nullptr, plan->d_twiddle_pass, plan->four_step_ctas};
+        return launch_spectrum64k(p, x, N, stream);
     });
 }
 

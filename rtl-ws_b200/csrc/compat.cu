@@ -25,11 +25,6 @@
 
 using namespace b200;
 
-extern "C" int b200_spectrum_exec_cs32(b200_spectrum_plan*, const int32_t*, int64_t, int, int64_t, float*, float*,
-                                       uint8_t*, void*);
-extern "C" int b200_spectrum_exec_rf32(b200_spectrum_plan*, const float*, int64_t, int, int64_t, float*, float*,
-                                       uint8_t*, void*);
-
 namespace {
 
 #define COMPAT_LOG(...)                                 \

@@ -322,11 +322,6 @@ __global__ void __launch_bounds__(T6_THREADS, 1) spectrum1024_tiled_kernel(const
 int launch_spectrum1024(const SpecParams& p, cudaStream_t stream)
 {
     const uint64_t total = (uint64_t) p.n_streams * (uint64_t) p.n_rows;
-    if (total == 0) return B200_OK;
-    if (total >= (1ull << 31)) {
-        set_error("spectrum: n_streams * n_rows = %llu exceeds 2^31 - 1 rows per launch", (unsigned long long) total);
-        return B200_ERR_ARG;
-    }
     const bool multi = p.K > 1;
     const bool window = p.window != nullptr;
     if (!multi && p.hop <= N1024 && p.row_hop == p.hop && p.n_rows >= 2 * T6_WARPS && p.db != nullptr && p.power == nullptr &&

@@ -251,11 +251,6 @@ __global__ void __launch_bounds__(S2K_THREADS, 1) spectrum2048_kernel(const Spec
 int launch_spectrum2048(const SpecParams& p, cudaStream_t stream)
 {
     const uint64_t total = (uint64_t) p.n_streams * (uint64_t) p.n_rows;
-    if (total == 0) return B200_OK;
-    if (total >= (1ull << 31)) {
-        set_error("spectrum: n_streams * n_rows = %llu exceeds 2^31 - 1 rows per launch", (unsigned long long) total);
-        return B200_ERR_ARG;
-    }
     auto kern = p.K > 1 ? (p.window ? spectrum2048_kernel<true, true> : spectrum2048_kernel<false, true>)
                         : (p.window ? spectrum2048_kernel<true, false> : spectrum2048_kernel<false, false>);
     if (int rc = ensure_dynamic_smem((const void*) kern, S2K_SMEM)) return rc;

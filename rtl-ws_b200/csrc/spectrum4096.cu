@@ -239,11 +239,6 @@ __global__ void __launch_bounds__(S4K_THREADS, 1) spectrum4096_kernel(const Spec
 int launch_spectrum4096(const SpecParams& p, cudaStream_t stream)
 {
     const uint64_t total = (uint64_t) p.n_streams * (uint64_t) p.n_rows;
-    if (total == 0) return B200_OK;
-    if (total >= (1ull << 31)) {
-        set_error("spectrum: n_streams * n_rows = %llu exceeds 2^31 - 1 rows per launch", (unsigned long long) total);
-        return B200_ERR_ARG;
-    }
     auto kern = p.K > 1 ? (p.window ? spectrum4096_kernel<true, true> : spectrum4096_kernel<false, true>)
                         : (p.window ? spectrum4096_kernel<true, false> : spectrum4096_kernel<false, false>);
     if (int rc = ensure_dynamic_smem((const void*) kern, S4K_SMEM)) return rc;

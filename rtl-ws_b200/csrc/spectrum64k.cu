@@ -235,7 +235,6 @@ template <int R>
 static int launch_scratch(const SpecParams& p, const Spec64kExtra& x, cudaStream_t stream)
 {
     const int64_t total = (int64_t) p.n_streams * p.n_rows;
-    if (total == 0) return B200_OK;
     auto kern = p.K > 1 ? (p.window ? spectrum64k_kernel<R, true, true> : spectrum64k_kernel<R, false, true>)
                         : (p.window ? spectrum64k_kernel<R, true, false> : spectrum64k_kernel<R, false, false>);
     if (int rc = ensure_dynamic_smem((const void*) kern, s64_smem(R))) return rc;
@@ -252,11 +251,8 @@ static int launch_scratch(const SpecParams& p, const Spec64kExtra& x, cudaStream
 // [N / 1024][1024], x.acc [scratch_ctas][N] floats when K > 1
 int launch_spectrum64k(const SpecParams& p, const Spec64kExtra& x, int N, cudaStream_t stream)
 {
-    if (N == 65536) return launch_scratch<64>(p, x, stream);
-    if (N == 32768) return launch_scratch<32>(p, x, stream);
-    if (N == 16384) return launch_scratch<16>(p, x, stream);
-    set_error("spectrum: the four-step kernel covers N = 16384, 32768, 65536 (got %d)", N);
-    return B200_ERR_ARG;
+    return N == 65536 ? launch_scratch<64>(p, x, stream)
+                      : (N == 32768 ? launch_scratch<32>(p, x, stream) : launch_scratch<16>(p, x, stream));
 }
 
 }  // namespace b200

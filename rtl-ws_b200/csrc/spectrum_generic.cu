@@ -172,12 +172,7 @@ int spectrum_generic_scratch_ctas()
 int launch_spectrum_generic(const SpecParams& p, int N, int kind, float2* scratch, float* acc_scratch, int scratch_ctas,
                             cudaStream_t stream)
 {
-    if (N < 16 || N > 65536 || (N & (N - 1)) != 0) {
-        set_error("spectrum: N = %d is not a power of two in [16, 65536]", N);
-        return B200_ERR_ARG;
-    }
     const int64_t total = (int64_t) p.n_streams * p.n_rows;
-    if (total == 0) return B200_OK;
     const int sample_bytes = kind == IN_CU8 ? 2 : (kind == IN_CS32 ? 8 : 4);
     int grid;
     int smem = 0;

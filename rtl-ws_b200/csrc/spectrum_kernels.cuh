@@ -20,8 +20,8 @@ struct SpecParams {
     float db_offset;              // 10*log10(g / (K * 2^14)): folds gain, /count and the 1/128 input scale
     const float2* twiddle;        // exp(-2*pi*i*k/N), k = 0..N-1 (device); the 1024-point table for u8 input at
                                   // N = 8192 and the four-step sizes (16384..65536)
-    const float2* twiddle_n;      // u8 input, N = 8192: [8][1024] W_N^(r k); N = 2048 / 4096: [N/64][64] W_N^(n2 k1);
-                                  // else null
+    const float2* twiddle_n;      // u8 input from N = 2048 up: the inter-pass table W_N^(r c), [N/64][64] below N = 8192,
+                                  // else [N/1024][1024] (the four-step kernel reads it as Spec64kExtra::twiddle_rk); else null
     const float* window;          // N floats (device) or null = rectangular
 };
 

@@ -247,11 +247,6 @@ __global__ void __launch_bounds__(MX_THREADS, 1) spectrum_mx1024_kernel(const Sp
 int launch_spectrum_mx1024(const SpecParams& p, cudaStream_t stream)
 {
     const uint64_t total = (uint64_t) p.n_streams * (uint64_t) p.n_rows;
-    if (total == 0) return B200_OK;
-    if (total >= (1ull << 31)) {
-        set_error("spectrum: n_streams * n_rows = %llu exceeds 2^31 - 1 rows per launch", (unsigned long long) total);
-        return B200_ERR_ARG;
-    }
     auto kern = p.K > 1 ? (p.window ? spectrum_mx1024_kernel<true, true> : spectrum_mx1024_kernel<false, true>)
                         : (p.window ? spectrum_mx1024_kernel<true, false> : spectrum_mx1024_kernel<false, false>);
     if (int rc = ensure_dynamic_smem((const void*) kern, MX_SMEM)) return rc;

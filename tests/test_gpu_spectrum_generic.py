@@ -390,10 +390,10 @@ def _hold_streams(torch, *streams):
 @pytest.mark.gpu
 def test_plan_scratch_shared_across_cuda_streams(pkg, cuda, synth):
     """Execs of one plan on two CUDA streams, enqueued back to back with no host synchronisation, share the plan's
-    scratch (the four-step kernel's x64.scratch for u8 N = 65536 and 16384, the generic kernel's global work arrays for
-    cs32 N = 16384): each result must equal its serial run bit for bit.  Each exec has fewer items than the kernel's
-    grid could hold twice over, so two unordered execs would be resident together and write the same scratch slots.
-    The last case alternates u8 and cs32 execs of one N = 16384 plan: one ordering event, two scratch arrays."""
+    scratch (the four-step kernel's work arrays for u8 N = 65536 and 16384, the generic kernel's for cs32 N = 16384):
+    each result must equal its serial run bit for bit.  Each exec has fewer items than the kernel's grid could hold
+    twice over, so two unordered execs would be resident together and write the same scratch slots.  The last case
+    alternates u8 and cs32 execs of one N = 16384 plan: one ordering event, one scratch that both kernels use."""
     torch = cuda
     s1, s2 = torch.cuda.Stream(), torch.cuda.Stream()
     u8_65536 = pkg.SpectrumPlan(65536, hop=32768, window=pkg.WINDOW_HANN)
