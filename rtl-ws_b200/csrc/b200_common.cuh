@@ -66,8 +66,6 @@ int launch_chain_fused(const uint8_t* d_iq, int64_t stride, int n_streams, int64
 
 int launch_fm_chain(const FmParams& p, cudaStream_t stream);
 int fm_history_samples(int R);
-int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream);
-int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream);
 int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int hist_samples,
                             cudaStream_t stream);
 int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream);
@@ -82,12 +80,36 @@ int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int 
                             int64_t n_audio_rows, const float* taps, int T, cudaStream_t stream);
 int fm_channels_fir_history_samples(int R, int T);
 int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h);
-// The channel filter of a block of n_rows [history | batch] rows at stream position 0, whose earlier work has all
-// finished: n_taps host taps (0 = the boxcar) replace d_taps / taps_count, and when the filter needs another history,
-// new rows with it, reset on `stream`, replace rows / row_bytes / hist.  On failure nothing changes.
-int set_channel_filter(const char* who, int R, int n_rows, int64_t max_batch, const float* h_taps, int n_taps,
-                       cudaStream_t stream, float*& d_taps, int& taps_count, uint8_t*& rows, int64_t& row_bytes,
-                       int& hist);
+
+// The device IQ rows of a session or a push stream: one row per stream, [history | batch], the history being the
+// last `hist` samples of the stream's previous batch (128 before the first).  The history is the FM chain's 32 R,
+// or the longer one the channel filter reaches back over.  Each call that launches work does it on `stream`.
+struct IqRows {
+    int R = 0;                     // down factor of the FM branch
+    int n_rows = 0;
+    int64_t max_batch = 0;         // samples
+    int hist = 0;                  // samples
+    int64_t pitch = 0;             // bytes per row: 2 * (hist + max_batch)
+    uint8_t* d_base = nullptr;     // [n_rows][pitch]
+    float* d_taps = nullptr;       // the channel filter's n_taps taps, nullptr = the boxcar
+    int n_taps = 0;
+
+    // rows with a 32 R history, reset and waited for; on failure free() releases what was allocated
+    int create(int R, int n_rows, int64_t max_batch, cudaStream_t stream);
+    void free();
+    uint8_t* batch(int i) const { return d_base + (int64_t) i * pitch + 2 * (int64_t) hist; }
+    // every row's history back to 128, waited for
+    int reset(cudaStream_t stream);
+    // the history of rows [i0, i0 + n) <- the last `hist` samples of their batch of n_samples
+    int carry(int i0, int n, int64_t n_samples, cudaStream_t stream);
+    // At stream position 0, with every earlier call on the rows finished: n_taps host taps (0 = the boxcar) become
+    // the filter, and when it needs another history, new rows with it, reset, replace the old ones.  Waits on
+    // `stream`.  On failure nothing changes.
+    int set_channel_filter(const char* who, const float* h_taps, int n_taps, cudaStream_t stream);
+
+private:
+    int alloc(int hist_samples, cudaStream_t stream);
+};
 
 // chain.cu: one batch of a host-buffer session, submitted without waiting (multi.cu drives one session per device)
 int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_bytes, int64_t n_samples, int gain_db,

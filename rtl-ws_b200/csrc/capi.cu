@@ -386,34 +386,37 @@ int b200_fm_history_samples(int R)
     return fm_history_samples(R);
 }
 
+// The checks the four history calls share.  The FM calls pass 32 R, or 0 for a down factor outside [1, 256].
+static bool history_args_ok(const char* who, const uint8_t* d_iq, int n_streams, int history_samples)
+{
+    if (d_iq != nullptr && n_streams >= 0 && history_samples >= 8 && history_samples % 8 == 0 &&
+        history_samples <= B200_IQ_MAX_HISTORY_SAMPLES)
+        return true;
+    set_error("%s: bad arguments (IQ %p, %d streams, a history of %d samples: it must be a positive multiple of 8, "
+              "at most 2^30 - 8)", who, (const void*) d_iq, n_streams, history_samples);
+    return false;
+}
+
 int b200_fm_history_reset(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int R, void* cuda_stream)
 {
-    if (d_iq == nullptr || R < 1 || R > 256 || n_streams < 0) {
-        set_error("fm history reset: bad arguments");
-        return B200_ERR_ARG;
-    }
-    return launch_fm_history_reset(d_iq, stream_stride_bytes, n_streams, R, reinterpret_cast<cudaStream_t>(cuda_stream));
+    const int h = R >= 1 && R <= 256 ? fm_history_samples(R) : 0;
+    if (!history_args_ok("fm history reset", d_iq, n_streams, h)) return B200_ERR_ARG;
+    return launch_iq_history_reset(d_iq, stream_stride_bytes, n_streams, h, reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 int b200_fm_history_carry(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples, int R,
                           void* cuda_stream)
 {
-    if (d_iq == nullptr || R < 1 || R > 256 || n_streams < 0) {
-        set_error("fm history carry: bad arguments");
-        return B200_ERR_ARG;
-    }
-    return launch_fm_history_carry(d_iq, stream_stride_bytes, n_streams, n_samples, R,
+    const int h = R >= 1 && R <= 256 ? fm_history_samples(R) : 0;
+    if (!history_args_ok("fm history carry", d_iq, n_streams, h)) return B200_ERR_ARG;
+    return launch_iq_history_carry(d_iq, stream_stride_bytes, n_streams, n_samples, h,
                                    reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 int b200_iq_history_reset(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int history_samples,
                           void* cuda_stream)
 {
-    if (d_iq == nullptr || n_streams < 0 || history_samples < 8 || history_samples % 8 != 0 ||
-        history_samples > B200_IQ_MAX_HISTORY_SAMPLES) {
-        set_error("iq history reset: bad arguments (history_samples %d must be a positive multiple of 8, at most 2^30 - 8)", history_samples);
-        return B200_ERR_ARG;
-    }
+    if (!history_args_ok("iq history reset", d_iq, n_streams, history_samples)) return B200_ERR_ARG;
     return launch_iq_history_reset(d_iq, stream_stride_bytes, n_streams, history_samples,
                                    reinterpret_cast<cudaStream_t>(cuda_stream));
 }
@@ -421,11 +424,7 @@ int b200_iq_history_reset(uint8_t* d_iq, int64_t stream_stride_bytes, int n_stre
 int b200_iq_history_carry(uint8_t* d_iq, int64_t stream_stride_bytes, int n_streams, int64_t n_samples,
                           int history_samples, void* cuda_stream)
 {
-    if (d_iq == nullptr || n_streams < 0 || history_samples < 8 || history_samples % 8 != 0 ||
-        history_samples > B200_IQ_MAX_HISTORY_SAMPLES) {
-        set_error("iq history carry: bad arguments (history_samples %d must be a positive multiple of 8, at most 2^30 - 8)", history_samples);
-        return B200_ERR_ARG;
-    }
+    if (!history_args_ok("iq history carry", d_iq, n_streams, history_samples)) return B200_ERR_ARG;
     return launch_iq_history_carry(d_iq, stream_stride_bytes, n_streams, n_samples, history_samples,
                                    reinterpret_cast<cudaStream_t>(cuda_stream));
 }

@@ -127,26 +127,62 @@ int b200_chain_exec_r(const uint8_t* d_iq, int64_t stream_stride_bytes, int n_st
 // ---- host-buffer session -----------------------------------------------------------------
 
 struct b200_session {
-    int n_streams;
-    int64_t max_samples;
-    int R;                     // down factor of the FM branch
-    int64_t tile;              // lcm(1024, 4R)
-    int hist_samples;          // 32 R, or the FIR channel filter's longer history (b200_session_set_channel_filter)
-    int64_t stride_bytes;      // per-stream row pitch in the device ring: history + batch
-    uint8_t* d_ring;           // [n_streams][stride_bytes]
-    float* d_db;               // [n_streams][max_samples]            (1024 bins per 1024 samples)
-    float* d_audio;            // [n_streams][max_samples / (4R)]
-    uint8_t* d_avg;            // [n_streams][1024] payload rows, allocated on first use (b200_session_products)
-    int64_t position;          // samples per stream consumed since create / reset (index of the next batch's first)
-    uint32_t* d_phase_inc;     // [n_streams][ch_cap], b200_session_channels, allocated on first use
-    float* d_ch_audio;         // [n_streams][ch_cap][max_samples / (4R)]
-    int ch_cap;                // channels the two buffers above hold
-    float* d_taps;             // FIR channel filter (b200_session_set_channel_filter), nullptr = the boxcar
-    int n_taps;
+    int n_streams = 0;
+    int64_t max_samples = 0;
+    int64_t tile = 0;                  // lcm(1024, 4R)
+    IqRows rows;                       // [n_streams] [history | batch], the down factor R and the channel filter
+    float* d_db = nullptr;             // [n_streams][max_samples]            (1024 bins per 1024 samples)
+    float* d_audio = nullptr;          // [n_streams][max_samples / (4R)]
+    uint8_t* d_avg = nullptr;          // [n_streams][1024] payload rows, allocated on first use (b200_session_products)
+    int64_t position = 0;              // samples per stream consumed since create / reset (index of the next batch's first)
+    uint32_t* d_phase_inc = nullptr;   // [n_streams][ch_cap], b200_session_channels, allocated on first use
+    float* d_ch_audio = nullptr;       // [n_streams][ch_cap][max_samples / (4R)]
+    int ch_cap = 0;                    // channels the two buffers above hold
     static constexpr int LANES = 4;
-    cudaStream_t streams[LANES];
-    int device;
+    cudaStream_t streams[LANES] = {};
+    int device = 0;
 };
+
+// A batch every session call takes: n_samples in [0, max_samples] and whole tiles, and with a channel filter set,
+// not shorter than its history (the carry copies the history from within the batch).
+static int session_batch_check(const char* who, const b200_session* s, const uint8_t* h_iq, int64_t n_samples)
+{
+    if (s == nullptr || h_iq == nullptr || n_samples < 0 || n_samples > s->max_samples || n_samples % s->tile != 0) {
+        set_error("%s: n_samples %lld must be a multiple of %lld and at most %lld", who, (long long) n_samples,
+                  s ? (long long) s->tile : 0ll, s ? (long long) s->max_samples : 0ll);
+        return B200_ERR_ARG;
+    }
+    if (n_samples > 0 && n_samples < s->rows.hist && s->rows.n_taps > 0) {
+        set_error("%s: a batch of %lld samples is shorter than the channel filter's history (%d samples)", who,
+                  (long long) n_samples, s->rows.hist);
+        return B200_ERR_ARG;
+    }
+    return B200_OK;
+}
+
+// One batch of every stream, in groups of ceil(n_streams / 16) streams taken round-robin by the lanes, so that
+// H2D copies, kernels and D2H copies of different groups overlap.  Per group: the 2-D copy of its IQ rows (iq_pitch
+// bytes apart in h_iq) into the device rows, step(s0, ns, d_batch, lane) for its launches and copies back, and the
+// history carry.
+template <class Step>
+static int session_groups(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch, int64_t n_samples, Step step)
+{
+    const int lanes = b200_session::LANES;
+    int group = (s->n_streams + 4 * lanes - 1) / (4 * lanes);
+    if (group < 1) group = 1;
+    int lane = 0;
+    for (int s0 = 0; s0 < s->n_streams; s0 += group, lane = (lane + 1) % lanes) {
+        const int ns = (s->n_streams - s0) < group ? (s->n_streams - s0) : group;
+        cudaStream_t st = s->streams[lane];
+        uint8_t* d_batch = s->rows.batch(s0);
+        B200_CUDA_TRY(cudaMemcpy2DAsync(d_batch, (size_t) s->rows.pitch, h_iq + (size_t) s0 * (size_t) iq_pitch,
+                                        (size_t) iq_pitch, (size_t) (2 * n_samples), (size_t) ns,
+                                        cudaMemcpyHostToDevice, st));
+        if (int rc = step(s0, ns, d_batch, st)) return rc;
+        if (int rc = s->rows.carry(s0, ns, n_samples, st)) return rc;
+    }
+    return B200_OK;
+}
 
 namespace b200 {
 
@@ -156,33 +192,13 @@ namespace b200 {
 int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_bytes, int64_t n_samples, int gain_db,
                          float* h_db, int64_t db_pitch, float* h_audio, int64_t audio_pitch, uint8_t* d_avg_u8, int K_avg)
 {
-    if (s == nullptr || h_iq == nullptr || n_samples < 0 || n_samples > s->max_samples || n_samples % s->tile != 0) {
-        set_error("session chain: n_samples %lld must be a multiple of %lld and at most %lld", (long long) n_samples,
-                  s ? (long long) s->tile : 0ll, s ? (long long) s->max_samples : 0ll);
-        return B200_ERR_ARG;
-    }
+    if (int rc = session_batch_check("session chain", s, h_iq, n_samples)) return rc;
     if (n_samples == 0) return B200_OK;
-    if (n_samples < s->hist_samples && s->n_taps > 0) {       // the carry below needs a whole history
-        set_error("session chain: a batch of %lld samples is shorter than the channel filter's history (%d samples)",
-                  (long long) n_samples, s->hist_samples);
-        return B200_ERR_ARG;
-    }
-    const int lanes = b200_session::LANES;
-    // stream groups small enough to pipeline H2D / kernels / D2H across the lanes
-    int group = (s->n_streams + 4 * lanes - 1) / (4 * lanes);
-    if (group < 1) group = 1;
-    const int64_t n_audio = n_samples / (4 * s->R);
-    int lane = 0;
-    for (int s0 = 0; s0 < s->n_streams; s0 += group, lane = (lane + 1) % lanes) {
-        const int ns = (s->n_streams - s0) < group ? (s->n_streams - s0) : group;
-        cudaStream_t st = s->streams[lane];
-        uint8_t* d_batch = s->d_ring + (int64_t) s0 * s->stride_bytes + 2 * (int64_t) s->hist_samples;
+    const int64_t n_audio = n_samples / (4 * s->rows.R);
+    const int rc = session_groups(s, h_iq, iq_pitch_bytes, n_samples, [&](int s0, int ns, uint8_t* d_batch, cudaStream_t st) {
         float* d_db = s->d_db + (size_t) s0 * (size_t) n_samples;
         float* d_audio = s->d_audio + (size_t) s0 * (size_t) n_audio;
-        B200_CUDA_TRY(cudaMemcpy2DAsync(d_batch, (size_t) s->stride_bytes, h_iq + (size_t) s0 * (size_t) iq_pitch_bytes,
-                                        (size_t) iq_pitch_bytes, (size_t) (2 * n_samples), (size_t) ns,
-                                        cudaMemcpyHostToDevice, st));
-        const int rc = b200_chain_exec_r(d_batch, s->stride_bytes, ns, n_samples, s->R, gain_db, h_db ? d_db : nullptr,
+        const int rc = b200_chain_exec_r(d_batch, s->rows.pitch, ns, n_samples, s->rows.R, gain_db, h_db ? d_db : nullptr,
                                          h_audio ? d_audio : nullptr, n_audio, d_avg_u8 ? d_avg_u8 + (size_t) s0 * 1024 : nullptr,
                                          K_avg, st);
         if (rc) return rc;
@@ -194,9 +210,9 @@ int session_chain_submit(b200_session* s, const uint8_t* h_iq, int64_t iq_pitch_
             B200_CUDA_TRY(cudaMemcpy2DAsync(h_audio + (size_t) s0 * (size_t) audio_pitch, sizeof(float) * (size_t) audio_pitch,
                                             d_audio, sizeof(float) * (size_t) n_audio, sizeof(float) * (size_t) n_audio,
                                             (size_t) ns, cudaMemcpyDeviceToHost, st));
-        const int rc2 = launch_iq_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->hist_samples, st);
-        if (rc2) return rc2;
-    }
+        return B200_OK;
+    });
+    if (rc) return rc;
     s->position += n_samples;
     return B200_OK;
 }
@@ -230,50 +246,39 @@ b200_session* b200_session_create_r(int n_streams, int64_t max_samples_per_batch
         return nullptr;
     }
     b200_session* s = new b200_session();
-    memset(s, 0, sizeof(*s));
     s->n_streams = n_streams;
     s->max_samples = max_samples_per_batch;
-    s->R = R;
     s->tile = tile;
-    s->hist_samples = fm_history_samples(R);
-    s->stride_bytes = 2 * ((int64_t) s->hist_samples + max_samples_per_batch);
     bool ok = cudaGetDevice(&s->device) == cudaSuccess;
-    ok = ok && cudaMalloc(&s->d_ring, (size_t) n_streams * (size_t) s->stride_bytes) == cudaSuccess;
     ok = ok && cudaMalloc(&s->d_db, sizeof(float) * (size_t) n_streams * (size_t) max_samples_per_batch) == cudaSuccess;
     ok = ok && cudaMalloc(&s->d_audio, sizeof(float) * (size_t) n_streams * (size_t) (max_samples_per_batch / (4 * R))) ==
                    cudaSuccess;
     for (int i = 0; ok && i < b200_session::LANES; ++i)
         ok = cudaStreamCreateWithFlags(&s->streams[i], cudaStreamNonBlocking) == cudaSuccess;
+    ok = ok && s->rows.create(R, n_streams, max_samples_per_batch, s->streams[0]) == B200_OK;
     if (!ok) {
         set_error("session: allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
         b200_session_destroy(s);
         return nullptr;
     }
-    b200_session_reset(s);
     return s;
 }
 
 void b200_session_destroy(b200_session* s)
 {
     if (s == nullptr) return;
-    for (int i = 0; i < b200_session::LANES; ++i)
-        if (s->streams[i]) cudaStreamDestroy(s->streams[i]);
-    if (s->d_ring) cudaFree(s->d_ring);
-    if (s->d_db) cudaFree(s->d_db);
-    if (s->d_audio) cudaFree(s->d_audio);
-    if (s->d_avg) cudaFree(s->d_avg);
-    if (s->d_phase_inc) cudaFree(s->d_phase_inc);
-    if (s->d_ch_audio) cudaFree(s->d_ch_audio);
-    if (s->d_taps) cudaFree(s->d_taps);
+    for (cudaStream_t st : s->streams)
+        if (st) cudaStreamDestroy(st);
+    s->rows.free();
+    for (void* d : std::initializer_list<void*>{s->d_db, s->d_audio, s->d_avg, s->d_phase_inc, s->d_ch_audio})
+        if (d != nullptr) cudaFree(d);
     delete s;
 }
 
 void b200_session_reset(b200_session* s)
 {
     if (s == nullptr) return;
-    launch_iq_history_reset(s->d_ring + 2 * (int64_t) s->hist_samples, s->stride_bytes, s->n_streams, s->hist_samples,
-                            s->streams[0]);
-    cudaStreamSynchronize(s->streams[0]);
+    s->rows.reset(s->streams[0]);
     s->position = 0;
 }
 
@@ -288,17 +293,8 @@ int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_sample
         set_error("session channels: n_channels %d outside [1, %d]", n_channels, B200_FM_MAX_CHANNELS);
         return B200_ERR_ARG;
     }
-    if (n_samples < 0 || n_samples > s->max_samples || n_samples % s->tile != 0) {
-        set_error("session channels: n_samples %lld must be a multiple of %lld and at most %lld", (long long) n_samples,
-                  (long long) s->tile, (long long) s->max_samples);
-        return B200_ERR_ARG;
-    }
+    if (int rc = session_batch_check("session channels", s, h_iq, n_samples)) return rc;
     if (n_samples == 0) return B200_OK;
-    if (n_samples < s->hist_samples && s->n_taps > 0) {
-        set_error("session channels: a batch of %lld samples is shorter than the channel filter's history (%d samples)",
-                  (long long) n_samples, s->hist_samples);
-        return B200_ERR_ARG;
-    }
     if (n_channels > s->ch_cap) {       // every earlier call has finished: the session calls wait for their work
         if (s->d_phase_inc) cudaFree(s->d_phase_inc);
         if (s->d_ch_audio) cudaFree(s->d_ch_audio);
@@ -307,38 +303,29 @@ int b200_session_channels(b200_session* s, const uint8_t* h_iq, int64_t n_sample
         s->ch_cap = 0;
         const size_t rows = (size_t) s->n_streams * (size_t) n_channels;
         B200_CUDA_TRY(cudaMalloc((void**) &s->d_phase_inc, sizeof(uint32_t) * rows));
-        B200_CUDA_TRY(cudaMalloc((void**) &s->d_ch_audio, sizeof(float) * rows * (size_t) (s->max_samples / (4 * s->R))));
+        B200_CUDA_TRY(cudaMalloc((void**) &s->d_ch_audio, sizeof(float) * rows * (size_t) (s->max_samples / (4 * s->rows.R))));
         s->ch_cap = n_channels;
     }
-    const int lanes = b200_session::LANES;
-    int group = (s->n_streams + 4 * lanes - 1) / (4 * lanes);
-    if (group < 1) group = 1;
-    const int64_t n_audio = n_samples / (4 * s->R);
-    int lane = 0;
-    for (int s0 = 0; s0 < s->n_streams; s0 += group, lane = (lane + 1) % lanes) {
-        const int ns = (s->n_streams - s0) < group ? (s->n_streams - s0) : group;
-        cudaStream_t st = s->streams[lane];
-        uint8_t* d_batch = s->d_ring + (int64_t) s0 * s->stride_bytes + 2 * (int64_t) s->hist_samples;
+    const int64_t n_audio = n_samples / (4 * s->rows.R);
+    const IqRows& r = s->rows;
+    int rc = session_groups(s, h_iq, 2 * n_samples, n_samples, [&](int s0, int ns, uint8_t* d_batch, cudaStream_t st) {
         const size_t row0 = (size_t) s0 * (size_t) n_channels;
         const size_t rows = (size_t) ns * (size_t) n_channels;
         uint32_t* d_inc = s->d_phase_inc + row0;
         float* d_audio = s->d_ch_audio + row0 * (size_t) n_audio;
-        B200_CUDA_TRY(cudaMemcpy2DAsync(d_batch, (size_t) s->stride_bytes, h_iq + (size_t) s0 * 2 * (size_t) n_samples,
-                                        (size_t) (2 * n_samples), (size_t) (2 * n_samples), (size_t) ns,
-                                        cudaMemcpyHostToDevice, st));
         B200_CUDA_TRY(cudaMemcpyAsync(d_inc, h_phase_inc + row0, sizeof(uint32_t) * rows, cudaMemcpyHostToDevice, st));
-        const int rc = s->n_taps > 0
-                           ? b200_fm_channels_exec_fir(d_batch, s->stride_bytes, ns, n_samples, s->R, s->position, d_inc,
-                                                       n_channels, d_audio, n_audio, nullptr, 0, s->d_taps, s->n_taps, st)
-                           : b200_fm_channels_exec(d_batch, s->stride_bytes, ns, n_samples, s->R, s->position, d_inc,
+        const int rc = r.n_taps > 0
+                           ? b200_fm_channels_exec_fir(d_batch, r.pitch, ns, n_samples, r.R, s->position, d_inc,
+                                                       n_channels, d_audio, n_audio, nullptr, 0, r.d_taps, r.n_taps, st)
+                           : b200_fm_channels_exec(d_batch, r.pitch, ns, n_samples, r.R, s->position, d_inc,
                                                    n_channels, d_audio, n_audio, nullptr, 0, st);
         if (rc) return rc;
         B200_CUDA_TRY(cudaMemcpyAsync(h_audio + row0 * (size_t) n_audio, d_audio, sizeof(float) * rows * (size_t) n_audio,
                                       cudaMemcpyDeviceToHost, st));
-        const int rc2 = launch_iq_history_carry(d_batch, s->stride_bytes, ns, n_samples, s->hist_samples, st);
-        if (rc2) return rc2;
-    }
-    const int rc = b200::session_wait(s);
+        return B200_OK;
+    });
+    if (rc) return rc;
+    rc = b200::session_wait(s);
     if (rc) return rc;
     s->position += n_samples;
     return B200_OK;
@@ -356,8 +343,7 @@ int b200_session_set_channel_filter(b200_session* s, const float* h_taps, int n_
         return B200_ERR_ARG;
     }
     // every earlier call has finished: the session calls wait for their work
-    return set_channel_filter("session channel filter", s->R, s->n_streams, s->max_samples, h_taps, n_taps,
-                              s->streams[0], s->d_taps, s->n_taps, s->d_ring, s->stride_bytes, s->hist_samples);
+    return s->rows.set_channel_filter("session channel filter", h_taps, n_taps, s->streams[0]);
 }
 
 int b200_session_chain(b200_session* s, const uint8_t* h_iq, int64_t n_samples, int gain_db, float* h_db,
@@ -368,7 +354,7 @@ int b200_session_chain(b200_session* s, const uint8_t* h_iq, int64_t n_samples, 
         return B200_ERR_ARG;
     }
     const int rc = b200::session_chain_submit(s, h_iq, 2 * n_samples, n_samples, gain_db, h_db, n_samples, h_audio,
-                                              n_samples / (4 * s->R), nullptr, 0);
+                                              n_samples / (4 * s->rows.R), nullptr, 0);
     if (rc) return rc;
     return b200::session_wait(s);
 }
@@ -382,7 +368,7 @@ int b200_session_products(b200_session* s, const uint8_t* h_iq, int64_t n_sample
     }
     if (s->d_avg == nullptr) B200_CUDA_TRY(cudaMalloc((void**) &s->d_avg, (size_t) s->n_streams * 1024));
     int rc = b200::session_chain_submit(s, h_iq, 2 * n_samples, n_samples, gain_db, nullptr, 0, h_audio,
-                                        n_samples / (4 * s->R), s->d_avg, K_avg);
+                                        n_samples / (4 * s->rows.R), s->d_avg, K_avg);
     if (rc) return rc;
     rc = b200::session_wait(s);
     if (rc) return rc;

@@ -387,7 +387,10 @@ int launch_iq_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t 
 int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist_samples, cudaStream_t stream)
 {
     const int hist_bytes = 2 * hist_samples;
-    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stride & 15) != 0) return B200_ERR_ALIGN;
+    if ((reinterpret_cast<uintptr_t>(iq) & 15) != 0 || (stride & 15) != 0) {
+        set_error("fm history reset: pointer and stride must be multiples of 16");
+        return B200_ERR_ALIGN;
+    }
     if (n_streams == 0) return B200_OK;
     const int64_t total = (int64_t) n_streams * (hist_bytes / 16);
     const int blocks = (int) ((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
@@ -396,14 +399,41 @@ int launch_iq_history_reset(uint8_t* iq, int64_t stride, int n_streams, int hist
     return B200_OK;
 }
 
-int launch_fm_history_carry(uint8_t* iq, int64_t stride, int n_streams, int64_t n_samples, int R, cudaStream_t stream)
+int IqRows::alloc(int hist_samples, cudaStream_t stream)
 {
-    return launch_iq_history_carry(iq, stride, n_streams, n_samples, fm_history_samples(R), stream);
+    hist = hist_samples;
+    pitch = 2 * ((int64_t) hist + max_batch);
+    B200_CUDA_TRY(cudaMalloc((void**) &d_base, (size_t) n_rows * (size_t) pitch));
+    return reset(stream);
 }
 
-int launch_fm_history_reset(uint8_t* iq, int64_t stride, int n_streams, int R, cudaStream_t stream)
+int IqRows::create(int R_, int n_rows_, int64_t max_batch_, cudaStream_t stream)
 {
-    return launch_iq_history_reset(iq, stride, n_streams, fm_history_samples(R), stream);
+    R = R_;
+    n_rows = n_rows_;
+    max_batch = max_batch_;
+    return alloc(fm_history_samples(R), stream);
+}
+
+void IqRows::free()
+{
+    cudaFree(d_base);
+    cudaFree(d_taps);
+    d_base = nullptr;
+    d_taps = nullptr;
+    n_taps = 0;
+}
+
+int IqRows::reset(cudaStream_t stream)
+{
+    if (int rc = launch_iq_history_reset(batch(0), pitch, n_rows, hist, stream)) return rc;
+    B200_CUDA_TRY(cudaStreamSynchronize(stream));
+    return B200_OK;
+}
+
+int IqRows::carry(int i0, int n, int64_t n_samples, cudaStream_t stream)
+{
+    return launch_iq_history_carry(batch(i0), pitch, n, n_samples, hist, stream);
 }
 
 }  // namespace b200

@@ -295,50 +295,49 @@ int fm_channels_fir_history_samples(int R, int T)
     return (h + 7) / 8 * 8;
 }
 
-int set_channel_filter(const char* who, int R, int n_rows, int64_t max_batch, const float* h_taps, int n_taps,
-                       cudaStream_t stream, float*& d_taps, int& taps_count, uint8_t*& rows, int64_t& row_bytes,
-                       int& hist)
+int IqRows::set_channel_filter(const char* who, const float* h_taps, int count, cudaStream_t stream)
 {
-    if (n_taps < 0 || n_taps > B200_FM_MAX_CHANNEL_TAPS || (n_taps > 0 && h_taps == nullptr)) {
-        set_error("%s: bad arguments (%d taps)", who, n_taps);
+    if (count < 0 || count > B200_FM_MAX_CHANNEL_TAPS || (count > 0 && h_taps == nullptr)) {
+        set_error("%s: bad arguments (%d taps)", who, count);
         return B200_ERR_ARG;
     }
-    const int h = n_taps > 0 ? fm_channels_fir_history_samples(R, n_taps) : fm_history_samples(R);
+    const int h = count > 0 ? fm_channels_fir_history_samples(R, count) : fm_history_samples(R);
     // the carry copies within a row: a history longer than the batch would overlap its own source
     if (h > max_batch) {
         set_error("%s: its history of %d samples is longer than the batch (%lld)", who, h, (long long) max_batch);
         return B200_ERR_ARG;
     }
-    const int64_t stride = 2 * ((int64_t) h + max_batch);
     float* taps = nullptr;
-    uint8_t* fresh = nullptr;
     cudaError_t e = cudaSuccess;
-    int rc = B200_OK;
-    if (n_taps > 0) {
-        e = cudaMalloc((void**) &taps, sizeof(float) * (size_t) n_taps);
+    if (count > 0) {
+        e = cudaMalloc((void**) &taps, sizeof(float) * (size_t) count);
         if (e == cudaSuccess)
-            e = cudaMemcpyAsync(taps, h_taps, sizeof(float) * (size_t) n_taps, cudaMemcpyHostToDevice, stream);
+            e = cudaMemcpyAsync(taps, h_taps, sizeof(float) * (size_t) count, cudaMemcpyHostToDevice, stream);
     }
-    if (e == cudaSuccess && h != hist) {        // rows with the new history; at position 0 nothing in them is kept
-        e = cudaMalloc((void**) &fresh, (size_t) n_rows * (size_t) stride);
-        if (e == cudaSuccess) rc = launch_iq_history_reset(fresh + 2 * (int64_t) h, stride, n_rows, h, stream);
+    IqRows fresh{R, n_rows, max_batch};     // rows with the new history; at position 0 nothing in the old ones is kept
+    int rc = B200_OK;
+    if (e == cudaSuccess && h != hist)
+        rc = fresh.alloc(h, stream);        // also waits for the taps
+    else if (e == cudaSuccess)
+        e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) {
+        set_error("%s: %s", who, cudaGetErrorString(e));
+        rc = B200_ERR_CUDA;
     }
-    if (e == cudaSuccess && rc == B200_OK) e = cudaStreamSynchronize(stream);
-    if (e != cudaSuccess || rc != B200_OK) {
-        if (e != cudaSuccess) set_error("%s: %s", who, cudaGetErrorString(e));
+    if (rc != B200_OK) {
         cudaFree(taps);
-        cudaFree(fresh);
-        return rc != B200_OK ? rc : B200_ERR_CUDA;
+        fresh.free();
+        return rc;
     }
-    if (fresh != nullptr) {
-        cudaFree(rows);
-        rows = fresh;
-        row_bytes = stride;
+    if (fresh.d_base != nullptr) {
+        cudaFree(d_base);
+        d_base = fresh.d_base;
+        pitch = fresh.pitch;
         hist = h;
     }
     cudaFree(d_taps);
     d_taps = taps;
-    taps_count = n_taps;
+    n_taps = count;
     return B200_OK;
 }
 

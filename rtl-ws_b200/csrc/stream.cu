@@ -37,52 +37,62 @@ constexpr int ST_GROUP = 16;       // streams submitted together when all of the
 }  // namespace
 
 struct b200_stream {
-    int n_streams;
-    int64_t batch;                 // samples per batch (multiple of 5120)
-    int gain_db;
-    int R;                         // down factor of the FM branch
-    int hist;                      // samples: 32 R, or the channel filter's H(R, T)
-    int64_t row_bytes;             // device row pitch: history + batch
-    uint8_t* d_rows;               // [n_streams][ST_SLOTS? no: one row per stream][row_bytes]
-    float* d_db;                   // [n_streams][batch]
-    float* d_audio;                // [n_streams][batch / (4R)]
-    uint8_t* h_in;                 // pinned [n_streams][ST_SLOTS][2 * batch]
-    float* h_db;                   // pinned [n_streams][ST_SLOTS][batch]
-    float* h_audio;                // pinned [n_streams][ST_SLOTS][batch / (4R)]
-    uint8_t* d_payload;            // [n_streams][1024]: K-frame averaged payload bytes of the batch start
-    uint8_t* h_payload;            // pinned [n_streams][ST_SLOTS][1024]
-    int payload_K;                 // 0 = no payload sink
-    b200_payload_sink payload_sink;
-    cudaStream_t lanes[ST_LANES];
-    int chan_max;                  // channel capacity per stream; 0 = no channel buffers yet
-    b200_channel_audio_sink chan_sink;
-    float* d_chan;                 // [n_streams][chan_max][batch / (4R)]
-    float* h_chan;                 // pinned [n_streams][ST_SLOTS][chan_max][batch / (4R)]
-    float* d_taps;                 // the channel filter (n_taps floats), nullptr = boxcar
-    int n_taps;
+    int n_streams = 0;
+    int64_t batch = 0;                   // samples per batch (multiple of 5120)
+    int gain_db = 0;
+    IqRows rows;                         // [n_streams] [history | batch], the down factor R and the channel filter
+    float* d_db = nullptr;               // [n_streams][batch]
+    float* d_audio = nullptr;            // [n_streams][batch / (4R)]
+    uint8_t* h_in = nullptr;             // pinned [n_streams][ST_SLOTS][2 * batch]
+    float* h_db = nullptr;               // pinned [n_streams][ST_SLOTS][batch]
+    float* h_audio = nullptr;            // pinned [n_streams][ST_SLOTS][batch / (4R)]
+    uint8_t* d_payload = nullptr;        // [n_streams][1024]: K-frame averaged payload bytes of the batch start
+    uint8_t* h_payload = nullptr;        // pinned [n_streams][ST_SLOTS][1024]
+    int payload_K = 0;                   // 0 = no payload sink
+    b200_payload_sink payload_sink = nullptr;
+    cudaStream_t lanes[ST_LANES] = {};
+    int chan_max = 0;                    // channel capacity per stream; 0 = no channel buffers yet
+    b200_channel_audio_sink chan_sink = nullptr;
+    float* d_chan = nullptr;             // [n_streams][chan_max][batch / (4R)]
+    float* h_chan = nullptr;             // pinned [n_streams][ST_SLOTS][chan_max][batch / (4R)]
     struct ChannelSet {
-        int n;
+        int n = 0;
         uint32_t inc[B200_FM_MAX_CHANNELS];
         int32_t id[B200_FM_MAX_CHANNELS];
     };
     struct PerStream {
-        int64_t fill;              // samples in the current slot
-        int slot;                  // slot being filled
-        int64_t batches_submitted;
-        int64_t batches_delivered;
-        cudaEvent_t done[ST_SLOTS];
-        bool in_flight[ST_SLOTS];
-        bool ready[ST_SLOTS];      // full, not yet submitted
-        bool has_db[ST_SLOTS];     // the submitted slot computed and copied per-frame dB rows
-        ChannelSet channels;       // current listener set (b200_stream_set_channels)
+        int64_t fill = 0;                // samples in the current slot
+        int slot = 0;                    // slot being filled
+        int64_t batches_submitted = 0;
+        int64_t batches_delivered = 0;
+        cudaEvent_t done[ST_SLOTS] = {};
+        bool in_flight[ST_SLOTS] = {};
+        bool ready[ST_SLOTS] = {};       // full, not yet submitted
+        bool has_db[ST_SLOTS] = {};      // the submitted slot computed and copied per-frame dB rows
+        ChannelSet channels;             // current listener set (b200_stream_set_channels)
         ChannelSet slot_channels[ST_SLOTS];     // the set of each full slot, taken when its last sample arrived
-        bool has_chan[ST_SLOTS];   // the submitted slot computed and copied channel audio
+        bool has_chan[ST_SLOTS] = {};    // the submitted slot computed and copied channel audio
     };
     std::vector<PerStream> st;
-    b200_spectrum_sink spectrum_sink;
-    b200_audio_sink audio_sink;
-    void* user;
+    b200_spectrum_sink spectrum_sink = nullptr;
+    b200_audio_sink audio_sink = nullptr;
+    void* user = nullptr;
 };
+
+// A device buffer of `bytes` and its pinned host mirror of ST_SLOTS times that, or neither: on failure both are null
+// and b200_last_error() says why, prefixed by `who`.
+template <class T>
+static bool alloc_slots(const char* who, T*& d, T*& h, size_t bytes)
+{
+    cudaError_t e = cudaMalloc(&d, bytes);
+    if (e == cudaSuccess) e = cudaHostAlloc(&h, ST_SLOTS * bytes, cudaHostAllocDefault);
+    if (e == cudaSuccess) return true;
+    set_error("%s: %s", who, cudaGetErrorString(e));
+    if (d) cudaFree(d);
+    d = nullptr;
+    h = nullptr;
+    return false;
+}
 
 static void stream_deliver(b200_stream* s, int i, bool block)
 {
@@ -102,10 +112,9 @@ static void stream_deliver(b200_stream* s, int i, bool block)
         // a sink installed after this batch was submitted without one gets nothing for it (there are no rows)
         if (s->spectrum_sink && p.has_db[slot])
             s->spectrum_sink(s->user, i, b * (s->batch / 1024), (int) (s->batch / 1024), s->h_db + off * (size_t) s->batch);
-        if (s->audio_sink)
-            s->audio_sink(s->user, i, b * (s->batch / (4 * s->R)), (int) (s->batch / (4 * s->R)), s->h_audio + off * (size_t) (s->batch / (4 * s->R)));
+        const int64_t n_audio = s->batch / (4 * s->rows.R);
+        if (s->audio_sink) s->audio_sink(s->user, i, b * n_audio, (int) n_audio, s->h_audio + off * (size_t) n_audio);
         if (s->chan_sink && p.has_chan[slot]) {
-            const int64_t n_audio = s->batch / (4 * s->R);
             const b200_stream::ChannelSet& cs = p.slot_channels[slot];
             for (int c = 0; c < cs.n; ++c)
                 s->chan_sink(s->user, i, cs.id[c], b * n_audio, (int) n_audio,
@@ -122,20 +131,20 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
 {
     const int n = b - a;
     const size_t batch = (size_t) s->batch;
-    const size_t n_audio = batch / (size_t) (4 * s->R);
+    const size_t n_audio = batch / (size_t) (4 * s->rows.R);
     cudaStream_t lane = s->lanes[(a / ST_GROUP) % ST_LANES];
     const size_t off = (size_t) a * ST_SLOTS + (size_t) slot;            // first stream's slot; next stream: + ST_SLOTS
-    uint8_t* d_batch = s->d_rows + (size_t) a * (size_t) s->row_bytes + 2 * (size_t) s->hist;
+    uint8_t* d_batch = s->rows.batch(a);
     // per-frame dB rows exist only once a spectrum sink has been installed (b200_stream_set_sinks allocates them)
     const bool want_db = s->spectrum_sink != nullptr && s->d_db != nullptr && s->h_db != nullptr;
     float* d_db = want_db ? s->d_db + (size_t) a * batch : nullptr;
     float* d_audio = s->d_audio + (size_t) a * n_audio;
     uint8_t* d_pay = s->d_payload + (size_t) a * 1024;
     const bool want_payload = s->payload_sink != nullptr && s->payload_K > 0;
-    B200_CUDA_TRY(cudaMemcpy2DAsync(d_batch, (size_t) s->row_bytes, s->h_in + off * 2 * batch, ST_SLOTS * 2 * batch, 2 * batch,
+    B200_CUDA_TRY(cudaMemcpy2DAsync(d_batch, (size_t) s->rows.pitch, s->h_in + off * 2 * batch, ST_SLOTS * 2 * batch, 2 * batch,
                                     (size_t) n, cudaMemcpyHostToDevice, lane));
     // without a per-frame sink the dB rows are not computed at all: the FM kernel and the K-frame average only
-    int rc = b200_chain_exec_r(d_batch, s->row_bytes, n, s->batch, s->R, s->gain_db, d_db, d_audio,
+    int rc = b200_chain_exec_r(d_batch, s->rows.pitch, n, s->batch, s->rows.R, s->gain_db, d_db, d_audio,
                                (int64_t) n_audio, want_payload ? d_pay : nullptr, want_payload ? s->payload_K : 0, lane);
     if (rc) return rc;
     // channels of the streams that have listeners: one runs-table launch over the group's rows
@@ -156,13 +165,13 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
             if (cs.n > chan_width) chan_width = cs.n;
         }
         if (n_runs > 0) {
-            rc = launch_fm_channels_runs(d_batch, s->row_bytes, n, s->batch, s->R, runs, n_runs,
+            rc = launch_fm_channels_runs(d_batch, s->rows.pitch, n, s->batch, s->rows.R, runs, n_runs,
                                          s->d_chan + (size_t) a * (size_t) s->chan_max * n_audio, (int64_t) n_audio,
-                                         (int64_t) n * s->chan_max, s->d_taps, s->n_taps, lane);
+                                         (int64_t) n * s->chan_max, s->rows.d_taps, s->rows.n_taps, lane);
             if (rc) return rc;
         }
     }
-    rc = launch_iq_history_carry(d_batch, s->row_bytes, n, s->batch, s->hist, lane);
+    rc = s->rows.carry(a, n, s->batch, lane);
     if (rc) return rc;
     // the per-frame dB rows cross PCIe only if somebody listens (4 bytes per sample; the payload is 1 KB per batch)
     if (want_db)
@@ -258,57 +267,16 @@ b200_stream* b200_stream_create_r(int n_streams, int64_t batch_samples, int gain
     s->n_streams = n_streams;
     s->batch = batch_samples;
     s->gain_db = gain_db;
-    s->R = R;
-    s->hist = fm_history_samples(R);
-    s->row_bytes = 2 * ((int64_t) s->hist + batch_samples);
-    s->d_rows = nullptr;
-    s->d_db = nullptr;
-    s->d_audio = nullptr;
-    s->h_in = nullptr;
-    s->h_db = nullptr;
-    s->h_audio = nullptr;
-    s->d_payload = nullptr;
-    s->h_payload = nullptr;
-    s->payload_K = 0;
-    s->payload_sink = nullptr;
-    s->spectrum_sink = nullptr;
-    s->audio_sink = nullptr;
-    s->user = nullptr;
-    s->chan_max = 0;
-    s->chan_sink = nullptr;
-    s->d_chan = nullptr;
-    s->h_chan = nullptr;
-    s->d_taps = nullptr;
-    s->n_taps = 0;
-    for (int i = 0; i < ST_LANES; ++i) s->lanes[i] = nullptr;
     const size_t ns = (size_t) n_streams;
-    bool ok = cudaMalloc(&s->d_rows, ns * (size_t) s->row_bytes) == cudaSuccess;
-    ok = ok && cudaMalloc(&s->d_audio, sizeof(float) * ns * (size_t) (batch_samples / (4 * R))) == cudaSuccess;
+    bool ok = alloc_slots("stream: allocation failed", s->d_audio, s->h_audio,
+                          sizeof(float) * ns * (size_t) (batch_samples / (4 * R)));
     ok = ok && cudaHostAlloc(&s->h_in, ns * ST_SLOTS * 2 * (size_t) batch_samples, cudaHostAllocDefault) == cudaSuccess;
-    ok = ok && cudaHostAlloc(&s->h_audio, sizeof(float) * ns * ST_SLOTS * (size_t) (batch_samples / (4 * R)), cudaHostAllocDefault) == cudaSuccess;
-    ok = ok && cudaMalloc(&s->d_payload, ns * 1024) == cudaSuccess;
-    ok = ok && cudaHostAlloc(&s->h_payload, ns * ST_SLOTS * 1024, cudaHostAllocDefault) == cudaSuccess;
+    ok = ok && alloc_slots("stream: allocation failed", s->d_payload, s->h_payload, ns * 1024);
     for (int i = 0; ok && i < ST_LANES; ++i) ok = cudaStreamCreateWithFlags(&s->lanes[i], cudaStreamNonBlocking) == cudaSuccess;
     s->st.resize(ns);
-    for (size_t i = 0; i < ns; ++i) {
-        s->st[i].fill = 0;
-        s->st[i].slot = 0;
-        s->st[i].batches_submitted = 0;
-        s->st[i].batches_delivered = 0;
-        s->st[i].channels.n = 0;
-        for (int k = 0; k < ST_SLOTS; ++k) {
-            s->st[i].done[k] = nullptr;
-            s->st[i].in_flight[k] = false;
-            s->st[i].ready[k] = false;
-            s->st[i].has_db[k] = false;
-            s->st[i].has_chan[k] = false;
-            s->st[i].slot_channels[k].n = 0;
-            if (ok) ok = cudaEventCreateWithFlags(&s->st[i].done[k], cudaEventDisableTiming) == cudaSuccess;
-        }
-    }
-    if (ok)
-        ok = launch_iq_history_reset(s->d_rows + 2 * (size_t) s->hist, s->row_bytes, n_streams, s->hist, s->lanes[0]) == B200_OK &&
-             cudaStreamSynchronize(s->lanes[0]) == cudaSuccess;
+    for (auto& p : s->st)
+        for (int k = 0; ok && k < ST_SLOTS; ++k) ok = cudaEventCreateWithFlags(&p.done[k], cudaEventDisableTiming) == cudaSuccess;
+    ok = ok && s->rows.create(R, n_streams, batch_samples, s->lanes[0]) == B200_OK;
     if (!ok) {
         set_error("stream: allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
         b200_stream_destroy(s);
@@ -320,25 +288,19 @@ b200_stream* b200_stream_create_r(int n_streams, int64_t batch_samples, int gain
 void b200_stream_destroy(b200_stream* s)
 {
     if (s == nullptr) return;
-    for (int i = 0; i < ST_LANES; ++i)
-        if (s->lanes[i]) {
-            cudaStreamSynchronize(s->lanes[i]);
-            cudaStreamDestroy(s->lanes[i]);
+    for (cudaStream_t lane : s->lanes)
+        if (lane) {
+            cudaStreamSynchronize(lane);
+            cudaStreamDestroy(lane);
         }
     for (auto& p : s->st)
-        for (int k = 0; k < ST_SLOTS; ++k)
-            if (p.done[k]) cudaEventDestroy(p.done[k]);
-    if (s->d_rows) cudaFree(s->d_rows);
-    if (s->d_db) cudaFree(s->d_db);
-    if (s->d_audio) cudaFree(s->d_audio);
-    if (s->h_in) cudaFreeHost(s->h_in);
-    if (s->h_db) cudaFreeHost(s->h_db);
-    if (s->h_audio) cudaFreeHost(s->h_audio);
-    if (s->d_payload) cudaFree(s->d_payload);
-    if (s->h_payload) cudaFreeHost(s->h_payload);
-    if (s->d_chan) cudaFree(s->d_chan);
-    if (s->h_chan) cudaFreeHost(s->h_chan);
-    if (s->d_taps) cudaFree(s->d_taps);
+        for (cudaEvent_t ev : p.done)
+            if (ev) cudaEventDestroy(ev);
+    s->rows.free();
+    for (void* d : std::initializer_list<void*>{s->d_db, s->d_audio, s->d_payload, s->d_chan})
+        if (d != nullptr) cudaFree(d);
+    for (void* h : std::initializer_list<void*>{s->h_in, s->h_db, s->h_audio, s->h_payload, s->h_chan})
+        if (h != nullptr) cudaFreeHost(h);
     delete s;
 }
 
@@ -347,18 +309,9 @@ void b200_stream_set_sinks(b200_stream* s, b200_spectrum_sink spectrum_sink, b20
     if (s == nullptr) return;
     // The per-frame dB rows (4 bytes per sample on the device, twice that pinned on the host: 420 MB for 256 streams
     // of 204800 samples) exist only for callers that listen to them: allocated when the first spectrum sink arrives.
-    if (spectrum_sink != nullptr && s->d_db == nullptr) {
-        const size_t ns = (size_t) s->n_streams;
-        bool ok = cudaMalloc(&s->d_db, sizeof(float) * ns * (size_t) s->batch) == cudaSuccess;
-        ok = ok && cudaHostAlloc(&s->h_db, sizeof(float) * ns * ST_SLOTS * (size_t) s->batch, cudaHostAllocDefault) == cudaSuccess;
-        if (!ok) {
-            set_error("stream: dB row buffers: %s", cudaGetErrorString(cudaGetLastError()));
-            if (s->d_db) cudaFree(s->d_db);
-            s->d_db = nullptr;
-            s->h_db = nullptr;
-            spectrum_sink = nullptr;      // reported through b200_last_error(); audio and payload keep working
-        }
-    }
+    if (spectrum_sink != nullptr && s->d_db == nullptr &&
+        !alloc_slots("stream: dB row buffers", s->d_db, s->h_db, sizeof(float) * (size_t) s->n_streams * (size_t) s->batch))
+        spectrum_sink = nullptr;      // reported through b200_last_error(); audio and payload keep working
     s->spectrum_sink = spectrum_sink;
     s->audio_sink = audio_sink;
     s->user = user;
@@ -437,17 +390,10 @@ int b200_stream_set_channel_sink(b200_stream* s, int max_channels, b200_channel_
         return B200_ERR_ARG;
     }
     if (s->chan_max == 0 && sink != nullptr) {      // the buffers come with the first sink, like the dB rows
-        const size_t rows = (size_t) s->n_streams * (size_t) max_channels;
-        const size_t n_audio = (size_t) (s->batch / (4 * s->R));
-        bool ok = cudaMalloc(&s->d_chan, sizeof(float) * rows * n_audio) == cudaSuccess;
-        ok = ok && cudaHostAlloc(&s->h_chan, sizeof(float) * rows * ST_SLOTS * n_audio, cudaHostAllocDefault) == cudaSuccess;
-        if (!ok) {
-            set_error("stream channel sink: buffers: %s", cudaGetErrorString(cudaGetLastError()));
-            if (s->d_chan) cudaFree(s->d_chan);
-            s->d_chan = nullptr;
-            s->h_chan = nullptr;
+        const size_t n_audio = (size_t) (s->batch / (4 * s->rows.R));
+        if (!alloc_slots("stream channel sink: buffers", s->d_chan, s->h_chan,
+                         sizeof(float) * (size_t) s->n_streams * (size_t) max_channels * n_audio))
             return B200_ERR_CUDA;
-        }
         s->chan_max = max_channels;
     }
     s->chan_sink = sink;
@@ -489,8 +435,7 @@ int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_ta
             set_error("stream channel filter: set it before anything is pushed");
             return B200_ERR_ARG;
         }
-    return set_channel_filter("stream channel filter", s->R, s->n_streams, s->batch, h_taps, n_taps, s->lanes[0],
-                              s->d_taps, s->n_taps, s->d_rows, s->row_bytes, s->hist);
+    return s->rows.set_channel_filter("stream channel filter", h_taps, n_taps, s->lanes[0]);
 }
 
 int64_t b200_stream_pending_samples(const b200_stream* s, int stream)
