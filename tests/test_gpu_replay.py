@@ -54,7 +54,11 @@ def test_virtual_dongles_feed_the_push_stream(pkg, cuda, po, synth):
     [t.start() for t in threads]
     [t.join() for t in threads]
     ps.flush()
-    assert pkg.launch_count() - before >= 5 * n_dongles
+    # a submission is one chain launch and one history carry.  Dongles that fill a batch together go out as one group
+    # (stream.cu), so the 5 batches of each dongle take between 5 and 5 * n_dongles submissions, depending on how the
+    # reader threads interleave
+    launches = pkg.launch_count() - before
+    assert 2 * 5 <= launches <= 2 * 5 * n_dongles, launches
     for i, c in enumerate(caps):
         assert ps.pending(i) == (n_buffers * BUF // 2) % 204800
         frames, audio = collect(ps, i)
