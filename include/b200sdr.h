@@ -270,6 +270,29 @@ int b200_debug_atan2(const int32_t* d_yx, int n, float* d_out, int which, void* 
 int64_t b200_audio_post_out_samples(int64_t n_audio, int flags);
 int b200_audio_post(const float* d_audio, int64_t audio_stride, int n_streams, int64_t n_audio, double audio_rate_hz,
                     int flags, float* d_state, float* d_out, int64_t out_stride, void* cuda_stream);
+/* The same arithmetic over a table of rows that each name their input, output and state row (the push stream's
+ * listeners come and go, and a listener's state belongs to it, not to its position).  Row k reads audio row
+ * audio_row of d_audio (audio_stride floats apart, n_audio_rows rows), writes output row out_row of d_out (out_stride
+ * floats apart, n_out_rows rows) and advances state row state_row of d_state (B200_AUDIO_POST_STATE_FLOATS floats
+ * apart, n_state_rows rows); fresh != 0 reads that state as all zero (stream start) without reading memory.  Row k's
+ * output and next state are bit for bit b200_audio_post's on that row with that state (zeroed if fresh), and the
+ * state layout is the same, so one state row may be advanced by either call in any order.  h_rows is host memory,
+ * read during the call only.  Two launches, like b200_audio_post.  Checked before anything is launched: B200_ERR_ARG
+ * for n_rows outside [1, B200_AUDIO_POST_MAX_ROWS], a row index outside its row count, two rows sharing an out_row
+ * or a state_row, audio_stride below n_audio or out_stride below b200_audio_post_out_samples(n_audio, flags), NULL
+ * pointers, overlapping audio, output and state blocks, and whatever b200_audio_post refuses; B200_ERR_ALIGN for a
+ * pointer that is not 4-byte aligned. */
+#define B200_AUDIO_POST_MAX_ROWS 1024
+typedef struct {
+    int32_t audio_row;   /* input row of d_audio */
+    int32_t out_row;     /* output row of d_out */
+    int32_t state_row;   /* B200_AUDIO_POST_STATE_FLOATS floats at d_state + state_row * that */
+    int32_t fresh;       /* nonzero: read the state as all zero (stream start); the next state is written either way */
+} b200_audio_post_row;
+int b200_audio_post_rows(const float* d_audio, int64_t audio_stride, int64_t n_audio_rows, int64_t n_audio,
+                         double audio_rate_hz, int flags, const b200_audio_post_row* h_rows, int n_rows,
+                         float* d_state, int64_t n_state_rows, float* d_out, int64_t out_stride, int64_t n_out_rows,
+                         void* cuda_stream);
 /* the resampler's 240 prototype taps (host), for whoever wants to check them; returns 240 */
 int b200_audio_resample_taps(float* h240);
 
@@ -345,7 +368,8 @@ int b200_session_set_channel_filter(b200_session* s, const float* h_taps, int n_
  * whatever is waiting.  One producer thread per b200_stream (as the reference has one sensor thread).
  * Finished batches are handed to the sinks from inside push / poll / flush, on the calling thread, in order:
  *   spectrum sink: n_frames rows of 1024 float dB (display order) starting at frame first_frame;
- *   audio sink:    n floats at fs/40 starting at audio sample first_sample.
+ *   audio sink:    n floats starting at audio sample first_sample: batch_samples / (4R) of them at fs / (4R) (fs/40
+ *                  at R = 10), or b200_audio_post_out_samples of that after b200_stream_set_audio_post (below).
  * The pointers passed to a sink are valid until it returns.  Batching is aligned to stream
  * start, so results do not depend on the chunking of the pushes (as with rf_decimator).
  */
@@ -354,7 +378,7 @@ typedef void (*b200_spectrum_sink)(void* user, int stream, int64_t first_frame, 
 typedef void (*b200_audio_sink)(void* user, int stream, int64_t first_sample, int n, const float* audio);
 b200_stream* b200_stream_create(int n_streams, int64_t batch_samples, int gain_db);
 /* any down factor (b200_stream_create is R = 10): batch_samples a multiple of b200_chain_tile_samples(R),
- * the audio sink gets batch_samples / (4R) floats per batch at fs / (4R) */
+ * the audio sink gets batch_samples / (4R) floats per batch at fs / (4R) (unless b200_stream_set_audio_post) */
 b200_stream* b200_stream_create_r(int n_streams, int64_t batch_samples, int gain_db, int R);
 void b200_stream_destroy(b200_stream* s);
 void b200_stream_set_sinks(b200_stream* s, b200_spectrum_sink spectrum_sink, b200_audio_sink audio_sink, void* user);
@@ -393,6 +417,20 @@ int b200_stream_set_channel_sink(b200_stream* s, int max_channels, b200_channel_
 int b200_stream_set_channels(b200_stream* s, int stream, int n_channels, const uint32_t* h_phase_inc,
                              const int32_t* h_channel_ids);
 int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_taps);
+/* De-emphasis and 48 kHz output on the push stream (opt-in; flags = 0, the default, leaves every output bit as it
+ * was).  flags and audio_rate_hz mean what they mean for b200_audio_post; the rate is fs / (4R), 51200 for the
+ * reference.  Only before anything is pushed, like b200_stream_set_channel_filter.  B200_ERR_ARG for whatever
+ * b200_audio_post refuses, and for B200_AUDIO_RESAMPLE_48K when batch_samples / (4R) is not a multiple of 16 (every
+ * batch at R = 10 is; a batch of 1024 at R = 256 is not).  From then on the audio sink and the channel sink get the
+ * post-processed audio: n = b200_audio_post_out_samples(batch_samples / (4R), flags) floats per batch (4800 per
+ * 204 800-sample batch with the resampler), first_sample counted at that output rate (batch b starts at b * n).
+ * Spectra and payloads do not change.  Each dongle's centre audio carries one state row from stream start.  Each
+ * channel carries state by listener id: a listener continues from where it was only if the same id was in the dongle's
+ * set in the previous batch and that batch had channel work (a channel sink); any other listener -- a new id, an id
+ * back after a gap, every listener of the first batch after batches without a channel sink -- starts from stream-start
+ * state.  Retuning an id or reordering the set keeps the state.  Each submitted run adds two launches for the centre
+ * audio (b200_audio_post) and, if it has listeners, two for its channels (b200_audio_post_rows). */
+int b200_stream_set_audio_post(b200_stream* s, int flags, double audio_rate_hz);
 
 /* ---- websocket wire formats: what the reference's main.c puts on the socket ----------------
  *

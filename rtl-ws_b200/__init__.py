@@ -11,7 +11,8 @@ from .binding import (  # noqa: F401
     B200Error, SpectrumPlan, StreamRing, Session, PushStream, RfDecimator, CicDelayLine,
     fm_exec, chain_exec, fm_channel_tune, fm_channels_exec, FM_MAX_CHANNELS, fm_channel_filter,
     fm_channels_exec_runs, FmChannelRun, FM_MAX_RUNS,
-    fm_channels_fir_history_samples, FM_MAX_CHANNEL_TAPS, init, lib, launch_count, fm_exec_cs32, FmDemod, debug_atan2, audio_post, resample_taps, Comm, Multi,
+    fm_channels_fir_history_samples, FM_MAX_CHANNEL_TAPS, init, lib, launch_count, fm_exec_cs32, FmDemod, debug_atan2, audio_post, resample_taps,
+    audio_post_rows, AudioPostRow, AUDIO_POST_MAX_ROWS, Comm, Multi,
     shard_count, shard_stream, FM_STATE_FLOATS, FM_SKIP_STAGE2, AUDIO_DEEMPH_50US, AUDIO_DEEMPH_75US,
     AUDIO_RESAMPLE_48K, AUDIO_POST_STATE_FLOATS,
     spectrum_alloc, spectrum_free, spectrum_add_cmplx_u8, spectrum_add_cmplx_s32, spectrum_add_real_f32,

@@ -41,6 +41,7 @@ EXPORTED_SYMBOLS = [
     "b200_host_alloc", "b200_host_free",
     "b200_fm_exec_cs32", "b200_fm_demod_create", "b200_fm_demod_destroy", "b200_fm_demod_reset", "b200_fm_demod_block",
     "b200_debug_atan2", "b200_audio_post", "b200_audio_post_out_samples", "b200_audio_resample_taps",
+    "b200_audio_post_rows", "b200_stream_set_audio_post",
     "b200_shard_count", "b200_shard_stream", "b200_comm_unique_id", "b200_comm_create", "b200_comm_create_all",
     "b200_comm_destroy", "b200_comm_world", "b200_comm_rank", "b200_comm_nccl_version", "b200_comm_gather_rows",
     "b200_comm_gather_rows_all", "b200_multi_create", "b200_multi_destroy", "b200_multi_chain",
@@ -72,6 +73,14 @@ CHANNEL_SINK = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_int32, C.c_int64, C.c_
 
 FM_MAX_CHANNELS = 32
 FM_MAX_RUNS = 64
+
+
+AUDIO_POST_MAX_ROWS = 1024
+
+
+class AudioPostRow(C.Structure):
+    """b200_audio_post_row: one row of the table of b200_audio_post_rows."""
+    _fields_ = [("audio_row", C.c_int32), ("out_row", C.c_int32), ("state_row", C.c_int32), ("fresh", C.c_int32)]
 
 
 class FmChannelRun(C.Structure):
@@ -166,6 +175,8 @@ def lib() -> C.CDLL:
     L.b200_audio_post_out_samples.restype = i64
     L.b200_audio_post_out_samples.argtypes = [i64, i32]
     L.b200_audio_resample_taps.argtypes = [vp]
+    L.b200_audio_post_rows.argtypes = [vp, i64, i64, i64, C.c_double, i32, vp, i32, vp, i64, vp, i64, i64, vp]
+    L.b200_stream_set_audio_post.argtypes = [vp, i32, C.c_double]
     L.b200_shard_count.argtypes = [i32, i32, i32]
     L.b200_shard_stream.argtypes = [i32, i32, i32, i32]
     L.b200_comm_unique_id.argtypes = [vp]
@@ -594,6 +605,34 @@ def audio_post(audio, state, flags: int, rate_hz: float = 51200.0, out=None, str
     return out
 
 
+def audio_post_rows(audio, rows, state, flags: int, rate_hz: float = 51200.0, out=None, stream=None):
+    """b200_audio_post_rows: audio_post over a table of rows.  rows is a sequence of (audio_row, out_row, state_row,
+    fresh); row k reads audio[audio_row], writes out[out_row] and advances state[state_row] (or starts from zero state
+    if fresh).  audio: cuda float32 [n_audio_rows, n] (rows may be slices of wider rows), state: cuda float32
+    [n_state_rows, AUDIO_POST_STATE_FLOATS], out (allocated if not given, one row per table row): float32
+    [n_out_rows, audio_post_out_samples(n)] rows with unit column stride."""
+    torch = _torch()
+    assert audio.is_cuda and audio.dtype == torch.float32 and audio.dim() == 2 and audio.stride(1) == 1
+    n = audio.shape[1]
+    n_out = int(lib().b200_audio_post_out_samples(n, flags))
+    if n_out < 0:
+        raise B200Error("audio_post_rows: the resampler takes multiples of 16 samples")
+    rows = list(rows)
+    table = (AudioPostRow * max(1, len(rows)))()
+    for k, (a, o, st, fresh) in enumerate(rows):
+        table[k].audio_row, table[k].out_row, table[k].state_row, table[k].fresh = a, o, st, int(bool(fresh))
+    if out is None:
+        out = torch.empty((max(1, len(rows)), n_out), dtype=torch.float32, device=audio.device)
+    _check_output("audio_post_rows out", out, torch.float32, (out.shape[0], n_out), audio.device, row_slices=True)
+    _check_output("audio_post_rows state", state, torch.float32, (state.shape[0], AUDIO_POST_STATE_FLOATS),
+                  audio.device)
+    _check(lib().b200_audio_post_rows(C.c_void_p(audio.data_ptr()), audio.stride(0), audio.shape[0], n, rate_hz, flags,
+                                      table, len(rows), C.c_void_p(state.data_ptr()), state.shape[0],
+                                      C.c_void_p(out.data_ptr()), out.stride(0), out.shape[0], _stream_ptr(stream)),
+           "b200_audio_post_rows")
+    return out
+
+
 def resample_taps() -> np.ndarray:
     h = np.empty(240, dtype=np.float32)
     assert lib().b200_audio_resample_taps(h.ctypes.data) == 240
@@ -788,6 +827,11 @@ class PushStream:
         h = np.zeros(0, np.float32) if h_taps is None else np.ascontiguousarray(h_taps, dtype=np.float32).reshape(-1)
         _check(lib().b200_stream_set_channel_filter(self.h, h.ctypes.data if h.size else None, int(h.size)),
                "b200_stream_set_channel_filter")
+
+    def set_audio_post(self, flags: int, rate_hz: float = 51200.0) -> None:
+        """b200_stream_set_audio_post: de-emphasis and / or 48 kHz output (AUDIO_* flags; 0 = raw audio) for the
+        centre and channel audio sinks.  rate_hz is fs / (4R).  Only before anything is pushed."""
+        _check(lib().b200_stream_set_audio_post(self.h, flags, rate_hz), "b200_stream_set_audio_post")
 
     def enable_frames(self) -> None:
         """Install the per-frame dB sink on a stream that was created without one (frames=False): the library

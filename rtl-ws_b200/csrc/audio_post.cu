@@ -26,6 +26,7 @@
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 
 #include "b200_common.cuh"
@@ -64,7 +65,11 @@ struct PostParams {
     int resample;
 };
 
-__global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams p)
+// One chunk (blockIdx.x) of one row (blockIdx.y).  ROWS: the row names its input, output and state rows and
+// whether it is fresh, i.e. reads the state as all zero (stream start) without touching it; otherwise all three are
+// row blockIdx.y and the state is read.  The next state is staged in the state row's [APS_NEXT..] either way.
+template <bool ROWS>
+__device__ __forceinline__ void audio_post_chunk(const PostParams& p, const b200_audio_post_row* rows)
 {
     __shared__ float e[AP_CHUNK + AP_HALO];      // e[i] = de-emphasised sample c0 - 16 + i
     __shared__ float taps[AP_TAPS];              // lanes read different phases: shared memory, not the constant port
@@ -74,8 +79,9 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
     const int s = blockIdx.y;
     const int64_t c0 = (int64_t) blockIdx.x * AP_CHUNK;
     const int n_here = (int) min((int64_t) AP_CHUNK, p.n - c0);
-    const float* x = p.in + (int64_t) s * p.in_stride;
-    float* st = p.state + (int64_t) s * B200_AUDIO_POST_STATE_FLOATS;
+    const float* x = p.in + (int64_t) (ROWS ? rows[s].audio_row : s) * p.in_stride;
+    float* st = p.state + (int64_t) (ROWS ? rows[s].state_row : s) * B200_AUDIO_POST_STATE_FLOATS;
+    const bool fresh = ROWS && rows[s].fresh != 0;
     const bool last = c0 + n_here == p.n;
 
     // ---- de-emphasis (or a plain copy) of samples [c0 - 16, c0 + n_here) into e[] ----
@@ -87,7 +93,7 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
                 float y;
                 int64_t g = g0 - p.runin;
                 if (g <= 0) {                                       // the run-in would cross the batch start: exact state
-                    y = st[APS_Y];
+                    y = fresh ? 0.0f : st[APS_Y];
                     g = 0;
                 } else {
                     y = 0.0f;
@@ -102,7 +108,7 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
                             y = fmaf(p.alpha, x[gg] - y, y);
                             e[i0 + k] = y;
                         } else {
-                            e[i0 + k] = gg >= -15 ? st[APS_HIST + 15 + (int) gg] : 0.0f;
+                            e[i0 + k] = gg >= -15 && !fresh ? st[APS_HIST + 15 + (int) gg] : 0.0f;
                         }
                     }
                 }
@@ -110,7 +116,8 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
 #pragma unroll
                 for (int k = 0; k < AP_PER_THREAD; ++k) {
                     const int64_t gg = g0 + k;
-                    if (i0 + k < n_here + AP_HALO) e[i0 + k] = gg >= 0 ? x[gg] : (gg >= -15 ? st[APS_HIST + 15 + (int) gg] : 0.0f);
+                    if (i0 + k < n_here + AP_HALO)
+                        e[i0 + k] = gg >= 0 ? x[gg] : (gg >= -15 && !fresh ? st[APS_HIST + 15 + (int) gg] : 0.0f);
                 }
             }
         }
@@ -118,7 +125,7 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
     __syncthreads();
 
     // ---- output ----
-    float* out = p.out + (int64_t) s * p.out_stride;
+    float* out = p.out + (int64_t) (ROWS ? rows[s].out_row : s) * p.out_stride;
     if (p.resample) {
         const int n_out = n_here / 16 * 15;                         // n is a multiple of 16
         const int64_t m0 = c0 / 16 * 15;
@@ -142,11 +149,35 @@ __global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams
     }
 }
 
+__global__ void __launch_bounds__(AP_THREADS) audio_post_kernel(const PostParams p)
+{
+    audio_post_chunk<false>(p, nullptr);
+}
+
+// The row table of b200_audio_post_rows, passed by value like FcRunsParams: 16 B a row, 16 KB in all
+struct PostRowsParams : PostParams {
+    b200_audio_post_row rows[B200_AUDIO_POST_MAX_ROWS];
+};
+
+__global__ void __launch_bounds__(AP_THREADS) audio_post_rows_kernel(const __grid_constant__ PostRowsParams p)
+{
+    audio_post_chunk<true>(p, p.rows);
+}
+
 __global__ void audio_post_commit_kernel(float* state, int n_streams)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_streams * 16) return;
     float* st = state + (int64_t) (i / 16) * B200_AUDIO_POST_STATE_FLOATS;
+    st[i % 16] = st[APS_NEXT + i % 16];
+}
+
+// the commit of the table's state rows (no two rows share one)
+__global__ void audio_post_commit_rows_kernel(const __grid_constant__ PostRowsParams p, int n_rows)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_rows * 16) return;
+    float* st = p.state + (int64_t) p.rows[i / 16].state_row * B200_AUDIO_POST_STATE_FLOATS;
     st[i % 16] = st[APS_NEXT + i % 16];
 }
 
@@ -187,9 +218,58 @@ static int ensure_taps()
     return B200_OK;
 }
 
+// The flag, rate and length rules every audio post path shares; alpha and runin (nullable) receive the kernel's
+// de-emphasis coefficient (0 = none) and run-in.
+int audio_post_check(const char* who, int flags, double audio_rate_hz, int64_t n_audio, float* alpha, int* runin)
+{
+    const int de = flags & (B200_AUDIO_DEEMPH_50US | B200_AUDIO_DEEMPH_75US);
+    if (n_audio < 0 || de == (B200_AUDIO_DEEMPH_50US | B200_AUDIO_DEEMPH_75US) || (flags & ~7) != 0 ||
+        !(audio_rate_hz > 0.0)) {
+        set_error("%s: bad arguments (flags = %d)", who, flags);
+        return B200_ERR_ARG;
+    }
+    if ((flags & B200_AUDIO_RESAMPLE_48K) && n_audio % 16 != 0) {
+        set_error("%s: the 15/16 resampler takes multiples of 16 samples, not %lld", who, (long long) n_audio);
+        return B200_ERR_ARG;
+    }
+    float a = 0.0f;
+    int L = AP_MIN_RUNIN;
+    if (de) {
+        const double tau = de == B200_AUDIO_DEEMPH_50US ? 50e-6 : 75e-6;
+        a = (float) (1.0 - exp(-1.0 / (audio_rate_hz * tau)));
+        // run-in after which a start from y = 0 is off by (1 - alpha)^L <= 1e-7 of the signal's peak (alpha = 0,
+        // a rate so high that alpha rounds away, would need an endless one)
+        const double need = ceil(log(1e-7) / log1p(-(double) a));
+        if (!(a > 0.0f) || !(need <= AP_MAX_RUNIN)) {
+            set_error("%s: de-emphasis at %g Hz needs a run-in of %g samples, more than %d", who, audio_rate_hz, need,
+                      AP_MAX_RUNIN);
+            return B200_ERR_ARG;
+        }
+        L = (int) need > AP_MIN_RUNIN ? ((int) need + 7) / 8 * 8 : AP_MIN_RUNIN;
+    }
+    if (alpha) *alpha = a;
+    if (runin) *runin = L;
+    return B200_OK;
+}
+
 }  // namespace b200
 
 using namespace b200;
+
+// bytes from the first float of `rows` rows `stride` floats apart to one past the last of the last row's `width`
+// floats; -1 for no rows or an extent past int64
+static int64_t block_bytes(int64_t rows, int64_t stride, int64_t width)
+{
+    if (rows < 1 || stride < 0 || width < 0 || width > INT64_MAX / 8) return -1;
+    if (stride > 0 && rows - 1 > (INT64_MAX / 4 - width) / stride) return -1;
+    return ((rows - 1) * stride + width) * 4;
+}
+
+static bool overlap(const void* a, int64_t a_bytes, const void* b, int64_t b_bytes)
+{
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + (uintptr_t) b_bytes && y < x + (uintptr_t) a_bytes;
+}
 
 extern "C" {
 
@@ -210,38 +290,18 @@ int b200_audio_resample_taps(float* h240)
 int b200_audio_post(const float* d_audio, int64_t audio_stride, int n_streams, int64_t n_audio, double audio_rate_hz,
                     int flags, float* d_state, float* d_out, int64_t out_stride, void* cuda_stream)
 {
-    const int de = flags & (B200_AUDIO_DEEMPH_50US | B200_AUDIO_DEEMPH_75US);
-    if (d_audio == nullptr || d_out == nullptr || d_state == nullptr || n_streams < 0 || n_audio < 0 ||
-        de == (B200_AUDIO_DEEMPH_50US | B200_AUDIO_DEEMPH_75US) || (flags & ~7) != 0 || !(audio_rate_hz > 0.0)) {
+    PostParams p;
+    if (d_audio == nullptr || d_out == nullptr || d_state == nullptr || n_streams < 0) {
         set_error("audio post: bad arguments (flags = %d)", flags);
         return B200_ERR_ARG;
     }
-    if ((flags & B200_AUDIO_RESAMPLE_48K) && n_audio % 16 != 0) {
-        set_error("audio post: the 15/16 resampler takes multiples of 16 samples, not %lld", (long long) n_audio);
-        return B200_ERR_ARG;
-    }
-    float alpha = 0.0f;
-    int runin = AP_MIN_RUNIN;
-    if (de) {
-        const double tau = de == B200_AUDIO_DEEMPH_50US ? 50e-6 : 75e-6;
-        alpha = (float) (1.0 - exp(-1.0 / (audio_rate_hz * tau)));
-        // run-in after which a start from y = 0 is off by (1 - alpha)^L <= 1e-7 of the signal's peak (alpha = 0,
-        // a rate so high that alpha rounds away, would need an endless one)
-        const double need = ceil(log(1e-7) / log1p(-(double) alpha));
-        if (!(alpha > 0.0f) || !(need <= AP_MAX_RUNIN)) {
-            set_error("audio post: de-emphasis at %g Hz needs a run-in of %g samples, more than %d", audio_rate_hz,
-                      need, AP_MAX_RUNIN);
-            return B200_ERR_ARG;
-        }
-        runin = (int) need > AP_MIN_RUNIN ? ((int) need + 7) / 8 * 8 : AP_MIN_RUNIN;
-    }
+    if (int rc = audio_post_check("audio post", flags, audio_rate_hz, n_audio, &p.alpha, &p.runin)) return rc;
     if (n_streams == 0 || n_audio == 0) return B200_OK;
     if (n_streams > 65535 || (n_audio + AP_CHUNK - 1) / AP_CHUNK >= (1ll << 31)) {
         set_error("audio post: too large for one launch");
         return B200_ERR_ARG;
     }
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(cuda_stream);
-    PostParams p;
     p.in = d_audio;
     p.in_stride = audio_stride;
     p.n = n_audio;
@@ -249,14 +309,90 @@ int b200_audio_post(const float* d_audio, int64_t audio_stride, int n_streams, i
     p.out_stride = out_stride;
     p.state = d_state;
     p.resample = (flags & B200_AUDIO_RESAMPLE_48K) != 0;
-    p.alpha = alpha;
-    p.runin = runin;
     if (p.resample)
         if (int rc = ensure_taps()) return rc;
     const unsigned chunks = (unsigned) ((n_audio + AP_CHUNK - 1) / AP_CHUNK);
     audio_post_kernel<<<dim3(chunks, (unsigned) n_streams), AP_THREADS, 0, stream>>>(p);
     B200_LAUNCH_CHECK();
     audio_post_commit_kernel<<<(n_streams * 16 + 255) / 256, 256, 0, stream>>>(d_state, n_streams);
+    B200_LAUNCH_CHECK();
+    return B200_OK;
+}
+
+int b200_audio_post_rows(const float* d_audio, int64_t audio_stride, int64_t n_audio_rows, int64_t n_audio,
+                         double audio_rate_hz, int flags, const b200_audio_post_row* h_rows, int n_rows,
+                         float* d_state, int64_t n_state_rows, float* d_out, int64_t out_stride, int64_t n_out_rows,
+                         void* cuda_stream)
+{
+    static thread_local PostRowsParams p;        // 16 KB: kept off the caller's stack
+    if (d_audio == nullptr || d_out == nullptr || d_state == nullptr || h_rows == nullptr || n_rows < 1 ||
+        n_rows > B200_AUDIO_POST_MAX_ROWS) {
+        set_error("audio post rows: null pointer or %d rows outside [1, %d]", n_rows, B200_AUDIO_POST_MAX_ROWS);
+        return B200_ERR_ARG;
+    }
+    if (int rc = audio_post_check("audio post rows", flags, audio_rate_hz, n_audio, &p.alpha, &p.runin)) return rc;
+    const int64_t n_out = b200_audio_post_out_samples(n_audio, flags);
+    // the byte extent of each block: rows past its stride would overlap and race
+    const int64_t in_bytes = block_bytes(n_audio_rows, audio_stride, n_audio);
+    const int64_t out_bytes = block_bytes(n_out_rows, out_stride, n_out);
+    const int64_t state_bytes = block_bytes(n_state_rows, B200_AUDIO_POST_STATE_FLOATS, B200_AUDIO_POST_STATE_FLOATS);
+    if (audio_stride < n_audio || out_stride < n_out || in_bytes < 0 || out_bytes < 0 || state_bytes < 0) {
+        set_error("audio post rows: %lld input rows %lld floats apart for %lld samples, %lld output rows %lld apart for "
+                  "%lld, %lld state rows", (long long) n_audio_rows, (long long) audio_stride, (long long) n_audio,
+                  (long long) n_out_rows, (long long) out_stride, (long long) n_out, (long long) n_state_rows);
+        return B200_ERR_ARG;
+    }
+    if (((reinterpret_cast<uintptr_t>(d_audio) | reinterpret_cast<uintptr_t>(d_out) |
+          reinterpret_cast<uintptr_t>(d_state)) & 3) != 0) {
+        set_error("audio post rows: audio, state and output must be 4-byte aligned");
+        return B200_ERR_ALIGN;
+    }
+    if (overlap(d_out, out_bytes, d_audio, in_bytes) || overlap(d_state, state_bytes, d_audio, in_bytes) ||
+        overlap(d_state, state_bytes, d_out, out_bytes)) {
+        set_error("audio post rows: the audio, output and state blocks may not overlap");
+        return B200_ERR_ARG;
+    }
+    int32_t out_rows[B200_AUDIO_POST_MAX_ROWS], state_rows[B200_AUDIO_POST_MAX_ROWS];
+    for (int k = 0; k < n_rows; ++k) {
+        const b200_audio_post_row& r = h_rows[k];
+        if (r.audio_row < 0 || r.audio_row >= n_audio_rows || r.out_row < 0 || r.out_row >= n_out_rows ||
+            r.state_row < 0 || r.state_row >= n_state_rows) {
+            set_error("audio post rows: row %d (audio row %d of %lld, output row %d of %lld, state row %d of %lld)", k,
+                      r.audio_row, (long long) n_audio_rows, r.out_row, (long long) n_out_rows, r.state_row,
+                      (long long) n_state_rows);
+            return B200_ERR_ARG;
+        }
+        out_rows[k] = r.out_row;
+        state_rows[k] = r.state_row;
+    }
+    // two rows writing one output row or one state row would race
+    std::sort(out_rows, out_rows + n_rows);
+    std::sort(state_rows, state_rows + n_rows);
+    for (int k = 1; k < n_rows; ++k)
+        if (out_rows[k] == out_rows[k - 1] || state_rows[k] == state_rows[k - 1]) {
+            set_error("audio post rows: two rows share output row %d or state row %d", out_rows[k], state_rows[k]);
+            return B200_ERR_ARG;
+        }
+    if (n_audio == 0) return B200_OK;
+    if ((n_audio + AP_CHUNK - 1) / AP_CHUNK >= (1ll << 31)) {
+        set_error("audio post rows: too large for one launch");
+        return B200_ERR_ARG;
+    }
+    p.in = d_audio;
+    p.in_stride = audio_stride;
+    p.n = n_audio;
+    p.out = d_out;
+    p.out_stride = out_stride;
+    p.state = d_state;
+    p.resample = (flags & B200_AUDIO_RESAMPLE_48K) != 0;
+    memcpy(p.rows, h_rows, sizeof(b200_audio_post_row) * (size_t) n_rows);
+    if (p.resample)
+        if (int rc = ensure_taps()) return rc;
+    cudaStream_t stream = reinterpret_cast<cudaStream_t>(cuda_stream);
+    const unsigned chunks = (unsigned) ((n_audio + AP_CHUNK - 1) / AP_CHUNK);
+    audio_post_rows_kernel<<<dim3(chunks, (unsigned) n_rows), AP_THREADS, 0, stream>>>(p);
+    B200_LAUNCH_CHECK();
+    audio_post_commit_rows_kernel<<<(n_rows * 16 + 255) / 256, 256, 0, stream>>>(p, n_rows);
     B200_LAUNCH_CHECK();
     return B200_OK;
 }

@@ -81,6 +81,10 @@ int launch_fm_channels_runs(const uint8_t* iq, int64_t stream_stride_bytes, int 
 int fm_channels_fir_history_samples(int R, int T);
 int fm_channel_filter_design(int R, int T, double cutoff_hz, double atten_db, double fs, float* h);
 
+// audio_post.cu: the flag, rate and length rules of b200_audio_post, b200_audio_post_rows and
+// b200_stream_set_audio_post (B200_ERR_ARG, b200_last_error() prefixed by `who`); alpha and runin are nullable
+int audio_post_check(const char* who, int flags, double audio_rate_hz, int64_t n_audio, float* alpha, int* runin);
+
 // The device IQ rows of a session or a push stream: one row per stream, [history | batch], the history being the
 // last `hist` samples of the stream's previous batch (128 before the first).  The history is the FM chain's 32 R,
 // or the longer one the channel filter reaches back over.  Each call that launches work does it on `stream`.

@@ -21,6 +21,10 @@
 // channels.  A batch takes the set that is current when its last sample is pushed (stored with the slot then), and a
 // submitted run adds one launch of the runs-table channel kernel over its streams that have channels, after the
 // chain kernel and before the history carry, and one 2-D copy back.
+//
+// Audio post-processing (b200_stream_set_audio_post, off by default): the centre audio of a run goes through
+// b200_audio_post with one state row per dongle, and its channels through one b200_audio_post_rows call whose state
+// rows belong to listener ids (stream_map_listeners).  The sinks then get the post-processed rows.
 #include <string.h>
 
 #include <vector>
@@ -72,8 +76,21 @@ struct b200_stream {
         ChannelSet channels;             // current listener set (b200_stream_set_channels)
         ChannelSet slot_channels[ST_SLOTS];     // the set of each full slot, taken when its last sample arrived
         bool has_chan[ST_SLOTS] = {};    // the submitted slot computed and copied channel audio
+        // post-processing state slots of the listeners of the last submitted batch with channel work
+        int64_t post_batch = -1;         // that batch's index; -1 = none
+        bool slot_used[B200_FM_MAX_CHANNELS] = {};
+        int32_t slot_id[B200_FM_MAX_CHANNELS];
     };
     std::vector<PerStream> st;
+    int post_flags = 0;                  // b200_audio_post flags; 0 = raw audio
+    double post_rate = 0.0;
+    float* d_post_audio = nullptr;       // [n_streams][batch / (4R)]: post output, n_out floats a row
+    float* d_post_state = nullptr;       // [n_streams][B200_AUDIO_POST_STATE_FLOATS]
+    float* d_post_chan = nullptr;        // [n_streams][chan_max][batch / (4R)]: post output, n_out floats a row
+    float* d_post_chan_state = nullptr;  // [n_streams][chan_max][B200_AUDIO_POST_STATE_FLOATS]: state slots
+    int64_t n_audio() const { return batch / (4 * rows.R); }
+    // audio samples a batch delivers per sink call
+    int64_t n_out() const { return post_flags ? b200_audio_post_out_samples(n_audio(), post_flags) : n_audio(); }
     b200_spectrum_sink spectrum_sink = nullptr;
     b200_audio_sink audio_sink = nullptr;
     void* user = nullptr;
@@ -112,17 +129,48 @@ static void stream_deliver(b200_stream* s, int i, bool block)
         // a sink installed after this batch was submitted without one gets nothing for it (there are no rows)
         if (s->spectrum_sink && p.has_db[slot])
             s->spectrum_sink(s->user, i, b * (s->batch / 1024), (int) (s->batch / 1024), s->h_db + off * (size_t) s->batch);
-        const int64_t n_audio = s->batch / (4 * s->rows.R);
-        if (s->audio_sink) s->audio_sink(s->user, i, b * n_audio, (int) n_audio, s->h_audio + off * (size_t) n_audio);
+        const int64_t n_audio = s->n_audio();      // the host rows' pitch
+        const int64_t n = s->n_out();
+        if (s->audio_sink) s->audio_sink(s->user, i, b * n, (int) n, s->h_audio + off * (size_t) n_audio);
         if (s->chan_sink && p.has_chan[slot]) {
             const b200_stream::ChannelSet& cs = p.slot_channels[slot];
             for (int c = 0; c < cs.n; ++c)
-                s->chan_sink(s->user, i, cs.id[c], b * n_audio, (int) n_audio,
+                s->chan_sink(s->user, i, cs.id[c], b * n, (int) n,
                              s->h_chan + (off * (size_t) s->chan_max + (size_t) c) * (size_t) n_audio);
         }
         p.in_flight[slot] = false;
         ++p.batches_delivered;
     }
+}
+
+// The post-processing state slots of stream p's listeners cs in the batch being submitted (its batches_submitted-th),
+// by id: a listener that was in the set of the stream's previous batch, when that batch had channel work, keeps its
+// slot; any other takes a free slot and starts fresh.  Slots of listeners that left are free again.
+static void stream_map_listeners(b200_stream::PerStream& p, const b200_stream::ChannelSet& cs, int* slot_of, bool* fresh)
+{
+    const bool carried = p.post_batch == p.batches_submitted - 1;
+    bool used[B200_FM_MAX_CHANNELS] = {};
+    for (int c = 0; c < cs.n; ++c) {
+        slot_of[c] = -1;
+        for (int k = 0; carried && k < B200_FM_MAX_CHANNELS; ++k)
+            if (p.slot_used[k] && p.slot_id[k] == cs.id[c]) {
+                slot_of[c] = k;
+                used[k] = true;
+                break;
+            }
+    }
+    int k = 0;      // cs.n <= chan_max slots, so a listener without one finds a free one below chan_max
+    for (int c = 0; c < cs.n; ++c) {
+        fresh[c] = slot_of[c] < 0;
+        if (fresh[c]) {
+            while (used[k]) ++k;
+            slot_of[c] = k;
+            used[k] = true;
+        }
+        p.slot_id[slot_of[c]] = cs.id[c];
+    }
+    memcpy(p.slot_used, used, sizeof(used));
+    p.post_batch = p.batches_submitted;
 }
 
 // Submit the ready slot `slot` of streams [a, b) as one unit.  All of them run on the lane of their group, so
@@ -131,7 +179,9 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
 {
     const int n = b - a;
     const size_t batch = (size_t) s->batch;
-    const size_t n_audio = batch / (size_t) (4 * s->rows.R);
+    const size_t n_audio = (size_t) s->n_audio();
+    const size_t n_out = (size_t) s->n_out();
+    const bool post = s->post_flags != 0;
     cudaStream_t lane = s->lanes[(a / ST_GROUP) % ST_LANES];
     const size_t off = (size_t) a * ST_SLOTS + (size_t) slot;            // first stream's slot; next stream: + ST_SLOTS
     uint8_t* d_batch = s->rows.batch(a);
@@ -153,8 +203,17 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
     if (want_chan) {
         b200_fm_channel_run runs[ST_GROUP];
         int n_runs = 0;
+        b200_audio_post_row rows[ST_GROUP * B200_FM_MAX_CHANNELS];
+        int n_rows = 0;
         for (int i = a; i < b; ++i) {
             const b200_stream::ChannelSet& cs = s->st[i].slot_channels[slot];
+            if (post) {
+                int slot_of[B200_FM_MAX_CHANNELS];
+                bool fresh[B200_FM_MAX_CHANNELS];
+                stream_map_listeners(s->st[i], cs, slot_of, fresh);
+                for (int c = 0; c < cs.n; ++c)
+                    rows[n_rows++] = {i * s->chan_max + c, i * s->chan_max + c, i * s->chan_max + slot_of[c], fresh[c]};
+            }
             if (cs.n == 0) continue;
             b200_fm_channel_run& r = runs[n_runs++];
             r.stream = i - a;
@@ -170,6 +229,19 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
                                          (int64_t) n * s->chan_max, s->rows.d_taps, s->rows.n_taps, lane);
             if (rc) return rc;
         }
+        if (n_rows > 0) {
+            const int64_t n_chan_rows = (int64_t) s->n_streams * s->chan_max;
+            rc = b200_audio_post_rows(s->d_chan, (int64_t) n_audio, n_chan_rows, (int64_t) n_audio, s->post_rate,
+                                      s->post_flags, rows, n_rows, s->d_post_chan_state, n_chan_rows, s->d_post_chan,
+                                      (int64_t) n_audio, n_chan_rows, lane);
+            if (rc) return rc;
+        }
+    }
+    if (post) {
+        rc = b200_audio_post(d_audio, (int64_t) n_audio, n, (int64_t) n_audio, s->post_rate, s->post_flags,
+                             s->d_post_state + (size_t) a * B200_AUDIO_POST_STATE_FLOATS,
+                             s->d_post_audio + (size_t) a * n_audio, (int64_t) n_audio, lane);
+        if (rc) return rc;
     }
     rc = s->rows.carry(a, n, s->batch, lane);
     if (rc) return rc;
@@ -177,17 +249,20 @@ static int stream_submit_run(b200_stream* s, int a, int b, int slot)
     if (want_db)
         B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_db + off * batch, ST_SLOTS * batch * sizeof(float), d_db, batch * sizeof(float),
                                         batch * sizeof(float), (size_t) n, cudaMemcpyDeviceToHost, lane));
-    B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_audio + off * n_audio, ST_SLOTS * n_audio * sizeof(float), d_audio,
-                                    n_audio * sizeof(float), n_audio * sizeof(float), (size_t) n, cudaMemcpyDeviceToHost, lane));
+    // post-processed rows hold n_out floats at the same pitch
+    B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_audio + off * n_audio, ST_SLOTS * n_audio * sizeof(float),
+                                    post ? s->d_post_audio + (size_t) a * n_audio : d_audio, n_audio * sizeof(float),
+                                    n_out * sizeof(float), (size_t) n, cudaMemcpyDeviceToHost, lane));
     if (want_payload)
         B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_payload + off * 1024, ST_SLOTS * 1024, d_pay, 1024, 1024, (size_t) n,
                                         cudaMemcpyDeviceToHost, lane));
-    // per stream, its first chan_width channel rows (rows past a stream's own count are not read on delivery)
+    // per stream, its first chan_width channel rows up to the last one's n_out floats (rows past a stream's own count
+    // are not read on delivery)
     if (chan_width > 0) {
         const size_t block = (size_t) s->chan_max * n_audio * sizeof(float);
         B200_CUDA_TRY(cudaMemcpy2DAsync(s->h_chan + off * (size_t) s->chan_max * n_audio, ST_SLOTS * block,
-                                        s->d_chan + (size_t) a * (size_t) s->chan_max * n_audio, block,
-                                        (size_t) chan_width * n_audio * sizeof(float), (size_t) n,
+                                        (post ? s->d_post_chan : s->d_chan) + (size_t) a * (size_t) s->chan_max * n_audio,
+                                        block, ((size_t) (chan_width - 1) * n_audio + n_out) * sizeof(float), (size_t) n,
                                         cudaMemcpyDeviceToHost, lane));
     }
     for (int i = a; i < b; ++i) {
@@ -240,6 +315,33 @@ static int stream_submit_ready(b200_stream* s)
         if (rc) return rc;
         // the same stream may hold a second full slot: look at it again
     }
+    return B200_OK;
+}
+
+// true once anything has been pushed: the settings that shape every batch are fixed from then on
+static bool stream_started(const b200_stream* s)
+{
+    for (const auto& p : s->st)
+        if (p.fill != 0 || p.batches_submitted != 0 || p.ready[0] || p.ready[1]) return true;
+    return false;
+}
+
+// The post-processing buffers the stream lacks with post-processing `flags` and its channel capacity: the centre
+// output and state rows (the state zeroed, waited for) and, with channels, their output rows and state slots (a slot
+// is read only after a fresh start has written it).  On failure b200_last_error() says why.
+static int stream_alloc_post(b200_stream* s, int flags)
+{
+    if (flags == 0) return B200_OK;
+    const size_t ns = (size_t) s->n_streams, n_audio = (size_t) s->n_audio(), nc = (size_t) s->chan_max;
+    const size_t state = sizeof(float) * B200_AUDIO_POST_STATE_FLOATS;
+    if (s->d_post_audio == nullptr) B200_CUDA_TRY(cudaMalloc(&s->d_post_audio, sizeof(float) * ns * n_audio));
+    if (s->d_post_state == nullptr) {
+        B200_CUDA_TRY(cudaMalloc(&s->d_post_state, state * ns));
+        B200_CUDA_TRY(cudaMemsetAsync(s->d_post_state, 0, state * ns, s->lanes[0]));
+        B200_CUDA_TRY(cudaStreamSynchronize(s->lanes[0]));
+    }
+    if (nc > 0 && s->d_post_chan == nullptr) B200_CUDA_TRY(cudaMalloc(&s->d_post_chan, sizeof(float) * ns * nc * n_audio));
+    if (nc > 0 && s->d_post_chan_state == nullptr) B200_CUDA_TRY(cudaMalloc(&s->d_post_chan_state, state * ns * nc));
     return B200_OK;
 }
 
@@ -297,7 +399,8 @@ void b200_stream_destroy(b200_stream* s)
         for (cudaEvent_t ev : p.done)
             if (ev) cudaEventDestroy(ev);
     s->rows.free();
-    for (void* d : std::initializer_list<void*>{s->d_db, s->d_audio, s->d_payload, s->d_chan})
+    for (void* d : std::initializer_list<void*>{s->d_db, s->d_audio, s->d_payload, s->d_chan, s->d_post_audio,
+                                                s->d_post_state, s->d_post_chan, s->d_post_chan_state})
         if (d != nullptr) cudaFree(d);
     for (void* h : std::initializer_list<void*>{s->h_in, s->h_db, s->h_audio, s->h_payload, s->h_chan})
         if (h != nullptr) cudaFreeHost(h);
@@ -396,6 +499,8 @@ int b200_stream_set_channel_sink(b200_stream* s, int max_channels, b200_channel_
             return B200_ERR_CUDA;
         s->chan_max = max_channels;
     }
+    if (sink != nullptr)
+        if (int rc = stream_alloc_post(s, s->post_flags)) return rc;
     s->chan_sink = sink;
     return B200_OK;
 }
@@ -430,12 +535,25 @@ int b200_stream_set_channel_filter(b200_stream* s, const float* h_taps, int n_ta
         set_error("stream channel filter: null stream");
         return B200_ERR_ARG;
     }
-    for (const auto& p : s->st)
-        if (p.fill != 0 || p.batches_submitted != 0 || p.ready[0] || p.ready[1]) {
-            set_error("stream channel filter: set it before anything is pushed");
-            return B200_ERR_ARG;
-        }
+    if (stream_started(s)) {
+        set_error("stream channel filter: set it before anything is pushed");
+        return B200_ERR_ARG;
+    }
     return s->rows.set_channel_filter("stream channel filter", h_taps, n_taps, s->lanes[0]);
+}
+
+int b200_stream_set_audio_post(b200_stream* s, int flags, double audio_rate_hz)
+{
+    if (s == nullptr || stream_started(s)) {
+        set_error("stream audio post: set it before anything is pushed");
+        return B200_ERR_ARG;
+    }
+    // a batch's audio is one call's n_audio: the resampler needs it a multiple of 16
+    if (int rc = audio_post_check("stream audio post", flags, audio_rate_hz, s->n_audio(), nullptr, nullptr)) return rc;
+    if (int rc = stream_alloc_post(s, flags)) return rc;
+    s->post_flags = flags;
+    s->post_rate = audio_rate_hz;
+    return B200_OK;
 }
 
 int64_t b200_stream_pending_samples(const b200_stream* s, int stream)

@@ -54,5 +54,13 @@ ps.set_channels(1, [0, pkg.fm_channel_tune(200e3, 2.048e6)], [4, 5])
 for s in range(2):
     ps.push(s, iq[s])
 ps.flush()
+# audio post-processing over a row table, and on the push stream's centre and channel audio
+pkg.audio_post_rows(audio[:, :368], [(2, 0, 1, 0), (0, 1, 0, 1)], st, pkg.AUDIO_DEEMPH_75US | pkg.AUDIO_RESAMPLE_48K)
+pp = pkg.PushStream(2, 5120 * 2, channel_capacity=2)
+pp.set_audio_post(pkg.AUDIO_DEEMPH_75US | pkg.AUDIO_RESAMPLE_48K)
+pp.set_channels(0, [pkg.fm_channel_tune(-200e3, 2.048e6)], [9])
+for s in range(2):
+    pp.push(s, iq[s])
+pp.flush()
 torch.cuda.synchronize()
 print("sanity ok", float(db.abs().max()) > 0, float(audio.abs().max()) >= 0)
