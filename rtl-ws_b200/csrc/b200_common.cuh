@@ -1,5 +1,5 @@
-// b200_common.cuh -- shared device helpers (sm_100a): mbarrier + 1-D bulk TMA copies,
-// error plumbing, and the one declaration of each internal host launcher and helper.
+// b200_common.cuh -- shared device helpers (sm_100a): mbarrier + 1-D bulk TMA copies, tensor
+// memory, error plumbing, and the one declaration of each internal host launcher and helper.
 // No CPU fallback anywhere: a failed CUDA call surfaces as B200_ERR_CUDA.
 #pragma once
 
@@ -184,6 +184,80 @@ __device__ __forceinline__ void tma_load_1d(void* dst_smem, const void* src_gmem
             smem_u32(dst_smem)),
         "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
         : "memory");
+}
+
+// ---- device: tensor memory (tcgen05, one CTA) -------------------------------------------
+// A TMEM address is lane << 16 | column.  A warp may only touch the 32 lanes of its quadrant, lanes
+// 32 (warp % 4) .. 32 (warp % 4) + 31; in the 32x32b shape thread t of the warp reads or writes lane
+// 32 (warp % 4) + t, 16 consecutive 32-bit columns from the address's column on (.x16).
+
+// Whole warp: allocate n_cols columns (a power of two, 32..512) of every lane; the base address lands in *slot.
+// Publish it to the other warps with tmem_fence_before_sync, a block barrier and tmem_fence_after_sync.
+__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t n_cols)
+{
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)),
+                 "r"(n_cols)
+                 : "memory");
+}
+
+// Whole warp: free what tmem_alloc returned.  Every allocation must be freed before the CTA exits.
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t n_cols)
+{
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(n_cols) : "memory");
+}
+
+// Whole warp: this CTA allocates no more, so a CTA waiting for tensor memory on this SM need not wait for it.
+__device__ __forceinline__ void tmem_relinquish_alloc_permit()
+{
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+
+// Whole warp: r[] -> 16 columns of this thread's lane.  Complete only after tmem_wait_st.
+__device__ __forceinline__ void tmem_st_32x32b_x16(uint32_t taddr, const uint32_t (&r)[16])
+{
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, "
+                 "%13, %14, %15, %16};" ::"r"(taddr),
+                 "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
+                 "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+                 : "memory");
+}
+
+// Whole warp: 16 columns of this thread's lane -> r[].  The load is asynchronous: r[] may be read only after
+// tmem_wait_ld(r), which also keeps the compiler from moving a use of r[] above the wait.
+__device__ __forceinline__ void tmem_ld_32x32b_x16(uint32_t taddr, uint32_t (&r)[16])
+{
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, "
+                 "%13, %14, %15}, [%16];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                   "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(taddr)
+                 : "memory");
+}
+
+// Whole warp: wait until every tcgen05.ld this thread issued has landed; r[] is the destination of the last one.
+__device__ __forceinline__ void tmem_wait_ld(uint32_t (&r)[16])
+{
+    asm volatile("tcgen05.wait::ld.sync.aligned;"
+                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
+                   "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
+                 :
+                 : "memory");
+}
+
+// Whole warp: wait until every tcgen05.st this thread issued has been written.
+__device__ __forceinline__ void tmem_wait_st()
+{
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+}
+
+// Order this thread's tcgen05 operations before (after) a thread synchronisation that follows (precedes) it.
+__device__ __forceinline__ void tmem_fence_before_sync()
+{
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_fence_after_sync()
+{
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 }
 
 // drop a 128-byte line from L2 without writing it back (its contents are dead)

@@ -14,8 +14,11 @@
 //   - one service job: 3 chunks, re-arm the TMA producer and run the two half-band decimators
 //     of the PREVIOUS tile -> 128 audio floats.
 // One CTA per SM of 18 warps; each warp takes the next job from a shared counter, so no warp is
-// tied to a role and none meets another at a block barrier.  The inter-pass twiddles come from
-// an 8 KB shared table instead of 62 registers per lane, which is what lets 18 warps fit.
+// tied to a role and none meets another at a block barrier between set-up and exit.  The
+// inter-pass twiddles come from a table in tensor memory (64 columns of every lane, filled once at
+// kernel start), read 16 columns at a time just before pass 2's first stage uses them: not 62
+// registers per lane, which would rule out 18 warps, and not shared memory, whose pipe the
+// transpose already keeps busy.
 // Tiles are independent (a tile's audio depends on input bytes only, through the history), so
 // CTAs stride over (stream, tile) with no inter-CTA communication.
 #include "b200_common.cuh"
@@ -42,9 +45,8 @@ constexpr int CF_RING_BYTES = CF_STAGES * CF_STAGE_BYTES;
 constexpr int CF_XCH_BYTES = CF_WARPS * FFT1024_XCH_BYTES;
 constexpr int CF_DEMOD_BYTES = CF_DBUF * CF_ND_PAD * 4;
 constexpr int CF_WORK_BYTES = CF_DBUF * CF_WORK * 4;
-constexpr int CF_BAR_BYTES = (2 * CF_STAGES + 2 * CF_DBUF) * 8 + 8;     // + the job counter
-constexpr int CF_TW_OFFSET = (CF_RING_BYTES + CF_XCH_BYTES + CF_DEMOD_BYTES + CF_WORK_BYTES + CF_BAR_BYTES + 127) / 128 * 128;
-constexpr int CF_SMEM = CF_TW_OFFSET + 32 * 32 * 8;                     // + the [n2][k1] twiddle table
+constexpr int CF_BAR_BYTES = (2 * CF_STAGES + 2 * CF_DBUF) * 8 + 8;     // + the job counter and the TMEM base
+constexpr int CF_SMEM = CF_RING_BYTES + CF_XCH_BYTES + CF_DEMOD_BYTES + CF_WORK_BYTES + CF_BAR_BYTES;
 static_assert(CF_SMEM <= 232448, "more shared memory than a CTA may have on sm_100");
 static_assert(CF_STAGE_BYTES % 128 == 0, "ring stages must stay 128-byte aligned");
 // A waiter tests the PARITY of a barrier phase, so it must never get two phases ahead of the barrier: no job of
@@ -74,8 +76,9 @@ struct ChainParams {
 // The six jobs of a tile (service + five frames) are not tied to particular warps: every warp takes the next job
 // from a shared counter, and a warp that drew the short service job simply comes back sooner.  Jobs are claimed in
 // order and only ever wait for lower-numbered jobs (ring refills, demod hand-off), so the lowest unfinished job can
-// always run: no deadlock whatever the interleaving.  The inter-pass twiddles W_1024^(n2 k1) come from a shared
-// [n2][k1] table (one LDS.64 per pair member, conflict-free).
+// always run: no deadlock whatever the interleaving.  The inter-pass twiddles W_1024^(n2 k1) come from tensor
+// memory: warps 0-3 write the same table into the four lane quadrants (lane k1 of a quadrant holds what lane k1 of a
+// warp needs, see fft1024_pass2_tmem_tw), and every warp reads its quadrant with four tcgen05.ld per frame.
 __global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -91,7 +94,7 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainPa
     uint64_t* demod_full = empty + CF_STAGES;
     uint64_t* demod_empty = demod_full + CF_DBUF;
     uint32_t* next_job = reinterpret_cast<uint32_t*>(demod_empty + CF_DBUF);
-    float2* tws = reinterpret_cast<float2*>(smem + CF_TW_OFFSET);                               // [n2][k1]
+    uint32_t* tmem_slot = next_job + 1;
 
     const uint32_t total_tiles = (uint32_t) p.n_streams * (uint32_t) p.tiles_per_stream;
     const uint32_t first = blockIdx.x;
@@ -128,6 +131,7 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainPa
         for (int r = 0; r < 4; ++r) out[32 * r + lane] = halfband_from(work + 2 * (32 * r + lane));
     };
 
+    if (warp == 0) tmem_alloc(tmem_slot, FFT1024_TMEM_COLS);
     if (warp == 0 && lane == 0) {
         for (int i = 0; i < CF_STAGES; ++i) {
             mbar_init(&full[i], 1);
@@ -141,8 +145,22 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainPa
         fence_mbar_init();
         for (uint32_t it = 0; it < CF_STAGES - 1 && it < n_mine; ++it) issue(it);
     }
-    for (int i = tid; i < 1024; i += CF_THREADS) tws[i] = __ldg(&p.twiddle[((i >> 5) * (i & 31)) & 1023]);
+    tmem_fence_before_sync();
     __syncthreads();
+    tmem_fence_after_sync();
+    const uint32_t tw_taddr = *tmem_slot + ((uint32_t) (32 * (warp % 4)) << 16);     // this warp's quadrant
+    if (warp < 4) {
+#pragma unroll 1
+        for (int c = 0; c < FFT1024_TMEM_COLS / FFT1024_TMEM_CHUNK; ++c) {
+            uint32_t r[FFT1024_TMEM_CHUNK];
+            fft1024_tmem_twiddles(p.twiddle, lane, c, r);
+            tmem_st_32x32b_x16(tw_taddr + FFT1024_TMEM_CHUNK * c, r);
+        }
+        tmem_wait_st();
+    }
+    tmem_fence_before_sync();
+    __syncthreads();
+    tmem_fence_after_sync();
 
     // jobs 6*it + pos: pos 0 = the tile's service job, 1..5 = frames 0..4; job 6*n_mine = the last tile's audio
     const uint32_t n_jobs = n_mine > 0 ? 6 * n_mine + 1 : 0;
@@ -190,7 +208,7 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainPa
             }
             fft1024_pass1<true>(a);
             c64 b[32];
-            fft1024_pass2_smem_tw<false>(a, tws + lane, xch, lane, b);
+            fft1024_pass2_tmem_tw(a, tw_taddr, xch, lane, b);
             float pw[32];
             fft1024_power(b, pw);
             // DC-position patch (spectrum.c:30-33): display index 512 takes display index 511's value
@@ -212,6 +230,15 @@ __global__ void __launch_bounds__(CF_THREADS, 1) chain_jobs_kernel(const ChainPa
             __syncwarp();
             if (it > 0) audio_job(it - 1);
         }
+    }
+
+    // every warp's last tcgen05.ld has completed (each pass 2 waits for its loads) before the table is freed
+    tmem_fence_before_sync();
+    __syncthreads();
+    if (warp == 0) {
+        tmem_fence_after_sync();
+        tmem_dealloc(*tmem_slot, FFT1024_TMEM_COLS);     // read again: a register held over the job loop costs more
+        tmem_relinquish_alloc_permit();
     }
 }
 

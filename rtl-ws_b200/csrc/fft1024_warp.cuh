@@ -120,12 +120,36 @@ __host__ __device__ constexpr int fft1024_col(int k2)
     return 32 * ((k2 + 16) & 31);
 }
 
-// pass 2 with the inter-pass twiddles in a shared [n2][k1] table (tws_lane = table + lane)
-template <bool SYNC_BEFORE>
-__device__ __forceinline__ void fft1024_pass2_smem_tw(c64 (&a)[32], const float2* tws_lane, float2* xch, int lane,
+// Tensor-memory table of the inter-pass twiddles: lane k1 of the warp's quadrant holds, in columns
+// 2g and 2g + 1, re and im of W_1024^(k1 * bitrev<32>(g)) for g = 0..31 (g = 0: 1) -- the order
+// fft_dit32_pretwiddled_chunks consumes them.  FFT1024_TMEM_COLS columns per lane.
+constexpr int FFT1024_TMEM_COLS = 64;
+// Columns per tcgen05.ld.  16 and not 32: at 18 warps per SM a thread has 96 registers (five warps share
+// one scheduler's 16 K), and 32 twiddle registers next to the 64 of the frame make ptxas spill.
+constexpr int FFT1024_TMEM_CHUNK = 16;
+
+// this lane's row of the table, FFT1024_TMEM_CHUNK columns at a time
+__device__ __forceinline__ void fft1024_tmem_twiddles(const float2* __restrict__ table, int lane, int c,
+                                                      uint32_t (&r)[FFT1024_TMEM_CHUNK])
+{
+#pragma unroll
+    for (int j = 0; j < FFT1024_TMEM_CHUNK; j += 2) {
+        const int g = (FFT1024_TMEM_CHUNK * c + j) / 2;
+        const float2 w = g == 0 ? make_float2(1.0f, 0.0f) : __ldg(&table[(lane * bitrev<32>(g)) & 1023]);
+        r[j] = __float_as_uint(w.x);
+        r[j + 1] = __float_as_uint(w.y);
+    }
+}
+
+// pass 2 with the inter-pass twiddles in tensor memory; tw_taddr = column 0 of this warp's quadrant of the
+// table.  The first chunk is requested before the exchange, so its latency hides behind the exchange's loads;
+// the other three are requested one at a time, each just before its four butterflies (tcgen05.wait::ld waits
+// for every outstanding load, and a second chunk in flight would not fit in the registers either).
+__device__ __forceinline__ void fft1024_pass2_tmem_tw(c64 (&a)[32], uint32_t tw_taddr, float2* xch, int lane,
                                                       c64 (&b)[32])
 {
-    if (SYNC_BEFORE) __syncwarp();
+    uint32_t tw[FFT1024_TMEM_CHUNK];
+    tmem_ld_32x32b_x16(tw_taddr, tw);
 #pragma unroll
     for (int k1 = 0; k1 < 32; ++k1) {
         float re, im;
@@ -139,7 +163,10 @@ __device__ __forceinline__ void fft1024_pass2_smem_tw(c64 (&a)[32], const float2
         b[bitrev<32>(2 * m)] = v.x;
         b[bitrev<32>(2 * m + 1)] = v.y;
     }
-    fft_dit32_pretwiddled_smem(b, tws_lane);
+    fft_dit32_pretwiddled_chunks(b, tw, [&](int c, uint32_t (&r)[FFT1024_TMEM_CHUNK]) {
+        if (c > 0) tmem_ld_32x32b_x16(tw_taddr + FFT1024_TMEM_CHUNK * c, r);
+        tmem_wait_ld(r);
+    });
 }
 
 // |X|^2 of the transform's output, as raw power (see FFT1024_POWER_SCALE)

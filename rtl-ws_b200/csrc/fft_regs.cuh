@@ -216,19 +216,27 @@ __device__ __forceinline__ void fft_dit32(c64 (&a)[32], const float2 (&tw)[32])
     }
 }
 
-// The same 32-point transform with the pre-multipliers read just in time from shared memory:
-// x[n] is multiplied by twp[32 * n] (n = 0 taken as 1).  twp already points at this lane's column
-// of a [32][32] table, so a warp load is 256 contiguous bytes.  Frees the 62 registers a
-// lane-private copy costs (chain_fused.cu runs 18 warps per SM at 95 registers with it).
-__device__ __forceinline__ void fft_dit32_pretwiddled_smem(c64 (&a)[32], const float2* twp)
+// The same 32-point transform with the pre-multipliers handed over C floats at a time, in the
+// order the first stage consumes them: floats 2g, 2g + 1 of the sequence are re, im of the
+// multiplier of input bitrev<32>(g) = register g (g = 0 is taken as 1; its pair is never read), so
+// chunk c covers registers C/2 c .. C/2 (c + 1) - 1.  fetch(c, tw) must leave chunk c in tw; it is
+// called for c = 0, 1, ... just before the butterflies that need the chunk, so only C registers
+// ever hold multipliers instead of the 62 a lane-private copy costs (chain_fused.cu reads them from
+// tensor memory).
+template <int C, class Fetch>
+__device__ __forceinline__ void fft_dit32_pretwiddled_chunks(c64 (&a)[32], uint32_t (&tw)[C], Fetch&& fetch)
 {
+    static_assert(C % 4 == 0 && 64 % C == 0, "a chunk holds whole butterflies");
 #pragma unroll
-    for (int g = 0; g < 32; g += 2) {
-        const int na = bitrev<32>(g);
-        const int nb = bitrev<32>(g + 1);
-        const float2 ta = na == 0 ? make_float2(1.0f, 0.0f) : twp[32 * na];
-        const float2 tb = twp[32 * nb];
-        dit_butterfly_pretwiddled(a[g], a[g + 1], na == 0, ta, tb);
+    for (int c = 0; c < 64 / C; ++c) {
+        fetch(c, tw);
+#pragma unroll
+        for (int j = 0; j < C; j += 4) {
+            const int g = (C * c + j) / 2;
+            const float2 ta = make_float2(__uint_as_float(tw[j]), __uint_as_float(tw[j + 1]));
+            const float2 tb = make_float2(__uint_as_float(tw[j + 2]), __uint_as_float(tw[j + 3]));
+            dit_butterfly_pretwiddled(a[g], a[g + 1], g == 0, ta, tb);
+        }
     }
 #pragma unroll
     for (int half = 2; half <= 16; half <<= 1) {
